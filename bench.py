@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port), rank 0 only
     python bench.py --gpus N --total-tracks 8192             # BASELINE configs[3] as named: 8192 tracks STRONG-sharded over N GPUs
     python bench.py --gpus 8 --config vit_768_h256_d12 --tracks 512     # BASELINE configs[4]: widest config, 4096 tracks on 8 GPUs
+    python bench.py --gpus 1 --steps K --dump-outputs DIR                # also write the last timed step's boxes as DIR/boxes.npy
 
 A "step" advances every track by one frame: crop + normalise + stem + 3 ViT blocks + head + Hann /
 arg-max / box decode (+ for N>1 one NCCL all-gather of the boxes).  Default workload per GPU (BASELINE.json
@@ -12,6 +13,11 @@ configs[2]): 1024 concurrent synthetic tracks over 64 distinct 720x1280 uint8 fr
 (177 MB > L2), open-loop seeded boxes re-seeded every step, stress-init weights; with N > 1 the line also
 carries `strong_8192` = configs[3] (8192 tracks / N per GPU) measured in the same run.  Prints ONE JSON line
 (see README / DESIGN.md for the keys).
+
+Every input is generated from fixed seeds, so a run with the same arguments sees the same inputs.  --dump-outputs DIR writes
+what the timed path returned in its last timed step as DIR/boxes.npy: x y w h confidence of every track in float64 (rank 0;
+--impl reference: its 256-track sample), at most 64 MB (beyond that a fixed, seeded sample of the tracks), so that two builds
+of the project can be compared output for output.
 """
 from __future__ import annotations
 
@@ -103,6 +109,22 @@ def hbm_rooflines(boxes_xywh, stages, peaks, S=256, factor=4.0):
     return out
 
 
+DUMP_LIMIT = 64 << 20         # bytes --dump-outputs may write
+
+
+def dump_outputs(out_dir, boxes):
+    """--dump-outputs: `boxes` as <out_dir>/boxes.npy in float64.  Beyond DUMP_LIMIT a fixed, seeded sample of its rows is kept and
+    their indices are written as <out_dir>/rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    boxes = np.asarray(boxes, dtype=np.float64)
+    if boxes.nbytes > DUMP_LIMIT:
+        keep = DUMP_LIMIT // (boxes[0].nbytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(len(boxes), keep, replace=False))
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+        boxes = boxes[rows]
+    np.save(os.path.join(out_dir, "boxes.npy"), boxes)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled every 200 ms while the timed region runs."""
     Q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
@@ -180,6 +202,7 @@ class CpuPath:
                             for i, b in enumerate(init_boxes)])
 
     def step(self, boxes, t):
+        """One frame for every track; returns [x, y, w, h, confidence] per track, as the reference's track() does."""
         O = self.O
         n = len(boxes)
         out_states = []
@@ -192,9 +215,10 @@ class CpuPath:
             out = self.model.forward(self.z[g0:g0 + len(crops)], torch.cat(crops))
             resp = self.win * out["score_map"]
             pb = self.model.cal_bbox(resp, out["size_map"], out["offset_map"])
+            conf = out["score_map"].flatten(1).max(1).values.tolist()
             for k, i in enumerate(idx):
                 pred = (pb[k] * 256 / rfs[k]).tolist()
-                out_states.append(O.clip_box(O.map_box_back(list(boxes[i]), pred, rfs[k]), FRAME_H, FRAME_W, margin=10))
+                out_states.append(O.clip_box(O.map_box_back(list(boxes[i]), pred, rfs[k]), FRAME_H, FRAME_W, margin=10) + [conf[k]])
         return out_states
 
 
@@ -266,9 +290,11 @@ def run_reference(args, rank, world):
     for s in range(args.steps):
         boxes = O.synth_boxes(tracks, FRAME_H, FRAME_W, seed=300 + s)
         ts = time.perf_counter()
-        cp.step(boxes, s)
+        last = cp.step(boxes, s)
         per_step.append(tracks / (time.perf_counter() - ts))
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     v = tracks * args.steps / el
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * el / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -448,12 +474,12 @@ class Workload:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for t in range(K):
-            self.step(W + t)
+            out = self.step(W + t)
         self.finish_gather()
         e1.record()
         self.barrier()
         ms = e0.elapsed_time(e1)
-        self.last_out = self.bt.out_boxes[:self.n].cpu().numpy().copy()            # boxes of the last timed step
+        self.step_out = out.cpu().numpy().copy()            # what the last timed step returned (all tracks by global id when sharded)
         stages = eng.profile_read()
         eng.profile(False)
         launches = eng.launch_count - launches0 + (K if self.world > 1 else 0)
@@ -570,7 +596,11 @@ def main():
     ap.add_argument("--no-strong-leg", action="store_true", help="skip the configs[3] leg a multi-GPU default run adds")
     ap.add_argument("--no-bind", action="store_true", help="do not pin the rank to its GPU's CPUs / NUMA node")
     ap.add_argument("--latency-frames", type=int, default=10000, help="open-loop frames of the batch-1 latency leg (SURVEY C2: 10000)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/boxes.npy (float64: x, y, w, h, confidence per track)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     widest = args.config == WIDEST["name"]
     if args.tracks <= 0:
@@ -618,8 +648,10 @@ def main():
     bt, pool, sharded = wl.bt, wl.pool, wl.sharded
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ms, stages, launches, clocks = wl.timed(W, K, sampler)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl.step_out)
     value = n * world * K / (ms / 1e3)
-    last_out = wl.last_out                                          # boxes of the last timed step
+    last_out = wl.step_out[:n]                                      # rank 0's boxes of the last timed step, as dumped
     try:
         parity = wl.parity_spot(W + K - 1, last_out, k=8 if widest else 32) if rank == 0 else None
     except Exception as e:                                         # secondary: never at the expense of the line

@@ -1,10 +1,10 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference (through oracle/ref_shim.py) in
 this container, and assert while doing so that oracle/vt_oracle.py reproduces it.
 
-    python oracle/make_golden.py          # needs /root/reference; writes tests/golden/
+    python oracle/make_golden.py          # needs a checkout of the original project at oracle/_ref (or $VT_REFERENCE_ROOT); writes tests/golden/
 
-TEST INFRASTRUCTURE.  The fixtures travel to the GPU box (which has no /root/reference); the parity
-tests there compare the CUDA path with these reference outputs and with the oracle.
+TEST INFRASTRUCTURE.  The tests compare the oracle and the CUDA path with these recorded reference outputs, so they need
+no copy of the reference.  Seeded inputs are stored as digests (oracle/golden.py), which keeps every file under 1 MB.
 """
 from __future__ import annotations
 
@@ -18,7 +18,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from oracle import ref_shim, vt_oracle as O  # noqa: E402
+from oracle import golden, ref_shim, vt_oracle as O  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
@@ -62,7 +62,8 @@ def golden_crops(ns):
 
 def golden_model(ns, frame):
     """Reference build_ostrack_dist(cfg).forward(z, x) on stress-init weights and real crops."""
-    sd = O.make_state_dict(seed=1, stress=True)
+    sd_kw = dict(seed=1, stress=True)
+    sd = O.make_state_dict(**sd_kw)
     cfg = ref_shim.reference_cfg()
     net = ns.build_ostrack_dist(cfg)
     net.load_state_dict(sd, strict=True)
@@ -91,7 +92,7 @@ def golden_model(ns, frame):
     resp = win * ref["score_map"]
     ref_boxes_win = net.box_head.cal_bbox(resp, ref["size_map"], ref["offset_map"])
     assert torch.equal(ref_boxes_win, om.cal_bbox(resp, out["size_map"], out["offset_map"]))
-    arrs = {f"w::{k}": v.numpy() for k, v in sd.items()}
+    arrs = golden.seeded("make_state_dict", "w::", **sd_kw)
     arrs.update(z_patch=np.stack(zp), x_patch=np.stack(xp), hann=win.numpy(),
                 pred_boxes=ref["pred_boxes"].numpy(), score_map=ref["score_map"].numpy(),
                 size_map=ref["size_map"].numpy(), offset_map=ref["offset_map"].numpy(),
@@ -107,9 +108,10 @@ def golden_model(ns, frame):
 def golden_track(ns, sd):
     """Reference Vit_dist.initialize()/track() closed loop, default and scale-stable weights."""
     H, W = 240, 320
-    frames = O.synth_frames(4, H, W, seed=21, smooth=True)
-    out = {"frames": frames}
-    for tag, sdict in (("stress", sd), ("stable", O.make_state_dict(seed=2, stress=True, stable_size=True))):
+    frames_kw, stable_kw = dict(n=4, H=H, W=W, seed=21, smooth=True), dict(seed=2, stress=True, stable_size=True)
+    frames = O.synth_frames(**frames_kw)
+    out = golden.seeded("synth_frames", "frames", **frames_kw)
+    for tag, sdict in (("stress", sd), ("stable", O.make_state_dict(**stable_kw))):
         with tempfile.TemporaryDirectory() as tmp:
             trk = ref_shim.build_reference_tracker(sdict, tmp)
         otrk = O.OracleTracker(O.OracleModel(sdict))
@@ -132,15 +134,14 @@ def golden_track(ns, sd):
         out[f"{tag}_states"] = np.array(states, dtype=np.float64)
         out[f"{tag}_conf"] = np.array(confs, dtype=np.float64)
         if tag == "stable":
-            for k, v in sdict.items():
-                out[f"w_stable::{k}"] = v.numpy()
+            out.update(golden.seeded("make_state_dict", "w_stable::", **stable_kw))
         print(f"track.npz[{tag}]: 8 closed-loop frames, reference == oracle exactly; last state {states[-1]}")
     np.savez_compressed(os.path.join(GOLDEN, "track.npz"), **out)
 
 
 def main():
     if not ref_shim.available():
-        raise SystemExit("reference not mounted; golden vectors can only be regenerated where /root/reference exists")
+        raise SystemExit(f"no checkout of the original project at {ref_shim.REFERENCE_ROOT}: golden vectors are recorded from it")
     os.makedirs(GOLDEN, exist_ok=True)
     torch.set_num_threads(1)          # deterministic reduction order for the recorded reference outputs
     ns = ref_shim.load_reference()

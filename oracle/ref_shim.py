@@ -1,6 +1,6 @@
-"""Import shim that lets the UNMODIFIED reference modules under /root/reference run on CPU in this
-container (TEST INFRASTRUCTURE; used only by oracle/make_golden.py and, when /root/reference is
-mounted, by tests that re-pin the oracle.  Never imported by the product; absent on the GPU box).
+"""Import shim that lets the UNMODIFIED reference modules of the original project run on CPU (TEST INFRASTRUCTURE; used only by
+oracle/make_golden.py and, where a checkout of the original is present, by tests that re-pin the oracle against it.  Never imported
+by the product).  The checkout is looked for at oracle/_ref (kept out of git) unless $VT_REFERENCE_ROOT names another place.
 
 The reference imports packages this image lacks (SURVEY.md 8c): timm, easydict, visdom, lmdb,
 jpeg4py, matplotlib, torch._six; hard-codes ``.cuda()`` (lib/test/tracker/vit_dist.py:27,34,
@@ -19,7 +19,7 @@ import types
 import torch
 import torch.nn as nn
 
-REFERENCE_ROOT = os.environ.get("VT_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("VT_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def available() -> bool:
@@ -142,7 +142,7 @@ def install() -> None:
     if _installed:
         return
     if not available():
-        raise RuntimeError(f"reference not mounted at {REFERENCE_ROOT}")
+        raise RuntimeError(f"no checkout of the original project at {REFERENCE_ROOT} (set VT_REFERENCE_ROOT to use another)")
 
     vt = dict(Block=Block, Attention=Attention, Mlp=Mlp, LayerScale=_Identityish, DropPath=_Identityish,
               PatchEmbed=_Identityish, Final=object, use_fused_attn=lambda *a, **k: False,
@@ -178,7 +178,7 @@ def install() -> None:
         _module("torch._six", string_classes=(str, bytes), int_classes=(int,), container_abcs=__import__("collections").abc)
         torch._six = sys.modules["torch._six"]
 
-    # .cuda() -> identity on this GPU-less box
+    # .cuda() -> identity: the reference runs on the CPU here
     torch.Tensor.cuda = lambda self, *a, **k: self
     nn.Module.cuda = lambda self, *a, **k: self
 

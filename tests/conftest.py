@@ -9,6 +9,8 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
+from oracle import golden  # noqa: E402
+
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
@@ -26,19 +28,19 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def golden_crops():
-    return np.load(os.path.join(GOLDEN, "crops.npz"))
+    return golden.load(os.path.join(GOLDEN, "crops.npz"))
 
 
 @pytest.fixture(scope="session")
 def golden_model():
-    return np.load(os.path.join(GOLDEN, "model.npz"))
+    return golden.load(os.path.join(GOLDEN, "model.npz"))
 
 
 @pytest.fixture(scope="session")
 def golden_track():
-    return np.load(os.path.join(GOLDEN, "track.npz"))
+    return golden.load(os.path.join(GOLDEN, "track.npz"))
 
 
 def state_dict_from_npz(npz, prefix="w::"):
     import torch
-    return {k[len(prefix):]: torch.from_numpy(np.array(npz[k])) for k in npz.files if k.startswith(prefix)}
+    return {k[len(prefix):]: torch.from_numpy(np.array(npz[k])) for k in npz if k.startswith(prefix)}

@@ -1,10 +1,13 @@
-"""The driver-facing contract of bench.py, checked without a GPU: the reference arm runs here (it is the CPU path), and the
-last recorded B200 line under profiles/ must carry every key the contract names."""
+"""The contract of bench.py: the reference arm runs without a GPU (it is the CPU path), the last recorded B200 line under
+profiles/ must carry every key the contract names, and on a GPU two runs with the same arguments dump identical outputs."""
 import glob
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -12,8 +15,9 @@ BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_ste
              "dtype", "data", "config", "cpu_baseline", "e2e"}
 
 
-def test_reference_arm_prints_one_contract_line():
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1"],
+def test_reference_arm_prints_one_contract_line(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                        "--dump-outputs", str(tmp_path / "out")],
                        capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
@@ -26,6 +30,9 @@ def test_reference_arm_prints_one_contract_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert "workload" in d["config"] and "model" not in d["config"]
+    boxes = np.load(tmp_path / "out" / "boxes.npy")
+    assert boxes.dtype == np.float64 and boxes.shape == (256, 5) and np.isfinite(boxes).all()
+    assert ((boxes[:, 4] > 0) & (boxes[:, 4] <= 1)).all()                       # confidence: the max of a sigmoid score map
 
 
 def test_recorded_b200_line_has_every_contract_key():
@@ -63,3 +70,40 @@ def test_secondary_figures_are_json_safe_and_sane():
     assert isinstance(bench.cpu_model_name(), str)
     sd = O.make_state_dict(seed=1, stress=True)
     assert bench.cpu_b1_sample(sd, 1, budget_s=0.5) > 0
+
+
+def test_dump_outputs_keeps_a_seeded_sample_within_the_limit(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    boxes = np.random.default_rng(1).standard_normal((1000, 5))
+    bench.dump_outputs(str(tmp_path / "all"), boxes)
+    assert np.array_equal(np.load(tmp_path / "all" / "boxes.npy"), boxes) and not (tmp_path / "all" / "rows.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 4800)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), boxes)
+    rows, got = np.load(tmp_path / "a" / "rows.npy"), np.load(tmp_path / "a" / "boxes.npy")
+    assert rows.dtype == got.dtype == np.float64 and rows.nbytes + got.nbytes <= 4800
+    idx = rows.astype(np.int64)
+    assert len(idx) == 100 and np.all(np.diff(idx) > 0) and np.array_equal(got, boxes[idx])
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy")) and np.array_equal(got, np.load(tmp_path / "b" / "boxes.npy"))
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_identical_from_run_to_run(tmp_path):
+    """Two runs with the same arguments see the same inputs, so the boxes of their last timed step must be identical; the dumped boxes
+    are the ones bench.py's parity leg re-runs bit for bit and checks against the CPU oracle."""
+    lines = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "3", "--tracks", "256",
+                            "--frames", "8", "--no-cpu-baseline", "--no-latency", "--no-gpu-eager", "--dump-outputs", str(tmp_path / run)],
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        lines.append(json.loads(r.stdout.strip().splitlines()[-1]))
+    assert all(d["steps"] == 3 for d in lines)
+    for d in lines:
+        p = d["parity_spot"]
+        assert p["rerun_bit_identical_to_timed_step"] is True and p["flips"] == 0 and p["status_nonzero"] == 0, p
+        assert p["max_box_err"] <= 1e-2 + 1e-3 * 1280 and p["max_conf_err"] < 1e-3, p
+    a, b = np.load(tmp_path / "a" / "boxes.npy"), np.load(tmp_path / "b" / "boxes.npy")
+    assert a.dtype == np.float64 and a.shape == (256, 5) and np.isfinite(a).all()
+    assert np.array_equal(a, b)

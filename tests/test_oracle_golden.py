@@ -1,13 +1,14 @@
 """CPU: the oracle against the golden vectors recorded from the reference (tests/golden, written by
-oracle/make_golden.py) and against OpenCV; re-pins against /root/reference itself when mounted."""
+oracle/make_golden.py) and against OpenCV; re-pins against the reference itself where a checkout of it is present."""
 import hashlib
+import json
 
 import numpy as np
 import pytest
 import torch
 
 from conftest import state_dict_from_npz
-from oracle import ref_shim, vt_oracle as O
+from oracle import golden, ref_shim, vt_oracle as O
 
 
 def sha(a):
@@ -93,12 +94,24 @@ def test_tracker_matches_reference_golden(golden_track, golden_model, tag):
         assert abs(float(out["confidence"]) - g[f"{tag}_conf"][t - 1]) < 1e-5
 
 
+def test_golden_seeded_inputs_are_regenerated_and_checked(tmp_path):
+    entry = golden.seeded("synth_frames", "frames", n=1, H=8, W=12, seed=3)
+    np.savez(tmp_path / "ok.npz", **entry, other=np.arange(3))
+    g = golden.load(str(tmp_path / "ok.npz"))
+    assert set(g) == {"frames", "other"} and np.array_equal(g["frames"], O.synth_frames(1, 8, 12, seed=3))
+    spec = json.loads(str(entry["seeded::frames"]))
+    spec["kw"]["seed"] = 4                                  # a generator that no longer gives the recorded input
+    np.savez(tmp_path / "bad.npz", **{"seeded::frames": np.array(json.dumps(spec))})
+    with pytest.raises(AssertionError, match="no longer reproduces"):
+        golden.load(str(tmp_path / "bad.npz"))
+
+
 def test_clip_box_python_semantics():
     assert O.clip_box([-5.0, 3.0, 20.0, 4.0], 100, 200, margin=10) == [0, 3.0, 15.0, 10]
     assert O.clip_box([195.0, 95.0, 20.0, 20.0], 100, 200, margin=10) == [190, 90, 10, 10]
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not ref_shim.available(), reason="no checkout of the original project at oracle/_ref or $VT_REFERENCE_ROOT")
 def test_oracle_repinned_against_reference_itself():
     ns = ref_shim.load_reference()
     im = O.synth_frames(1, 180, 240, seed=3, smooth=True)[0]
@@ -121,7 +134,7 @@ def test_oracle_repinned_against_reference_itself():
         assert (ref[k] - out[k]).abs().max().item() <= 1e-6
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not ref_shim.available(), reason="no checkout of the original project at oracle/_ref or $VT_REFERENCE_ROOT")
 @pytest.mark.parametrize("C,heads,depth,hc", [(96, 3, 2, 64), (40, 5, 1, 24)])
 def test_oracle_generic_family_against_reference_itself(C, heads, depth, hc):
     """The generic-configuration path (BASELINE configs[4]) is checked on the GPU against the oracle at other widths / head counts /

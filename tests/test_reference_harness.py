@@ -1,9 +1,9 @@
 """The drop-in tracker class under the REFERENCE'S OWN evaluation harness (lib/test/evaluation/tracker.py:66-152 `_track_sequence`,
 lib/test/evaluation/running.py:14-102 `_save_tracker_output`), beside the reference's own `Vit_dist` on the same sequence and weights.
 
-Runs where /root/reference is mounted (this container; the harness is imported through oracle/ref_shim.py and is NOT modified).  There
-is no GPU here, so the CUDA engine behind `vittracker_b200.tracker.Vit_dist` is replaced - in this test only - by a stand-in that
-answers the engine's calls (tracks_init / tracks_set_state / tracks_step / crop_normalize) with the CPU oracle.  What is under test is
+The harness test runs where a checkout of the original project is present (oracle/_ref or $VT_REFERENCE_ROOT; imported through
+oracle/ref_shim.py and NOT modified); without it, the drop-in class is held to the reference's recorded closed loop (tests/golden).
+These tests run on the CPU, so the CUDA engine behind `vittracker_b200.tracker.Vit_dist` is replaced by a stand-in that the engine's calls (tracks_init / tracks_set_state / tracks_step / crop_normalize) with the CPU oracle.  What is under test is
 everything of the product that the harness touches: the plugin surface (`__init__(params, dataset_name)`, `params.save_all_boxes`,
 `initialize` returning None, `track` returning `target_bbox` / `confidence`), the host-side float64 box arithmetic, the aliasing of
 `target_bbox` and `state`, `z_patch_arr`, and the result-file writer.  The kernels themselves are covered by the `-m gpu` tests."""
@@ -13,9 +13,8 @@ import numpy as np
 import pytest
 import torch
 
+from conftest import state_dict_from_npz
 from oracle import ref_shim, vt_oracle as O
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference not mounted")
 
 
 class OracleEngine:
@@ -93,6 +92,29 @@ def sequence(tmp_path):
     return frames, paths, [120.5, 80.25, 60.0, 44.0]
 
 
+@pytest.mark.parametrize("tag", ["stress", "stable"])
+def test_dropin_class_reproduces_the_recorded_reference_closed_loop(golden_track, golden_model, tag, monkeypatch):
+    """The reference's own Vit_dist.initialize()/track() on 8 frames, recorded by oracle/make_golden.py, against the drop-in class on the same
+    frames and weights: the same Python numbers frame by frame (the host-side float64 map-back and clip), `target_bbox` aliasing the state."""
+    g = golden_track
+    sd = state_dict_from_npz(golden_model) if tag == "stress" else state_dict_from_npz(g, "w_stable::")
+    torch.set_num_threads(1)                                    # the reduction order the reference was recorded with
+    import vittracker_b200.tracker as vt_tracker
+    from vittracker_b200 import parameters
+    monkeypatch.setattr(vt_tracker, "build_ostrack_dist", lambda cfg, depth=3, **kw: FakeNetwork(sd))
+    params = parameters("vit_48_h32_noKD")
+    params.state_dict = sd
+    trk = vt_tracker.get_tracker_class()(params, "synthetic")
+    frames = g["frames"]
+    assert trk.initialize(frames[0], {"init_bbox": [float(v) for v in g[f"{tag}_init"]]}) is None
+    for t in range(1, 9):
+        out = trk.track(frames[t % 4], {})
+        assert out["target_bbox"] is trk.state
+        assert [float(v) for v in out["target_bbox"]] == g[f"{tag}_states"][t - 1].tolist(), (tag, t)
+        assert float(out["confidence"]) == g[f"{tag}_conf"][t - 1], (tag, t)
+
+
+@pytest.mark.skipif(not ref_shim.available(), reason="no checkout of the original project at oracle/_ref or $VT_REFERENCE_ROOT")
 def test_dropin_class_under_the_reference_harness(tmp_path, sequence, monkeypatch):
     ref = ref_shim.load_reference()
     import importlib

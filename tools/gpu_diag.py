@@ -11,7 +11,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-from oracle import vt_oracle as O  # noqa: E402
+from oracle import golden, vt_oracle as O  # noqa: E402
 from vittracker_b200 import BatchedTracker, FramePool, load_cfg  # noqa: E402
 from vittracker_b200.engine import Engine  # noqa: E402
 
@@ -29,8 +29,8 @@ def section(name, fn):
     sys.stdout.flush()
 
 
-g = np.load(os.path.join(ROOT, "tests", "golden", "model.npz"))
-sd = {k[3:]: torch.from_numpy(np.array(g[k])) for k in g.files if k.startswith("w::")}
+g = golden.load(os.path.join(ROOT, "tests", "golden", "model.npz"))
+sd = {k[3:]: torch.from_numpy(np.array(g[k])) for k in g if k.startswith("w::")}
 eng = Engine(cfg, max_tracks=512, chunk_tracks=128, blocks_impl=blocks)
 eng.load_state_dict(sd)
 

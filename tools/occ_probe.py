@@ -1,5 +1,5 @@
-import ctypes as C, sys
-sys.path.insert(0,'/root/repo')
+import ctypes as C, os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 torch.cuda.init(); torch.zeros(1,device='cuda')
 from vittracker_b200 import _lib
