@@ -201,6 +201,34 @@ int vt_profile_read(VtHandle h, double* stage_ms, int64_t* stage_launches, int64
 int vt_upload_frame_rect(const uint8_t* image, int32_t H, int32_t W, int32_t y0, int32_t y1, int32_t x0, int32_t x1,
                          uint8_t* staging, uint8_t* staging_dev, uint8_t* frame_dev, void* stream);
 
+/* YUV 4:2:0 frames, as video decoders hand them out.  Replaces cv2.cvtColor(frame, COLOR_YUV2RGB_NV12 / COLOR_YUV2RGB_I420)
+ * in front of sample_target, bit for bit (OpenCV 4.13.0, modules/imgproc/src/color_yuv.simd.hpp, 20 fractional bits):
+ *     y = max(0, Y - 16) * 1220542
+ *     R = sat_u8((y + (1 << 19) + 1673527 (V - 128)) >> 20)
+ *     G = sat_u8((y + (1 << 19) -  852492 (V - 128) - 409993 (U - 128)) >> 20)
+ *     B = sat_u8((y + (1 << 19) + 2116026 (U - 128)) >> 20)
+ * with one (U, V) sample per 2x2 luma block and no interpolation.  A frame is the array cvtColor takes: uint8 (H*3/2) x W,
+ * contiguous, pitch W, H and W even.  NV12: the H x W Y plane, then H/2 rows of W interleaved bytes U V U V ...; I420
+ * (yuv420p): the Y plane, then U (H/2 x W/2), then V (H/2 x W/2).  The result is the H x W x 3 RGB frame every other entry
+ * point takes; the tracking kernels read it unchanged. */
+#define VT_FRAME_NV12 1
+#define VT_FRAME_I420 2
+
+/* n whole frames, device -> device.  src + src_offsets[i]: a (H*3/2) x W YUV frame, frame_hw[i] = (H, W) (even);
+ * dst + dst_offsets[i]: the H x W x 3 RGB frame the other entry points take.  Arrays are device pointers.  Offsets may be
+ * any byte offset.  The sizes are read on the device: an item whose H or W is odd or below 2 is skipped (its destination is
+ * not written); a caller that cannot vouch for its sizes checks them on the host.  One kernel launch. */
+int vt_yuv420_to_rgb(VtHandle h, int32_t format, const uint8_t* src, const int64_t* src_offsets, const int32_t* frame_hw,
+                     uint8_t* dst, const int64_t* dst_offsets, int32_t n, void* stream);
+
+/* The YUV counterpart of vt_upload_frame_rect: rows [y0, y1) x columns [x0, x1) of a host YUV frame (`image`, pageable memory
+ * is fine; H and W even), widened to even bounds, are packed (Y rows, then the chroma rows), cross the link as one contiguous
+ * copy into staging_dev and are converted straight into frame_rgb_dev at their place in the H x W x 3 frame.  Nothing outside
+ * the widened rectangle is written.  `staging` (pinned host) and `staging_dev` (device, required) hold at least
+ * rows * cols * 3/2 bytes of the widened rectangle; they may be reused once `stream` has passed the conversion. */
+int vt_upload_yuv420_rect(VtHandle h, int32_t format, const uint8_t* image, int32_t H, int32_t W, int32_t y0, int32_t y1,
+                          int32_t x0, int32_t x1, uint8_t* staging, uint8_t* staging_dev, uint8_t* frame_rgb_dev, void* stream);
+
 /* Development aid: which profiled stage launches (vt_profile_enable) have started / finished.  Non-blocking;
  * meant for a watchdog thread while the owning thread waits in a synchronisation (tools/hang_probe.py,
  * tests/test_gpu_soak.py).  out[i] = stage * 4 + (started ? 1 : 0) + (finished ? 2 : 0); returns the count. */

@@ -57,6 +57,9 @@ SIGNATURES = {
     "vt_profile_read": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "vt_upload_frame_rect": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "vt_debug_pending": (C.c_int, [_P, C.POINTER(C.c_int32), C.c_int32]),
+    "vt_yuv420_to_rgb": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, C.c_int32, _P]),
+    "vt_upload_yuv420_rect": (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                        _P, _P, _P, _P]),
 }
 
 _lib = None

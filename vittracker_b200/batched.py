@@ -12,7 +12,7 @@ from typing import Optional, Sequence, Tuple
 import numpy as np
 import torch
 
-from .engine import Engine
+from .engine import Engine, yuv420_frame_hw, yuv_format
 
 
 class FramePool:
@@ -29,11 +29,41 @@ class FramePool:
         self.data = frames.to(device, non_blocking=True).contiguous()
         self.frame_bytes = self.H * self.W * 3
 
+    @classmethod
+    def from_yuv420(cls, engine: Engine, frames, format: str) -> "FramePool":
+        """RGB pool converted on the device from YUV 4:2:0 frames [F, H*3/2, W] uint8 ("nv12" or "i420", each frame laid out as
+        cv2.cvtColor takes it), on the host or already on the device (decoder output): the pool holds, bit for bit,
+        cv2.cvtColor(frame, COLOR_YUV2RGB_NV12 / _I420) of every frame."""
+        yuv_format(format)
+        if isinstance(frames, np.ndarray):
+            frames = torch.from_numpy(np.ascontiguousarray(frames))
+        if frames.dim() != 3:
+            raise ValueError("frames must be uint8 [F, H*3/2, W]")
+        H, W = yuv420_frame_hw(frames[0] if frames.shape[0] else frames.new_zeros((0, 0)))
+        F, dev = int(frames.shape[0]), engine.device
+        if frames.device.type == "cpu":
+            frames = frames.pin_memory() if torch.cuda.is_available() else frames
+        src = frames.to(dev, non_blocking=True).contiguous()
+        pool = cls(torch.empty((F, H, W, 3), dtype=torch.uint8, device=dev), dev)
+        conv = _YuvBatch(F, H, W, dev)
+        engine.yuv420_to_rgb(src, conv.src_off, conv.hw, pool.data, conv.dst_off, format)
+        return pool
+
     def offsets(self, index: torch.Tensor) -> torch.Tensor:
         return index.to(torch.int64) * self.frame_bytes
 
     def hw(self, n: int) -> torch.Tensor:
         return torch.tensor([[self.H, self.W]], dtype=torch.int32, device=self.data.device).expand(n, 2).contiguous()
+
+
+class _YuvBatch:
+    """Offsets and sizes of F contiguous (H*3/2) x W YUV frames and of their H x W x 3 RGB counterparts, on the device."""
+
+    def __init__(self, F: int, H: int, W: int, device: torch.device):
+        idx = torch.arange(F, dtype=torch.int64)
+        self.src_off = (idx * (H * W * 3 // 2)).to(device)
+        self.dst_off = (idx * (H * W * 3)).to(device)
+        self.hw = torch.tensor([[H, W]], dtype=torch.int32).expand(F, 2).contiguous().to(device)
 
 
 class BatchedTracker:
@@ -91,10 +121,27 @@ class PipelinedFrameFeeder:
 
     Every host-to-device copy of a step goes through the copy stream, small ones first: a copy engine serves its
     queue in submission order, so a small upload issued on the compute stream would wait behind the next step's
-    frames and stall the step that needs it."""
+    frames and stall the step that needs it.
 
-    def __init__(self, F: int, H: int, W: int, device: torch.device, max_tracks: int = 0):
+    ``frame_format="nv12"`` or ``"i420"`` (``engine`` required): host frames are YUV 4:2:0 [F, H*3/2, W], half the bytes of
+    RGB on the link.  They land in one of two YUV upload pools; ``acquire()`` converts that pool on the compute stream
+    (vt_yuv420_to_rgb, bit for bit cv2.cvtColor) into its paired RGB pool and returns the RGB pool; ``release()``
+    covers both."""
+
+    def __init__(self, F: int, H: int, W: int, device: torch.device, max_tracks: int = 0, frame_format: str = "rgb",
+                 engine: Optional[Engine] = None):
         self.device = device
+        self.frame_format = frame_format
+        self.yuv = None
+        if frame_format != "rgb":
+            yuv_format(frame_format)
+            if engine is None:
+                raise ValueError("a YUV frame_format needs the engine that converts the frames")
+            if H < 2 or W < 2 or H % 2 or W % 2:
+                raise ValueError(f"YUV 4:2:0 frames need an even H and W (got {H} x {W})")
+            self.engine = engine
+            self.yuv = [torch.zeros((F, H * 3 // 2, W), dtype=torch.uint8, device=device) for _ in range(2)]
+            self._conv = _YuvBatch(F, H, W, device)
         self.pools = [FramePool(torch.zeros((F, H, W, 3), dtype=torch.uint8), device) for _ in range(2)]
         for p in self.pools:
             p.boxes = torch.zeros((max_tracks, 4), dtype=torch.float64, device=device) if max_tracks > 0 else None
@@ -112,13 +159,16 @@ class PipelinedFrameFeeder:
                 self.copy_stream.wait_event(self._free[i])
             if host_boxes is not None:
                 self.pools[i].boxes[: host_boxes.shape[0]].copy_(host_boxes, non_blocking=True)
-            self.pools[i].data.copy_(host_frames, non_blocking=True)
+            (self.pools[i].data if self.yuv is None else self.yuv[i]).copy_(host_frames, non_blocking=True)
             self._ready[i].record(self.copy_stream)
         self._pending.append(i)
 
     def acquire(self) -> FramePool:
         i = self._pending.pop(0)
         torch.cuda.current_stream(self.device).wait_event(self._ready[i])
+        if self.yuv is not None:
+            c = self._conv
+            self.engine.yuv420_to_rgb(self.yuv[i], c.src_off, c.hw, self.pools[i].data, c.dst_off, self.frame_format)
         return self.pools[i]
 
     def release(self, pool: FramePool) -> None:

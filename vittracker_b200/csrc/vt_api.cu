@@ -360,6 +360,59 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
     return VT_OK;
 }
 
+// Host rows -> device, the part of a frame upload that scales with its size.  `runs` are packed back to back into the pinned
+// `staging` and cross the link into `dev` at the same offsets; dev == NULL: packed only (the caller copies from `staging`).
+// Packing is a plain memory copy: a single thread moves ~25 GB/s, a few OpenMP threads (the runtime's pool stays warm between
+// frames) ~45 GB/s, the link 55 GB/s.  The rows go in up to four pieces of >= 384 KB, so that a piece crosses the link while the
+// next one is packed.  A strided host -> device copy runs at half the link's rate (the DMA engine walks the rows), a contiguous one
+// at all of it: each piece crosses in one copy.
+struct PackRun {
+    const uint8_t* src;
+    size_t pitch, bytes;       // `rows` rows of `bytes` bytes, `pitch` apart
+    int rows;
+};
+
+cudaError_t pack_upload(const PackRun* runs, int nruns, uint8_t* staging, uint8_t* dev, cudaStream_t st) {
+    int rows = 0;
+    size_t total = 0;
+    for (int k = 0; k < nruns; ++k) { rows += runs[k].rows; total += (size_t)runs[k].rows * runs[k].bytes; }
+    auto offset_of = [&](int row) {            // packed byte offset of global row `row`
+        size_t off = 0;
+        for (int k = 0; k < nruns && row > 0; ++k) {
+            const int m = row < runs[k].rows ? row : runs[k].rows;
+            off += (size_t)m * runs[k].bytes;
+            row -= m;
+        }
+        return off;
+    };
+    int pieces = (int)(total / (384u << 10));
+    pieces = pieces < 1 ? 1 : pieces > 4 ? 4 : pieces;
+    if (!dev) pieces = 1;
+    const int cap = omp_get_max_threads() < 8 ? omp_get_max_threads() : 8;
+    cudaError_t e = cudaSuccess;
+    for (int p = 0; p < pieces && e == cudaSuccess; ++p) {
+        const int r0 = (int)((long long)rows * p / pieces), r1 = (int)((long long)rows * (p + 1) / pieces);
+        const size_t off = offset_of(r0), len = offset_of(r1) - off;
+        int nt = (int)(len / (96u << 10));
+        nt = nt < 1 ? 1 : nt > cap ? cap : nt;
+        size_t base = 0;
+        for (int k = 0, g0 = 0; k < nruns; g0 += runs[k].rows, base += (size_t)runs[k].rows * runs[k].bytes, ++k) {
+            const int a = (r0 > g0 ? r0 : g0) - g0, b = (r1 < g0 + runs[k].rows ? r1 : g0 + runs[k].rows) - g0;
+            const PackRun& R = runs[k];
+            uint8_t* out = staging + base;
+            if (a >= b) continue;
+            if (nt == 1) {
+                for (int i = a; i < b; ++i) memcpy(out + (size_t)i * R.bytes, R.src + (size_t)i * R.pitch, R.bytes);
+            } else {
+#pragma omp parallel for num_threads(nt) schedule(static)
+                for (int i = a; i < b; ++i) memcpy(out + (size_t)i * R.bytes, R.src + (size_t)i * R.pitch, R.bytes);
+            }
+        }
+        if (dev) e = cudaMemcpyAsync(dev + off, staging + off, len, cudaMemcpyHostToDevice, st);
+    }
+    return e;
+}
+
 }  // namespace
 
 extern "C" {
@@ -956,42 +1009,74 @@ int vt_upload_frame_rect(const uint8_t* image, int32_t H, int32_t W, int32_t y0,
     if (!image || !staging || !frame_dev || H <= 0 || W <= 0 || y0 < 0 || y1 > H || y0 >= y1 || x0 < 0 || x1 > W || x0 >= x1) return VT_ERR_INVALID_ARG;
     const size_t pitch = (size_t)W * 3, wb = (size_t)(x1 - x0) * 3;
     const int rows = y1 - y0;
-    const uint8_t* src = image + (size_t)y0 * pitch + (size_t)x0 * 3;
-    // Packing is a plain memory copy and the only host work of a frame that scales with its size: a single thread moves ~25 GB/s, a few
-    // OpenMP threads (the runtime's pool stays warm between frames) ~45 GB/s, the link 55 GB/s.  The rectangle goes in up to four pieces
-    // of >= 384 KB, so that a piece crosses the link while the next one is packed.  A strided host -> device copy runs at half the
-    // link's rate (the DMA engine walks the rows), a contiguous one at all of it: the packed pieces cross in one copy each and are
-    // spread over the frame's rows by one device-to-device copy at the end.
     cudaStream_t st = (cudaStream_t)stream;
     uint8_t* dst = frame_dev + (size_t)y0 * pitch + (size_t)x0 * 3;
-    const size_t total = (size_t)rows * wb;
-    int pieces = (int)(total / (384u << 10));
-    pieces = pieces < 1 ? 1 : pieces > 4 ? 4 : pieces;
-    const int cap = omp_get_max_threads() < 8 ? omp_get_max_threads() : 8;
     const bool direct = wb == pitch;                       // full rows: the packed layout is the frame's
-    if (!direct && !staging_dev) pieces = 1;
-    cudaError_t e = cudaSuccess;
-    for (int p = 0; p < pieces && e == cudaSuccess; ++p) {
-        const int r0 = (int)((long long)rows * p / pieces), r1 = (int)((long long)rows * (p + 1) / pieces);
-        int nt = (int)((size_t)(r1 - r0) * wb / (96u << 10));
-        nt = nt < 1 ? 1 : nt > cap ? cap : nt;
-        if (nt == 1) {
-            for (int i = r0; i < r1; ++i) memcpy(staging + (size_t)i * wb, src + (size_t)i * pitch, wb);
-        } else {
-#pragma omp parallel for num_threads(nt) schedule(static)
-            for (int i = r0; i < r1; ++i) memcpy(staging + (size_t)i * wb, src + (size_t)i * pitch, wb);
-        }
-        const size_t off = (size_t)r0 * wb, len = (size_t)(r1 - r0) * wb;
-        if (direct) e = cudaMemcpyAsync(dst + off, staging + off, len, cudaMemcpyHostToDevice, st);
-        else if (staging_dev) e = cudaMemcpyAsync(staging_dev + off, staging + off, len, cudaMemcpyHostToDevice, st);
-        else e = cudaMemcpy2DAsync(dst, pitch, staging, wb, wb, (size_t)rows, cudaMemcpyHostToDevice, st);
-    }
-    if (e == cudaSuccess && !direct && staging_dev)
-        e = cudaMemcpy2DAsync(dst, pitch, staging_dev, wb, wb, (size_t)rows, cudaMemcpyDeviceToDevice, st);
+    const PackRun run{image + (size_t)y0 * pitch + (size_t)x0 * 3, pitch, wb, rows};
+    cudaError_t e = pack_upload(&run, 1, staging, direct ? dst : staging_dev, st);
+    if (e == cudaSuccess && !direct)
+        e = staging_dev ? cudaMemcpy2DAsync(dst, pitch, staging_dev, wb, wb, (size_t)rows, cudaMemcpyDeviceToDevice, st)
+                        : cudaMemcpy2DAsync(dst, pitch, staging, wb, wb, (size_t)rows, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) {
         cudaGetLastError();
         return VT_ERR_CUDA;
     }
+    return VT_OK;
+}
+
+int vt_upload_yuv420_rect(VtHandle h, int32_t format, const uint8_t* image, int32_t H, int32_t W, int32_t y0, int32_t y1,
+                          int32_t x0, int32_t x1, uint8_t* staging, uint8_t* staging_dev, uint8_t* frame_rgb_dev, void* stream) {
+    if (!h) return VT_ERR_INVALID_ARG;
+    if (format != VT_FRAME_NV12 && format != VT_FRAME_I420) return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: unknown format %d", format);
+    if (!image || !staging || !staging_dev || !frame_rgb_dev) return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: null pointer");
+    if (H < 2 || W < 2 || (H & 1) || (W & 1)) return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: frame %d x %d: H and W must be even and positive", H, W);
+    if (y0 < 0 || y1 > H || y0 >= y1 || x0 < 0 || x1 > W || x0 >= x1)
+        return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: rectangle [%d, %d) x [%d, %d) is empty or leaves the %d x %d frame", y0, y1, x0, x1, H, W);
+    // widen to even bounds: a 2x2 block shares one chroma sample
+    y0 &= ~1; x0 &= ~1; y1 = (y1 + 1) & ~1; x1 = (x1 + 1) & ~1;
+    const int rows = y1 - y0, cols = x1 - x0;
+    const uint8_t* chroma = image + (size_t)H * W;
+    PackRun runs[3];
+    int nruns = 0;
+    runs[nruns++] = {image + (size_t)y0 * W + x0, (size_t)W, (size_t)cols, rows};
+    if (format == VT_FRAME_NV12) {
+        runs[nruns++] = {chroma + (size_t)(y0 / 2) * W + x0, (size_t)W, (size_t)cols, rows / 2};
+    } else {
+        const size_t cw = (size_t)W / 2;
+        runs[nruns++] = {chroma + (size_t)(y0 / 2) * cw + x0 / 2, cw, (size_t)cols / 2, rows / 2};
+        runs[nruns++] = {chroma + (size_t)(H / 2) * cw + (size_t)(y0 / 2) * cw + x0 / 2, cw, (size_t)cols / 2, rows / 2};
+    }
+    DeviceGuard dg(h->cfg.device);
+    VT_CUDA(h, dg.err);
+    cudaStream_t st = (cudaStream_t)stream;
+    VT_CUDA(h, pack_upload(runs, nruns, staging, staging_dev, st));
+    YuvDesc d{};
+    d.y = staging_dev;
+    d.u = staging_dev + (size_t)rows * cols;
+    d.y_pitch = cols;
+    d.c_pitch = format == VT_FRAME_NV12 ? cols : cols / 2;
+    d.v = d.u + (size_t)(rows / 2) * (cols / 2);
+    d.dst = frame_rgb_dev + ((size_t)y0 * W + x0) * 3;
+    d.dst_pitch = (int64_t)W * 3;
+    d.w = cols; d.h = rows;
+    const int k = launch_yuv420_rect(format, d, h->num_sms, st);
+    if (k < 0) return fail(h, VT_ERR_CUDA, "vt_upload_yuv420_rect: kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    h->launches += k;
+    return VT_OK;
+}
+
+int vt_yuv420_to_rgb(VtHandle h, int32_t format, const uint8_t* src, const int64_t* src_offsets, const int32_t* frame_hw,
+                     uint8_t* dst, const int64_t* dst_offsets, int32_t n, void* stream) {
+    if (!h) return VT_ERR_INVALID_ARG;
+    if (format != VT_FRAME_NV12 && format != VT_FRAME_I420) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_to_rgb: unknown format %d", format);
+    if (n < 0) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_to_rgb: negative n");
+    if (n == 0) return VT_OK;
+    if (!src || !src_offsets || !frame_hw || !dst || !dst_offsets) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_to_rgb: null pointer");
+    DeviceGuard dg(h->cfg.device);
+    VT_CUDA(h, dg.err);
+    const int k = launch_yuv420_to_rgb(format, src, src_offsets, frame_hw, dst, dst_offsets, n, h->num_sms, (cudaStream_t)stream);
+    if (k < 0) return fail(h, VT_ERR_CUDA, "vt_yuv420_to_rgb: kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    h->launches += k;
     return VT_OK;
 }
 

@@ -228,6 +228,22 @@ struct DeviceGuard {
 };
 
 // ---- kernel launchers (each returns the number of kernels it launched, or <0 on a CUDA error) -----
+// YUV 4:2:0 -> RGB (vt_yuv.cu).  One work item: an even w x h image whose luma rows are y_pitch apart and whose chroma rows
+// (one per two luma rows) are c_pitch apart; NV12 reads interleaved U V pairs at u, I420 reads U at u and V at v.
+constexpr int kYuvNV12 = 1, kYuvI420 = 2;
+struct YuvDesc {
+    const uint8_t* y;
+    const uint8_t* u;
+    const uint8_t* v;
+    uint8_t* dst;                  // w x h x 3 RGB, rows dst_pitch apart
+    int64_t y_pitch, c_pitch, dst_pitch;
+    int32_t w, h;
+};
+// n whole frames laid out as cv2.cvtColor takes them ((H*3/2) x W, pitch W); items whose H or W is odd or < 2 are skipped.
+int launch_yuv420_to_rgb(int format, const uint8_t* src, const int64_t* src_offsets, const int32_t* frame_hw, uint8_t* dst,
+                         const int64_t* dst_offsets, int n, int num_sms, cudaStream_t st);
+int launch_yuv420_rect(int format, const YuvDesc& d, int num_sms, cudaStream_t st);
+
 int launch_crop_normalize(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
                           const double* boxes, double factor, int S, int n, const float* lut,
                           float* out_nchw, uint8_t* out_u8, uint8_t* out_mask, double* out_rf,

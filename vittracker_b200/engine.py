@@ -18,6 +18,25 @@ def _ptr(t: Optional[torch.Tensor]):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+YUV_FORMATS = {"nv12": 1, "i420": 2}          # VT_FRAME_NV12, VT_FRAME_I420
+
+
+def yuv_format(name: str) -> int:
+    if name not in YUV_FORMATS:
+        raise ValueError(f"unknown YUV format {name!r}: expected one of {sorted(YUV_FORMATS)}")
+    return YUV_FORMATS[name]
+
+
+def yuv420_frame_hw(frame) -> Tuple[int, int]:
+    """(H, W) of a YUV 4:2:0 frame laid out as cv2.cvtColor takes it: uint8 (H*3/2) x W with H and W even."""
+    if frame.dtype not in (np.uint8, torch.uint8) or frame.ndim != 2:
+        raise ValueError("a YUV 4:2:0 frame must be a 2-D uint8 array of shape (H*3/2, W)")
+    rows, W = int(frame.shape[0]), int(frame.shape[1])
+    if rows % 3 or (rows * 2 // 3) % 2 or W % 2 or rows == 0 or W == 0:
+        raise ValueError(f"YUV 4:2:0 frame of shape {tuple(frame.shape)}: expected (H*3/2, W) with H and W even and positive")
+    return rows * 2 // 3, W
+
+
 def hann2d_window(sz: int = 16) -> torch.Tensor:
     """Cosine window the reference builds once per tracker (lib/test/utils/hann.py:6-16,
     centered=True): w[k] = 0.5 (1 - cos(2 pi k / (sz + 1))), k = 1..sz, outer product -> (1,1,sz,sz)."""
@@ -168,6 +187,38 @@ class Engine:
         with torch.cuda.device(dev):
             self._check(self.lib.vt_cal_bbox(self.handle, _ptr(score), _ptr(size_map), _ptr(offset_map), int(n), _ptr(boxes), self._stream()))
         return boxes
+
+    # ------------------------------------------------------------------------------------------
+    def yuv420_to_rgb(self, src: torch.Tensor, src_offsets: torch.Tensor, frame_hw: torch.Tensor, dst: torch.Tensor,
+                      dst_offsets: torch.Tensor, format: str) -> torch.Tensor:
+        """cv2.cvtColor(COLOR_YUV2RGB_NV12 / _I420) of n frames, bit for bit, device -> device: the (H*3/2) x W YUV frame at byte
+        ``src_offsets[i]`` of ``src`` becomes the H x W x 3 frame at byte ``dst_offsets[i]`` of ``dst``.  uint8 buffers, int64
+        offsets [n], int32 frame_hw [n, 2] (even), all on this engine's device.  Returns ``dst``."""
+        fmt = yuv_format(format)
+        for t, dt in ((src, torch.uint8), (dst, torch.uint8), (src_offsets, torch.int64), (dst_offsets, torch.int64), (frame_hw, torch.int32)):
+            if t.dtype != dt or t.device != self.device or not t.is_contiguous():
+                raise ValueError(f"yuv420_to_rgb: expected a contiguous {dt} tensor on {self.device}")
+        n = int(src_offsets.shape[0])
+        if dst_offsets.shape != (n,) or frame_hw.shape != (n, 2):
+            raise ValueError("yuv420_to_rgb: src_offsets [n], dst_offsets [n] and frame_hw [n, 2] required")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_yuv420_to_rgb(self.handle, fmt, _ptr(src), _ptr(src_offsets), _ptr(frame_hw), _ptr(dst),
+                                                  _ptr(dst_offsets), n, self._stream()))
+        return dst
+
+    def upload_yuv420_rect(self, format: str, image: np.ndarray, y0: int, y1: int, x0: int, x1: int, staging: torch.Tensor,
+                           staging_dev: torch.Tensor, frame_rgb: torch.Tensor) -> None:
+        """Rows [y0, y1) x columns [x0, x1) of the host YUV frame ``image`` ((H*3/2) x W uint8), widened to even bounds, into the
+        H x W x 3 device frame ``frame_rgb`` through ``staging`` (pinned) and ``staging_dev`` (vt_upload_yuv420_rect)."""
+        fmt = yuv_format(format)
+        H, W = yuv420_frame_hw(image)
+        image = np.ascontiguousarray(image)
+        need = H * W * 3 // 2
+        if staging.numel() < need or staging_dev.numel() < need or frame_rgb.numel() < H * W * 3:
+            raise ValueError("upload_yuv420_rect: staging buffers need (H*3/2) x W bytes and frame_rgb H x W x 3")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_upload_yuv420_rect(self.handle, fmt, image.ctypes.data, H, W, int(y0), int(y1), int(x0), int(x1),
+                                                       _ptr(staging), _ptr(staging_dev), _ptr(frame_rgb), self._stream()))
 
     # ------------------------------------------------------------------------------------------
     def tracks_init(self, frames, frame_offsets, frame_hw, boxes, first: int = 0) -> torch.Tensor:

@@ -14,9 +14,17 @@ from typing import Optional
 import numpy as np
 import torch
 
+from .engine import yuv420_frame_hw, yuv_format
 from .model import build_ostrack_dist
 from .sequences import crop_rect
 from .weights import load_checkpoint
+
+
+def even_rect(rect, H: int, W: int) -> tuple:
+    """``rect`` = (ya, yb, xa, xb) widened to even bounds inside an even H x W frame: the rectangle vt_upload_yuv420_rect converts
+    (a 2x2 luma block shares one chroma sample)."""
+    ya, yb, xa, xb = rect
+    return ya & ~1, min(H, (yb + 1) & ~1), xa & ~1, min(W, (xb + 1) & ~1)
 
 
 def clip_box(box: list, H, W, margin=0):
@@ -88,6 +96,11 @@ class Vit_dist(BaseTracker):
         self._out_boxes = self._out_dev[:5].view(1, 5)
         self._out_detail = self._out_dev[5:].view(1, 8)
         self._graph, self._graph_key = None, None
+        # params.frame_format: "rgb" (H x W x 3, the reference's input) or a YUV 4:2:0 layout as decoders hand it out, "nv12" or
+        # "i420" ((H*3/2) x W, as cv2.cvtColor takes it), converted on the device bit for bit as cv2.cvtColor(COLOR_YUV2RGB_*) would
+        self.frame_format = getattr(params, "frame_format", "rgb")
+        if self.frame_format != "rgb":
+            yuv_format(self.frame_format)
 
     # ------------------------------------------------------------------------------------------
     def _pinned(self, t: torch.Tensor) -> torch.Tensor:
@@ -98,11 +111,17 @@ class Vit_dist(BaseTracker):
             torch.cuda.current_stream(self._dev).synchronize()
 
     def _upload(self, image: np.ndarray, box, factor: float):
-        """Stage the rows of ``image`` the crop will read into the device frame buffer."""
-        if image.dtype != np.uint8 or image.ndim != 3 or image.shape[2] != 3:
-            raise ValueError("image must be HxWx3 uint8")
+        """Stage the rows of ``image`` the crop will read into the device frame buffer (as RGB, whatever the frame format)."""
+        yuv = self.frame_format != "rgb"
+        if yuv:
+            if not isinstance(image, np.ndarray):
+                raise ValueError(f"image must be a ({self.frame_format}) numpy array")
+            H, W = yuv420_frame_hw(image)
+        else:
+            if image.dtype != np.uint8 or image.ndim != 3 or image.shape[2] != 3:
+                raise ValueError("image must be HxWx3 uint8")
+            H, W, _ = image.shape
         image = np.ascontiguousarray(image)
-        H, W, _ = image.shape
         if (H, W) != self._hw:
             # zero-filled: the crop kernels read the first pixels of a row with weight 0 for taps in the padding
             self._frame_dev = torch.zeros((H * W * 3,), dtype=torch.uint8, device=self._dev)
@@ -119,7 +138,11 @@ class Vit_dist(BaseTracker):
         if rect is None:
             raise ValueError("crop lies outside the image (undefined in the reference)")
         ya, yb, xa, xb = rect
-        if self._dev.type == "cuda":
+        if yuv:
+            # the even-widened rectangle (a superset of crop_rect) crosses the link as YUV and is converted into the RGB frame
+            ya, yb, xa, xb = even_rect(rect, H, W)
+            self.engine.upload_yuv420_rect(self.frame_format, image, ya, yb, xa, xb, self._frame_pin, self._frame_stage, self._frame_dev)
+        elif self._dev.type == "cuda":
             with torch.cuda.device(self._dev):
                 rc = self.engine.lib.vt_upload_frame_rect(image.ctypes.data, H, W, ya, yb, xa, xb, self._frame_pin.data_ptr(),
                                                           self._frame_stage.data_ptr(), self._frame_dev.data_ptr(),
