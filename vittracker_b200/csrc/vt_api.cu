@@ -472,6 +472,7 @@ int vt_create(const VtConfig* cfg, VtHandle* out) {
     } else {
         h->gw.C = cfg->embed_dim; h->gw.heads = cfg->num_heads; h->gw.depth = cfg->depth; h->gw.hc = cfg->head_channels;
         h->gw.use_img = (cfg->blocks_impl != VT_BLOCKS_SIMT_FP32 && cfg->embed_dim % 128 == 0) ? 1 : 0;
+        h->gw.fp32_only = cfg->blocks_impl == VT_BLOCKS_SIMT_FP32 ? 1 : 0;
         size_t off[kGenWorkSlots];
         const size_t tot = gen_work_floats(h->gw, h->chunk, off);
         A((void**)&h->d_gwork, tot * sizeof(float));

@@ -1,6 +1,6 @@
 // Generic-configuration path: OstrackDist.forward for ANY member of the vit_dist family (embed dim C, heads, depth,
 // head width), used for every configuration other than vit_48_h32 - in particular the widest one (C = 768, 12 heads,
-// depth 12, head 256; BASELINE configs[4]).  Same arithmetic as the reference graph, fp32 on CUDA cores:
+// depth 12, head 256; BASELINE configs[4]).  Same arithmetic as the reference graph:
 //   LevitPatchEmbedding   lib/models/vit_dist/vit_dist.py:10-54   conv3x3 s2 + BN(eval, folded) [+ Hardswish] x4
 //   OstrackDist.forward   lib/models/vit_dist/vit_dist.py:77-100  pos-embed add, cat(z, x), blocks, LayerNorm
 //   timm Block            tracking/onnxexport.py:126-225          LN -> qkv -> MHSA (h heads) -> proj, LN -> fc1 -> GELU -> fc2
@@ -8,6 +8,10 @@
 // Convolutions are im2col (NHWC, k = (ky, kx, ci)) + one tiled GEMM with a fused bias / activation / residual epilogue;
 // attention is two batched GEMMs (batch = track x head) around a row softmax.  The decode is the code the fused head
 // kernels use (vt_decode.cuh).  This path favours coverage over speed; the tuned kernels are vit_48_h32's.
+// Precision: under blocks_impl "simt" (GenModelW::fp32_only) every GEMM runs on the fp32 CUDA-core kernel (sgemm_kernel).  Otherwise
+// the GEMMs whose shapes allow it run on the tensor cores with fp16 hi / lo operand splits (three products: hi*hi + lo*hi + hi*lo),
+// gemm_tc_kernel converting fp32 operands per tile and, for C a multiple of 128, gemm_img_kernel reading pre-split images; the rest
+// stays on sgemm_kernel.  tests/test_generic_edges.py maps which configuration reaches which kernel.
 #include <stdlib.h>
 #include <string.h>
 
@@ -39,6 +43,7 @@ struct GemmArgs {
     // optional: write the result as the split image of a matrix with img_K columns instead of C (tensor-core kernel only):
     // element (m, n) of batch z lands at image row z1 * img_rows1 + m, column z2 * img_cols2 + n
     uint8_t* Cimg; int img_K; long long img_rows1; int img_cols2;
+    int tile_y0, z0;     // row tile and batch index of blockIdx.y = 0 / blockIdx.z = 0 (launch_pieces)
 };
 
 constexpr int kBM = 64, kBN = 64, kBK = 16;
@@ -48,12 +53,12 @@ template <bool NN>
 __global__ void __launch_bounds__(256) sgemm_kernel(GemmArgs g) {
     __shared__ float As[kBK][kBM + 4];
     __shared__ float Bs[kBK][kBN + 4];
-    const int z = blockIdx.z, z1 = z / g.nh, z2 = z % g.nh;
+    const int z = blockIdx.z + g.z0, z1 = z / g.nh, z2 = z % g.nh;
     const float* A = g.A + z1 * g.sa1 + z2 * g.sa2;
     const float* B = g.B + z1 * g.sb1 + z2 * g.sb2;
     float* C = g.C + z1 * g.sc1 + z2 * g.sc2;
     const float* R = g.R ? g.R + z1 * g.sr1 + z2 * g.sr2 : nullptr;
-    const int m0 = blockIdx.y * kBM, n0 = blockIdx.x * kBN;
+    const int m0 = (blockIdx.y + g.tile_y0) * kBM, n0 = blockIdx.x * kBN;
     const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
     float acc[4][4];
 #pragma unroll
@@ -140,12 +145,12 @@ __global__ void __launch_bounds__(kTcGemmThreads) gemm_tc_kernel(GemmArgs g) {
     uint64_t* bar_acc = bar_empty + kTcStages;
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bar_acc + 1);
     const int tid = threadIdx.x, warp = tid >> 5;
-    const int z = blockIdx.z, z1 = z / g.nh, z2 = z % g.nh;
+    const int z = blockIdx.z + g.z0, z1 = z / g.nh, z2 = z % g.nh;
     const float* A = g.A + z1 * g.sa1 + z2 * g.sa2;
     const float* B = g.B + z1 * g.sb1 + z2 * g.sb2;
     float* C = g.C + z1 * g.sc1 + z2 * g.sc2;
     const float* R = g.R ? g.R + z1 * g.sr1 + z2 * g.sr2 : nullptr;
-    const int m0 = blockIdx.y * kTcBM, n0 = blockIdx.x * kTcBN;
+    const int m0 = (blockIdx.y + g.tile_y0) * kTcBM, n0 = blockIdx.x * kTcBN;
     const int ksteps = (g.K + kTcBK - 1) / kTcBK;
 
     if (warp == 8) tc::tmem_alloc(s_tmem, 128);
@@ -269,13 +274,25 @@ bool gemm_tc_ok(const GemmArgs& g, bool nn) {
     return nn || (g.ldb % 4 == 0 && al16(g.B) && g.sb1 % 4 == 0 && g.sb2 % 4 == 0);     // B[k][n] is read with scalar loads
 }
 
+// gridDim.y and gridDim.z are limited to 65535 (stem conv1 of the search crop has 256 row tiles per track): a launch takes at most
+// that many row tiles and batch entries, and the kernels add tile_y0 / z0.  Every output element is computed by the same thread
+// arithmetic whatever the piece, so the split changes no bit.  Returns the number of launches.
+constexpr int kMaxGridYZ = 65535;
+template <typename Launch>
+int launch_pieces(GemmArgs g, int tiles_x, int tiles_y, int batch, Launch launch) {
+    int launched = 0;
+    for (g.z0 = 0; g.z0 < batch; g.z0 += kMaxGridYZ)
+        for (g.tile_y0 = 0; g.tile_y0 < tiles_y; g.tile_y0 += kMaxGridYZ, ++launched)
+            launch(g, dim3(tiles_x, min(kMaxGridYZ, tiles_y - g.tile_y0), min(kMaxGridYZ, batch - g.z0)));
+    return cudaGetLastError() == cudaSuccess ? launched : -1;
+}
+
 template <bool NN>
 int launch_gemm_tc(const GemmArgs& g, int batch, cudaStream_t st) {
     static DeviceOnce once;
     if (!ensure_dyn_smem(once, gemm_tc_kernel<NN>, kTcGemmSmem)) return -1;
-    dim3 grid((g.N + kTcBN - 1) / kTcBN, (g.M + kTcBM - 1) / kTcBM, batch);
-    gemm_tc_kernel<NN><<<grid, kTcGemmThreads, kTcGemmSmem, st>>>(g);
-    return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    return launch_pieces(g, (g.N + kTcBN - 1) / kTcBN, (g.M + kTcBM - 1) / kTcBM, batch,
+                         [&](const GemmArgs& p, dim3 grid) { gemm_tc_kernel<NN><<<grid, kTcGemmThreads, kTcGemmSmem, st>>>(p); });
 }
 
 // ---- split-image GEMM: C = act(A B^T + bias) + R with BOTH operands already in the tensor cores' shared-memory layout -------------------
@@ -294,6 +311,7 @@ struct ImgGemmArgs {
     uint8_t* Cimg;          // image of the result (K' = N), or null
     int rmod;               // > 0: residual row = m % rmod (the positional embedding, broadcast over tracks)
     int c_group, c_stride;  // c_group > 0: output row of m = (m / c_group) * c_stride + m % c_group (tokens of a track inside [320][C])
+    int tile_y0;            // row tile of blockIdx.y = 0 (run_gemm_img splits the grid like launch_pieces)
 };
 constexpr int kIgStages = 3;
 constexpr int kIgStageBytes = 2 * kImgBlockBytes;                                   // A block | B block
@@ -307,7 +325,7 @@ __global__ void __launch_bounds__(kIgThreads) gemm_img_kernel(ImgGemmArgs g) {
     uint64_t* bar_acc = bar_empty + kIgStages;
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bar_acc + 1);
     const int tid = threadIdx.x, warp = tid >> 5;
-    const int m0 = blockIdx.y * 128, n0 = blockIdx.x * 128;
+    const int ty = blockIdx.y + g.tile_y0, m0 = ty * 128, n0 = blockIdx.x * 128;
     const int ksteps = g.K / 32;
     if (warp == 9) tc::tmem_alloc(s_tmem, 128);
     if (tid == 0) {
@@ -322,7 +340,7 @@ __global__ void __launch_bounds__(kIgThreads) gemm_img_kernel(ImgGemmArgs g) {
 
     if (warp == 8) {
         // ---- bulk copies: block (row tile, K panel) of each operand, kIgStages in flight ----
-        const uint8_t* ab = g.A + (size_t)blockIdx.y * ksteps * kImgBlockBytes;
+        const uint8_t* ab = g.A + (size_t)ty * ksteps * kImgBlockBytes;
         const uint8_t* bb = g.B + (size_t)blockIdx.x * ksteps * kImgBlockBytes;
 #pragma unroll 1
         for (int ks = 0; ks < ksteps; ++ks) {
@@ -405,14 +423,17 @@ __global__ void __launch_bounds__(kIgThreads) gemm_img_kernel(ImgGemmArgs g) {
     if (warp == 9) tc::tmem_dealloc(tbase, 128);
 }
 
-int run_gemm_img(const ImgGemmArgs& g, cudaStream_t st) {
-    if (g.M <= 0) return 0;
-    if (g.N % 16 != 0 || g.K % 32 != 0 || (g.C && (g.ldc % 4 != 0)) || (g.Cimg && g.N % 32 != 0)) return -1;
+int run_gemm_img(const ImgGemmArgs& g0, cudaStream_t st) {
+    if (g0.M <= 0) return 0;
+    if (g0.N % 16 != 0 || g0.K % 32 != 0 || (g0.C && (g0.ldc % 4 != 0)) || (g0.Cimg && g0.N % 32 != 0)) return -1;
     static DeviceOnce once;
     if (!ensure_dyn_smem(once, gemm_img_kernel, kIgSmem)) return -1;
-    dim3 grid((g.N + 127) / 128, (g.M + 127) / 128);
-    gemm_img_kernel<<<grid, kIgThreads, kIgSmem, st>>>(g);
-    return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    const int tiles_y = (g0.M + 127) / 128;
+    int launched = 0;
+    ImgGemmArgs g = g0;
+    for (g.tile_y0 = 0; g.tile_y0 < tiles_y; g.tile_y0 += kMaxGridYZ, ++launched)
+        gemm_img_kernel<<<dim3((g.N + 127) / 128, min(kMaxGridYZ, tiles_y - g.tile_y0)), kIgThreads, kIgSmem, st>>>(g);
+    return cudaGetLastError() == cudaSuccess ? launched : -1;
 }
 
 // LayerNorm over the last dim C (eps 1e-5), one warp per row (same arithmetic as layernorm_kernel), result written as a split image
@@ -446,7 +467,21 @@ __global__ void __launch_bounds__(256) layernorm_img_kernel(const float* __restr
     }
 }
 
-int run_gemm(const GemmArgs& g, int batch, bool nn, cudaStream_t st);
+// fp32 rows [rows][K] (K a multiple of 8) -> split image, thread = (row, 8-wide chunk)
+__global__ void __launch_bounds__(256) rows_img_kernel(const float* __restrict__ in, uint8_t* __restrict__ img, long long rows, int K) {
+    const int chunks = K / 8;
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < rows * chunks; i += (long long)gridDim.x * 256) {
+        const long long row = i / chunks;
+        const int kc = (int)(i % chunks);
+        const float4* p = reinterpret_cast<const float4*>(in + row * K + 8 * kc);
+        uint4 hi, lo;
+        gen_split8(p[0], p[1], hi, lo);
+        *reinterpret_cast<uint4*>(img + gen_img_offset(row, kc, K, 0)) = hi;
+        *reinterpret_cast<uint4*>(img + gen_img_offset(row, kc, K, 1)) = lo;
+    }
+}
+
+int run_gemm(const GemmArgs& g, int batch, bool nn, const GenModelW& w, cudaStream_t st);
 
 }  // namespace
 
@@ -473,14 +508,15 @@ void gen_pack_weight_image(const float* w, int N, int K, uint8_t* img) {
 
 namespace {
 
-int run_gemm(const GemmArgs& g, int batch, bool nn, cudaStream_t st) {
+// w.fp32_only (blocks_impl "simt"): every GEMM on the fp32 CUDA-core kernel, no fp16 operand anywhere
+int run_gemm(const GemmArgs& g, int batch, bool nn, const GenModelW& w, cudaStream_t st) {
     if (g.M <= 0 || g.N <= 0 || batch <= 0) return 0;
-    if (gemm_tc_ok(g, nn)) return nn ? launch_gemm_tc<true>(g, batch, st) : launch_gemm_tc<false>(g, batch, st);
+    if (!w.fp32_only && gemm_tc_ok(g, nn)) return nn ? launch_gemm_tc<true>(g, batch, st) : launch_gemm_tc<false>(g, batch, st);
     if (g.Cimg) return -1;                      // the image epilogue exists on the tensor-core kernel only
-    dim3 grid((g.N + kBN - 1) / kBN, (g.M + kBM - 1) / kBM, batch);
-    if (nn) sgemm_kernel<true><<<grid, 256, 0, st>>>(g);
-    else sgemm_kernel<false><<<grid, 256, 0, st>>>(g);
-    return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    return launch_pieces(g, (g.N + kBN - 1) / kBN, (g.M + kBM - 1) / kBM, batch, [&](const GemmArgs& p, dim3 grid) {
+        if (nn) sgemm_kernel<true><<<grid, 256, 0, st>>>(p);
+        else sgemm_kernel<false><<<grid, 256, 0, st>>>(p);
+    });
 }
 
 GemmArgs gemm_args(const float* A, int lda, const float* B, int ldb, float* C, int ldc, int M, int N, int K, const float* bias, int act) {
@@ -691,13 +727,13 @@ int gen_launch_stem(const float* img, int S, int n, const GenModelW& w, const Ge
         else GEN_TRY(run_im2col(false, acts[l - 1], (long long)H * H * ch[l], ch[l], 0, ch[l], H, 2, n, ws.col, st));
         if (l < 3) {
             GemmArgs g = gemm_args(ws.col, K, w.stem_w[l], K, acts[l], ch[l + 1], n * Ho * Ho, ch[l + 1], K, w.stem_b[l], ACT_HSWISH);
-            GEN_TRY(run_gemm(g, 1, false, st));
+            GEN_TRY(run_gemm(g, 1, false, w, st));
         } else {
             // last layer: one GEMM per track (batch), rows = tokens, + positional embedding (broadcast residual)
             GemmArgs g = gemm_args(ws.col, K, w.stem_w[l], K, tokens + (size_t)tok_off * C, C, Ho * Ho, C, K, w.stem_b[l], ACT_NONE);
             g.sa1 = (long long)Ho * Ho * K; g.sc1 = (long long)tok_stride_rows * C;
             g.R = (S == kSx) ? w.pos_x : w.pos_z; g.ldr = C;
-            GEN_TRY(run_gemm(g, n, false, st));
+            GEN_TRY(run_gemm(g, n, false, w, st));
         }
         H = Ho;
     }
@@ -740,7 +776,7 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
                 g.sa1 = g.sb1 = (long long)kN * 3 * C; g.sa2 = g.sb2 = hd;
                 g.sc1 = (long long)w.heads * kN * kN; g.sc2 = (long long)kN * kN;
                 g.alpha = 1.f / sqrtf((float)hd);
-                GEN_TRY(run_gemm(g, n * w.heads, false, st));
+                GEN_TRY(run_gemm(g, n * w.heads, false, w, st));
             }
             {
                 const long long srows = (long long)n * w.heads * kN;
@@ -754,8 +790,16 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
                 g.sa1 = (long long)w.heads * kN * kN; g.sa2 = (long long)kN * kN;
                 g.sb1 = (long long)kN * 3 * C; g.sb2 = hd;
                 g.sc1 = (long long)kN * C; g.sc2 = hd;
-                g.Cimg = img_attn; g.img_K = C; g.img_rows1 = kN; g.img_cols2 = hd;
-                GEN_TRY(run_gemm(g, n * w.heads, true, st));
+                if (gemm_tc_ok(g, true) && hd % 8 == 0) {          // the image epilogue writes whole 8-column chunks of one head
+                    g.Cimg = img_attn; g.img_K = C; g.img_rows1 = kN; g.img_cols2 = hd;
+                    GEN_TRY(run_gemm(g, n * w.heads, true, w, st));
+                } else {                                            // head width < 64: fp32 P V, then the image
+                    GEN_TRY(run_gemm(g, n * w.heads, true, w, st));
+                    const long long chunks = (long long)rows * (C / 8);
+                    rows_img_kernel<<<(int)((chunks + 255) / 256 < 148 * 32 ? (chunks + 255) / 256 : 148 * 32), 256, 0, st>>>(ws.attn, img_attn, rows, C);
+                    if (cudaGetLastError() != cudaSuccess) return -1;
+                    ++total;
+                }
             }
             GEN_TRY(lin(img_attn, B.iwproj, C, C, tokens, B.bproj, ACT_NONE, tokens, nullptr));
             GEN_TRY(ln_img(tokens, B.ln2g, B.ln2b));
@@ -765,14 +809,14 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
             continue;
         }
         GEN_TRY(ln(tokens, ws.ln, B.ln1g, B.ln1b));
-        GEN_TRY(run_gemm(gemm_args(ws.ln, C, B.wqkv, C, ws.qkv, 3 * C, rows, 3 * C, C, B.bqkv, ACT_NONE), 1, false, st));
+        GEN_TRY(run_gemm(gemm_args(ws.ln, C, B.wqkv, C, ws.qkv, 3 * C, rows, 3 * C, C, B.bqkv, ACT_NONE), 1, false, w, st));
         {   // scores[b][h] = (q k^T) * hd^-0.5, batch = track x head
             GemmArgs g = gemm_args(ws.qkv, 3 * C, ws.qkv + C, 3 * C, ws.scores, kN, kN, kN, hd, nullptr, ACT_NONE);
             g.nh = w.heads;
             g.sa1 = g.sb1 = (long long)kN * 3 * C; g.sa2 = g.sb2 = hd;
             g.sc1 = (long long)w.heads * kN * kN; g.sc2 = (long long)kN * kN;
             g.alpha = 1.f / sqrtf((float)hd);
-            GEN_TRY(run_gemm(g, n * w.heads, false, st));
+            GEN_TRY(run_gemm(g, n * w.heads, false, w, st));
         }
         {
             const long long srows = (long long)n * w.heads * kN;
@@ -786,19 +830,19 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
             g.sa1 = (long long)w.heads * kN * kN; g.sa2 = (long long)kN * kN;
             g.sb1 = (long long)kN * 3 * C; g.sb2 = hd;
             g.sc1 = (long long)kN * C; g.sc2 = hd;
-            GEN_TRY(run_gemm(g, n * w.heads, true, st));
+            GEN_TRY(run_gemm(g, n * w.heads, true, w, st));
         }
         {   // x = x + proj(attn)
             GemmArgs g = gemm_args(ws.attn, C, B.wproj, C, tokens, C, rows, C, C, B.bproj, ACT_NONE);
             g.R = tokens; g.ldr = C;
-            GEN_TRY(run_gemm(g, 1, false, st));
+            GEN_TRY(run_gemm(g, 1, false, w, st));
         }
         GEN_TRY(ln(tokens, ws.ln, B.ln2g, B.ln2b));
-        GEN_TRY(run_gemm(gemm_args(ws.ln, C, B.wfc1, C, ws.hid, 4 * C, rows, 4 * C, C, B.bfc1, ACT_GELU), 1, false, st));
+        GEN_TRY(run_gemm(gemm_args(ws.ln, C, B.wfc1, C, ws.hid, 4 * C, rows, 4 * C, C, B.bfc1, ACT_GELU), 1, false, w, st));
         {
             GemmArgs g = gemm_args(ws.hid, 4 * C, B.wfc2, 4 * C, tokens, C, rows, C, 4 * C, B.bfc2, ACT_NONE);
             g.R = tokens; g.ldr = C;
-            GEN_TRY(run_gemm(g, 1, false, st));
+            GEN_TRY(run_gemm(g, 1, false, w, st));
         }
         if (taps && cudaMemcpyAsync(taps + (size_t)(b + 1) * tap_stride, tokens, tok_bytes, cudaMemcpyDeviceToDevice, st) != cudaSuccess) return -1;
     }
@@ -817,10 +861,10 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
         const int r2 = run_gemm_img(g, st);
         return r2 < 0 ? r2 : r + r2;
     };
-    if (w.ihead_w1) GEN_TRY(conv_img(ws.ln + (size_t)kNz * C, (long long)kN * C, C, 0, C, w.ihead_w1, w.head_b1, ws.t1, 3 * hc, 3 * hc));
+    if (w.ihead_w1 && (3 * hc) % 16 == 0) GEN_TRY(conv_img(ws.ln + (size_t)kNz * C, (long long)kN * C, C, 0, C, w.ihead_w1, w.head_b1, ws.t1, 3 * hc, 3 * hc));
     else {
         GEN_TRY(run_im2col(false, ws.ln + (size_t)kNz * C, (long long)kN * C, C, 0, C, kFeat, 1, n, ws.col, st));
-        GEN_TRY(run_gemm(gemm_args(ws.col, 9 * C, w.head_w1, 9 * C, ws.t1, 3 * hc, prow, 3 * hc, 9 * C, w.head_b1, ACT_RELU), 1, false, st));
+        GEN_TRY(run_gemm(gemm_args(ws.col, 9 * C, w.head_w1, 9 * C, ws.t1, 3 * hc, prow, 3 * hc, 9 * C, w.head_b1, ACT_RELU), 1, false, w, st));
     }
     float* tbuf[4] = {ws.t1, ws.t2, ws.t3, ws.t4};
     for (int l = 1; l < 4; ++l)
@@ -831,14 +875,14 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
                 continue;
             }
             GEN_TRY(run_im2col(false, tbuf[l - 1], (long long)256 * 3 * ci, 3 * ci, t * ci, ci, kFeat, 1, n, ws.col, st));
-            GEN_TRY(run_gemm(gemm_args(ws.col, 9 * ci, w.head_w[t][l - 1], 9 * ci, tbuf[l] + t * cn, 3 * cn, prow, cn, 9 * ci, w.head_b[t][l - 1], ACT_RELU), 1, false, st));
+            GEN_TRY(run_gemm(gemm_args(ws.col, 9 * ci, w.head_w[t][l - 1], 9 * ci, tbuf[l] + t * cn, 3 * cn, prow, cn, 9 * ci, w.head_b[t][l - 1], ACT_RELU), 1, false, w, st));
         }
     {   // conv5 (1x1): tower t -> its columns of raw5 (ctr 0 | offset 1, 2 | size 3, 4)
         const int c4 = co[4];
         const int col0[3] = {0, 1, 3}, outs[3] = {1, 2, 2};
         for (int t = 0; t < 3; ++t)
             GEN_TRY(run_gemm(gemm_args(ws.t4 + t * c4, 3 * c4, w.head_w5 + (size_t)col0[t] * c4, c4, ws.raw5 + col0[t], 5, prow, outs[t], c4,
-                                       w.head_b5 + col0[t], ACT_NONE), 1, false, st));
+                                       w.head_b5 + col0[t], ACT_NONE), 1, false, w, st));
     }
     gen_decode_kernel<<<n, 256, 0, st>>>(ws.raw5, a, w.hann, ws.ln, C);
     if (cudaGetLastError() != cudaSuccess) return -1;

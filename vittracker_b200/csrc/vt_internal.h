@@ -309,8 +309,9 @@ int launch_cal_bbox(const float* score, const float* size_map, const float* offs
                     cudaStream_t st);
 
 // ---- generic-configuration path (vt_generic.cu): any embed dim / heads / depth / head width of the vit_dist family ----
-// (BASELINE configs[4]: the widest config, C = 768, 12 heads, depth 12, head 256).  fp32 CUDA-core kernels: im2col + tiled
-// GEMM with fused bias / activation / residual epilogues, LayerNorm, softmax, and the shared decode.  Activations are NHWC
+// (BASELINE configs[4]: the widest config, C = 768, 12 heads, depth 12, head 256).  im2col + tiled GEMM (fp32 CUDA cores, or
+// tensor cores with fp16 hi / lo splits unless fp32_only) with fused bias / activation / residual epilogues, LayerNorm, softmax,
+// and the shared decode.  Activations are NHWC
 // (= token-major), weights keep the reference's [out][in] layout (conv: [cout][ky][kx][cin], BN folded).
 constexpr int kGenMaxDepth = 32;
 struct GenBlockW {
@@ -329,6 +330,7 @@ void gen_pack_weight_image(const float* w, int N, int K, uint8_t* img);     // h
 struct GenModelW {
     int C, heads, depth, hc;
     int use_img;                                             // Linear layers of the blocks on the split-image GEMM (C % 128 == 0)
+    int fp32_only;                                           // blocks_impl "simt": every GEMM on the fp32 CUDA-core kernel
     const float* stem_w[4]; const float* stem_b[4];          // [cout][9 cin], [cout]
     GenBlockW blk[kGenMaxDepth];
     const float *norm_g, *norm_b, *pos_z, *pos_x;
