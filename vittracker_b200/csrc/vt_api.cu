@@ -1,6 +1,6 @@
-// C-ABI layer of libvittrack_b200.so: handle, weight ingestion (BN folding + layout packing),
+// C-ABI layer of libvittrack_b200.so: handle, weight ingestion (BN folding into the fp32 layouts; each tensor-core weight blob is packed
+// by the file of the kernel that reads it),
 // workspace, and the entry points declared in include/vittrack_b200.h.
-#include <cuda_fp16.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -153,6 +153,29 @@ struct Packer {
     }
 };
 
+// Tensor lookup of the finalisers: a tensor that was never set yields null and is listed in `missing`
+struct TensorLookup {
+    VtHandle h;
+    std::string missing;
+    const float* operator()(const std::string& n) {
+        auto it = h->tensors.find(n);
+        if (it == h->tensors.end()) { if (missing.size() < 300) missing += n + " "; return nullptr; }
+        return it->second.data.data();
+    }
+};
+
+// The packed weights -> h->d_weights (reallocated when it has grown); returns once the copy is done, as pk is the caller's local
+int upload_weights(VtHandle h, const Packer& pk, cudaStream_t st) {
+    if (h->d_weights && h->weights_floats < pk.buf.size()) { cudaFree(h->d_weights); h->d_weights = nullptr; }
+    if (!h->d_weights) {
+        VT_CUDA(h, cudaMalloc((void**)&h->d_weights, pk.buf.size() * sizeof(float)));
+        h->weights_floats = pk.buf.size();
+    }
+    VT_CUDA(h, cudaMemcpyAsync(h->d_weights, pk.buf.data(), pk.buf.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+    VT_CUDA(h, cudaStreamSynchronize(st));
+    return VT_OK;
+}
+
 void free_all(VtHandle h) {
     for (auto& r : h->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
     for (auto e : h->evpool) cudaEventDestroy(e);
@@ -226,12 +249,7 @@ void fill_hann_and_lut(VtHandle h, float* hann, float* lut) {
 int finalize_generic(VtHandle h, cudaStream_t st) {
     const VtConfig& c = h->cfg;
     const int C = c.embed_dim, hc = c.head_channels, hid = c.mlp_ratio * C;
-    std::string missing;
-    auto T = [&](const std::string& n) -> const float* {
-        auto it = h->tensors.find(n);
-        if (it == h->tensors.end()) { if (missing.size() < 300) missing += n + " "; return nullptr; }
-        return it->second.data.data();
-    };
+    TensorLookup T{h};
     Packer pk;
     auto put = [&](const float* src, size_t n) { const size_t o = pk.alloc(n); if (src) memcpy(&pk.buf[o], src, n * sizeof(float)); return o; };
     const double eps = 1e-5;
@@ -272,7 +290,7 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
         const int wn[4] = {3 * C, C, hid, C}, wk[4] = {C, C, C, hid};
         for (int b = 0; b < c.depth; ++b)
             for (int j = 0; j < 4; ++j) io[b].v[j] = pk.alloc(gen_img_bytes(wn[j], wk[j]) / 4);
-        if (missing.empty())
+        if (T.missing.empty())
             for (int b = 0; b < c.depth; ++b)
                 for (int j = 0; j < 4; ++j)
                     gen_pack_weight_image(&pk.buf[bo[b].v[wi[j]]], wn[j], wk[j], reinterpret_cast<uint8_t*>(&pk.buf[io[b].v[j]]));
@@ -308,7 +326,7 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
             }
         }
     }
-    if (!missing.empty()) return fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", missing.c_str());
+    if (!T.missing.empty()) return fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", T.missing.c_str());
     const size_t o_hann = pk.alloc(256), o_lut = pk.alloc(768);
     fill_hann_and_lut(h, &pk.buf[o_hann], &pk.buf[o_lut]);
     // split images of the folded convolution weights (K = 9 cin must be a whole number of 32-wide panels)
@@ -324,13 +342,7 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
     for (int t = 0; t < 3; ++t)
         for (int l = 0; l < 3; ++l) ihw[t][l] = conv_img(hw[t][l], hch[l + 2], hch[l + 1]);
 
-    if (h->d_weights && h->weights_floats < pk.buf.size()) { cudaFree(h->d_weights); h->d_weights = nullptr; }
-    if (!h->d_weights) {
-        VT_CUDA(h, cudaMalloc((void**)&h->d_weights, pk.buf.size() * sizeof(float)));
-        h->weights_floats = pk.buf.size();
-    }
-    VT_CUDA(h, cudaMemcpyAsync(h->d_weights, pk.buf.data(), pk.buf.size() * sizeof(float), cudaMemcpyHostToDevice, st));
-    VT_CUDA(h, cudaStreamSynchronize(st));
+    if (const int rc = upload_weights(h, pk, st)) return rc;
     const float* base = h->d_weights;
     GenModelW& g = h->gw;
     for (int l = 0; l < 4; ++l) { g.stem_w[l] = base + sw[l]; g.stem_b[l] = base + sb[l]; }
@@ -536,12 +548,7 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     DeviceGuard dg(h->cfg.device);
     VT_CUDA(h, dg.err);
     if (h->generic) return finalize_generic(h, st);
-    std::string missing;
-    auto T = [&](const std::string& n) -> const float* {
-        auto it = h->tensors.find(n);
-        if (it == h->tensors.end()) { if (missing.size() < 300) missing += n + " "; return nullptr; }
-        return it->second.data.data();
-    };
+    TensorLookup T{h};
     Packer pk;
     auto slot = [&](size_t n) { return pk.alloc(n); };
     const double eps = 1e-5;     // BatchNorm2d default eps
@@ -575,26 +582,15 @@ int vt_finalize_weights(VtHandle h, void* stream) {
             stc_b[i] = slot(lnpad[i]);
             uint8_t* hi8 = reinterpret_cast<uint8_t*>(&pk.buf[stc_w[i]]);
             for (int co = 0; co < lcout[i]; ++co) pk.buf[stc_b[i] + co] = pk.buf[stem_b[l] + co];
-            stem_tc_pack_weights(lcin[i], lcch[i], lcout[i], lnpad[i], &pk.buf[stem_w[l]], hi8, hi8 + bytes / 2,
-                                 [](float v, uint16_t* hi, uint16_t* lo) {
-                                     const __half h2 = __float2half_rn(v);
-                                     const __half l2 = __float2half_rn(v - __half2float(h2));
-                                     memcpy(hi, &h2, 2);
-                                     memcpy(lo, &l2, 2);
-                                 });
+            stem_tc_pack_weights(lcin[i], lcch[i], lcout[i], lnpad[i], &pk.buf[stem_w[l]], hi8, hi8 + bytes / 2);
         }
     }
     // ---- stem conv1 for the fused tensor-core front (vt_stem_fused.cu): pixel normalisation folded into the weights / border-variant biases
     const size_t s1_w = slot(kStem1TcWBytes / 4), s1_p = slot(kStem1TcParFloats);
-    stem1_tc_pack(&pk.buf[stem_w[0]], &pk.buf[stem_b[0]], reinterpret_cast<uint8_t*>(&pk.buf[s1_w]), &pk.buf[s1_p],
-                  [](float v, uint16_t* hi, uint16_t* lo) {
-                      const __half h2 = __float2half_rn(v);
-                      const __half l2 = __float2half_rn(v - __half2float(h2));
-                      memcpy(hi, &h2, 2);
-                      memcpy(lo, &l2, 2);
-                  });
+    stem1_tc_pack(&pk.buf[stem_w[0]], &pk.buf[stem_b[0]], reinterpret_cast<uint8_t*>(&pk.buf[s1_w]), &pk.buf[s1_p]);
     // ---- blocks: Linear weights [out][in] -> K-major [in][out]
     struct BOff { size_t ln1g, ln1b, wqkv, bqkv, wproj, bproj, ln2g, ln2b, wfc1, bfc1, wfc2, bfc2; } bo[kDepth];
+    BlockTensors bt[kDepth];
     auto copyv = [&](size_t o, const float* src, size_t n) { if (src) memcpy(&pk.buf[o], src, n * sizeof(float)); };
     auto transp = [&](size_t o, const float* src, int rows_out, int cols_in) {     // src [out][in] -> dst [in][out]
         if (!src) return;
@@ -603,63 +599,29 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     };
     for (int b = 0; b < kDepth; ++b) {
         const std::string p = "blocks." + std::to_string(b) + ".";
-        bo[b].ln1g = slot(kC); copyv(bo[b].ln1g, T(p + "norm1.weight"), kC);
-        bo[b].ln1b = slot(kC); copyv(bo[b].ln1b, T(p + "norm1.bias"), kC);
-        bo[b].wqkv = slot(kC * 3 * kC); transp(bo[b].wqkv, T(p + "attn.qkv.weight"), 3 * kC, kC);
-        bo[b].bqkv = slot(3 * kC); copyv(bo[b].bqkv, T(p + "attn.qkv.bias"), 3 * kC);
-        bo[b].wproj = slot(kC * kC); transp(bo[b].wproj, T(p + "attn.proj.weight"), kC, kC);
-        bo[b].bproj = slot(kC); copyv(bo[b].bproj, T(p + "attn.proj.bias"), kC);
-        bo[b].ln2g = slot(kC); copyv(bo[b].ln2g, T(p + "norm2.weight"), kC);
-        bo[b].ln2b = slot(kC); copyv(bo[b].ln2b, T(p + "norm2.bias"), kC);
-        bo[b].wfc1 = slot(kC * kHid); transp(bo[b].wfc1, T(p + "mlp.fc1.weight"), kHid, kC);
-        bo[b].bfc1 = slot(kHid); copyv(bo[b].bfc1, T(p + "mlp.fc1.bias"), kHid);
-        bo[b].wfc2 = slot(kHid * kC); transp(bo[b].wfc2, T(p + "mlp.fc2.weight"), kC, kHid);
-        bo[b].bfc2 = slot(kC); copyv(bo[b].bfc2, T(p + "mlp.fc2.bias"), kC);
+        BlockTensors& t = bt[b];
+        t = {T(p + "norm1.weight"), T(p + "norm1.bias"), T(p + "attn.qkv.weight"), T(p + "attn.qkv.bias"), T(p + "attn.proj.weight"),
+             T(p + "attn.proj.bias"), T(p + "norm2.weight"), T(p + "norm2.bias"), T(p + "mlp.fc1.weight"), T(p + "mlp.fc1.bias"),
+             T(p + "mlp.fc2.weight"), T(p + "mlp.fc2.bias")};
+        bo[b].ln1g = slot(kC); copyv(bo[b].ln1g, t.ln1_g, kC);
+        bo[b].ln1b = slot(kC); copyv(bo[b].ln1b, t.ln1_b, kC);
+        bo[b].wqkv = slot(kC * 3 * kC); transp(bo[b].wqkv, t.wqkv, 3 * kC, kC);
+        bo[b].bqkv = slot(3 * kC); copyv(bo[b].bqkv, t.bqkv, 3 * kC);
+        bo[b].wproj = slot(kC * kC); transp(bo[b].wproj, t.wproj, kC, kC);
+        bo[b].bproj = slot(kC); copyv(bo[b].bproj, t.bproj, kC);
+        bo[b].ln2g = slot(kC); copyv(bo[b].ln2g, t.ln2_g, kC);
+        bo[b].ln2b = slot(kC); copyv(bo[b].ln2b, t.ln2_b, kC);
+        bo[b].wfc1 = slot(kC * kHid); transp(bo[b].wfc1, t.wfc1, kHid, kC);
+        bo[b].bfc1 = slot(kHid); copyv(bo[b].bfc1, t.bfc1, kHid);
+        bo[b].wfc2 = slot(kHid * kC); transp(bo[b].wfc2, t.wfc2, kC, kHid);
+        bo[b].bfc2 = slot(kC); copyv(bo[b].bfc2, t.bfc2, kC);
     }
-    // ---- tensor-core operands: fp16 hi/lo split, UMMA no-swizzle K-major [k/8][n][8] ------------------
+    // ---- the same blocks for the tensor cores (vt_block_tc.cu), packed only when every tensor looked up so far is present
     size_t tc_wa[kDepth], tc_wb[kDepth], tc_par[kDepth];
-    auto pack_kmajor = [&](uint8_t* dst_hi, uint8_t* dst_lo, const float* W, int N, int K) {   // W: [N][K] (torch Linear weight)
-        for (int n = 0; n < N; ++n)
-            for (int k = 0; k < K; ++k) {
-                const float v = W[(size_t)n * K + k];
-                const __half hi = __float2half_rn(v);
-                const __half lo = __float2half_rn(v - __half2float(hi));
-                const size_t off = ((size_t)(k / 8) * N + n) * 16 + (k % 8) * 2;
-                memcpy(dst_hi + off, &hi, 2);
-                memcpy(dst_lo + off, &lo, 2);
-            }
-    };
     for (int b = 0; b < kDepth; ++b) {
-        const std::string p = "blocks." + std::to_string(b) + ".";
         tc_wa[b] = slot(kTcWaBytes / 4); tc_wb[b] = slot(kTcWbBytes / 4); tc_par[b] = slot(kTcParFloats);
-        const float *wqkv = T(p + "attn.qkv.weight"), *wproj = T(p + "attn.proj.weight"), *w1 = T(p + "mlp.fc1.weight"), *w2 = T(p + "mlp.fc2.weight");
-        if (!(wqkv && wproj && w1 && w2)) continue;
-        uint8_t* wa = reinterpret_cast<uint8_t*>(&pk.buf[tc_wa[b]]);
-        uint8_t* wb = reinterpret_cast<uint8_t*>(&pk.buf[tc_wb[b]]);
-        // attention output projection folded into the value projection: (P V) Wp^T = P (V Wp^T), V Wp^T = LN(x) (Wp Wv)^T + Wp bv
-        // (products accumulated in float64; the block kernel then needs no separate proj GEMM)
-        const float* bqkv = T(p + "attn.qkv.bias");
-        std::vector<float> wf(wqkv, wqkv + 144 * 48), bvp(48, 0.f);
-        for (int o = 0; o < 48; ++o) {
-            for (int i = 0; i < 48; ++i) {
-                double acc = 0.0;
-                for (int j = 0; j < 48; ++j) acc += (double)wproj[o * 48 + j] * (double)wqkv[(96 + j) * 48 + i];
-                wf[(96 + o) * 48 + i] = (float)acc;
-            }
-            double accb = 0.0;
-            for (int j = 0; j < 48 && bqkv; ++j) accb += (double)wproj[o * 48 + j] * (double)bqkv[96 + j];
-            bvp[o] = (float)accb;
-        }
-        pack_kmajor(wa, wa + 13824, wf.data(), 144, 48);
-        pack_kmajor(wb, wb + 18432, w1, 192, 48);
-        pack_kmajor(wb + 36864, wb + 36864 + 18432, w2, 48, 192);
-        float* par = &pk.buf[tc_par[b]];
-        const float* src[8] = {T(p + "norm1.weight"), T(p + "norm1.bias"), T(p + "attn.qkv.bias"), T(p + "attn.proj.bias"),
-                               T(p + "norm2.weight"), T(p + "norm2.bias"), T(p + "mlp.fc1.bias"), T(p + "mlp.fc2.bias")};
-        const int cnt[8] = {48, 48, 144, 48, 48, 48, 192, 48};
-        int o = 0;
-        for (int i = 0; i < 8; ++i) { if (src[i]) memcpy(par + o, src[i], cnt[i] * sizeof(float)); o += cnt[i]; }
-        memcpy(par + 96 + 96, bvp.data(), 48 * sizeof(float));          // bias of the folded value projection
+        if (T.missing.empty())
+            block_tc_pack(bt[b], reinterpret_cast<uint8_t*>(&pk.buf[tc_wa[b]]), reinterpret_cast<uint8_t*>(&pk.buf[tc_wb[b]]), &pk.buf[tc_par[b]]);
     }
     const size_t o_ng = slot(kC), o_nb = slot(kC), o_pz = slot(kNz * kC), o_px = slot(kNx * kC);
     copyv(o_ng, T("norm.weight"), kC); copyv(o_nb, T("norm.bias"), kC);
@@ -685,68 +647,11 @@ int vt_finalize_weights(VtHandle h, void* stream) {
             }
         }
     }
-    // head conv1 / conv2 for the tensor cores (fp16 hi | lo, K-major [k/8][n][8]); see vt_head.cu
-    const size_t o_htc = slot(18 * kHeadTcPieceBytes / 4), o_htc2 = slot(kHeadTcW2Bytes / 4), o_htc3 = slot(kHeadTcW3Bytes / 4);
-    {
-        auto put = [&](uint8_t* hi8, uint8_t* lo8, size_t off, float v) {
-            const __half hi = __float2half_rn(v);
-            const __half lo = __float2half_rn(v - __half2float(hi));
-            memcpy(hi8 + off, &hi, 2);
-            memcpy(lo8 + off, &lo, 2);
-        };
-        uint8_t* base8 = reinterpret_cast<uint8_t*>(&pk.buf[o_htc]);
-        const float* w1 = &pk.buf[hw[0]];                       // folded, [ci][ky*3+kx][96]
-        // conv1: piece p = (h * 3 + ky) * 3 + ks holds one K step (input channels 16 ks .. 16 ks + 15) of vertical tap ky for ALL three
-        // horizontal taps: B[n = kx * 48 + (co - 48 h)][k = ci], [hi | lo] x [chunk 2][n 144][8] - one N = 144 MMA feeds the three
-        // per-kx accumulators (adjacent TMEM columns) from a single read of the A operand
-        for (int h2 = 0; h2 < 2; ++h2)
-            for (int ky = 0; ky < 3; ++ky)
-                for (int ks = 0; ks < 3; ++ks) {
-                    uint8_t* hi8 = base8 + (size_t)((h2 * 3 + ky) * 3 + ks) * kHeadTcPieceBytes;
-                    uint8_t* lo8 = hi8 + kHeadTcPieceBytes / 2;
-                    for (int kx = 0; kx < 3; ++kx)
-                        for (int n = 0; n < 48; ++n)
-                            for (int e = 0; e < 16; ++e) {
-                                const int ci = 16 * ks + e;
-                                put(hi8, lo8, ((size_t)(e / 8) * 144 + kx * 48 + n) * 16 + (e % 8) * 2, w1[((size_t)ci * 9 + ky * 3 + kx) * 96 + h2 * 48 + n]);
-                            }
-                }
-        uint8_t* base2 = reinterpret_cast<uint8_t*>(&pk.buf[o_htc2]);
-        const float* w2 = &pk.buf[hw[1]];                       // folded, [ci][ky*3+kx][tower][16]
-        for (int t = 0; t < 3; ++t) {                           // blob (tower): B[n = kx * 16 + co][k = ky * 32 + ci], [hi | lo] x [k/8 12][n 48][8]
-            uint8_t* hi8 = base2 + (size_t)t * 18432;
-            uint8_t* lo8 = hi8 + 9216;
-            for (int kx = 0; kx < 3; ++kx)
-                for (int n = 0; n < 16; ++n)
-                    for (int ky = 0; ky < 3; ++ky)
-                        for (int ci = 0; ci < 32; ++ci) {
-                            const int k = ky * 32 + ci;
-                            put(hi8, lo8, ((size_t)(k / 8) * 48 + kx * 16 + n) * 16 + (k % 8) * 2, w2[(((size_t)ci * 9 + ky * 3 + kx) * 3 + t) * 16 + n]);
-                        }
-        }
-    }
-    {
-        auto put = [&](uint8_t* hi8, uint8_t* lo8, size_t off, float v) {
-            const __half hi = __float2half_rn(v);
-            const __half lo = __float2half_rn(v - __half2float(hi));
-            memcpy(hi8 + off, &hi, 2);
-            memcpy(lo8 + off, &lo, 2);
-        };
-        uint8_t* base3 = reinterpret_cast<uint8_t*>(&pk.buf[o_htc3]);
-        memset(base3, 0, kHeadTcW3Bytes);                       // output columns 24..31 are padding
-        const float* w3 = &pk.buf[hw[2]];                       // folded, [ci][ky*3+kx][tower][8]
-        for (int t = 0; t < 3; ++t) {                           // blob (tower): B[n = kx * 8 + co][k = ky * 16 + ci], [hi | lo] x [k/8 6][n 32][8]
-            uint8_t* hi8 = base3 + (size_t)t * 6144;
-            uint8_t* lo8 = hi8 + 3072;
-            for (int kx = 0; kx < 3; ++kx)
-                for (int n = 0; n < 8; ++n)
-                    for (int ky = 0; ky < 3; ++ky)
-                        for (int ci = 0; ci < 16; ++ci) {
-                            const int k = ky * 16 + ci;
-                            put(hi8, lo8, ((size_t)(k / 8) * 32 + kx * 8 + n) * 16 + (k % 8) * 2, w3[(((size_t)ci * 9 + ky * 3 + kx) * 3 + t) * 8 + n]);
-                        }
-        }
-    }
+    // head conv1 - conv3 for the tensor cores (vt_head.cu)
+    size_t o_htc[3];
+    for (int i = 0; i < 3; ++i) o_htc[i] = slot(head_tc_weight_bytes(i) / 4);
+    head_tc_pack(&pk.buf[hw[0]], &pk.buf[hw[1]], &pk.buf[hw[2]], reinterpret_cast<uint8_t*>(&pk.buf[o_htc[0]]),
+                 reinterpret_cast<uint8_t*>(&pk.buf[o_htc[1]]), reinterpret_cast<uint8_t*>(&pk.buf[o_htc[2]]));
     hw[4] = slot(3 * 4 * 2); hb[4] = slot(3 * 2);
     for (int t = 0; t < 3; ++t) {
         const std::string p = std::string("box_head.conv5_") + kTowers[t] + ".";
@@ -758,19 +663,13 @@ int vt_finalize_weights(VtHandle h, void* stream) {
             for (int c = 0; c < 4; ++c) pk.buf[hw[4] + (t * 4 + c) * 2 + o] = w[o * 4 + c];
         }
     }
-    if (!missing.empty()) return fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", missing.c_str());
+    if (!T.missing.empty()) return fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", T.missing.c_str());
 
     // ---- Hann window (hann.py:6-16) and normalisation table (data_utils.py:8-14) -----------------
     const size_t o_hann = slot(256), o_lut = slot(768);
     fill_hann_and_lut(h, &pk.buf[o_hann], &pk.buf[o_lut]);
 
-    if (h->d_weights && h->weights_floats < pk.buf.size()) { cudaFree(h->d_weights); h->d_weights = nullptr; }
-    if (!h->d_weights) {
-        VT_CUDA(h, cudaMalloc((void**)&h->d_weights, pk.buf.size() * sizeof(float)));
-        h->weights_floats = pk.buf.size();
-    }
-    VT_CUDA(h, cudaMemcpyAsync(h->d_weights, pk.buf.data(), pk.buf.size() * sizeof(float), cudaMemcpyHostToDevice, st));
-    VT_CUDA(h, cudaStreamSynchronize(st));          // pk.buf is a local
+    if (const int rc = upload_weights(h, pk, st)) return rc;
     const float* base = h->d_weights;
     ModelW& m = h->mw;
     for (int l = 0; l < 4; ++l) { m.stem[l].w = base + stem_w[l]; m.stem[l].b = base + stem_b[l]; }
@@ -779,8 +678,6 @@ int vt_finalize_weights(VtHandle h, void* stream) {
         B.ln1_g = base + bo[b].ln1g; B.ln1_b = base + bo[b].ln1b; B.wqkv = base + bo[b].wqkv; B.bqkv = base + bo[b].bqkv;
         B.wproj = base + bo[b].wproj; B.bproj = base + bo[b].bproj; B.ln2_g = base + bo[b].ln2g; B.ln2_b = base + bo[b].ln2b;
         B.wfc1 = base + bo[b].wfc1; B.bfc1 = base + bo[b].bfc1; B.wfc2 = base + bo[b].wfc2; B.bfc2 = base + bo[b].bfc2;
-    }
-    for (int b = 0; b < kDepth; ++b) {
         m.tc[b].wa = reinterpret_cast<const uint8_t*>(base + tc_wa[b]);
         m.tc[b].wb = reinterpret_cast<const uint8_t*>(base + tc_wb[b]);
         m.tc[b].par = base + tc_par[b];
@@ -789,9 +686,9 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     m.head.w1 = base + hw[0]; m.head.b1 = base + hb[0]; m.head.w2 = base + hw[1]; m.head.b2 = base + hb[1];
     m.head.w3 = base + hw[2]; m.head.b3 = base + hb[2]; m.head.w4 = base + hw[3]; m.head.b4 = base + hb[3];
     m.head.w5 = base + hw[4]; m.head.b5 = base + hb[4];
-    m.head_tc_w1 = reinterpret_cast<const uint8_t*>(base + o_htc);
-    m.head_tc_w2 = reinterpret_cast<const uint8_t*>(base + o_htc2);
-    m.head_tc_w3 = reinterpret_cast<const uint8_t*>(base + o_htc3);
+    m.head_tc_w1 = reinterpret_cast<const uint8_t*>(base + o_htc[0]);
+    m.head_tc_w2 = reinterpret_cast<const uint8_t*>(base + o_htc[1]);
+    m.head_tc_w3 = reinterpret_cast<const uint8_t*>(base + o_htc[2]);
     for (int i = 0; i < 3; ++i) { m.stem_tc_w[i] = reinterpret_cast<const uint8_t*>(base + stc_w[i]); m.stem_tc_b[i] = base + stc_b[i]; }
     m.stem1_tc_w = reinterpret_cast<const uint8_t*>(base + s1_w); m.stem1_tc_par = base + s1_p;
     m.hann = base + o_hann; m.lut = base + o_lut;

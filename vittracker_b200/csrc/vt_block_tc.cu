@@ -20,6 +20,8 @@
 //
 // Algorithmic work per track: 112.07 MFLOP (SURVEY 8d); issued MMA work is 3x that (split) x 1.2
 // (padding of the third tile).
+#include <vector>
+
 #include "vt_internal.h"
 #include "vt_tc.cuh"
 
@@ -74,25 +76,34 @@ constexpr uint32_t kColOpa = 368;      // [368,512): three 48-column A-operand s
 constexpr uint32_t kColHA = 0, kColHB = 192;       // 192 columns each
 constexpr uint32_t kColYA = 384, kColYB = 432;     // 48 columns each
 
+// ---- one block's weight blobs (block_tc_pack), byte offsets: fp16 hi | lo halves, UMMA no-swizzle K-major [k/8][n][8] ------------
+//   wa: [Wq; Wk; Wproj Wv] (N 144, K 48) hi | lo           wb: W1 (N 192, K 48) hi | lo, then W2 (N 48, K 192) hi | lo
+constexpr int kWaLo = 3 * kC * kC * 2;                    // 13824
+constexpr int kWbW1Lo = kHid * kC * 2;                    // 18432
+constexpr int kWbW2Hi = 2 * kWbW1Lo;                      // 36864 = W1 hi | lo
+constexpr int kWbW2Lo = kWbW2Hi + kC * kHid * 2;          // 55296
+static_assert(kTcWaBytes == 2 * kWaLo && kTcWbBytes == kWbW2Lo + kC * kHid * 2, "block weight blobs");
+
 // ---- shared memory (bytes) -------------------------------------------------------------------------
 constexpr int kSmWa = 0;                                  // Wqkv hi|lo, Wproj hi|lo (bulk copied per block)
 constexpr int kSmX = kSmWa + kTcWaBytes;                  // attention: K hi|lo, V hi|lo ; MLP: W1 hi|lo, W2 hi|lo
 constexpr int kKBytes = kN * kC * 2;                      // 30720 per precision
 constexpr int kSmKhi = kSmX, kSmKlo = kSmX + kKBytes, kSmVhi = kSmX + 2 * kKBytes, kSmVlo = kSmX + 3 * kKBytes;
-constexpr int kSmW2hi = kSmX, kSmW2lo = kSmX + 18432;       // W2 hi|lo overlays K (streamed in once attention is over)
+constexpr int kSmW2hi = kSmX, kSmW2lo = kSmX + (kWbW2Lo - kWbW2Hi);   // W2 hi|lo overlays K (streamed in once attention is over)
 constexpr int kSmW1 = kSmX + 4 * kKBytes;                 // W1 hi|lo in its own region: prefetched during attention
-constexpr int kSmW1hi = kSmW1, kSmW1lo = kSmW1 + 18432;
-constexpr int kSmPar = kSmW1 + 36864;                     // fp32 parameters of all blocks
+constexpr int kSmW1hi = kSmW1, kSmW1lo = kSmW1 + kWbW1Lo;
+constexpr int kSmPar = kSmW1 + kWbW2Hi;                   // fp32 parameters of all blocks
 constexpr int kSmRed = kSmPar + kDepth * kTcParFloats * 4;   // 6 arrays x kNS column groups x 128 rows fp32
 constexpr int kSmBar = kSmRed + 6 * kNS * 128 * 4;        // mbarriers
 constexpr int kSmTmem = kSmBar + 20 * 8;
 static_assert(kSmTmem + 16 <= 227 * 1024, "shared memory");
 constexpr int kTcSmemBytes = kSmTmem + 16;
-static_assert(kTcWbBytes == 2 * 36864 && 36864 <= 4 * kKBytes, "W2 overlays the K/V region");
+static_assert(kTcWbBytes - kWbW2Hi <= 4 * kKBytes, "W2 overlays the K/V region");
 static_assert(kSmBar % 8 == 0 && kSmX % 128 == 0, "alignment");
 
 // parameter offsets inside one block's fp32 parameter vector
 constexpr int kPLn1g = 0, kPLn1b = 48, kPBqkv = 96, kPBproj = 240, kPLn2g = 288, kPLn2b = 336, kPBfc1 = 384, kPBfc2 = 576;
+static_assert(kPBfc2 + kC == kTcParFloats, "parameter vector");
 
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory"); }
 
@@ -296,8 +307,8 @@ blocks_tc_kernel(const float* __restrict__ tok_z, int z_stride_rows, const float
             const uint32_t id192 = instr_desc_f16(128, 192, false);
             auto wait_go = [&]() { TC_TRACE(0); mbar_wait(mb_go, go_ph); go_ph ^= 1; tc_fence_after(); TC_TRACE(0); };
             auto load_wa = [&](int blk) { bulk_g2s_elect(smem + kSmWa, w.tc[blk].wa, kTcWaBytes, mb_wa); };
-            auto load_w1 = [&](int blk) { bulk_g2s_elect(smem + kSmW1, w.tc[blk].wb, 36864, mb_w1); };
-            auto load_w2 = [&](int blk) { bulk_g2s_elect(smem + kSmX, w.tc[blk].wb + 36864, 36864, mb_wb); };
+            auto load_w1 = [&](int blk) { bulk_g2s_elect(smem + kSmW1, w.tc[blk].wb, kWbW2Hi, mb_w1); };
+            auto load_w2 = [&](int blk) { bulk_g2s_elect(smem + kSmX, w.tc[blk].wb + kWbW2Hi, kTcWbBytes - kWbW2Hi, mb_wb); };
             // D[d_col] = A(opa slot t, K = 48) x B^T, B K-major [k/8][N][8] at byte offsets b_hi / b_lo
             auto gemm_k48 = [&](int t, uint32_t d_col, uint32_t b_hi, uint32_t b_lo, int N, uint32_t idesc) {
                 const uint32_t a = tbase + kColOpa + 48 * t;
@@ -310,7 +321,7 @@ blocks_tc_kernel(const float* __restrict__ tok_z, int z_stride_rows, const float
                     mma_ts_elect(tbase + d_col, a + 8 * ks, bl, idesc, true);             // hi * lo
                 }
             };
-            auto qkv = [&](int t, uint32_t d_col) { gemm_k48(t, d_col, kSmWa, kSmWa + 13824, 144, id144); };
+            auto qkv = [&](int t, uint32_t d_col) { gemm_k48(t, d_col, kSmWa, kSmWa + kWaLo, 144, id144); };
             auto fc1 = [&](int t, uint32_t h_col) { gemm_k48(t, h_col, kSmW1hi, kSmW1lo, 192, id192); };
             // S = q k^T over 320 keys as two N = 160 halves; K operand K-major [k/8][320][8]
             auto scores_half = [&](int t, int half) {
@@ -695,6 +706,40 @@ int launch_blocks_tc(const float* tok_z, int z_stride_rows, const float* tok_x, 
     if (scores_terms == 1) blocks_tc_kernel<1><<<grid, kTcThreads, kTcSmemBytes, st>>>(tok_z, z_stride_rows, tok_x, x_stride_rows, out, n, w, taps, tap_stride);
     else blocks_tc_kernel<3><<<grid, kTcThreads, kTcSmemBytes, st>>>(tok_z, z_stride_rows, tok_x, x_stride_rows, out, n, w, taps, tap_stride);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
+}
+
+// Host side: one block's checkpoint tensors -> its blobs wa, wb and parameter vector par (layouts above).
+// The attention output projection is folded into the value projection: (P V) Wp^T = P (V Wp^T), V Wp^T = LN(x) (Wp Wv)^T + Wp bv
+// (products accumulated in float64; the kernel then needs no separate proj GEMM).
+void block_tc_pack(const BlockTensors& t, uint8_t* wa, uint8_t* wb, float* par) {
+    auto pack_kmajor = [](uint8_t* dst_hi, uint8_t* dst_lo, const float* W, int N, int K) {     // W: [N][K] (torch Linear weight)
+        for (int n = 0; n < N; ++n)
+            for (int k = 0; k < K; ++k) put_kmajor_f16(dst_hi, dst_lo, N, n, k, W[(size_t)n * K + k]);
+    };
+    std::vector<float> wf(t.wqkv, t.wqkv + 3 * kC * kC), bvp(kC);
+    for (int o = 0; o < kC; ++o) {
+        for (int i = 0; i < kC; ++i) {
+            double acc = 0.0;
+            for (int j = 0; j < kC; ++j) acc += (double)t.wproj[o * kC + j] * (double)t.wqkv[(2 * kC + j) * kC + i];
+            wf[(2 * kC + o) * kC + i] = (float)acc;
+        }
+        double accb = 0.0;
+        for (int j = 0; j < kC; ++j) accb += (double)t.wproj[o * kC + j] * (double)t.bqkv[2 * kC + j];
+        bvp[o] = (float)accb;
+    }
+    pack_kmajor(wa, wa + kWaLo, wf.data(), 3 * kC, kC);
+    pack_kmajor(wb, wb + kWbW1Lo, t.wfc1, kHid, kC);
+    pack_kmajor(wb + kWbW2Hi, wb + kWbW2Lo, t.wfc2, kC, kHid);
+    auto put = [&](int o, const float* src, int n) { memcpy(par + o, src, n * sizeof(float)); };
+    put(kPLn1g, t.ln1_g, kC);
+    put(kPLn1b, t.ln1_b, kC);
+    put(kPBqkv, t.bqkv, 2 * kC);                     // bq, bk
+    put(kPBqkv + 2 * kC, bvp.data(), kC);            // bias of the folded value projection
+    put(kPBproj, t.bproj, kC);
+    put(kPLn2g, t.ln2_g, kC);
+    put(kPLn2b, t.ln2_b, kC);
+    put(kPBfc1, t.bfc1, kHid);
+    put(kPBfc2, t.bfc2, kC);
 }
 
 }  // namespace vt

@@ -492,9 +492,8 @@ void gen_pack_weight_image(const float* w, int N, int K, uint8_t* img) {
     auto work = [&](int n_lo, int n_hi) {
         for (int n = n_lo; n < n_hi; ++n)
             for (int k = 0; k < K; ++k) {
-                const float v = w[(size_t)n * K + k];
-                const __half hi = __float2half_rn(v);
-                const __half lo = __float2half_rn(v - __half2float(hi));
+                uint16_t hi, lo;
+                tc::split_f16(w[(size_t)n * K + k], &hi, &lo);
                 const size_t off = gen_img_offset(n, k / 8, K, 0) + (k % 8) * 2;
                 memcpy(img + off, &hi, 2);
                 memcpy(img + off + 8192, &lo, 2);

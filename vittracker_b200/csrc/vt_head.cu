@@ -76,8 +76,12 @@ constexpr size_t kHeadTcSmemBytes = kT_Bar + (2 * kT_RingSlots + 9) * 8;
 constexpr int kT_TokBytes = 256 * kC * 4;               // a track's search tokens, staged in R1 (dead until conv1's first epilogue) for the LayerNorm
 static_assert(kT_TokBytes <= 2 * kT_R1Half, "token staging");
 constexpr int kT_Issue1 = 2, kT_Issue2 = 6;             // warps issuing conv1's (one per M tile) and conv2's (one per tower x M tile) MMAs
-constexpr int kT_W2Bytes = 3 * 2 * 12 * 48 * 16;        // conv2 weights: (tower) x [hi | lo] x K-major [12 chunks][n = kx*16 + co][8] = 55296
-static_assert(kT_W2Bytes <= kT_R0Bytes && kT_Out4 + 12 * kPlane * 4 <= kT_R0 + kT_R0Bytes && kT_W3 + kHeadTcW3Bytes <= kT_R1 && kT_W3 % 128 == 0, "head tc smem plan");
+// conv2 / conv3 weights: one blob per tower, hi | lo halves, each K-major [k/8][n][8] (head_tc_pack)
+constexpr int kT_W2Half = 12 * 48 * 16;                  // conv2: [12 chunks][n = kx*16 + co][8], k = ky*32 + ci
+constexpr int kT_W2Tower = 2 * kT_W2Half, kT_W2Bytes = 3 * kT_W2Tower;
+constexpr int kT_W3Half = 6 * 32 * 16;                   // conv3: [6 chunks][n = kx*8 + co, 32 (24 used)][8], k = ky*16 + ci
+constexpr int kT_W3Tower = 2 * kT_W3Half, kT_W3Bytes = 3 * kT_W3Tower;
+static_assert(kT_W2Bytes <= kT_R0Bytes && kT_Out4 + 12 * kPlane * 4 <= kT_R0 + kT_R0Bytes && kT_W3 + kT_W3Bytes <= kT_R1 && kT_W3 % 128 == 0, "head tc smem plan");
 static_assert(kHeadTcSmemBytes <= 227 * 1024 && kT_Bar % 8 == 0 && kT_R1 % 128 == 0, "head smem (tc)");
 
 __device__ __forceinline__ void cp_async16(float* dst_smem, const float* src_gmem) {
@@ -474,10 +478,10 @@ __global__ void __launch_bounds__(kHeadThreads, 1) head_tc_kernel(HeadArgs a, Mo
             tc::tc_fence_after();
             HEAD_TRACE(12 + 3 * h);
             if (h == 1 && warp == 0) {           // conv1's operand and weight ring are dead: conv2's and conv3's weights stream into their place
-                tc::bulk_g2s_elect(sm8 + kT_R0, w.head_tc_w2, kT_W2Bytes / 3, bar_w2);
-                tc::bulk_g2s_elect(sm8 + kT_R0 + kT_W2Bytes / 3, w.head_tc_w2 + kT_W2Bytes / 3, kT_W2Bytes / 3, bar_w2t);
-                tc::bulk_g2s_elect(sm8 + kT_R0 + 2 * (kT_W2Bytes / 3), w.head_tc_w2 + 2 * (kT_W2Bytes / 3), kT_W2Bytes / 3, bar_w2t + 1);
-                tc::bulk_g2s_elect(sm8 + kT_W3, w.head_tc_w3, kHeadTcW3Bytes, bar_w3);
+                tc::bulk_g2s_elect(sm8 + kT_R0, w.head_tc_w2, kT_W2Tower, bar_w2);
+                tc::bulk_g2s_elect(sm8 + kT_R0 + kT_W2Tower, w.head_tc_w2 + kT_W2Tower, kT_W2Tower, bar_w2t);
+                tc::bulk_g2s_elect(sm8 + kT_R0 + 2 * kT_W2Tower, w.head_tc_w2 + 2 * kT_W2Tower, kT_W2Tower, bar_w2t + 1);
+                tc::bulk_g2s_elect(sm8 + kT_W3, w.head_tc_w3, kT_W3Bytes, bar_w3);
             }
             // epilogue: combine the three horizontal taps, bias, ReLU -> conv2's operand image (channels 48 h ..)
             {
@@ -527,7 +531,7 @@ __global__ void __launch_bounds__(kHeadThreads, 1) head_tc_kernel(HeadArgs a, Mo
         tc::mbar_wait(tw == 0 ? bar_w2 : bar_w2t + (tw - 1), 0);
         tc::tc_fence_after();
         const uint32_t d = tbase + (tw * 2 + tl) * 48;
-        const uint32_t wb = sbase + kT_R0 + tw * 18432;
+        const uint32_t wb = sbase + kT_R0 + tw * kT_W2Tower;
 #pragma unroll
         for (int ky = 0; ky < 3; ++ky)
 #pragma unroll
@@ -536,7 +540,7 @@ __global__ void __launch_bounds__(kHeadThreads, 1) head_tc_kernel(HeadArgs a, Mo
                 const uint64_t ah = tc::smem_desc(sbase + aoff, kTcAChunk, 128);
                 const uint64_t al = tc::smem_desc(sbase + aoff + kT_R1Half, kTcAChunk, 128);
                 const uint64_t bh = tc::smem_desc(wb + (ky * 4 + 2 * kp) * 768, 768, 128);
-                const uint64_t bl = tc::smem_desc(wb + 9216 + (ky * 4 + 2 * kp) * 768, 768, 128);
+                const uint64_t bl = tc::smem_desc(wb + kT_W2Half + (ky * 4 + 2 * kp) * 768, 768, 128);
                 tc::mma_ss_elect(d, ah, bh, id48, (ky | kp) != 0);
                 tc::mma_ss_elect(d, al, bh, id48, 1);
                 tc::mma_ss_elect(d, ah, bl, id48, 1);
@@ -596,14 +600,14 @@ __global__ void __launch_bounds__(kHeadThreads, 1) head_tc_kernel(HeadArgs a, Mo
         tc::mbar_wait(bar_w3, 0);
         tc::tc_fence_after();
         const uint32_t d = tbase + 288 + (tw * 2 + tl) * 32;
-        const uint32_t wb = sbase + kT_W3 + tw * 6144;
+        const uint32_t wb = sbase + kT_W3 + tw * kT_W3Tower;
 #pragma unroll
         for (int ky = 0; ky < 3; ++ky) {
             const uint32_t aoff = kT_R1 + (2 * tw) * kTcAChunk + (8 * tl + ky) * 256;
             const uint64_t ah = tc::smem_desc(sbase + aoff, kTcAChunk, 128);
             const uint64_t al = tc::smem_desc(sbase + aoff + kT_R1Half, kTcAChunk, 128);
             const uint64_t bh = tc::smem_desc(wb + (ky * 2) * 512, 512, 128);
-            const uint64_t bl = tc::smem_desc(wb + 3072 + (ky * 2) * 512, 512, 128);
+            const uint64_t bl = tc::smem_desc(wb + kT_W3Half + (ky * 2) * 512, 512, 128);
             tc::mma_ss_elect(d, ah, bh, id32, ky != 0);
             tc::mma_ss_elect(d, al, bh, id32, 1);
             tc::mma_ss_elect(d, ah, bl, id32, 1);
@@ -670,6 +674,39 @@ int launch_head(const HeadArgs& a, const ModelW& w, cudaStream_t st) {
     }
     else head_kernel<<<a.n, kHeadThreads, kHeadSmemBytes, st>>>(a, w);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
+}
+
+size_t head_tc_weight_bytes(int layer) { return layer == 0 ? (size_t)18 * kT_PieceBytes : layer == 1 ? kT_W2Bytes : kT_W3Bytes; }
+
+// Host side: the folded fp32 weights (HeadW: w1 [ci][ky*3+kx][96], w2 [ci][ky*3+kx][tower][16], w3 [ci][ky*3+kx][tower][8]) -> the
+// fp16 hi | lo blobs head_tc_kernel reads.
+void head_tc_pack(const float* w1, const float* w2, const float* w3, uint8_t* blob1, uint8_t* blob2, uint8_t* blob3) {
+    // conv1: piece p = (h * 3 + ky) * 3 + ks holds one K step (input channels 16 ks .. 16 ks + 15) of vertical tap ky for ALL three
+    // horizontal taps: B[n = kx * 48 + (co - 48 h)][k = ci], [hi | lo] x [chunk 2][n 144][8] - one N = 144 MMA feeds the three
+    // per-kx accumulators (adjacent TMEM columns) from a single read of the A operand
+    for (int h = 0; h < 2; ++h)
+        for (int ky = 0; ky < 3; ++ky)
+            for (int ks = 0; ks < 3; ++ks) {
+                uint8_t* piece = blob1 + (size_t)((h * 3 + ky) * 3 + ks) * kT_PieceBytes;
+                for (int kx = 0; kx < 3; ++kx)
+                    for (int n = 0; n < 48; ++n)
+                        for (int e = 0; e < 16; ++e)
+                            tc::put_kmajor_f16(piece, piece + kT_PieceBytes / 2, 144, kx * 48 + n, e,
+                                               w1[((size_t)(16 * ks + e) * 9 + ky * 3 + kx) * 96 + h * 48 + n]);
+            }
+    // conv2 / conv3, one blob per tower t: B[n = kx * co_n + co][k = ky * ci_n + ci], N = npad
+    auto towers = [](uint8_t* blob, int tower_bytes, int ci_n, int co_n, int npad, const float* wf) {
+        for (int t = 0; t < 3; ++t)
+            for (int kx = 0; kx < 3; ++kx)
+                for (int n = 0; n < co_n; ++n)
+                    for (int ky = 0; ky < 3; ++ky)
+                        for (int ci = 0; ci < ci_n; ++ci)
+                            tc::put_kmajor_f16(blob + t * tower_bytes, blob + t * tower_bytes + tower_bytes / 2, npad, kx * co_n + n, ky * ci_n + ci,
+                                               wf[(((size_t)ci * 9 + ky * 3 + kx) * 3 + t) * co_n + n]);
+    };
+    towers(blob2, kT_W2Tower, 32, 16, 48, w2);
+    memset(blob3, 0, kT_W3Bytes);                        // conv3's output columns 24..31 are padding
+    towers(blob3, kT_W3Tower, 16, 8, 32, w3);
 }
 
 // box_head.cal_bbox(score, size_map, offset_map) on caller-provided maps (head.py:142-160).

@@ -119,13 +119,10 @@ struct HeadW {               // CENTER head, BN folded, towers ordered ctr, offs
     const float *w5, *b5;    // [3][4][2] (ctr uses column 0), [3][2]
 };
 
-// Tensor-core block kernel operands (vt_block_tc.cu): fp16 hi/lo split weights in the UMMA
+// Tensor-core block kernel operands (vt_block_tc.cu: block_tc_pack): fp16 hi/lo split weights in the UMMA
 // no-swizzle K-major layout [k/8][n][8], one bulk-copyable blob per phase, plus fp32 parameters.
 constexpr int kTcWaBytes = 2 * (144 * 48 * 2);                         // [Wq; Wk; Wproj Wv] hi|lo = 27648 (the output projection is folded into V)
 constexpr int kTcWbBytes = 2 * (192 * 48 * 2) + 2 * (48 * 192 * 2);     // W1 hi|lo, W2 hi|lo     = 73728
-constexpr int kHeadTcPieceBytes = 2 * (48 * 48 * 2);       // one (half, ky, K step) piece of head conv1: hi | lo, N = 144 (kx, co), K = 16 -> 9216
-constexpr int kHeadTcW3Bytes = 3 * 2 * (48 * 32 * 2);      // head conv3: 3 tower blobs of hi | lo, N = 32 (kx, co; 24 used), K = 48 -> 18432
-constexpr int kHeadTcW2Bytes = 9 * 2 * (96 * 16 * 2);      // head conv2: 3 tower blobs of hi | lo, N = 48 (kx, co), K = 96 -> 55296
 constexpr int kStem1TcWBytes = 4 * 512;     // fused stem, conv1 on tcgen05 (vt_stem_fused.cu): [variant 2][K step 2] x (2 chunks x 16 n x 16 B)
 constexpr int kStem1TcParFloats = 40;       // bias[4 border variants][8], 2^-s at [32]
 constexpr int kTcParFloats = 624;   // ln1_g 48 | ln1_b 48 | bq 48 | bk 48 | Wproj bv 48 | bproj 48 | ln2_g 48 | ln2_b 48 | bfc1 192 | bfc2 48
@@ -134,6 +131,9 @@ struct BlockTcW {
     const uint8_t* wb;     // kTcWbBytes
     const float* par;      // kTcParFloats
 };
+// One ViT block's tensors as the checkpoint holds them (host memory; Linear weights [out][in])
+struct BlockTensors { const float *ln1_g, *ln1_b, *wqkv, *bqkv, *wproj, *bproj, *ln2_g, *ln2_b, *wfc1, *bfc1, *wfc2, *bfc2; };
+void block_tc_pack(const BlockTensors& t, uint8_t* wa, uint8_t* wb, float* par);
 
 struct ModelW {
     StemLayerW stem[4];
@@ -267,10 +267,9 @@ int launch_stem34_tc(const uint8_t* planes3, int n, const ModelW& w, uint8_t* pl
 // Fused front of the search-branch stem (vt_stem_fused.cu): tap tables + crop gather -> conv1 -> conv2 on tcgen05 -> planes3
 int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes, double factor,
                              int n, const ModelW& w, int32_t* out_status, void* tap_tables, uint8_t* planes3, cudaStream_t st);
-void stem1_tc_pack(const float* wf, const float* bf, uint8_t* blob, float* par, void (*split)(float, uint16_t*, uint16_t*));
+void stem1_tc_pack(const float* wf, const float* bf, uint8_t* blob, float* par);
 size_t stem_tc_weight_bytes(int layer);
-void stem_tc_pack_weights(int cin, int cch, int cout, int npad, const float* wf, uint8_t* hi8, uint8_t* lo8,
-                          void (*split)(float, uint16_t*, uint16_t*));
+void stem_tc_pack_weights(int cin, int cch, int cout, int npad, const float* wf, uint8_t* hi8, uint8_t* lo8);
 
 // Crop + stem straight from raw uint8 frames (the first conv layer gathers its tile from the frame).
 int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
@@ -304,6 +303,10 @@ struct HeadArgs {
     int use_tc;               // first (48 -> 96) convolution on the tcgen05 tensor cores
 };
 int launch_head(const HeadArgs& a, const ModelW& w, cudaStream_t st);
+// Weights of the tensor-core head (vt_head.cu): blob sizes (0: conv1, 1: conv2, 2: conv3) and the host packer that fills them from
+// the folded HeadW layouts w1, w2, w3.
+size_t head_tc_weight_bytes(int layer);
+void head_tc_pack(const float* w1, const float* w2, const float* w3, uint8_t* blob1, uint8_t* blob2, uint8_t* blob3);
 
 int launch_cal_bbox(const float* score, const float* size_map, const float* offset_map, int n, float* boxes,
                     cudaStream_t st);

@@ -508,7 +508,7 @@ int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets
 //   (K step 0: ky = 0 | ky = 1; K step 1: ky = 2 | zeros); k = 3 * pixel + ci over the chunk's two pixels.
 //   variant 0: pixel 0 -> kx = 1, pixel 1 -> kx = 2;  variant 1 (A operand one chunk earlier): pixel 1 -> kx = 0.
 //   par: bias[4][8] (variant = 2 * (y == 0) + (x == 0): taps in the convolution's zero padding left out), par[32] = 2^-s.
-void stem1_tc_pack(const float* wf, const float* bf, uint8_t* blob, float* par, void (*split)(float, uint16_t*, uint16_t*)) {
+void stem1_tc_pack(const float* wf, const float* bf, uint8_t* blob, float* par) {
     const double mean[3] = {0.485, 0.456, 0.406}, stdv[3] = {0.229, 0.224, 0.225};
     auto W = [&](int ci, int ky, int kx, int co) { return (double)wf[(((size_t)ci * 3 + ky) * 3 + kx) * 6 + co]; };
     double maxabs = 0.0;
@@ -535,7 +535,7 @@ void stem1_tc_pack(const float* wf, const float* bf, uint8_t* blob, float* par, 
                         if (v == 0) kx = 1 + pix; else { if (pix == 0) continue; kx = 0; }
                         const float val = (float)(W(ci, ky, kx, co) / (255.0 * stdv[ci]) * scale);
                         uint16_t h, l;
-                        split(val, &h, &l);
+                        split_f16(val, &h, &l);
                         uint8_t* base = blob + (v * 2 + ks) * 512 + c * 256 + k * 2;
                         memcpy(base + co * 16, &h, 2);
                         memcpy(base + (8 + co) * 16, &l, 2);

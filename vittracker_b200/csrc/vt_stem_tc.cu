@@ -296,8 +296,7 @@ size_t stem_tc_weight_bytes(int layer) {      // layer 0: conv2, 1: conv3, 2: co
 }
 
 // Host side of the K-step schedule: weight blob of one layer (fp16 hi | lo), `wf` = folded weights [ci][ky][kx][cout].
-void stem_tc_pack_weights(int cin, int cch, int cout, int npad, const float* wf, uint8_t* hi8, uint8_t* lo8,
-                          void (*split)(float, uint16_t*, uint16_t*)) {
+void stem_tc_pack_weights(int cin, int cch, int cout, int npad, const float* wf, uint8_t* hi8, uint8_t* lo8) {
     int slot = 0;
     for (int acc = 0; acc < 2; ++acc)
         for (int s = 0; s < tcs_nsteps(cch, acc); ++s, ++slot) {
@@ -312,7 +311,7 @@ void stem_tc_pack_weights(int cin, int cch, int cout, int npad, const float* wf,
                         float v = 0.f;
                         if (!(half == 1 && zero1) && ci < cin && n < cout) v = wf[(((size_t)ci * 3 + ky) * 3 + kx) * cout + n];
                         uint16_t h, l;
-                        split(v, &h, &l);
+                        split_f16(v, &h, &l);
                         const size_t off = ((size_t)(slot * 2 + half) * npad + n) * 16 + e * 2;
                         memcpy(hi8 + off, &h, 2);
                         memcpy(lo8 + off, &l, 2);

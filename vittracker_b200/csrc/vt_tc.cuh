@@ -6,6 +6,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <string.h>
 
 namespace vt {
 namespace tc {
@@ -274,6 +275,22 @@ __device__ __forceinline__ void split_pack2(float v0, float v1, uint32_t& hi, ui
         : "=&r"(hi), "=f"(l0), "=f"(l1)
         : "f"(v0), "f"(v1));
     asm("cvt.rn.f16x2.f32 %0, %2, %1;" : "=r"(lo) : "f"(l0), "f"(l1));
+}
+
+// The same split on the host, for the weight packers: fp16 bit patterns of hi and lo.
+inline void split_f16(float v, uint16_t* hi, uint16_t* lo) {
+    const __half h = __float2half_rn(v);
+    const __half l = __float2half_rn(v - __half2float(h));
+    memcpy(hi, &h, 2);
+    memcpy(lo, &l, 2);
+}
+// Host: element (n, k) of a no-swizzle K-major UMMA operand [k/8][N][8], split into the hi and lo images
+inline void put_kmajor_f16(uint8_t* hi, uint8_t* lo, int N, int n, int k, float v) {
+    uint16_t h, l;
+    split_f16(v, &h, &l);
+    const size_t off = ((size_t)(k / 8) * N + n) * 16 + (k % 8) * 2;
+    memcpy(hi + off, &h, 2);
+    memcpy(lo + off, &l, 2);
 }
 
 }  // namespace tc
