@@ -255,7 +255,8 @@ size_t stem_scratch_floats(int S);
 // planes (tensor-core path only): zero-initialised buffer of plane_tracks * tc_planes_bytes_per_track() bytes
 int launch_stem(const float* img, int S, int n, const ModelW& w, float* scratch, float* tokens,
                 int tok_stride_rows, int tok_off, uint8_t* planes, int plane_tracks, cudaStream_t st);
-// Search-branch conv3 + conv4 on the tensor cores (a2: conv2 output [n][12][64][64]; a3: scratch for conv3 output)
+// Search-branch conv2 + conv3 + conv4 on the tensor cores, for launch_stem: planes2 is conv2's operand image (written by conv1), planes3
+// and planes4 receive conv3's and conv4's
 int launch_stem234_tc(const uint8_t* planes2, int n, const ModelW& w, uint8_t* planes3, uint8_t* planes4, float* tokens,
                       int tok_stride_rows, int tok_off, cudaStream_t st);
 __host__ __device__ constexpr size_t tc_planes_bytes_per_track() {

@@ -8,8 +8,6 @@
 // in shared memory as [cin][ky][kx][cout]; a thread owns P output pixels x QG output channels and
 // reads its weights with broadcast vector loads.  The last layer writes tokens (row = y*16+x,
 // token-major [token][48]) with the positional embedding added (vit_dist.py:53,81-82).
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "vt_geom.cuh"
@@ -346,7 +344,7 @@ constexpr int kCc1TileSide = 2 * 32 + 1;                                // 65 re
 constexpr int kCc1WFloats = 2 * Conv1Cfg::kWFloats;                    // conv1 weights duplicated {w, w} for the packed FMAs
 constexpr size_t kCc1SmemBytes = Conv1Cfg::kSmemBytes + Conv1Cfg::kWFloats * sizeof(float) + 64 + 2 * 80 * sizeof(int4);     // 4 CTAs / SM
 
-template <int S, int TCOUT_CCH>
+template <int S>
 __global__ void __launch_bounds__(kCc1Threads, 4)
 crop_conv1_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict__ frame_offsets,
                   const int4* __restrict__ taps, const float* __restrict__ wg,
@@ -455,7 +453,7 @@ crop_conv1_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict_
     }
     asm volatile("cp.async.wait_group 0;\n" ::: "memory");
     __syncthreads();
-    conv_compute<3, 6, 6, 4, 32, 32, true, false, TCOUT_CCH, true>(tile, ws, bs, tx0, ty0, Hout, Hout, item, out, nullptr, 0, 0);
+    conv_compute<3, 6, 6, 4, 32, 32, true, false, 0, true>(tile, ws, bs, tx0, ty0, Hout, Hout, item, out, nullptr, 0, 0);
 }
 
 template <int CIN, int COUT, int QG, int P, int TW, int TH, bool HSWISH, bool TOKENS, int TCOUT_CCH = 0>
@@ -487,10 +485,10 @@ size_t stem_scratch_floats(int S) {
 
 size_t crop_taps_bytes(int n) { return (size_t)n * 2 * kTapPitch * sizeof(int4) + 256; }      // + the fused front's work counter
 
-template <int S, int TCOUT_CCH>
+template <int S>
 static int run_crop_conv1(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
                           double factor, int n, const ModelW& w, float* out, int32_t* out_status, int4* taps, cudaStream_t st) {
-    auto kern = crop_conv1_kernel<S, TCOUT_CCH>;
+    auto kern = crop_conv1_kernel<S>;
     static DeviceOnce once;
     if (!ensure_dyn_smem(once, kern, kCc1SmemBytes)) return -1;
     constexpr int tiles = (S / 64) * (S / 64);
@@ -499,9 +497,7 @@ static int run_crop_conv1(const uint8_t* frames, const int64_t* frame_offsets, c
     for (int first = 0; first < n; first += 32768) {
         const int m = min(32768, n - first);
         kern<<<dim3(tiles, m), kCc1Threads, kCc1SmemBytes, st>>>(frames, frame_offsets + first, taps + (size_t)first * 2 * kTapPitch,
-                                                                 w.stem[0].w, w.stem[0].b,
-                                                                 TCOUT_CCH > 0 ? reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(out) + (size_t)first * tc_planes_bytes(TCOUT_CCH, S / 4))
-                                                                               : out + (size_t)first * 6 * (S / 2) * (S / 2));
+                                                                 w.stem[0].w, w.stem[0].b, out + (size_t)first * 6 * (S / 2) * (S / 2));
         ++launched;
     }
     return cudaGetLastError() == cudaSuccess ? launched : -1;
@@ -519,26 +515,17 @@ int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const 
     const float* pos = (S == kSx) ? w.pos_x : w.pos_z;
     int total = 0, r;
     if (planes && S == kSx && n <= plane_tracks) {
-        // search branch: conv1 writes conv2's tensor-core operand image; layers 2-4 run on tcgen05
-        uint8_t* planes2 = planes;
-        uint8_t* planes3 = planes2 + (size_t)plane_tracks * tc_planes_bytes(kConv2Cch, kConv2Wout);
+        // search branch: crop + conv1 + conv2 in one tcgen05 kernel (vt_stem_fused.cu), then layers 3-4 on tcgen05.  The planes
+        // buffer keeps conv2's operand image first (launch_stem writes it), so conv3's image starts after it.
+        uint8_t* planes3 = planes + (size_t)plane_tracks * tc_planes_bytes(kConv2Cch, kConv2Wout);
         uint8_t* planes4 = planes3 + (size_t)plane_tracks * tc_planes_bytes(kConv3Cch, kConv3Wout);
-        // default: crop + conv1 + conv2 in one tcgen05 kernel (vt_stem_fused.cu); VT_STEM_UNFUSED=1 keeps the previous three-kernel
-        // front (CUDA-core conv1 writing conv2's operand image to HBM) for A / B comparisons
-        static const bool unfused = [] { const char* e = getenv("VT_STEM_UNFUSED"); return e && e[0] == '1'; }();
-        if (!unfused) {
-            if ((r = launch_crop_stem12_fused(frames, frame_offsets, frame_hw, boxes, factor, n, w, out_status, tap_tables, planes3, st)) < 0) return r;
-            total += r;
-            if ((r = launch_stem34_tc(planes3, n, w, planes4, tokens, tok_stride_rows, tok_off, st)) < 0) return r;
-            return total + r;
-        }
-        if ((r = run_crop_conv1<256, kConv2Cch>(frames, frame_offsets, frame_hw, boxes, factor, n, w, reinterpret_cast<float*>(planes2), out_status, taps, st)) < 0) return r;
+        if ((r = launch_crop_stem12_fused(frames, frame_offsets, frame_hw, boxes, factor, n, w, out_status, tap_tables, planes3, st)) < 0) return r;
         total += r;
-        if ((r = launch_stem234_tc(planes2, n, w, planes3, planes4, tokens, tok_stride_rows, tok_off, st)) < 0) return r;
+        if ((r = launch_stem34_tc(planes3, n, w, planes4, tokens, tok_stride_rows, tok_off, st)) < 0) return r;
         return total + r;
     }
-    if (S == 256) r = run_crop_conv1<256, 0>(frames, frame_offsets, frame_hw, boxes, factor, n, w, a1, out_status, taps, st);
-    else if (S == 128) r = run_crop_conv1<128, 0>(frames, frame_offsets, frame_hw, boxes, factor, n, w, a1, out_status, taps, st);
+    if (S == 256) r = run_crop_conv1<256>(frames, frame_offsets, frame_hw, boxes, factor, n, w, a1, out_status, taps, st);
+    else if (S == 128) r = run_crop_conv1<128>(frames, frame_offsets, frame_hw, boxes, factor, n, w, a1, out_status, taps, st);
     else return -1;
     if (r < 0) return r;
     total += r;

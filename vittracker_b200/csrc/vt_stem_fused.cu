@@ -11,8 +11,8 @@
 // the padded pixel is 0; its share of the second sum is left out of the bias: four bias variants (interior, top row, left column,
 // corner).  Zero padding of the CROP (pixels outside the frame) is pixel value 0, as in the reference, and needs nothing special.
 //
-// Work item = (track, band of BR2 conv2 output rows).  Per item, with 512 threads:
-//   1. gather: the band needs resized-crop rows 4 oy0 - 3 .. 4 oy0 + 4 BR2 - 1; a thread owns one PAIR of adjacent columns (2x, 2x + 1)
+// Work item = (track, band of kBR2 = 4 conv2 output rows).  Per item, with 512 threads:
+//   1. gather: the band needs resized-crop rows 4 oy0 - 3 .. 4 oy0 + 4 kBR2 - 1; a thread owns one PAIR of adjacent columns (2x, 2x + 1)
 //      and walks down the rows (same integer arithmetic as crop_conv1_kernel: aligned word loads, funnel shifts, byte permute + dp2a,
 //      11-bit fixed point).  The six bytes of the pair become six fp16 = one 16-byte K chunk {R G B R G B 0 0} - one STS.128.  A row is
 //      stored as a zero chunk followed by its 128 pair chunks.
@@ -23,7 +23,6 @@
 //   3. epilogue 1: (hi + lo) * 2^-s + bias variant, Hardswish, fp16 hi/lo split -> conv2's parity-plane operand image in shared memory.
 //   4. conv2 + epilogue 2: as conv_s2_tc_kernel (vt_stem_tc.cu), reading that image; writes conv3's operand image to global memory.
 #include <math.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "vt_geom.cuh"
@@ -54,13 +53,13 @@ namespace {
 constexpr int kFThreads = 512;
 constexpr int kIPitch = 129 * 16;              // one resized-crop row in shared memory: a zero chunk + 128 pixel-pair chunks of 16 bytes
 
-template <int BR2>
 struct Fused {
-    using C2 = TcConv<kConv2Cch, 12, 16, kConv2Wout, BR2>;       // conv2: band geometry (A operand planes) and weight blob
-    static constexpr int kBands = kConv2Wout / BR2;
+    static constexpr int kBR2 = 4;                                // conv2 output rows of a band
+    using C2 = TcConv<kConv2Cch, 12, 16, kConv2Wout, kBR2>;      // conv2: band geometry (A operand planes) and weight blob
+    static constexpr int kBands = kConv2Wout / kBR2;
     static constexpr int kUnitBands = 4;                          // consecutive bands of one track a CTA takes at a time (work unit), at most
-    static constexpr int kIRows = 4 * BR2 + 3;                    // resized-crop rows of a band
-    static constexpr int kA1Rows = 2 * BR2 + 1;                   // conv1 output rows of a band
+    static constexpr int kIRows = 4 * kBR2 + 3;                   // resized-crop rows of a band
+    static constexpr int kA1Rows = 2 * kBR2 + 1;                  // conv1 output rows of a band
     static constexpr int kOffI = 0;
     static constexpr int kIBytes = (kIRows * kIPitch + 16 + 127) / 128 * 128;     // + one trailing zero chunk
     static constexpr int kOffA1 = kOffI + kIBytes;
@@ -107,14 +106,13 @@ __device__ __forceinline__ uint32_t pack_u8_f16x2(int a, int b) {
 
 }  // namespace
 
-template <int BR2>
-__global__ void __launch_bounds__(kFThreads, Fused<BR2>::kCtasPerSm)
+__global__ void __launch_bounds__(kFThreads, Fused::kCtasPerSm)
 stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict__ frame_offsets, const int4* __restrict__ taps,
                     const uint8_t* __restrict__ w1g, const float* __restrict__ par1g, const uint8_t* __restrict__ w2g,
                     const float* __restrict__ bias2g, uint8_t* __restrict__ planes3, int n_units, int n_big, int unit_bands,
                     int* __restrict__ work_counter) {
-    using F = Fused<BR2>;
-    using C2 = typename F::C2;
+    using F = Fused;
+    using C2 = F::C2;
     extern __shared__ __align__(128) uint8_t sm[];
 #ifdef VT_FUSED_TRACE
     if (threadIdx.x == 0 && blockIdx.x < 1024) {
@@ -155,7 +153,7 @@ stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restric
 
     // reuse: the item is the band below the one whose rows are in the slots - its first three rows are that band's last three
     auto gather = [&](int item, bool reuse) {
-        const int b = item / F::kBands, oy0 = (item % F::kBands) * BR2;
+        const int b = item / F::kBands, oy0 = (item % F::kBands) * F::kBR2;
         const int i0 = 4 * oy0 - 3;                                   // resized-crop row held by slot 0
         const uint8_t* __restrict__ im = frames + frame_offsets[b];
         const int4* __restrict__ tcol = taps + (size_t)b * 2 * kTapPitch + 1;    // record of resized-crop column d at [d]
@@ -230,7 +228,7 @@ stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restric
     // dependent chain (record -> pixel addresses -> pixels) that every warp of the CTA walks at the same time.
     auto prefetch_taps = [&](int item) {
         if (tid >= 32 && tid < 72) {
-            const int b = item / F::kBands, oy0 = (item % F::kBands) * BR2;
+            const int b = item / F::kBands, oy0 = (item % F::kBands) * F::kBR2;
             const int4* tcol = taps + (size_t)b * 2 * kTapPitch;
             const int l = tid - 32;
             const int4* p = l < 34 ? tcol + 8 * l : tcol + kTapPitch + max(4 * oy0 - 3, 0) + 8 * (l - 34);
@@ -238,7 +236,7 @@ stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restric
         }
     };
     auto issue_conv1 = [&](int item) {
-        const int oy0 = (item % F::kBands) * BR2;
+        const int oy0 = (item % F::kBands) * F::kBR2;
         // ---- 2. conv1: per output row r (y = 2 oy0 - 1 + r) four MMAs into columns [16 r, 16 r + 16)
         if (warp == 0) {                     // convergent; one elected lane issues
             const uint32_t idesc1 = instr_desc_f16(128, 16, false);
@@ -260,7 +258,7 @@ stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restric
         }
     };
     auto epilogue1 = [&](int item) {
-        const int oy0 = (item % F::kBands) * BR2;
+        const int oy0 = (item % F::kBands) * F::kBR2;
         // ---- 3. epilogue 1: thread = (pixel x = TMEM lane, row group); -> conv2's operand image (parity planes, fp16 hi | lo)
         {
             const int q = warp & 3, g = warp >> 2;
@@ -327,7 +325,7 @@ stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restric
         }
     };
     auto epilogue2 = [&](int item) {
-        const int b = item / F::kBands, oy0 = (item % F::kBands) * BR2;
+        const int b = item / F::kBands, oy0 = (item % F::kBands) * F::kBR2;
         // ---- 5. epilogue 2: 16 warps = (channel half) x (tile of a pair) x (TMEM lane quarter); thread = one output pixel x 8 channels
         {
             const int q = warp & 3, tsel = (warp >> 2) & 1, half = warp >> 3;
@@ -460,17 +458,13 @@ stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restric
     if (warp == 0) tmem_dealloc(tbase, F::kTmemCols);
 }
 
-#ifndef VT_FUSED_BR
-#define VT_FUSED_BR 4
-#endif
-
 // Search crop of n tracks straight from the raw frames -> conv3's operand image (planes3): tap tables + the fused kernel.
 // tap_tables: crop_taps_bytes(n) bytes; the fused kernel's work counter sits behind the n tables.
 int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes, double factor,
                              int n, const ModelW& w, int32_t* out_status, void* tap_tables, uint8_t* planes3, cudaStream_t st) {
     if (n <= 0) return 0;
-    using F = Fused<VT_FUSED_BR>;
-    auto kern = stem12_fused_kernel<VT_FUSED_BR>;
+    using F = Fused;
+    auto kern = stem12_fused_kernel;
     static int grid_caps[kMaxDevices] = {};
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) return -1;
@@ -481,10 +475,7 @@ int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets
         grid_caps[dev] = sms * resident_ctas_per_sm(kern, kFThreads, F::kSmemBytes, F::kTmemCols, dev);
     }
     // few tracks (the batch-1 latency path): single bands, so that a track spreads over kBands CTAs instead of kBands / kUnitBands
-    static const int forced = [] { const char* e = getenv("VT_FUSED_UNIT_BANDS"); return e ? atoi(e) : 0; }();      // A / B aid: 1, 2 or 4
-    // few tracks (the batch-1 latency path): single bands, so that a track spreads over kBands CTAs instead of kBands / kUnitBands
-    const int unit_bands = (forced == 1 || forced == 2 || forced == 4) ? forced
-                           : (long long)n * (F::kBands / F::kUnitBands) >= 2LL * grid_caps[dev] ? F::kUnitBands : 1;
+    const int unit_bands = (long long)n * (F::kBands / F::kUnitBands) >= 2LL * grid_caps[dev] ? F::kUnitBands : 1;
     const long long bands = (long long)n * F::kBands;
     if (bands > 0x7fffffffLL) return -1;
     // the last sixteenth of the bands (at least two rounds of the grid) is handed out band by band
@@ -573,8 +564,8 @@ extern "C" int vt_fused_trace_read(long long* host, int* n) {
 
 // Development aid (not part of the ABI): what the occupancy API answers for the fused kernel on the current device.
 extern "C" int vt_debug_fused_occupancy(int* out) {
-    using F = vt::Fused<VT_FUSED_BR>;
-    auto kern = vt::stem12_fused_kernel<VT_FUSED_BR>;
+    using F = vt::Fused;
+    auto kern = vt::stem12_fused_kernel;
     int a = -1, b = -1, c = -1;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, kern, vt::kFThreads, F::kSmemBytes);
     cudaError_t e1 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, F::kSmemBytes);

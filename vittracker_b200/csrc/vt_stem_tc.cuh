@@ -40,13 +40,7 @@ __host__ __device__ inline void tcs_step(int cch, int acc, int s, int& tap0, int
     tap0 = a; tap1 = b;
 }
 
-#ifndef VT_CONV2_BR
-#define VT_CONV2_BR 4
-#endif
-#ifndef VT_CONV3_BR
-#define VT_CONV3_BR 4
-#endif
-constexpr int kConv2BR = VT_CONV2_BR, kConv3BR = VT_CONV3_BR;     // output rows per CTA
+constexpr int kConv2BR = 4, kConv3BR = 4;     // output rows per CTA
 
 template <int CCH, int COUT, int NPAD, int WOUT, int BR>
 struct TcConv {

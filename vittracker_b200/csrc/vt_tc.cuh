@@ -60,30 +60,15 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 }
 #else
 // Spin on try_wait (a hardware-bounded suspend per try).  A suspend-time hint (mbarrier.try_wait ..., hint -> TRYWAIT + NANOSLEEP.SYNCS)
-// was measured: every tcgen05 kernel got 1 - 3 % SLOWER (wake-up latency), so the plain spin stays; -DVT_MBAR_HINT_NS=<ns> re-enables it.
+// was measured: every tcgen05 kernel got 1 - 3 % SLOWER (wake-up latency), so the plain spin stays.
 // The loop doubles as an always-on watchdog: a wait that outlasts 2^26 tries (seconds; every legitimate wait here is far below a
 // millisecond) is a protocol deadlock - the kernel traps (the launch fails with an error the host sees) instead of hanging the GPU.
-#ifndef VT_MBAR_HINT_NS
-#define VT_MBAR_HINT_NS 0
-#endif
 #ifndef VT_MBAR_WATCHDOG_TRIES
 #define VT_MBAR_WATCHDOG_TRIES (1u << 26)
 #endif
-__device__ __forceinline__ bool mbar_try_wait_hint(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok)
-                 : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)VT_MBAR_HINT_NS)
-                 : "memory");
-    return ok != 0;
-}
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     uint32_t n = 0;
-#if VT_MBAR_HINT_NS > 0
-    while (!mbar_try_wait_hint(bar, parity)) {
-#else
     while (!mbar_try_wait(bar, parity)) {
-#endif
         if (++n > VT_MBAR_WATCHDOG_TRIES) __trap();
     }
 }
@@ -257,14 +242,6 @@ __device__ __forceinline__ void mbar_arrive_expect_tx_elect(uint64_t* bar, uint3
 // fma.rn.f32.f16: an fp16 product accumulated onto an fp32 addend, exact here) gives v - hi without unpacking, one packed conversion
 // gives both lo halves.
 __device__ __forceinline__ void split_pack2(float v0, float v1, uint32_t& hi, uint32_t& lo) {
-#ifdef VT_OLD_SPLIT
-    const __half2 h = __floats2half2_rn(v0, v1);
-    const float2 hf = __half22float2(h);
-    const __half2 l = __floats2half2_rn(v0 - hf.x, v1 - hf.y);
-    hi = *reinterpret_cast<const uint32_t*>(&h);
-    lo = *reinterpret_cast<const uint32_t*>(&l);
-    return;
-#endif
     float l0, l1;
     asm("{\n\t.reg .b16 h0, h1, m;\n\t"
         "cvt.rn.f16x2.f32 %0, %4, %3;\n\t"
