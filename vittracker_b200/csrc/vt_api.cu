@@ -86,85 +86,109 @@ int fail(VtHandle h, int code, const char* fmt, ...) {
     } while (0)
 
 const char* kTowers[3] = {"ctr", "offset", "size"};
+std::string stem_prefix(int l) { return "patch_embed.net." + std::to_string(2 * l) + "."; }
+std::string head_prefix(int layer, int tower) { return "box_head.conv" + std::to_string(layer + 1) + "_" + kTowers[tower] + "."; }
 
-bool expected_shape(const VtConfig& c, const std::string& name, std::vector<int64_t>& shp) {
-    const int C = c.embed_dim, hc = c.head_channels;
-    char buf[128];
-    if (name == "pos_embed_z") { shp = {1, 64, C}; return true; }
-    if (name == "pos_embed_x") { shp = {1, 256, C}; return true; }
-    if (name == "norm.weight" || name == "norm.bias") { shp = {C}; return true; }
-    if (name == "tracker.output_window") { shp = {1, 1, 16, 16}; return true; }
-    const int ch[5] = {3, C / 8, C / 4, C / 2, C};
-    for (int i = 0; i < 4; ++i) {
-        snprintf(buf, sizeof buf, "patch_embed.net.%d.", 2 * i);
-        if (name.rfind(buf, 0) == 0) {
-            const std::string leaf = name.substr(strlen(buf));
-            if (leaf == "c.weight") { shp = {ch[i + 1], ch[i], 3, 3}; return true; }
-            if (leaf == "bn.weight" || leaf == "bn.bias" || leaf == "bn.running_mean" || leaf == "bn.running_var") { shp = {ch[i + 1]}; return true; }
-            return false;
-        }
+// Every tensor of the reference's state_dict for configuration c: name -> shape.  tracker.output_window is optional (the window is
+// computed when the tracker's own tensor was not handed over).
+std::map<std::string, std::vector<int64_t>> tensor_table(const VtConfig& c) {
+    const int64_t C = c.embed_dim, hc = c.head_channels, hid = (int64_t)c.mlp_ratio * C;
+    std::map<std::string, std::vector<int64_t>> t;
+    t["pos_embed_z"] = {1, 64, C};
+    t["pos_embed_x"] = {1, 256, C};
+    t["norm.weight"] = {C};
+    t["norm.bias"] = {C};
+    t["tracker.output_window"] = {1, 1, 16, 16};
+    const int64_t ch[5] = {3, C / 8, C / 4, C / 2, C};
+    for (int l = 0; l < 4; ++l) {
+        const std::string p = stem_prefix(l);
+        t[p + "c.weight"] = {ch[l + 1], ch[l], 3, 3};
+        for (const char* leaf : {"bn.weight", "bn.bias", "bn.running_mean", "bn.running_var"}) t[p + leaf] = {ch[l + 1]};
     }
     for (int b = 0; b < c.depth; ++b) {
-        snprintf(buf, sizeof buf, "blocks.%d.", b);
-        if (name.rfind(buf, 0) == 0) {
-            const std::string leaf = name.substr(strlen(buf));
-            const int hid = c.mlp_ratio * C;
-            if (leaf == "norm1.weight" || leaf == "norm1.bias" || leaf == "norm2.weight" || leaf == "norm2.bias") { shp = {C}; return true; }
-            if (leaf == "attn.qkv.weight") { shp = {3 * C, C}; return true; }
-            if (leaf == "attn.qkv.bias") { shp = {3 * C}; return true; }
-            if (leaf == "attn.proj.weight") { shp = {C, C}; return true; }
-            if (leaf == "attn.proj.bias") { shp = {C}; return true; }
-            if (leaf == "mlp.fc1.weight") { shp = {hid, C}; return true; }
-            if (leaf == "mlp.fc1.bias") { shp = {hid}; return true; }
-            if (leaf == "mlp.fc2.weight") { shp = {C, hid}; return true; }
-            if (leaf == "mlp.fc2.bias") { shp = {C}; return true; }
-            return false;
-        }
+        const std::string p = "blocks." + std::to_string(b) + ".";
+        for (const char* leaf : {"norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias", "attn.proj.bias", "mlp.fc2.bias"}) t[p + leaf] = {C};
+        t[p + "attn.qkv.weight"] = {3 * C, C};
+        t[p + "attn.qkv.bias"] = {3 * C};
+        t[p + "attn.proj.weight"] = {C, C};
+        t[p + "mlp.fc1.weight"] = {hid, C};
+        t[p + "mlp.fc1.bias"] = {hid};
+        t[p + "mlp.fc2.weight"] = {C, hid};
     }
-    const int hch[5] = {C, hc, hc / 2, hc / 4, hc / 8};
-    const int outs[3] = {1, 2, 2};
-    for (int t = 0; t < 3; ++t) {
+    const int64_t hch[5] = {C, hc, hc / 2, hc / 4, hc / 8}, outs[3] = {1, 2, 2};
+    for (int k = 0; k < 3; ++k) {
         for (int i = 0; i < 4; ++i) {
-            snprintf(buf, sizeof buf, "box_head.conv%d_%s.", i + 1, kTowers[t]);
-            if (name.rfind(buf, 0) == 0) {
-                const std::string leaf = name.substr(strlen(buf));
-                if (leaf == "0.weight") { shp = {hch[i + 1], hch[i], 3, 3}; return true; }
-                if (leaf == "0.bias" || leaf == "1.weight" || leaf == "1.bias" || leaf == "1.running_mean" || leaf == "1.running_var") { shp = {hch[i + 1]}; return true; }
-                return false;
-            }
+            const std::string p = head_prefix(i, k);
+            t[p + "0.weight"] = {hch[i + 1], hch[i], 3, 3};
+            for (const char* leaf : {"0.bias", "1.weight", "1.bias", "1.running_mean", "1.running_var"}) t[p + leaf] = {hch[i + 1]};
         }
-        snprintf(buf, sizeof buf, "box_head.conv5_%s.", kTowers[t]);
-        if (name.rfind(buf, 0) == 0) {
-            const std::string leaf = name.substr(strlen(buf));
-            if (leaf == "weight") { shp = {outs[t], hch[4], 1, 1}; return true; }
-            if (leaf == "bias") { shp = {outs[t]}; return true; }
-            return false;
-        }
+        const std::string p = std::string("box_head.conv5_") + kTowers[k] + ".";
+        t[p + "weight"] = {outs[k], hch[4], 1, 1};
+        t[p + "bias"] = {outs[k]};
     }
-    return false;
+    return t;
 }
 
+// First step of finalisation: every tensor of the table that is not optional must have been set.  Past it, every lookup succeeds.
+int check_missing(VtHandle h) {
+    std::string missing;
+    for (const auto& e : tensor_table(h->cfg))
+        if (e.first != "tracker.output_window" && !h->tensors.count(e.first) && missing.size() < 300) missing += e.first + " ";
+    return missing.empty() ? VT_OK : fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", missing.c_str());
+}
+
+const float* tensor(VtHandle h, const std::string& name) { return h->tensors.at(name).data.data(); }
+
+BlockTensors block_tensors(VtHandle h, int b) {
+    const std::string p = "blocks." + std::to_string(b) + ".";
+    return {tensor(h, p + "norm1.weight"), tensor(h, p + "norm1.bias"), tensor(h, p + "attn.qkv.weight"), tensor(h, p + "attn.qkv.bias"),
+            tensor(h, p + "attn.proj.weight"), tensor(h, p + "attn.proj.bias"), tensor(h, p + "norm2.weight"), tensor(h, p + "norm2.bias"),
+            tensor(h, p + "mlp.fc1.weight"), tensor(h, p + "mlp.fc1.bias"), tensor(h, p + "mlp.fc2.weight"), tensor(h, p + "mlp.fc2.bias")};
+}
+
+// Conv2d (with its bias when `conv_bias`) and BatchNorm2d (eval) folded in float64 (Conv2d_BN.fuse vit_dist.py:22-33; head conv + bias
+// -> BN, head.py:16-21): w [co][ci][3][3] in the conv's order, b [co]; co and ci are the conv weight's stored shape.
+struct FoldedConv {
+    int co, ci;
+    std::vector<float> w, b;
+};
+FoldedConv fold_conv_bn(VtHandle h, const std::string& conv, const std::string& bn, bool conv_bias) {
+    const HostTensor& wt = h->tensors.at(conv + "weight");
+    const float *w = wt.data.data(), *cb = conv_bias ? tensor(h, conv + "bias") : nullptr;
+    const float *g = tensor(h, bn + "weight"), *b = tensor(h, bn + "bias"), *m = tensor(h, bn + "running_mean"), *v = tensor(h, bn + "running_var");
+    FoldedConv f{(int)wt.shape[0], (int)wt.shape[1], std::vector<float>(wt.data.size()), std::vector<float>(wt.shape[0])};
+    const size_t kn = wt.data.size() / f.co;                                  // ci * 9 weights per output channel
+    for (int co = 0; co < f.co; ++co) {
+        const double s = (double)g[co] / sqrt((double)v[co] + 1e-5);         // BatchNorm2d's default eps
+        f.b[co] = (float)(((cb ? (double)cb[co] : 0.0) - (double)m[co]) * s + (double)b[co]);
+        for (size_t k = 0; k < kn; ++k) f.w[co * kn + k] = (float)((double)w[co * kn + k] * s);
+    }
+    return f;
+}
+
+// The packed weights: one fp32 buffer of 16-byte aligned slots.  slot() allocates one for the ModelW / GenModelW member that will
+// point at it and returns its host offset; upload_weights() points every such member into the device buffer.
 struct Packer {
     std::vector<float> buf;
-    size_t alloc(size_t n) {                     // 16-byte aligned slots
+    std::vector<std::pair<const float**, size_t>> fslots;
+    std::vector<std::pair<const uint8_t**, size_t>> bslots;
+    size_t alloc(size_t n) {
         const size_t off = buf.size();
         buf.resize(off + (n + 3) / 4 * 4, 0.f);
         return off;
     }
-};
-
-// Tensor lookup of the finalisers: a tensor that was never set yields null and is listed in `missing`
-struct TensorLookup {
-    VtHandle h;
-    std::string missing;
-    const float* operator()(const std::string& n) {
-        auto it = h->tensors.find(n);
-        if (it == h->tensors.end()) { if (missing.size() < 300) missing += n + " "; return nullptr; }
-        return it->second.data.data();
+    size_t slot(const float*& member, size_t n) { fslots.push_back({&member, alloc(n)}); return fslots.back().second; }
+    size_t slot(const uint8_t*& member, size_t n) { bslots.push_back({&member, alloc(n)}); return bslots.back().second; }
+    size_t put(const float*& member, const float* src, size_t n) {
+        const size_t o = slot(member, n);
+        memcpy(&buf[o], src, n * sizeof(float));
+        return o;
     }
+    uint8_t* bytes(size_t o) { return reinterpret_cast<uint8_t*>(&buf[o]); }
 };
 
-// The packed weights -> h->d_weights (reallocated when it has grown); returns once the copy is done, as pk is the caller's local
+// The packed weights -> h->d_weights (reallocated when it has grown), then every slot's member -> its place there; returns once the
+// copy is done, as pk is the caller's local
 int upload_weights(VtHandle h, const Packer& pk, cudaStream_t st) {
     if (h->d_weights && h->weights_floats < pk.buf.size()) { cudaFree(h->d_weights); h->d_weights = nullptr; }
     if (!h->d_weights) {
@@ -173,6 +197,8 @@ int upload_weights(VtHandle h, const Packer& pk, cudaStream_t st) {
     }
     VT_CUDA(h, cudaMemcpyAsync(h->d_weights, pk.buf.data(), pk.buf.size() * sizeof(float), cudaMemcpyHostToDevice, st));
     VT_CUDA(h, cudaStreamSynchronize(st));
+    for (const auto& e : pk.fslots) *e.first = h->d_weights + e.second;
+    for (const auto& e : pk.bslots) *e.first = reinterpret_cast<const uint8_t*>(h->d_weights + e.second);
     return VT_OK;
 }
 
@@ -222,6 +248,44 @@ int run_blocks(VtHandle h, const float* tokz, int zs, const float* tokx, int xs,
 }
 
 
+// HeadArgs of a forward pass over rows [first, first + m) of the caller's output arrays (each nullable)
+HeadArgs forward_head_args(int first, int m, float* pred_boxes, float* score_map, float* size_map, float* offset_map) {
+    HeadArgs a{};
+    a.n = m;
+    a.pred_boxes = pred_boxes ? pred_boxes + (size_t)first * 4 : nullptr;
+    a.score_map = score_map ? score_map + (size_t)first * 256 : nullptr;
+    a.size_map = size_map ? size_map + (size_t)first * 512 : nullptr;
+    a.offset_map = offset_map ? offset_map + (size_t)first * 512 : nullptr;
+    return a;
+}
+
+// The maps of the last tracking step from track `first` on: kept planar per array, score [max_tracks][256] | size [max_tracks][512] |
+// offset [max_tracks][512]
+struct LastMaps { float *score, *size, *offset; };
+LastMaps last_maps(VtHandle h, int first) {
+    const size_t mt = h->cfg.max_tracks;
+    return {h->d_maps + (size_t)first * 256, h->d_maps + mt * 256 + (size_t)first * 512, h->d_maps + mt * 768 + (size_t)first * 512};
+}
+
+// HeadArgs of a tracking step over tracks [first + c0, first + c0 + m); frame_hw, out_boxes and out_detail are the step's arrays,
+// which start at track `first`
+HeadArgs track_head_args(VtHandle h, int first, int c0, int m, const int32_t* frame_hw, double* out_boxes, double* out_detail,
+                         int update_state) {
+    const int t0 = first + c0;
+    const LastMaps maps = last_maps(h, t0);
+    HeadArgs a{};
+    a.n = m;
+    a.score_map = maps.score; a.size_map = maps.size; a.offset_map = maps.offset;
+    a.state = h->d_state + (size_t)t0 * 4;
+    a.frame_hw = frame_hw + 2 * c0;
+    a.status = h->d_status + t0;
+    a.out_boxes = out_boxes + (size_t)c0 * 5;
+    a.out_detail = out_detail ? out_detail + (size_t)c0 * 8 : nullptr;
+    a.update_state = update_state;
+    a.search_factor = h->cfg.search_factor;
+    return a;
+}
+
 // Hann window (hann.py:6-16; the tracker's own tensor when it was handed over) and normalisation table (data_utils.py:8-14)
 void fill_hann_and_lut(VtHandle h, float* hann, float* lut) {
     auto it = h->tensors.find("tracker.output_window");
@@ -244,130 +308,84 @@ void fill_hann_and_lut(VtHandle h, float* hann, float* lut) {
         }
 }
 
-// Weights of the generic path: the reference's own layouts ([out][in]; conv [cout][ky][kx][cin]) with BatchNorm(eval) folded
-// in float64 (Conv2d_BN.fuse vit_dist.py:22-33; head conv + bias -> BN, head.py:16-21).
+// Weights of the generic path: the reference's own layouts ([out][in]; conv [cout][ky][kx][cin]) with BatchNorm(eval) folded.
 int finalize_generic(VtHandle h, cudaStream_t st) {
-    const VtConfig& c = h->cfg;
-    const int C = c.embed_dim, hc = c.head_channels, hid = c.mlp_ratio * C;
-    TensorLookup T{h};
-    Packer pk;
-    auto put = [&](const float* src, size_t n) { const size_t o = pk.alloc(n); if (src) memcpy(&pk.buf[o], src, n * sizeof(float)); return o; };
-    const double eps = 1e-5;
-    // conv [co][ci][3][3] (+ optional conv bias) with BN -> [co][(ky, kx, ci)], bias
-    auto fold_conv = [&](const float* w, const float* cb, const float* g, const float* b, const float* m, const float* v, int co_n, int ci_n,
-                         size_t& ow, size_t& ob) {
-        ow = pk.alloc((size_t)co_n * 9 * ci_n); ob = pk.alloc(co_n);
-        if (!(w && g && b && m && v)) return;
-        for (int co = 0; co < co_n; ++co) {
-            const double sc = (double)g[co] / sqrt((double)v[co] + eps);
-            pk.buf[ob + co] = (float)((((cb ? (double)cb[co] : 0.0) - (double)m[co]) * sc) + (double)b[co]);
-            for (int ci = 0; ci < ci_n; ++ci)
-                for (int k = 0; k < 9; ++k)
-                    pk.buf[ow + ((size_t)co * 9 + k) * ci_n + ci] = (float)((double)w[((size_t)co * ci_n + ci) * 9 + k] * sc);
-        }
-    };
-    const int ch[5] = {3, C / 8, C / 4, C / 2, C};
-    size_t sw[4], sb[4];
-    for (int l = 0; l < 4; ++l) {
-        const std::string p = "patch_embed.net." + std::to_string(2 * l) + ".";
-        fold_conv(T(p + "c.weight"), nullptr, T(p + "bn.weight"), T(p + "bn.bias"), T(p + "bn.running_mean"), T(p + "bn.running_var"), ch[l + 1], ch[l], sw[l], sb[l]);
-    }
-    struct BO { size_t v[12]; };
-    std::vector<BO> bo(c.depth);
-    for (int b = 0; b < c.depth; ++b) {
-        const std::string p = "blocks." + std::to_string(b) + ".";
-        const char* names[12] = {"norm1.weight", "norm1.bias", "attn.qkv.weight", "attn.qkv.bias", "attn.proj.weight", "attn.proj.bias",
-                                 "norm2.weight", "norm2.bias", "mlp.fc1.weight", "mlp.fc1.bias", "mlp.fc2.weight", "mlp.fc2.bias"};
-        const size_t cnt[12] = {(size_t)C, (size_t)C, (size_t)3 * C * C, (size_t)3 * C, (size_t)C * C, (size_t)C,
-                                (size_t)C, (size_t)C, (size_t)hid * C, (size_t)hid, (size_t)C * hid, (size_t)C};
-        for (int i = 0; i < 12; ++i) bo[b].v[i] = put(T(p + names[i]), cnt[i]);
-    }
-    // split images of the blocks' Linear weights for the bulk-copy GEMM (same bytes as the fp32 matrices; packed on a few host threads)
-    struct IO { size_t v[4]; };
-    std::vector<IO> io(c.depth);
-    if (h->gw.use_img) {
-        const int wi[4] = {2, 4, 8, 10};                                       // qkv, proj, fc1, fc2 in `names`
-        const int wn[4] = {3 * C, C, hid, C}, wk[4] = {C, C, C, hid};
-        for (int b = 0; b < c.depth; ++b)
-            for (int j = 0; j < 4; ++j) io[b].v[j] = pk.alloc(gen_img_bytes(wn[j], wk[j]) / 4);
-        if (T.missing.empty())
-            for (int b = 0; b < c.depth; ++b)
-                for (int j = 0; j < 4; ++j)
-                    gen_pack_weight_image(&pk.buf[bo[b].v[wi[j]]], wn[j], wk[j], reinterpret_cast<uint8_t*>(&pk.buf[io[b].v[j]]));
-    }
-    const size_t o_ng = put(T("norm.weight"), C), o_nb = put(T("norm.bias"), C);
-    const size_t o_pz = put(T("pos_embed_z"), (size_t)kNz * C), o_px = put(T("pos_embed_x"), (size_t)kNx * C);
-    // head: layer 1 merged over the towers (ctr | offset | size), layers 2-4 per tower, conv5 rows ctr, off x, off y, size w, size h
-    const int hch[5] = {C, hc, hc / 2, hc / 4, hc / 8};
-    const size_t o_w1 = pk.alloc((size_t)3 * hc * 9 * C), o_b1 = pk.alloc((size_t)3 * hc);
-    size_t hw[3][3], hb[3][3];
-    for (int t = 0; t < 3; ++t) {
-        for (int i = 0; i < 4; ++i) {
-            const std::string p = std::string("box_head.conv") + std::to_string(i + 1) + "_" + kTowers[t] + ".";
-            size_t ow, ob;
-            fold_conv(T(p + "0.weight"), T(p + "0.bias"), T(p + "1.weight"), T(p + "1.bias"), T(p + "1.running_mean"), T(p + "1.running_var"),
-                      hch[i + 1], hch[i], ow, ob);
-            if (i == 0) {       // copy into the merged layer (alloc moves pk.buf: index, do not hold pointers)
-                for (size_t k = 0; k < (size_t)hc * 9 * C; ++k) pk.buf[o_w1 + (size_t)t * hc * 9 * C + k] = pk.buf[ow + k];
-                for (int k = 0; k < hc; ++k) pk.buf[o_b1 + (size_t)t * hc + k] = pk.buf[ob + k];
-            } else { hw[t][i - 1] = ow; hb[t][i - 1] = ob; }
-        }
-    }
-    const size_t o_w5 = pk.alloc((size_t)5 * hch[4]), o_b5 = pk.alloc(5);
-    {
-        const int row0[3] = {0, 1, 3}, outs[3] = {1, 2, 2};
-        for (int t = 0; t < 3; ++t) {
-            const std::string p = std::string("box_head.conv5_") + kTowers[t] + ".";
-            const float *w = T(p + "weight"), *b = T(p + "bias");
-            if (!(w && b)) continue;
-            for (int o = 0; o < outs[t]; ++o) {
-                pk.buf[o_b5 + row0[t] + o] = b[o];
-                for (int k = 0; k < hch[4]; ++k) pk.buf[o_w5 + (size_t)(row0[t] + o) * hch[4] + k] = w[(size_t)o * hch[4] + k];
-            }
-        }
-    }
-    if (!T.missing.empty()) return fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", T.missing.c_str());
-    const size_t o_hann = pk.alloc(256), o_lut = pk.alloc(768);
-    fill_hann_and_lut(h, &pk.buf[o_hann], &pk.buf[o_lut]);
-    // split images of the folded convolution weights (K = 9 cin must be a whole number of 32-wide panels)
-    size_t isw[4] = {0, 0, 0, 0}, ihw1 = 0, ihw[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
-    auto conv_img = [&](size_t w_off, int co_n, int ci_n) -> size_t {
-        if (!h->gw.use_img || ci_n % 32 != 0) return 0;
-        const size_t o = pk.alloc(gen_img_bytes(co_n, 9 * ci_n) / 4);
-        gen_pack_weight_image(&pk.buf[w_off], co_n, 9 * ci_n, reinterpret_cast<uint8_t*>(&pk.buf[o]));
-        return o;
-    };
-    for (int l = 1; l < 4; ++l) isw[l] = conv_img(sw[l], ch[l + 1], ch[l]);
-    ihw1 = conv_img(o_w1, 3 * hc, C);
-    for (int t = 0; t < 3; ++t)
-        for (int l = 0; l < 3; ++l) ihw[t][l] = conv_img(hw[t][l], hch[l + 2], hch[l + 1]);
-
-    if (const int rc = upload_weights(h, pk, st)) return rc;
-    const float* base = h->d_weights;
+    const int C = h->cfg.embed_dim, hc = h->cfg.head_channels, hid = h->cfg.mlp_ratio * C;
     GenModelW& g = h->gw;
-    for (int l = 0; l < 4; ++l) { g.stem_w[l] = base + sw[l]; g.stem_b[l] = base + sb[l]; }
-    for (int b = 0; b < c.depth; ++b) {
-        const float* q[12];
-        for (int i = 0; i < 12; ++i) q[i] = base + bo[b].v[i];
-        g.blk[b] = GenBlockW{q[0], q[1], q[2], q[3], q[4], q[5], q[6], q[7], q[8], q[9], q[10], q[11], nullptr, nullptr, nullptr, nullptr};
-        if (g.use_img) {
-            const uint8_t* ib[4];
-            for (int j = 0; j < 4; ++j) ib[j] = reinterpret_cast<const uint8_t*>(base + io[b].v[j]);
-            g.blk[b].iwqkv = ib[0]; g.blk[b].iwproj = ib[1]; g.blk[b].iwfc1 = ib[2]; g.blk[b].iwfc2 = ib[3];
+    Packer pk;
+    // split images of the folded convolutions whose K = 9 cin is a whole number of 32-wide panels, packed after the fp32 weights
+    struct ConvImg { const uint8_t** img; size_t w; int co, ci; };
+    std::vector<ConvImg> imgs;
+    auto want_img = [&](const uint8_t*& img, size_t w, int co, int ci) { if (g.use_img && ci % 32 == 0) imgs.push_back({&img, w, co, ci}); };
+    auto conv_rows = [&](const FoldedConv& f, size_t ow, size_t ob) {          // -> [co][(ky, kx, ci)] at ow, bias at ob
+        for (int co = 0; co < f.co; ++co) {
+            pk.buf[ob + co] = f.b[co];
+            for (int ci = 0; ci < f.ci; ++ci)
+                for (int k = 0; k < 9; ++k) pk.buf[ow + ((size_t)co * 9 + k) * f.ci + ci] = f.w[((size_t)co * f.ci + ci) * 9 + k];
+        }
+    };
+    for (int l = 0; l < 4; ++l) {
+        const FoldedConv f = fold_conv_bn(h, stem_prefix(l) + "c.", stem_prefix(l) + "bn.", false);
+        const size_t ow = pk.slot(g.stem_w[l], f.w.size()), ob = pk.slot(g.stem_b[l], f.co);
+        conv_rows(f, ow, ob);
+        want_img(g.istem_w[l], ow, f.co, f.ci);
+    }
+    for (int b = 0; b < h->cfg.depth; ++b) {
+        const BlockTensors t = block_tensors(h, b);
+        GenBlockW& B = g.blk[b];
+        pk.put(B.ln1g, t.ln1_g, C); pk.put(B.ln1b, t.ln1_b, C);
+        pk.put(B.wqkv, t.wqkv, (size_t)3 * C * C); pk.put(B.bqkv, t.bqkv, (size_t)3 * C);
+        pk.put(B.wproj, t.wproj, (size_t)C * C); pk.put(B.bproj, t.bproj, C);
+        pk.put(B.ln2g, t.ln2_g, C); pk.put(B.ln2b, t.ln2_b, C);
+        pk.put(B.wfc1, t.wfc1, (size_t)hid * C); pk.put(B.bfc1, t.bfc1, hid);
+        pk.put(B.wfc2, t.wfc2, (size_t)C * hid); pk.put(B.bfc2, t.bfc2, C);
+    }
+    // split images of the blocks' Linear weights for the bulk-copy GEMM (same bytes as the fp32 matrices)
+    for (int b = 0; b < h->cfg.depth && g.use_img; ++b) {
+        const BlockTensors t = block_tensors(h, b);
+        GenBlockW& B = g.blk[b];
+        const struct { const uint8_t*& img; const float* w; int n, k; } lin[4] = {
+            {B.iwqkv, t.wqkv, 3 * C, C}, {B.iwproj, t.wproj, C, C}, {B.iwfc1, t.wfc1, hid, C}, {B.iwfc2, t.wfc2, C, hid}};
+        for (const auto& L : lin) {
+            const size_t o = pk.slot(L.img, gen_img_bytes(L.n, L.k) / 4);
+            gen_pack_weight_image(L.w, L.n, L.k, pk.bytes(o));
         }
     }
-    g.norm_g = base + o_ng; g.norm_b = base + o_nb; g.pos_z = base + o_pz; g.pos_x = base + o_px;
-    g.head_w1 = base + o_w1; g.head_b1 = base + o_b1;
+    pk.put(g.norm_g, tensor(h, "norm.weight"), C); pk.put(g.norm_b, tensor(h, "norm.bias"), C);
+    pk.put(g.pos_z, tensor(h, "pos_embed_z"), (size_t)kNz * C); pk.put(g.pos_x, tensor(h, "pos_embed_x"), (size_t)kNx * C);
+    // head: layer 1 merged over the towers (ctr | offset | size), layers 2-4 per tower, conv5 rows ctr, off x, off y, size w, size h
+    const size_t w1 = pk.slot(g.head_w1, (size_t)3 * hc * 9 * C), b1 = pk.slot(g.head_b1, (size_t)3 * hc);
+    want_img(g.ihead_w1, w1, 3 * hc, C);
     for (int t = 0; t < 3; ++t)
-        for (int l = 0; l < 3; ++l) { g.head_w[t][l] = base + hw[t][l]; g.head_b[t][l] = base + hb[t][l]; }
-    g.head_w5 = base + o_w5; g.head_b5 = base + o_b5;
-    g.hann = base + o_hann;
-    auto imgp = [&](size_t o) { return o ? reinterpret_cast<const uint8_t*>(base + o) : nullptr; };
-    for (int l = 0; l < 4; ++l) g.istem_w[l] = imgp(isw[l]);
-    g.ihead_w1 = imgp(ihw1);
-    for (int t = 0; t < 3; ++t)
-        for (int l = 0; l < 3; ++l) g.ihead_w[t][l] = imgp(ihw[t][l]);
-    h->mw.hann = base + o_hann; h->mw.lut = base + o_lut;         // the crop kernel reads the table through ModelW
+        for (int i = 0; i < 4; ++i) {
+            const FoldedConv f = fold_conv_bn(h, head_prefix(i, t) + "0.", head_prefix(i, t) + "1.", true);
+            if (i == 0) {      // the merged layer's rows of this tower (the tower's own layer-1 slot is not read)
+                const size_t ow = pk.alloc(f.w.size()), ob = pk.alloc(f.co);
+                conv_rows(f, ow, ob);
+                conv_rows(f, w1 + (size_t)t * hc * 9 * C, b1 + (size_t)t * hc);
+                continue;
+            }
+            const size_t ow = pk.slot(g.head_w[t][i - 1], f.w.size()), ob = pk.slot(g.head_b[t][i - 1], f.co);
+            conv_rows(f, ow, ob);
+            want_img(g.ihead_w[t][i - 1], ow, f.co, f.ci);
+        }
+    const int c5 = hc / 8, row0[3] = {0, 1, 3}, outs[3] = {1, 2, 2};
+    const size_t w5 = pk.slot(g.head_w5, (size_t)5 * c5), b5 = pk.slot(g.head_b5, 5);
+    for (int t = 0; t < 3; ++t) {
+        const std::string p = std::string("box_head.conv5_") + kTowers[t] + ".";
+        const float *w = tensor(h, p + "weight"), *b = tensor(h, p + "bias");
+        for (int o = 0; o < outs[t]; ++o) {
+            pk.buf[b5 + row0[t] + o] = b[o];
+            for (int k = 0; k < c5; ++k) pk.buf[w5 + (size_t)(row0[t] + o) * c5 + k] = w[(size_t)o * c5 + k];
+        }
+    }
+    const size_t hann = pk.slot(g.hann, 256), lut = pk.slot(h->mw.lut, 768);         // the crop kernel reads the table through ModelW
+    fill_hann_and_lut(h, &pk.buf[hann], &pk.buf[lut]);
+    for (const ConvImg& c : imgs) {
+        const size_t o = pk.slot(*c.img, gen_img_bytes(c.co, 9 * c.ci) / 4);       // (allocating moves pk.buf: index, hold no pointer)
+        gen_pack_weight_image(&pk.buf[c.w], c.co, 9 * c.ci, pk.bytes(o));
+    }
+    if (const int rc = upload_weights(h, pk, st)) return rc;
     h->finalized = true;
     return VT_OK;
 }
@@ -523,9 +541,11 @@ int vt_set_tensor(VtHandle h, const char* name, const float* data_host, const in
     const std::string nm(name);
     const char* nbt = "num_batches_tracked";
     if (nm.size() >= strlen(nbt) && nm.compare(nm.size() - strlen(nbt), strlen(nbt), nbt) == 0) return VT_OK;   // accepted, unused in eval
-    std::vector<int64_t> want;
-    if (!expected_shape(h->cfg, nm, want)) return fail(h, VT_ERR_WEIGHTS, "unknown tensor '%s' (ignored, as load_state_dict(strict=False) would)", name);
+    const auto table = tensor_table(h->cfg);
+    const auto it = table.find(nm);
+    if (it == table.end()) return fail(h, VT_ERR_WEIGHTS, "unknown tensor '%s' (ignored, as load_state_dict(strict=False) would)", name);
     if (!data_host) return fail(h, VT_ERR_INVALID_ARG, "vt_set_tensor: null data for '%s'", name);
+    const std::vector<int64_t>& want = it->second;
     std::vector<int64_t> got(shape, shape + ndim);
     if (got != want) {
         std::string g, w;
@@ -547,151 +567,96 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
     DeviceGuard dg(h->cfg.device);
     VT_CUDA(h, dg.err);
+    if (const int rc = check_missing(h)) return rc;
     if (h->generic) return finalize_generic(h, st);
-    TensorLookup T{h};
     Packer pk;
-    auto slot = [&](size_t n) { return pk.alloc(n); };
-    const double eps = 1e-5;     // BatchNorm2d default eps
+    ModelW& m = h->mw;
 
-    // ---- stem: fold BN (Conv2d_BN.fuse, vit_dist.py:22-33), repack [co][ci][3][3] -> [ci][ky][kx][co]
-    const int ch[5] = {3, 6, 12, 24, 48};
+    // ---- stem: BN folded, [co][ci][3][3] -> [ci][ky][kx][co]
     size_t stem_w[4], stem_b[4];
     for (int l = 0; l < 4; ++l) {
-        const std::string p = "patch_embed.net." + std::to_string(2 * l) + ".";
-        const float *w = T(p + "c.weight"), *g = T(p + "bn.weight"), *b = T(p + "bn.bias"), *m = T(p + "bn.running_mean"), *v = T(p + "bn.running_var");
-        const int ci_n = ch[l], co_n = ch[l + 1];
-        stem_w[l] = slot((size_t)ci_n * 9 * co_n);
-        stem_b[l] = slot(co_n);
-        if (!(w && g && b && m && v)) continue;
-        for (int co = 0; co < co_n; ++co) {
-            const double s = (double)g[co] / sqrt((double)v[co] + eps);
-            pk.buf[stem_b[l] + co] = (float)((double)b[co] - (double)m[co] * s);
-            for (int ci = 0; ci < ci_n; ++ci)
-                for (int k = 0; k < 9; ++k)
-                    pk.buf[stem_w[l] + ((size_t)ci * 9 + k) * co_n + co] = (float)((double)w[((size_t)co * ci_n + ci) * 9 + k] * s);
-        }
+        const FoldedConv f = fold_conv_bn(h, stem_prefix(l) + "c.", stem_prefix(l) + "bn.", false);
+        stem_w[l] = pk.slot(m.stem[l].w, f.w.size());
+        stem_b[l] = pk.put(m.stem[l].b, f.b.data(), f.co);
+        for (int co = 0; co < f.co; ++co)
+            for (int ci = 0; ci < f.ci; ++ci)
+                for (int k = 0; k < 9; ++k) pk.buf[stem_w[l] + ((size_t)ci * 9 + k) * f.co + co] = f.w[((size_t)co * f.ci + ci) * 9 + k];
     }
-    // ---- stem conv3 / conv4 for the tensor cores: fp16 hi | lo weight blobs in the kernels' K-step order (vt_stem_tc.cu)
-    size_t stc_w[3], stc_b[3];
+    // ---- stem conv2 / conv3 / conv4 for the tensor cores: fp16 hi | lo weight blobs in the kernels' K-step order (vt_stem_tc.cu)
     {
         const int lcin[3] = {6, 12, 24}, lcch[3] = {kConv2Cch, kConv3Cch, kConv4Cch}, lcout[3] = {12, 24, 48}, lnpad[3] = {16, 32, 48};
         for (int i = 0; i < 3; ++i) {
-            const int l = 1 + i;
             const size_t bytes = stem_tc_weight_bytes(i);
-            stc_w[i] = slot(bytes / 4);
-            stc_b[i] = slot(lnpad[i]);
-            uint8_t* hi8 = reinterpret_cast<uint8_t*>(&pk.buf[stc_w[i]]);
-            for (int co = 0; co < lcout[i]; ++co) pk.buf[stc_b[i] + co] = pk.buf[stem_b[l] + co];
-            stem_tc_pack_weights(lcin[i], lcch[i], lcout[i], lnpad[i], &pk.buf[stem_w[l]], hi8, hi8 + bytes / 2);
+            const size_t w = pk.slot(m.stem_tc_w[i], bytes / 4), b = pk.slot(m.stem_tc_b[i], lnpad[i]);
+            for (int co = 0; co < lcout[i]; ++co) pk.buf[b + co] = pk.buf[stem_b[i + 1] + co];
+            stem_tc_pack_weights(lcin[i], lcch[i], lcout[i], lnpad[i], &pk.buf[stem_w[i + 1]], pk.bytes(w), pk.bytes(w) + bytes / 2);
         }
     }
     // ---- stem conv1 for the fused tensor-core front (vt_stem_fused.cu): pixel normalisation folded into the weights / border-variant biases
-    const size_t s1_w = slot(kStem1TcWBytes / 4), s1_p = slot(kStem1TcParFloats);
-    stem1_tc_pack(&pk.buf[stem_w[0]], &pk.buf[stem_b[0]], reinterpret_cast<uint8_t*>(&pk.buf[s1_w]), &pk.buf[s1_p]);
+    const size_t s1_w = pk.slot(m.stem1_tc_w, kStem1TcWBytes / 4), s1_p = pk.slot(m.stem1_tc_par, kStem1TcParFloats);
+    stem1_tc_pack(&pk.buf[stem_w[0]], &pk.buf[stem_b[0]], pk.bytes(s1_w), &pk.buf[s1_p]);
     // ---- blocks: Linear weights [out][in] -> K-major [in][out]
-    struct BOff { size_t ln1g, ln1b, wqkv, bqkv, wproj, bproj, ln2g, ln2b, wfc1, bfc1, wfc2, bfc2; } bo[kDepth];
-    BlockTensors bt[kDepth];
-    auto copyv = [&](size_t o, const float* src, size_t n) { if (src) memcpy(&pk.buf[o], src, n * sizeof(float)); };
     auto transp = [&](size_t o, const float* src, int rows_out, int cols_in) {     // src [out][in] -> dst [in][out]
-        if (!src) return;
         for (int r = 0; r < rows_out; ++r)
             for (int c = 0; c < cols_in; ++c) pk.buf[o + (size_t)c * rows_out + r] = src[(size_t)r * cols_in + c];
     };
     for (int b = 0; b < kDepth; ++b) {
-        const std::string p = "blocks." + std::to_string(b) + ".";
-        BlockTensors& t = bt[b];
-        t = {T(p + "norm1.weight"), T(p + "norm1.bias"), T(p + "attn.qkv.weight"), T(p + "attn.qkv.bias"), T(p + "attn.proj.weight"),
-             T(p + "attn.proj.bias"), T(p + "norm2.weight"), T(p + "norm2.bias"), T(p + "mlp.fc1.weight"), T(p + "mlp.fc1.bias"),
-             T(p + "mlp.fc2.weight"), T(p + "mlp.fc2.bias")};
-        bo[b].ln1g = slot(kC); copyv(bo[b].ln1g, t.ln1_g, kC);
-        bo[b].ln1b = slot(kC); copyv(bo[b].ln1b, t.ln1_b, kC);
-        bo[b].wqkv = slot(kC * 3 * kC); transp(bo[b].wqkv, t.wqkv, 3 * kC, kC);
-        bo[b].bqkv = slot(3 * kC); copyv(bo[b].bqkv, t.bqkv, 3 * kC);
-        bo[b].wproj = slot(kC * kC); transp(bo[b].wproj, t.wproj, kC, kC);
-        bo[b].bproj = slot(kC); copyv(bo[b].bproj, t.bproj, kC);
-        bo[b].ln2g = slot(kC); copyv(bo[b].ln2g, t.ln2_g, kC);
-        bo[b].ln2b = slot(kC); copyv(bo[b].ln2b, t.ln2_b, kC);
-        bo[b].wfc1 = slot(kC * kHid); transp(bo[b].wfc1, t.wfc1, kHid, kC);
-        bo[b].bfc1 = slot(kHid); copyv(bo[b].bfc1, t.bfc1, kHid);
-        bo[b].wfc2 = slot(kHid * kC); transp(bo[b].wfc2, t.wfc2, kC, kHid);
-        bo[b].bfc2 = slot(kC); copyv(bo[b].bfc2, t.bfc2, kC);
+        const BlockTensors t = block_tensors(h, b);
+        BlockW& B = m.blk[b];
+        pk.put(B.ln1_g, t.ln1_g, kC); pk.put(B.ln1_b, t.ln1_b, kC);
+        transp(pk.slot(B.wqkv, kC * 3 * kC), t.wqkv, 3 * kC, kC);
+        pk.put(B.bqkv, t.bqkv, 3 * kC);
+        transp(pk.slot(B.wproj, kC * kC), t.wproj, kC, kC);
+        pk.put(B.bproj, t.bproj, kC);
+        pk.put(B.ln2_g, t.ln2_g, kC); pk.put(B.ln2_b, t.ln2_b, kC);
+        transp(pk.slot(B.wfc1, kC * kHid), t.wfc1, kHid, kC);
+        pk.put(B.bfc1, t.bfc1, kHid);
+        transp(pk.slot(B.wfc2, kHid * kC), t.wfc2, kC, kHid);
+        pk.put(B.bfc2, t.bfc2, kC);
     }
-    // ---- the same blocks for the tensor cores (vt_block_tc.cu), packed only when every tensor looked up so far is present
-    size_t tc_wa[kDepth], tc_wb[kDepth], tc_par[kDepth];
+    // ---- the same blocks for the tensor cores (vt_block_tc.cu)
     for (int b = 0; b < kDepth; ++b) {
-        tc_wa[b] = slot(kTcWaBytes / 4); tc_wb[b] = slot(kTcWbBytes / 4); tc_par[b] = slot(kTcParFloats);
-        if (T.missing.empty())
-            block_tc_pack(bt[b], reinterpret_cast<uint8_t*>(&pk.buf[tc_wa[b]]), reinterpret_cast<uint8_t*>(&pk.buf[tc_wb[b]]), &pk.buf[tc_par[b]]);
+        const size_t wa = pk.slot(m.tc[b].wa, kTcWaBytes / 4), wb = pk.slot(m.tc[b].wb, kTcWbBytes / 4), par = pk.slot(m.tc[b].par, kTcParFloats);
+        block_tc_pack(block_tensors(h, b), pk.bytes(wa), pk.bytes(wb), &pk.buf[par]);
     }
-    const size_t o_ng = slot(kC), o_nb = slot(kC), o_pz = slot(kNz * kC), o_px = slot(kNx * kC);
-    copyv(o_ng, T("norm.weight"), kC); copyv(o_nb, T("norm.bias"), kC);
-    copyv(o_pz, T("pos_embed_z"), kNz * kC); copyv(o_px, T("pos_embed_x"), kNx * kC);
+    pk.put(m.norm_g, tensor(h, "norm.weight"), kC); pk.put(m.norm_b, tensor(h, "norm.bias"), kC);
+    pk.put(m.pos_z, tensor(h, "pos_embed_z"), kNz * kC); pk.put(m.pos_x, tensor(h, "pos_embed_x"), kNx * kC);
 
     // ---- head: conv(+bias) -> BN folded; layer i weights laid out [ci][k][tower][co_t]
-    const int hch[5] = {kC, kHeadC, kHeadC / 2, kHeadC / 4, kHeadC / 8};
-    size_t hw[5], hb[5];
+    const float** head_w[4] = {&m.head.w1, &m.head.w2, &m.head.w3, &m.head.w4};
+    const float** head_b[4] = {&m.head.b1, &m.head.b2, &m.head.b3, &m.head.b4};
+    size_t hw[4];
     for (int i = 0; i < 4; ++i) {
-        const int ci_n = hch[i], co_n = hch[i + 1];
-        hw[i] = slot((size_t)ci_n * 9 * 3 * co_n);
-        hb[i] = slot(3 * co_n);
-        for (int t = 0; t < 3; ++t) {
-            const std::string p = std::string("box_head.conv") + std::to_string(i + 1) + "_" + kTowers[t] + ".";
-            const float *w = T(p + "0.weight"), *cb = T(p + "0.bias"), *g = T(p + "1.weight"), *b = T(p + "1.bias"), *m = T(p + "1.running_mean"), *v = T(p + "1.running_var");
-            if (!(w && cb && g && b && m && v)) continue;
+        FoldedConv f[3];
+        for (int t = 0; t < 3; ++t) f[t] = fold_conv_bn(h, head_prefix(i, t) + "0.", head_prefix(i, t) + "1.", true);
+        const int ci_n = f[0].ci, co_n = f[0].co;
+        hw[i] = pk.slot(*head_w[i], (size_t)ci_n * 9 * 3 * co_n);
+        const size_t hb = pk.slot(*head_b[i], 3 * co_n);
+        for (int t = 0; t < 3; ++t)
             for (int co = 0; co < co_n; ++co) {
-                const double s = (double)g[co] / sqrt((double)v[co] + eps);
-                pk.buf[hb[i] + t * co_n + co] = (float)(((double)cb[co] - (double)m[co]) * s + (double)b[co]);
+                pk.buf[hb + t * co_n + co] = f[t].b[co];
                 for (int ci = 0; ci < ci_n; ++ci)
                     for (int k = 0; k < 9; ++k)
-                        pk.buf[hw[i] + (((size_t)ci * 9 + k) * 3 + t) * co_n + co] = (float)((double)w[((size_t)co * ci_n + ci) * 9 + k] * s);
+                        pk.buf[hw[i] + (((size_t)ci * 9 + k) * 3 + t) * co_n + co] = f[t].w[((size_t)co * ci_n + ci) * 9 + k];
             }
-        }
     }
     // head conv1 - conv3 for the tensor cores (vt_head.cu)
-    size_t o_htc[3];
-    for (int i = 0; i < 3; ++i) o_htc[i] = slot(head_tc_weight_bytes(i) / 4);
-    head_tc_pack(&pk.buf[hw[0]], &pk.buf[hw[1]], &pk.buf[hw[2]], reinterpret_cast<uint8_t*>(&pk.buf[o_htc[0]]),
-                 reinterpret_cast<uint8_t*>(&pk.buf[o_htc[1]]), reinterpret_cast<uint8_t*>(&pk.buf[o_htc[2]]));
-    hw[4] = slot(3 * 4 * 2); hb[4] = slot(3 * 2);
+    const size_t htc1 = pk.slot(m.head_tc_w1, head_tc_weight_bytes(0) / 4), htc2 = pk.slot(m.head_tc_w2, head_tc_weight_bytes(1) / 4),
+                 htc3 = pk.slot(m.head_tc_w3, head_tc_weight_bytes(2) / 4);
+    head_tc_pack(&pk.buf[hw[0]], &pk.buf[hw[1]], &pk.buf[hw[2]], pk.bytes(htc1), pk.bytes(htc2), pk.bytes(htc3));
+    const size_t w5 = pk.slot(m.head.w5, 3 * 4 * 2), b5 = pk.slot(m.head.b5, 3 * 2);
     for (int t = 0; t < 3; ++t) {
         const std::string p = std::string("box_head.conv5_") + kTowers[t] + ".";
-        const float *w = T(p + "weight"), *b = T(p + "bias");
-        if (!(w && b)) continue;
-        const int outs = t == 0 ? 1 : 2;
-        for (int o = 0; o < outs; ++o) {
-            pk.buf[hb[4] + t * 2 + o] = b[o];
-            for (int c = 0; c < 4; ++c) pk.buf[hw[4] + (t * 4 + c) * 2 + o] = w[o * 4 + c];
+        const float *w = tensor(h, p + "weight"), *b = tensor(h, p + "bias");
+        for (int o = 0; o < (t == 0 ? 1 : 2); ++o) {
+            pk.buf[b5 + t * 2 + o] = b[o];
+            for (int c = 0; c < 4; ++c) pk.buf[w5 + (t * 4 + c) * 2 + o] = w[o * 4 + c];
         }
     }
-    if (!T.missing.empty()) return fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", T.missing.c_str());
-
     // ---- Hann window (hann.py:6-16) and normalisation table (data_utils.py:8-14) -----------------
-    const size_t o_hann = slot(256), o_lut = slot(768);
-    fill_hann_and_lut(h, &pk.buf[o_hann], &pk.buf[o_lut]);
-
+    const size_t hann = pk.slot(m.hann, 256), lut = pk.slot(m.lut, 768);
+    fill_hann_and_lut(h, &pk.buf[hann], &pk.buf[lut]);
     if (const int rc = upload_weights(h, pk, st)) return rc;
-    const float* base = h->d_weights;
-    ModelW& m = h->mw;
-    for (int l = 0; l < 4; ++l) { m.stem[l].w = base + stem_w[l]; m.stem[l].b = base + stem_b[l]; }
-    for (int b = 0; b < kDepth; ++b) {
-        BlockW& B = m.blk[b];
-        B.ln1_g = base + bo[b].ln1g; B.ln1_b = base + bo[b].ln1b; B.wqkv = base + bo[b].wqkv; B.bqkv = base + bo[b].bqkv;
-        B.wproj = base + bo[b].wproj; B.bproj = base + bo[b].bproj; B.ln2_g = base + bo[b].ln2g; B.ln2_b = base + bo[b].ln2b;
-        B.wfc1 = base + bo[b].wfc1; B.bfc1 = base + bo[b].bfc1; B.wfc2 = base + bo[b].wfc2; B.bfc2 = base + bo[b].bfc2;
-        m.tc[b].wa = reinterpret_cast<const uint8_t*>(base + tc_wa[b]);
-        m.tc[b].wb = reinterpret_cast<const uint8_t*>(base + tc_wb[b]);
-        m.tc[b].par = base + tc_par[b];
-    }
-    m.norm_g = base + o_ng; m.norm_b = base + o_nb; m.pos_z = base + o_pz; m.pos_x = base + o_px;
-    m.head.w1 = base + hw[0]; m.head.b1 = base + hb[0]; m.head.w2 = base + hw[1]; m.head.b2 = base + hb[1];
-    m.head.w3 = base + hw[2]; m.head.b3 = base + hb[2]; m.head.w4 = base + hw[3]; m.head.b4 = base + hb[3];
-    m.head.w5 = base + hw[4]; m.head.b5 = base + hb[4];
-    m.head_tc_w1 = reinterpret_cast<const uint8_t*>(base + o_htc[0]);
-    m.head_tc_w2 = reinterpret_cast<const uint8_t*>(base + o_htc[1]);
-    m.head_tc_w3 = reinterpret_cast<const uint8_t*>(base + o_htc[2]);
-    for (int i = 0; i < 3; ++i) { m.stem_tc_w[i] = reinterpret_cast<const uint8_t*>(base + stc_w[i]); m.stem_tc_b[i] = base + stc_b[i]; }
-    m.stem1_tc_w = reinterpret_cast<const uint8_t*>(base + s1_w); m.stem1_tc_par = base + s1_p;
-    m.hann = base + o_hann; m.lut = base + o_lut;
     h->finalized = true;
     return VT_OK;
 }
@@ -731,12 +696,7 @@ int vt_forward(VtHandle h, const float* z, const float* x, int32_t n, float* pre
             const int m = (n - first < h->chunk) ? n - first : h->chunk;
             VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_forward/stem(z)", gen_launch_stem(z + (size_t)first * 3 * kTz * kTz, kTz, m, h->gw, h->gws, h->gws.tok, kN, 0, st));
             VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_forward/stem(x)", gen_launch_stem(x + (size_t)first * 3 * kSx * kSx, kSx, m, h->gw, h->gws, h->gws.tok, kN, kNz, st));
-            HeadArgs a{};
-            a.n = m;
-            a.pred_boxes = pred_boxes ? pred_boxes + (size_t)first * 4 : nullptr;
-            a.score_map = score_map ? score_map + (size_t)first * 256 : nullptr;
-            a.size_map = size_map ? size_map + (size_t)first * 512 : nullptr;
-            a.offset_map = offset_map ? offset_map + (size_t)first * 512 : nullptr;
+            const HeadArgs a = forward_head_args(first, m, pred_boxes, score_map, size_map, offset_map);
             VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_forward/blocks+head",
                       gen_launch_blocks_head(h->gws.tok, m, h->gw, h->gws, a, taps ? taps + (size_t)first * kN * C : nullptr, gtap, st));
         }
@@ -749,12 +709,8 @@ int vt_forward(VtHandle h, const float* z, const float* x, int32_t n, float* pre
         VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_forward/stem(x)", launch_stem(x + (size_t)first * 3 * kSx * kSx, kSx, m, h->mw, h->d_scratch, h->d_tokx, kNx, 0, h->d_planes, h->chunk, st));
         VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_forward/blocks", run_blocks(h, h->d_tokz, kNz, h->d_tokx, kNx, h->d_tok, m,
                                                       taps ? taps + (size_t)first * kN * kC : nullptr, tap_stride, st));
-        HeadArgs a{};
-        a.tokens = h->d_tok; a.n = m;
-        a.pred_boxes = pred_boxes ? pred_boxes + (size_t)first * 4 : nullptr;
-        a.score_map = score_map ? score_map + (size_t)first * 256 : nullptr;
-        a.size_map = size_map ? size_map + (size_t)first * 512 : nullptr;
-        a.offset_map = offset_map ? offset_map + (size_t)first * 512 : nullptr;
+        HeadArgs a = forward_head_args(first, m, pred_boxes, score_map, size_map, offset_map);
+        a.tokens = h->d_tok;
         a.tokens_norm = taps ? taps + (size_t)(kDepth + 1) * tap_stride + (size_t)first * kN * kC : nullptr;
         a.use_tc = h->cfg.blocks_impl != VT_BLOCKS_SIMT_FP32;
         VT_LAUNCH(h, VT_STAGE_HEAD, m, st, "vt_forward/head", launch_head(a, h->mw, st));
@@ -827,18 +783,7 @@ int vt_tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offse
             VT_CUDA(h, cudaMemcpy2DAsync(h->gws.tok, (size_t)kN * C * sizeof(float), h->d_tmpl + (size_t)t0 * kNz * C, (size_t)kNz * C * sizeof(float),
                                          (size_t)kNz * C * sizeof(float), m, cudaMemcpyDeviceToDevice, st));
             VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_step/stem", gen_launch_stem(h->gws.crop, kSx, m, h->gw, h->gws, h->gws.tok, kN, kNz, st));
-            HeadArgs a{};
-            a.n = m;
-            a.score_map = h->d_maps + (size_t)t0 * 256;
-            a.size_map = h->d_maps + (size_t)h->cfg.max_tracks * 256 + (size_t)t0 * 512;
-            a.offset_map = h->d_maps + (size_t)h->cfg.max_tracks * 768 + (size_t)t0 * 512;
-            a.state = h->d_state + (size_t)t0 * 4;
-            a.frame_hw = frame_hw + 2 * c0;
-            a.status = h->d_status + t0;
-            a.out_boxes = out_boxes + (size_t)c0 * 5;
-            a.out_detail = out_detail ? out_detail + (size_t)c0 * 8 : nullptr;
-            a.update_state = update_state;
-            a.search_factor = h->cfg.search_factor;
+            const HeadArgs a = track_head_args(h, first, c0, m, frame_hw, out_boxes, out_detail, update_state);
             VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_tracks_step/blocks+head", gen_launch_blocks_head(h->gws.tok, m, h->gw, h->gws, a, nullptr, 0, st));
         }
         h->last_first = first; h->last_n = n;
@@ -857,19 +802,8 @@ int vt_tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offse
         const int m = n;
         VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_tracks_step/blocks",
                   run_blocks(h, h->d_tmpl + (size_t)first * kNz * kC, kNz, h->d_tokx, kNx, h->d_tok, m, nullptr, 0, st));
-        HeadArgs a{};
-        a.tokens = h->d_tok; a.n = m;
-        // maps of the last step are kept planar per array: score [max][256] | size [max][512] | offset [max][512]
-        a.score_map = h->d_maps + (size_t)first * 256;
-        a.size_map = h->d_maps + (size_t)h->cfg.max_tracks * 256 + (size_t)first * 512;
-        a.offset_map = h->d_maps + (size_t)h->cfg.max_tracks * 768 + (size_t)first * 512;
-        a.state = h->d_state + (size_t)first * 4;
-        a.frame_hw = frame_hw;
-        a.status = h->d_status + first;
-        a.out_boxes = out_boxes;
-        a.out_detail = out_detail;
-        a.update_state = update_state;
-        a.search_factor = h->cfg.search_factor;
+        HeadArgs a = track_head_args(h, first, 0, m, frame_hw, out_boxes, out_detail, update_state);
+        a.tokens = h->d_tok;
         a.use_tc = h->cfg.blocks_impl != VT_BLOCKS_SIMT_FP32;
         VT_LAUNCH(h, VT_STAGE_HEAD, m, st, "vt_tracks_step/head", launch_head(a, h->mw, st));
     }
@@ -895,10 +829,10 @@ int vt_tracks_last_maps(VtHandle h, int32_t first, int32_t n, float* score_map, 
     if (!h) return VT_ERR_INVALID_ARG;
     if (first < h->last_first || n < 0 || first + n > h->last_first + h->last_n) return fail(h, VT_ERR_STATE, "vt_tracks_last_maps: tracks [%d, %d) were not part of the last step", first, first + n);
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t mt = h->cfg.max_tracks;
-    if (score_map) VT_CUDA(h, cudaMemcpyAsync(score_map, h->d_maps + (size_t)first * 256, (size_t)n * 256 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    if (size_map) VT_CUDA(h, cudaMemcpyAsync(size_map, h->d_maps + mt * 256 + (size_t)first * 512, (size_t)n * 512 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    if (offset_map) VT_CUDA(h, cudaMemcpyAsync(offset_map, h->d_maps + mt * 768 + (size_t)first * 512, (size_t)n * 512 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    const LastMaps maps = last_maps(h, first);
+    if (score_map) VT_CUDA(h, cudaMemcpyAsync(score_map, maps.score, (size_t)n * 256 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (size_map) VT_CUDA(h, cudaMemcpyAsync(size_map, maps.size, (size_t)n * 512 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (offset_map) VT_CUDA(h, cudaMemcpyAsync(offset_map, maps.offset, (size_t)n * 512 * sizeof(float), cudaMemcpyDeviceToDevice, st));
     return VT_OK;
 }
 
