@@ -229,6 +229,30 @@ int vt_yuv420_to_rgb(VtHandle h, int32_t format, const uint8_t* src, const int64
 int vt_upload_yuv420_rect(VtHandle h, int32_t format, const uint8_t* image, int32_t H, int32_t W, int32_t y0, int32_t y1,
                           int32_t x0, int32_t x1, uint8_t* staging, uint8_t* staging_dev, uint8_t* frame_rgb_dev, void* stream);
 
+/* Device-resident YUV surfaces (a hardware decoder's output: pitched planes, the chroma plane wherever the decoder put it),
+ * converted only where a crop reads them.  For item i of n:
+ *   planes     [n][3] device addresses of the Y plane, the U plane (NV12: the interleaved U V plane) and the V plane (I420; NV12
+ *              ignores it).  Any byte alignment.
+ *   pitches    [n][2] int32 byte distance between rows of the luma plane and of the chroma plane(s): at least W for luma and for
+ *              NV12 chroma, at least W/2 for I420 chroma (U and V share it).
+ *   frame_hw   [n][2] int32 (H, W) of the picture (even; a decoder surface's padding rows below H are never read).
+ *   boxes_xywh [n][4] float64 boxes, or NULL: the current state of tracks [first, first + n) (what vt_tracks_step will crop).
+ *   factor     the crop factor (the configuration's template_factor before vt_tracks_init, search_factor before vt_tracks_step).
+ *   dst + dst_offsets[i]: the item's H x W x 3 RGB frame, the one passed to vt_tracks_init / vt_tracks_step afterwards.
+ * The box's crop geometry is computed on the device by the code the crop kernels run: crop_sz = ceil(sqrt(w h) factor),
+ * x1 = round(x + w/2 - crop_sz/2), y1 = round(y + h/2 - crop_sz/2) (half to even).  Only rows [max(0, y1), min(H, y1 + crop_sz))
+ * x columns [max(0, x1 - 1), min(W, x1 + crop_sz + 1)) - what sample_target reads plus one spare column on either side - widened
+ * to even bounds (a 2x2 block shares one chroma sample) are read and converted, with the cvtColor arithmetic above, at their place
+ * in the RGB frame.  No other byte of dst is written.  Nothing is written for an item whose crop is degenerate (VT_TRACK_TOO_SMALL
+ * or VT_TRACK_OUT_OF_DOMAIN), whose H or W is odd or below 2, or whose pitch is below its row width.  The rest of the RGB frame
+ * keeps what it held: zero-fill it once (the crop kernels read the first pixels of a row with weight 0).
+ * All arrays are device pointers.  No allocation and no host synchronisation: the call can be captured in a CUDA graph.
+ * Bad host arguments (format, null pointers, n < 0, factor <= 0, first + n > max_tracks when the state is used) return
+ * VT_ERR_INVALID_ARG before any launch.  One kernel launch. */
+int vt_yuv420_crop_to_rgb(VtHandle h, int32_t format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw,
+                          const double* boxes_xywh, double factor, int32_t first, int32_t n, uint8_t* dst,
+                          const int64_t* dst_offsets, void* stream);
+
 /* Development aid: which profiled stage launches (vt_profile_enable) have started / finished.  Non-blocking;
  * meant for a watchdog thread while the owning thread waits in a synchronisation (tools/hang_probe.py,
  * tests/test_gpu_soak.py).  out[i] = stage * 4 + (started ? 1 : 0) + (finished ? 2 : 0); returns the count. */

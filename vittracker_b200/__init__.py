@@ -19,7 +19,7 @@ def __getattr__(name):
     if name in ("Vit_dist", "get_tracker_class", "BaseTracker", "clip_box"):
         from . import tracker
         return getattr(tracker, name)
-    if name in ("BatchedTracker", "ShardedTracker", "FramePool", "PipelinedFrameFeeder", "shard_range"):
+    if name in ("BatchedTracker", "ShardedTracker", "FramePool", "PipelinedFrameFeeder", "YuvSurfaces", "shard_range"):
         from . import batched
         return getattr(batched, name)
     if name in ("Sequence", "MultiSequenceRunner", "BatchedBackend", "run_sequences", "save_tracker_output", "read_image"):

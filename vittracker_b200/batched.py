@@ -12,7 +12,7 @@ from typing import Optional, Sequence, Tuple
 import numpy as np
 import torch
 
-from .engine import Engine, yuv420_frame_hw, yuv_format
+from .engine import YUV_FORMATS, Engine, yuv420_frame_hw, yuv_format
 
 
 class FramePool:
@@ -66,6 +66,108 @@ class _YuvBatch:
         self.hw = torch.tensor([[H, W]], dtype=torch.int32).expand(F, 2).contiguous().to(device)
 
 
+def _planes(x, what: str) -> list:
+    """2-D uint8 planes from a 3-D tensor [n, rows, cols] (one plane per item), a 2-D tensor (one item) or a sequence of 2-D tensors;
+    objects with ``__cuda_array_interface__`` (CuPy, Numba, decoder bindings) go through ``torch.as_tensor``, which shares their memory."""
+    def tensor(a):
+        return a if torch.is_tensor(a) else torch.as_tensor(a)
+    if torch.is_tensor(x) or hasattr(x, "__cuda_array_interface__"):
+        x = tensor(x)
+        if x.dim() == 2:
+            return [x]
+        if x.dim() != 3:
+            raise ValueError(f"{what}: expected a 2-D plane or a 3-D batch of planes, got shape {tuple(x.shape)}")
+        return list(x.unbind(0))
+    return [tensor(a) for a in x]
+
+
+class YuvSurfaces:
+    """n device-resident YUV 4:2:0 surfaces ("nv12" or "i420") of one picture size H x W, as a hardware decoder hands them out:
+    every plane is a strided 2-D uint8 CUDA tensor whose rows are ``stride(0)`` bytes apart (the surface pitch, >= the row width) and
+    whose columns are adjacent.  ``luma`` [H, W]; ``chroma`` NV12: the interleaved U V plane [H/2, W]; I420: the U plane [H/2, W/2],
+    with ``v`` the V plane [H/2, W/2] at the same pitch.  Each argument is a 3-D tensor [n, rows, cols], a sequence of 2-D planes or
+    one 2-D plane; planes may sit anywhere (padding bytes and padding surface rows are never read).
+
+    ``planes`` (int64 [n, 3] device addresses Y, U or UV, V), ``pitches`` (int32 [n, 2] luma, chroma) and ``hw`` (int32 [n, 2]) live on
+    the device; the object keeps the plane tensors alive.  The surfaces' contents may change between calls (a decoder reusing them):
+    what is read is what they hold when the conversion runs on the stream."""
+
+    def __init__(self, format: str, luma, chroma, v=None):
+        i420 = yuv_format(format) == YUV_FORMATS["i420"]
+        ys, us = _planes(luma, "luma"), _planes(chroma, "chroma")
+        if i420 and v is None:
+            raise ValueError("I420 surfaces need the V planes")
+        if not i420 and v is not None:
+            raise ValueError("NV12 surfaces have no separate V plane (the chroma plane interleaves U and V)")
+        vs = _planes(v, "v") if i420 else None
+        n = len(ys)
+        if n == 0 or len(us) != n or (vs is not None and len(vs) != n):
+            raise ValueError(f"{n} luma planes, {len(us)} chroma planes{'' if vs is None else f', {len(vs)} V planes'}: expected as many of each, at least one")
+        for p in ys + us + (vs or []):
+            if p.dtype != torch.uint8 or p.dim() != 2:
+                raise ValueError(f"YUV planes must be 2-D uint8 tensors (got {p.dtype}, shape {tuple(p.shape)})")
+        H, W = int(ys[0].shape[0]), int(ys[0].shape[1])
+        if H < 2 or W < 2 or H % 2 or W % 2:
+            raise ValueError(f"YUV 4:2:0 surfaces need an even H and W of at least 2 (got {H} x {W})")
+        cshape = (H // 2, W // 2) if i420 else (H // 2, W)
+
+        def check(p, shape, name):
+            if tuple(p.shape) != shape:
+                raise ValueError(f"{name} plane of shape {tuple(p.shape)}: expected {shape} for {format} surfaces of {H} x {W}")
+            if p.stride(1) != 1 or not shape[1] <= p.stride(0) < 2 ** 31:
+                raise ValueError(f"{name} plane with strides {p.stride()}: expected (pitch, 1) with {shape[1]} <= pitch < 2^31")
+
+        for k in range(n):
+            check(ys[k], (H, W), "luma")
+            check(us[k], cshape, "U" if i420 else "chroma")
+            if i420:
+                check(vs[k], cshape, "V")
+                if vs[k].stride(0) != us[k].stride(0):
+                    raise ValueError(f"I420 U and V planes must share one pitch (got {us[k].stride(0)} and {vs[k].stride(0)})")
+        devices = {p.device for p in ys + us + (vs or [])}
+        if len(devices) != 1 or next(iter(devices)).type != "cuda":
+            raise ValueError(f"YUV surfaces must be CUDA tensors on one device (got {sorted(map(str, devices))})")
+        self.format, self.n, self.H, self.W = format, n, H, W
+        self.device = next(iter(devices))
+        addr = [[ys[k].data_ptr(), us[k].data_ptr(), vs[k].data_ptr() if i420 else 0] for k in range(n)]
+        self.planes = torch.tensor(addr, dtype=torch.int64).to(self.device)
+        self.pitches = torch.tensor([[ys[k].stride(0), us[k].stride(0)] for k in range(n)], dtype=torch.int32).to(self.device)
+        self.hw = torch.tensor([[H, W]], dtype=torch.int32).expand(n, 2).contiguous().to(self.device)
+        self._keep = (ys, us, vs)
+
+    @classmethod
+    def from_frames(cls, frames, format: str, height: Optional[int] = None, surface_rows: Optional[int] = None) -> "YuvSurfaces":
+        """Surfaces from one uint8 CUDA tensor [n, rows, W] (or [rows, W] for one) whose rows are ``stride(-2)`` bytes apart (the pitch):
+        per frame the luma plane is rows [0, H), and the chroma starts at row ``surface_rows`` (default H; a decoder's padded surface
+        height, e.g. 1088 for 1080p).  NV12: chroma rows [S, S + H/2).  I420: the U plane at byte S * pitch with rows pitch/2 apart,
+        the V plane (S/2) * (pitch/2) bytes after it.  With the defaults and pitch W, a frame is laid out as cv2.cvtColor takes it,
+        (H*3/2) x W.  ``height`` defaults to rows * 2/3."""
+        yuv_format(format)
+        f = frames if torch.is_tensor(frames) else torch.as_tensor(frames)
+        if f.dim() == 2:
+            f = f.unsqueeze(0)
+        if f.dim() != 3 or f.dtype != torch.uint8 or f.stride(2) != 1:
+            raise ValueError("frames must be a uint8 tensor [n, rows, W] with adjacent columns")
+        n, R, W = (int(v) for v in f.shape)
+        H = R * 2 // 3 if height is None else int(height)
+        if height is None and R != H * 3 // 2:
+            raise ValueError(f"frames of {R} rows: give the picture height, or use the (H*3/2) x W layout")
+        S = H if surface_rows is None else int(surface_rows)
+        P = f.stride(1)
+        if H < 2 or H % 2 or S < H or S % 2:
+            raise ValueError(f"picture height {H} / surface rows {S}: expected even values with surface rows >= height")
+        if format == "nv12":
+            if S + H // 2 > R:
+                raise ValueError(f"NV12 frames of {R} rows cannot hold {S} surface rows + {H // 2} chroma rows")
+            return cls(format, f[:, :H], f[:, S:S + H // 2])
+        if P % 2 or S * P + (S // 2) * (P // 2) + (H // 2) * (P // 2) > R * P:
+            raise ValueError(f"I420 frames of {R} rows x pitch {P} cannot hold {S} surface rows and two chroma planes (pitch must be even)")
+        base = f.storage_offset() + S * P
+        u = f.as_strided((n, H // 2, W // 2), (f.stride(0), P // 2, 1), base)
+        v = f.as_strided((n, H // 2, W // 2), (f.stride(0), P // 2, 1), base + (S // 2) * (P // 2))
+        return cls(format, f[:, :H], u, v)
+
+
 class BatchedTracker:
     """``initialize(pool, frame_index, boxes)`` / ``track(pool, frame_index)`` for n tracks at once:
     the batched counterpart of ``Vit_dist.initialize`` / ``Vit_dist.track``."""
@@ -80,6 +182,9 @@ class BatchedTracker:
         self.n = 0
         self._hw = None
         self.out_boxes = torch.zeros((max_tracks, 5), dtype=torch.float64, device=self.device)
+        self.template_factor, self.search_factor = float(cfg.TEST.TEMPLATE_FACTOR), float(cfg.TEST.SEARCH_FACTOR)
+        self._yuv_rgb: Optional[torch.Tensor] = None             # initialize_yuv / track_yuv: one RGB frame per track
+        self._yuv_off: Optional[torch.Tensor] = None
 
     def initialize(self, pool: FramePool, frame_index: torch.Tensor, boxes) -> torch.Tensor:
         boxes = torch.as_tensor(boxes, dtype=torch.float64).reshape(-1, 4).to(self.device).contiguous()
@@ -108,6 +213,45 @@ class BatchedTracker:
         r = self.engine.tracks_step(frames, offsets, self._hw, first=0, n=self.n, out_boxes=out,
                                     update_state=update_state, detail=detail)
         return r
+
+    def _yuv_frames(self, surfaces: YuvSurfaces) -> Tuple[torch.Tensor, torch.Tensor]:
+        if surfaces.n > self.max_tracks:
+            raise ValueError(f"{surfaces.n} surfaces > max_tracks {self.max_tracks}")
+        if surfaces.device != self.device:
+            raise ValueError(f"surfaces on {surfaces.device}, tracker on {self.device}")
+        if self._yuv_rgb is None or tuple(self._yuv_rgb.shape[1:3]) != (surfaces.H, surfaces.W):
+            self._yuv_rgb = None
+            # zero-filled once: the crop kernels read the first pixels of a row with weight 0 for taps in the padding
+            self._yuv_rgb = torch.zeros((self.max_tracks, surfaces.H, surfaces.W, 3), dtype=torch.uint8, device=self.device)
+            self._yuv_off = torch.arange(self.max_tracks, dtype=torch.int64, device=self.device) * (surfaces.H * surfaces.W * 3)
+        return self._yuv_rgb, self._yuv_off[: surfaces.n]
+
+    def initialize_yuv(self, surfaces: YuvSurfaces, boxes) -> torch.Tensor:
+        """``initialize`` for tracks 0..n-1 from device-resident YUV surfaces (``YuvSurfaces``, track i on surface i): only the rectangle
+        each template crop reads is converted (vt_yuv420_crop_to_rgb, bit for bit cv2.cvtColor), into an RGB frame per track that
+        this tracker owns, then vt_tracks_init runs on it on the same stream.  Those frames cost max_tracks x H x W x 3 bytes of
+        device memory (2.76 MB per track at 720p, 6.2 MB at 1080p), allocated at the first call for a picture size."""
+        boxes = torch.as_tensor(boxes, dtype=torch.float64).reshape(-1, 4).to(self.device).contiguous()
+        if boxes.shape[0] != surfaces.n:
+            raise ValueError(f"{boxes.shape[0]} boxes for {surfaces.n} surfaces")
+        frames, offs = self._yuv_frames(surfaces)
+        self.engine.yuv420_crop_to_rgb(surfaces.format, surfaces.planes, surfaces.pitches, surfaces.hw, frames, offs,
+                                       self.template_factor, boxes=boxes)
+        self.n = surfaces.n
+        self._hw = surfaces.hw
+        return self.engine.tracks_init(frames, offs, self._hw, boxes, first=0)
+
+    def track_yuv(self, surfaces: YuvSurfaces, update_state: bool = True, detail: bool = False):
+        """``track`` from device-resident YUV surfaces (surface i for track i): the rectangle each search crop reads is computed on the
+        device from the track's current state - the host never waits for it - and converted; then vt_tracks_step runs on the same
+        stream.  No allocation after the first call for a picture size, so a step can be captured in a CUDA graph."""
+        if surfaces.n != self.n:
+            raise ValueError(f"{surfaces.n} surfaces for {self.n} tracks")
+        frames, offs = self._yuv_frames(surfaces)
+        self.engine.yuv420_crop_to_rgb(surfaces.format, surfaces.planes, surfaces.pitches, surfaces.hw, frames, offs,
+                                       self.search_factor, boxes=None, first=0)
+        self._hw = surfaces.hw
+        return self.track_offsets(frames, offs, update_state=update_state, detail=detail)
 
 
 class PipelinedFrameFeeder:

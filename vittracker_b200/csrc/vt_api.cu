@@ -912,6 +912,26 @@ int vt_yuv420_to_rgb(VtHandle h, int32_t format, const uint8_t* src, const int64
     return VT_OK;
 }
 
+int vt_yuv420_crop_to_rgb(VtHandle h, int32_t format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw,
+                          const double* boxes_xywh, double factor, int32_t first, int32_t n, uint8_t* dst, const int64_t* dst_offsets,
+                          void* stream) {
+    if (!h) return VT_ERR_INVALID_ARG;
+    if (format != VT_FRAME_NV12 && format != VT_FRAME_I420) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: unknown format %d", format);
+    if (n < 0) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: negative n");
+    if (n == 0) return VT_OK;
+    if (!planes || !pitches || !frame_hw || !dst || !dst_offsets) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: null pointer");
+    if (!(factor > 0)) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: factor must be positive");
+    if (!boxes_xywh && (first < 0 || first + n > h->cfg.max_tracks))
+        return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: tracks [%d, %d) exceed max_tracks %d", first, first + n, h->cfg.max_tracks);
+    DeviceGuard dg(h->cfg.device);
+    VT_CUDA(h, dg.err);
+    const double* boxes = boxes_xywh ? boxes_xywh : h->d_state + (size_t)first * 4;
+    const int k = launch_yuv420_crop_to_rgb(format, planes, pitches, frame_hw, boxes, factor, dst, dst_offsets, n, h->num_sms, (cudaStream_t)stream);
+    if (k < 0) return fail(h, VT_ERR_CUDA, "vt_yuv420_crop_to_rgb: kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    h->launches += k;
+    return VT_OK;
+}
+
 int64_t vt_launch_count(VtHandle h) { return h ? h->launches : 0; }
 
 int vt_profile_enable(VtHandle h, int32_t enable) {

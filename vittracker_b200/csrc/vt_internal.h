@@ -243,6 +243,11 @@ struct YuvDesc {
 int launch_yuv420_to_rgb(int format, const uint8_t* src, const int64_t* src_offsets, const int32_t* frame_hw, uint8_t* dst,
                          const int64_t* dst_offsets, int n, int num_sms, cudaStream_t st);
 int launch_yuv420_rect(int format, const YuvDesc& d, int num_sms, cudaStream_t st);
+// Per item, only the even-widened rectangle the crop of boxes[i] (factor) reads, from pitched planes (planes [n][3] device addresses
+// Y, U or UV, V; pitches [n][2] luma, chroma) into the H x W x 3 frame at dst + dst_offsets[i]; degenerate crops, odd or tiny sizes
+// and pitches below the row width are skipped.
+int launch_yuv420_crop_to_rgb(int format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw, const double* boxes,
+                              double factor, uint8_t* dst, const int64_t* dst_offsets, int n, int num_sms, cudaStream_t st);
 
 int launch_crop_normalize(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
                           const double* boxes, double factor, int S, int n, const float* lut,

@@ -7,11 +7,14 @@
 // and every 2x2 luma block uses its one chroma sample (no interpolation).  Every term fits in int32.
 //
 // It writes the RGB frames the tracking kernels read; they are unchanged.  Bound: HBM, 1.5 bytes read and 3 written per pixel.
+// Three callers: whole contiguous frames, one packed rectangle (the host upload), and per item only the rectangle its crop reads, from
+// pitched planes (decoder surfaces), with the rectangle computed on the device from the box (yuv420_crop_to_rgb_kernel).
 //
 // One work unit = one chroma row (two luma rows) x kSegPx columns of one item; a thread converts a run of two 2x2 blocks (one
 // chroma load feeds four pixels).  Sources and destinations may sit at any byte offset: loads are aligned words joined with a
 // funnel shift (only words that hold a wanted byte are read), and each output row segment is assembled in shared memory and
 // written as aligned words plus single head / tail bytes, so no byte outside the item is touched.
+#include "vt_geom.cuh"
 #include "vt_internal.h"
 
 namespace vt {
@@ -57,12 +60,47 @@ __device__ __forceinline__ bool make_desc(const YuvBatch& b, const YuvDesc& one,
     return true;
 }
 
+// The rectangle of a crop (vt_yuv420_crop_to_rgb): the box's crop geometry, computed by the code the crop kernels run, gives rows
+// [max(0, y1), min(H, y1 + crop_sz)) x columns [max(0, x1 - 1), min(W, x1 + crop_sz + 1)) (sequences.py crop_rect), widened to even
+// bounds (tracker.py even_rect); the descriptor addresses it inside the item's own planes and RGB frame.  False: nothing to write
+// (degenerate crop, odd or tiny frame, a pitch below its row's width).
+struct YuvCropBatch {
+    const uint64_t* planes;                               // [n][3] Y, U (NV12: UV), V
+    const int32_t* pitches;                               // [n][2] luma, chroma
+    const int32_t* hw;
+    const double* boxes;                                  // [n][4]
+    double factor;
+    uint8_t* dst;
+    const int64_t* dst_off;
+};
+
 template <int Layout>
-__global__ void __launch_bounds__(kYuvThreads)
-yuv420_to_rgb_kernel(YuvBatch b, YuvDesc one) {
-    __shared__ uint32_t s_row[2][kRowWords];
-    YuvDesc d;
-    if (!make_desc<Layout>(b, one, blockIdx.y, d)) return;
+__device__ __forceinline__ bool make_crop_desc(const YuvCropBatch& b, int item, YuvDesc& d) {
+    const int H = b.hw[2 * item], W = b.hw[2 * item + 1];
+    const int yp = b.pitches[2 * item], cp = b.pitches[2 * item + 1];
+    if (H < 2 || W < 2 || (H & 1) || (W & 1) || yp < W || cp < (Layout == kYuvI420 ? W / 2 : W)) return false;
+    const double* bx = b.boxes + 4 * item;
+    const CropGeom g = crop_geometry(bx[0], bx[1], bx[2], bx[3], b.factor, 1, H, W);
+    if (g.status != 0) return false;
+    const long long y0 = max(0, g.y1), y1 = min((long long)H, (long long)g.y1 + g.crop_sz);
+    const long long x0 = max(0, g.x1 - 1), x1 = min((long long)W, (long long)g.x1 + g.crop_sz + 1);
+    if (y1 <= y0 || x1 <= x0) return false;
+    const int ya = (int)y0 & ~1, yb = min(H, (int)(y1 + 1) & ~1), xa = (int)x0 & ~1, xb = min(W, (int)(x1 + 1) & ~1);
+    const uint64_t* p = b.planes + 3 * item;
+    d.y = reinterpret_cast<const uint8_t*>(p[0]) + (int64_t)ya * yp + xa;
+    d.u = reinterpret_cast<const uint8_t*>(p[1]) + (int64_t)(ya / 2) * cp + (Layout == kYuvI420 ? xa / 2 : xa);
+    d.v = Layout == kYuvI420 ? reinterpret_cast<const uint8_t*>(p[2]) + (int64_t)(ya / 2) * cp + xa / 2 : d.u;
+    d.dst = b.dst + b.dst_off[item] + ((int64_t)ya * W + xa) * 3;
+    d.y_pitch = yp;
+    d.c_pitch = cp;
+    d.dst_pitch = (int64_t)W * 3;
+    d.w = xb - xa; d.h = yb - ya;
+    return true;
+}
+
+// The CTA's share of the item d (units blockIdx.x, blockIdx.x + gridDim.x, ...); no byte outside d's rectangle is written.
+template <int Layout>
+__device__ __forceinline__ void convert_units(const YuvDesc& d, uint32_t (&s_row)[2][kRowWords]) {
     const int t = threadIdx.x;
     const int nseg = (d.w + kSegPx - 1) / kSegPx;
     const int units = (d.h / 2) * nseg;
@@ -132,6 +170,25 @@ yuv420_to_rgb_kernel(YuvBatch b, YuvDesc one) {
     }
 }
 
+template <int Layout>
+__global__ void __launch_bounds__(kYuvThreads)
+yuv420_to_rgb_kernel(YuvBatch b, YuvDesc one) {
+    __shared__ uint32_t s_row[2][kRowWords];
+    YuvDesc d;
+    if (!make_desc<Layout>(b, one, blockIdx.y, d)) return;
+    convert_units<Layout>(d, s_row);
+}
+
+// CTAs of an item whose rectangle has fewer units than blockIdx.x exit at once.
+template <int Layout>
+__global__ void __launch_bounds__(kYuvThreads)
+yuv420_crop_to_rgb_kernel(YuvCropBatch b) {
+    __shared__ uint32_t s_row[2][kRowWords];
+    YuvDesc d;
+    if (!make_crop_desc<Layout>(b, blockIdx.y, d)) return;
+    convert_units<Layout>(d, s_row);
+}
+
 namespace {
 
 int launch(int format, const YuvBatch& b, const YuvDesc& one, dim3 grid, cudaStream_t st) {
@@ -165,6 +222,27 @@ int launch_yuv420_rect(int format, const YuvDesc& d, int num_sms, cudaStream_t s
     if (units <= 0) return 0;
     const YuvBatch b{nullptr, nullptr, nullptr, nullptr, nullptr};
     return launch(format, b, d, dim3(min(units, num_sms * 32), 1), st);
+}
+
+int launch_yuv420_crop_to_rgb(int format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw, const double* boxes,
+                              double factor, uint8_t* dst, const int64_t* dst_offsets, int n, int num_sms, cudaStream_t st) {
+    if (n <= 0) return 0;
+    // the rectangles are known on the device only: a fixed number of CTAs per item, as for whole frames, sized for a search crop
+    // (a 400 x 402 rectangle of a 100 x 100 box is ~400 units)
+    const int per_item = max(1, min(256, num_sms * 32 * 2 / min(n, 32768)));
+    int launched = 0;
+    for (int first = 0; first < n; first += 32768) {
+        const int m = min(32768, n - first);
+        const YuvCropBatch b{planes + 3 * first, pitches + 2 * first, frame_hw + 2 * first, boxes + 4 * first, factor, dst,
+                             dst_offsets + first};
+        const dim3 grid(per_item, m);
+        if (format == kYuvNV12) yuv420_crop_to_rgb_kernel<kYuvNV12><<<grid, kYuvThreads, 0, st>>>(b);
+        else if (format == kYuvI420) yuv420_crop_to_rgb_kernel<kYuvI420><<<grid, kYuvThreads, 0, st>>>(b);
+        else return -1;
+        if (cudaPeekAtLastError() != cudaSuccess) return -1;
+        ++launched;
+    }
+    return launched;
 }
 
 }  // namespace vt

@@ -220,6 +220,25 @@ class Engine:
             self._check(self.lib.vt_upload_yuv420_rect(self.handle, fmt, image.ctypes.data, H, W, int(y0), int(y1), int(x0), int(x1),
                                                        _ptr(staging), _ptr(staging_dev), _ptr(frame_rgb), self._stream()))
 
+    def yuv420_crop_to_rgb(self, format: str, planes: torch.Tensor, pitches: torch.Tensor, frame_hw: torch.Tensor, dst: torch.Tensor,
+                           dst_offsets: torch.Tensor, factor: float, boxes: Optional[torch.Tensor] = None, first: int = 0) -> torch.Tensor:
+        """vt_yuv420_crop_to_rgb: per item, only the even-widened rectangle the crop of its box (``boxes`` float64 [n, 4], or None: the
+        state of tracks [first, first + n)) reads, from pitched planes (``planes`` int64 [n, 3] device addresses Y, U or UV, V;
+        ``pitches`` int32 [n, 2]) into the H x W x 3 frame at byte ``dst_offsets[i]`` of ``dst``, bit for bit cv2.cvtColor.  No
+        allocation and no synchronisation (capturable in a CUDA graph).  Returns ``dst``."""
+        fmt = yuv_format(format)
+        n = int(planes.shape[0])
+        want = [(planes, torch.int64, (n, 3)), (pitches, torch.int32, (n, 2)), (frame_hw, torch.int32, (n, 2)), (dst_offsets, torch.int64, (n,))]
+        if boxes is not None:
+            want.append((boxes, torch.float64, (n, 4)))
+        for t, dt, shape in want + [(dst, torch.uint8, tuple(dst.shape))]:
+            if t.dtype != dt or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape:
+                raise ValueError(f"yuv420_crop_to_rgb: expected a contiguous {dt} tensor of shape {shape} on {self.device}")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_yuv420_crop_to_rgb(self.handle, fmt, _ptr(planes), _ptr(pitches), _ptr(frame_hw), _ptr(boxes),
+                                                       float(factor), int(first), n, _ptr(dst), _ptr(dst_offsets), self._stream()))
+        return dst
+
     # ------------------------------------------------------------------------------------------
     def tracks_init(self, frames, frame_offsets, frame_hw, boxes, first: int = 0) -> torch.Tensor:
         n = boxes.shape[0]

@@ -14,6 +14,7 @@ from typing import Optional
 import numpy as np
 import torch
 
+from .batched import YuvSurfaces
 from .engine import yuv420_frame_hw, yuv_format
 from .model import build_ostrack_dist
 from .sequences import crop_rect
@@ -97,7 +98,9 @@ class Vit_dist(BaseTracker):
         self._out_detail = self._out_dev[5:].view(1, 8)
         self._graph, self._graph_key = None, None
         # params.frame_format: "rgb" (H x W x 3, the reference's input) or a YUV 4:2:0 layout as decoders hand it out, "nv12" or
-        # "i420" ((H*3/2) x W, as cv2.cvtColor takes it), converted on the device bit for bit as cv2.cvtColor(COLOR_YUV2RGB_*) would
+        # "i420" ((H*3/2) x W, as cv2.cvtColor takes it), converted on the device bit for bit as cv2.cvtColor(COLOR_YUV2RGB_*) would.
+        # A YUV frame may also be on the device already (decoder output): a CUDA tensor (H*3/2) x W with any row pitch, or a
+        # (luma, chroma[, v]) tuple of strided CUDA planes (see batched.YuvSurfaces); only the crop's rectangle is converted.
         self.frame_format = getattr(params, "frame_format", "rgb")
         if self.frame_format != "rgb":
             yuv_format(self.frame_format)
@@ -110,18 +113,36 @@ class Vit_dist(BaseTracker):
         if self._dev.type == "cuda":
             torch.cuda.current_stream(self._dev).synchronize()
 
-    def _upload(self, image: np.ndarray, box, factor: float):
+    def _surfaces(self, image) -> YuvSurfaces:
+        """A YUV frame already on the device: one CUDA tensor (H*3/2) x W with any row pitch, or a (luma, chroma[, v]) tuple of planes."""
+        if torch.is_tensor(image):
+            if not image.is_cuda:
+                raise ValueError(f"a {self.frame_format} frame tensor must be on the device (host frames are numpy arrays)")
+            s = YuvSurfaces.from_frames(image, self.frame_format)
+        else:
+            s = YuvSurfaces(self.frame_format, *image)
+        if s.n != 1 or s.device != self._dev:
+            raise ValueError(f"expected one {self.frame_format} frame on {self._dev}")
+        return s
+
+    def _upload(self, image, box, factor: float):
         """Stage the rows of ``image`` the crop will read into the device frame buffer (as RGB, whatever the frame format)."""
         yuv = self.frame_format != "rgb"
+        surfaces = None
         if yuv:
-            if not isinstance(image, np.ndarray):
-                raise ValueError(f"image must be a ({self.frame_format}) numpy array")
-            H, W = yuv420_frame_hw(image)
+            if isinstance(image, np.ndarray):
+                H, W = yuv420_frame_hw(image)
+            elif torch.is_tensor(image) or isinstance(image, (tuple, list)):
+                surfaces = self._surfaces(image)
+                H, W = surfaces.H, surfaces.W
+            else:
+                raise ValueError(f"image must be a ({self.frame_format}) numpy array, a CUDA tensor or a tuple of CUDA planes")
         else:
             if image.dtype != np.uint8 or image.ndim != 3 or image.shape[2] != 3:
                 raise ValueError("image must be HxWx3 uint8")
             H, W, _ = image.shape
-        image = np.ascontiguousarray(image)
+        if surfaces is None:
+            image = np.ascontiguousarray(image)
         if (H, W) != self._hw:
             # zero-filled: the crop kernels read the first pixels of a row with weight 0 for taps in the padding
             self._frame_dev = torch.zeros((H * W * 3,), dtype=torch.uint8, device=self._dev)
@@ -138,7 +159,14 @@ class Vit_dist(BaseTracker):
         if rect is None:
             raise ValueError("crop lies outside the image (undefined in the reference)")
         ya, yb, xa, xb = rect
-        if yuv:
+        if surfaces is not None:
+            # the frame is on the device already: the same rectangle is computed there from the device box and converted from the
+            # surface's planes (vt_yuv420_crop_to_rgb); nothing crosses the link but the box
+            self._set_box(box)
+            self.engine.yuv420_crop_to_rgb(self.frame_format, surfaces.planes, surfaces.pitches, surfaces.hw, self._frame_dev, self._off_dev,
+                                           factor, boxes=self._box_dev)
+            self._last_surfaces = surfaces                      # its address arrays stay alive while the conversion is queued
+        elif yuv:
             # the even-widened rectangle (a superset of crop_rect) crosses the link as YUV and is converted into the RGB frame
             ya, yb, xa, xb = even_rect(rect, H, W)
             self.engine.upload_yuv420_rect(self.frame_format, image, ya, yb, xa, xb, self._frame_pin, self._frame_stage, self._frame_dev)
