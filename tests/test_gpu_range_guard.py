@@ -27,7 +27,8 @@ def _scaled(sd, key, factor, rows=None):
 CASES = [
     ("stem conv1 output", "patch_embed.net.0.c.weight", 1e5, None),
     ("stem conv3 output", "patch_embed.net.4.c.weight", 1e6, None),
-    ("attention keys", "blocks.0.attn.qkv.weight", 3e5, (48, 96)),
+    # q and k rows together: scaling k alone (or q alone) only moves scale between them, which weight ingest rebalances away
+    ("attention queries and keys", "blocks.0.attn.qkv.weight", 3e5, (0, 96)),
     ("attention values", "blocks.1.attn.qkv.weight", 1e6, (96, 144)),
     ("MLP hidden (GELU output)", "blocks.2.mlp.fc1.weight", 1e6, None),
     ("head conv1 output", "box_head.conv1_ctr.0.weight", 1e7, None),

@@ -1,5 +1,5 @@
-// C-ABI layer of libvittrack_b200.so: handle, weight ingestion (BN folding into the fp32 layouts; each tensor-core weight blob is packed
-// by the file of the kernel that reads it),
+// C-ABI layer of libvittrack_b200.so: handle, weight ingestion (power-of-two rebalancing of scale between layers, BN folding into the
+// fp32 layouts; each tensor-core weight blob is packed by the file of the kernel that reads it),
 // workspace, and the entry points declared in include/vittrack_b200.h.
 #include <math.h>
 #include <stdarg.h>
@@ -25,13 +25,14 @@ struct HostTensor {
     std::vector<float> data;
     std::vector<int64_t> shape;
 };
+using TensorMap = std::map<std::string, HostTensor>;
 
 }  // namespace
 
 struct VtContext {
     VtConfig cfg;
     std::string err;
-    std::map<std::string, HostTensor> tensors;
+    TensorMap tensors;
     bool finalized = false;
     bool tracks_ready = false;
     int64_t launches = 0;
@@ -137,13 +138,13 @@ int check_missing(VtHandle h) {
     return missing.empty() ? VT_OK : fail(h, VT_ERR_WEIGHTS, "missing tensors: %s", missing.c_str());
 }
 
-const float* tensor(VtHandle h, const std::string& name) { return h->tensors.at(name).data.data(); }
+const float* tensor(const TensorMap& ts, const std::string& name) { return ts.at(name).data.data(); }
 
-BlockTensors block_tensors(VtHandle h, int b) {
+BlockTensors block_tensors(const TensorMap& ts, int b) {
     const std::string p = "blocks." + std::to_string(b) + ".";
-    return {tensor(h, p + "norm1.weight"), tensor(h, p + "norm1.bias"), tensor(h, p + "attn.qkv.weight"), tensor(h, p + "attn.qkv.bias"),
-            tensor(h, p + "attn.proj.weight"), tensor(h, p + "attn.proj.bias"), tensor(h, p + "norm2.weight"), tensor(h, p + "norm2.bias"),
-            tensor(h, p + "mlp.fc1.weight"), tensor(h, p + "mlp.fc1.bias"), tensor(h, p + "mlp.fc2.weight"), tensor(h, p + "mlp.fc2.bias")};
+    return {tensor(ts, p + "norm1.weight"), tensor(ts, p + "norm1.bias"), tensor(ts, p + "attn.qkv.weight"), tensor(ts, p + "attn.qkv.bias"),
+            tensor(ts, p + "attn.proj.weight"), tensor(ts, p + "attn.proj.bias"), tensor(ts, p + "norm2.weight"), tensor(ts, p + "norm2.bias"),
+            tensor(ts, p + "mlp.fc1.weight"), tensor(ts, p + "mlp.fc1.bias"), tensor(ts, p + "mlp.fc2.weight"), tensor(ts, p + "mlp.fc2.bias")};
 }
 
 // Conv2d (with its bias when `conv_bias`) and BatchNorm2d (eval) folded in float64 (Conv2d_BN.fuse vit_dist.py:22-33; head conv + bias
@@ -152,10 +153,10 @@ struct FoldedConv {
     int co, ci;
     std::vector<float> w, b;
 };
-FoldedConv fold_conv_bn(VtHandle h, const std::string& conv, const std::string& bn, bool conv_bias) {
-    const HostTensor& wt = h->tensors.at(conv + "weight");
-    const float *w = wt.data.data(), *cb = conv_bias ? tensor(h, conv + "bias") : nullptr;
-    const float *g = tensor(h, bn + "weight"), *b = tensor(h, bn + "bias"), *m = tensor(h, bn + "running_mean"), *v = tensor(h, bn + "running_var");
+FoldedConv fold_conv_bn(const TensorMap& ts, const std::string& conv, const std::string& bn, bool conv_bias) {
+    const HostTensor& wt = ts.at(conv + "weight");
+    const float *w = wt.data.data(), *cb = conv_bias ? tensor(ts, conv + "bias") : nullptr;
+    const float *g = tensor(ts, bn + "weight"), *b = tensor(ts, bn + "bias"), *m = tensor(ts, bn + "running_mean"), *v = tensor(ts, bn + "running_var");
     FoldedConv f{(int)wt.shape[0], (int)wt.shape[1], std::vector<float>(wt.data.size()), std::vector<float>(wt.shape[0])};
     const size_t kn = wt.data.size() / f.co;                                  // ci * 9 weights per output channel
     for (int co = 0; co < f.co; ++co) {
@@ -164,6 +165,67 @@ FoldedConv fold_conv_bn(VtHandle h, const std::string& conv, const std::string& 
         for (size_t k = 0; k < kn; ++k) f.w[co * kn + k] = (float)((double)w[co * kn + k] * s);
     }
     return f;
+}
+
+// Nearest integer to log2(v / unit), as v's exponent plus a function of its mantissa alone: octave(v * 2^k, unit) == octave(v, unit) + k
+// exactly.  0 for a v that is zero or not finite.
+int octave(double v, double unit) {
+    if (!(v > 0.0) || !std::isfinite(v)) return 0;
+    int e = 0;
+    const double m = frexp(v, &e);
+    return e + (int)lround(log2(m / unit));
+}
+
+// Power-of-two rebalancing of the model's scale, on the copy of the tensors that finalisation packs.  A checkpoint may split scale freely
+// between a LayerNorm or BatchNorm affine and the next layer's weights, between the q and k rows of a block's qkv, or between its v rows
+// and the output projection: the model is the same, but the tensor-core paths split each operand into fp16 hi + lo, which keeps its
+// ~22 bits only while both halves are normal fp16 numbers.  Each producer -> consumer pair below moves 2^-p onto the factor its statistic
+// reads and 2^p onto the other, p = octave(statistic): the operands come out near the magnitudes of a random-init model whatever the
+// checkpoint's split.  Properties that the tests rely on (tests/test_scale_invariance.py):
+// - multiplying by a power of two is exact, and so is the rewrite as a whole: the fp32 layers keep their bits, and no kernel changes;
+// - scaling a pair's factors by 2^-k and 2^k shifts its p by exactly k, so the packed weights are the same bits.  For that, each
+//   statistic reads only tensors that no other pair rescales (qkv.weight is shared by three pairs: the q / k statistic is a ratio of
+//   its rows, which ln1's uniform scale leaves alone);
+// - p = 0 for random-init weights, so such a model packs exactly the tensors it was handed.
+// Returns the final LayerNorm's p: its output, the tokens_norm tap, is scaled back by 2^p.
+int rebalance(const VtConfig& c, TensorMap& ts) {
+    const size_t C = c.embed_dim;
+    auto amax = [&](const std::string& name, size_t first = 0, size_t count = 0) {
+        const std::vector<float>& d = ts.at(name).data;
+        double m = 0.0;
+        for (size_t i = first, end = count ? first + count : d.size(); i < end; ++i) m = fmax(m, fabs((double)d[i]));
+        return m;
+    };
+    auto scale = [&](const std::string& name, int p, size_t first = 0, size_t count = 0) {
+        std::vector<float>& d = ts.at(name).data;
+        for (size_t i = first, end = count ? first + count : d.size(); i < end; ++i) d[i] = ldexpf(d[i], p);
+    };
+    // a LayerNorm / BatchNorm affine (weight and bias): its output is about as large as the larger of the two
+    auto affine_to = [&](const std::string& norm, const std::vector<std::string>& consumers) {
+        const int p = octave(fmax(amax(norm + "weight"), amax(norm + "bias")), 1.0);
+        scale(norm + "weight", -p);
+        scale(norm + "bias", -p);
+        for (const std::string& w : consumers) scale(w, p);
+        return p;
+    };
+    for (int b = 0; b < c.depth; ++b) {
+        const std::string p = "blocks." + std::to_string(b) + ".", qkv = p + "attn.qkv.";
+        const int pqk = octave(sqrt(amax(qkv + "weight", 0, C * C) / amax(qkv + "weight", C * C, C * C)), 1.0);
+        const int pv = octave(amax(p + "attn.proj.weight"), 1.0 / sqrt((double)C));     // random-init Linear weights: |w| < C^-1/2
+        affine_to(p + "norm1.", {qkv + "weight"});
+        affine_to(p + "norm2.", {p + "mlp.fc1.weight"});
+        scale(qkv + "weight", -pqk, 0, C * C);   scale(qkv + "bias", -pqk, 0, C);
+        scale(qkv + "weight", pqk, C * C, C * C); scale(qkv + "bias", pqk, C, C);
+        scale(qkv + "weight", pv, 2 * C * C, C * C); scale(qkv + "bias", pv, 2 * C, C);
+        scale(p + "attn.proj.weight", -pv);
+    }
+    std::vector<std::string> conv1;
+    for (int t = 0; t < 3; ++t) conv1.push_back(head_prefix(0, t) + "0.weight");
+    const int pnorm = affine_to("norm.", conv1);
+    for (int t = 0; t < 3; ++t)
+        for (int i = 0; i < 4; ++i)
+            affine_to(head_prefix(i, t) + "1.", {i < 3 ? head_prefix(i + 1, t) + "0.weight" : std::string("box_head.conv5_") + kTowers[t] + ".weight"});
+    return pnorm;
 }
 
 // The packed weights: one fp32 buffer of 16-byte aligned slots.  slot() allocates one for the ModelW / GenModelW member that will
@@ -287,9 +349,9 @@ HeadArgs track_head_args(VtHandle h, int first, int c0, int m, const int32_t* fr
 }
 
 // Hann window (hann.py:6-16; the tracker's own tensor when it was handed over) and normalisation table (data_utils.py:8-14)
-void fill_hann_and_lut(VtHandle h, float* hann, float* lut) {
-    auto it = h->tensors.find("tracker.output_window");
-    if (it != h->tensors.end()) {
+void fill_hann_and_lut(const TensorMap& ts, float* hann, float* lut) {
+    auto it = ts.find("tracker.output_window");
+    if (it != ts.end()) {
         memcpy(hann, it->second.data.data(), 256 * sizeof(float));
     } else {
         float w1[16];
@@ -309,9 +371,10 @@ void fill_hann_and_lut(VtHandle h, float* hann, float* lut) {
 }
 
 // Weights of the generic path: the reference's own layouts ([out][in]; conv [cout][ky][kx][cin]) with BatchNorm(eval) folded.
-int finalize_generic(VtHandle h, cudaStream_t st) {
+int finalize_generic(VtHandle h, const TensorMap& ts, int pnorm, cudaStream_t st) {
     const int C = h->cfg.embed_dim, hc = h->cfg.head_channels, hid = h->cfg.mlp_ratio * C;
     GenModelW& g = h->gw;
+    g.norm_tap_scale = ldexpf(1.f, pnorm);
     Packer pk;
     // split images of the folded convolutions whose K = 9 cin is a whole number of 32-wide panels, packed after the fp32 weights
     struct ConvImg { const uint8_t** img; size_t w; int co, ci; };
@@ -325,13 +388,13 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
         }
     };
     for (int l = 0; l < 4; ++l) {
-        const FoldedConv f = fold_conv_bn(h, stem_prefix(l) + "c.", stem_prefix(l) + "bn.", false);
+        const FoldedConv f = fold_conv_bn(ts, stem_prefix(l) + "c.", stem_prefix(l) + "bn.", false);
         const size_t ow = pk.slot(g.stem_w[l], f.w.size()), ob = pk.slot(g.stem_b[l], f.co);
         conv_rows(f, ow, ob);
         want_img(g.istem_w[l], ow, f.co, f.ci);
     }
     for (int b = 0; b < h->cfg.depth; ++b) {
-        const BlockTensors t = block_tensors(h, b);
+        const BlockTensors t = block_tensors(ts, b);
         GenBlockW& B = g.blk[b];
         pk.put(B.ln1g, t.ln1_g, C); pk.put(B.ln1b, t.ln1_b, C);
         pk.put(B.wqkv, t.wqkv, (size_t)3 * C * C); pk.put(B.bqkv, t.bqkv, (size_t)3 * C);
@@ -342,7 +405,7 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
     }
     // split images of the blocks' Linear weights for the bulk-copy GEMM (same bytes as the fp32 matrices)
     for (int b = 0; b < h->cfg.depth && g.use_img; ++b) {
-        const BlockTensors t = block_tensors(h, b);
+        const BlockTensors t = block_tensors(ts, b);
         GenBlockW& B = g.blk[b];
         const struct { const uint8_t*& img; const float* w; int n, k; } lin[4] = {
             {B.iwqkv, t.wqkv, 3 * C, C}, {B.iwproj, t.wproj, C, C}, {B.iwfc1, t.wfc1, hid, C}, {B.iwfc2, t.wfc2, C, hid}};
@@ -351,14 +414,14 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
             gen_pack_weight_image(L.w, L.n, L.k, pk.bytes(o));
         }
     }
-    pk.put(g.norm_g, tensor(h, "norm.weight"), C); pk.put(g.norm_b, tensor(h, "norm.bias"), C);
-    pk.put(g.pos_z, tensor(h, "pos_embed_z"), (size_t)kNz * C); pk.put(g.pos_x, tensor(h, "pos_embed_x"), (size_t)kNx * C);
+    pk.put(g.norm_g, tensor(ts, "norm.weight"), C); pk.put(g.norm_b, tensor(ts, "norm.bias"), C);
+    pk.put(g.pos_z, tensor(ts, "pos_embed_z"), (size_t)kNz * C); pk.put(g.pos_x, tensor(ts, "pos_embed_x"), (size_t)kNx * C);
     // head: layer 1 merged over the towers (ctr | offset | size), layers 2-4 per tower, conv5 rows ctr, off x, off y, size w, size h
     const size_t w1 = pk.slot(g.head_w1, (size_t)3 * hc * 9 * C), b1 = pk.slot(g.head_b1, (size_t)3 * hc);
     want_img(g.ihead_w1, w1, 3 * hc, C);
     for (int t = 0; t < 3; ++t)
         for (int i = 0; i < 4; ++i) {
-            const FoldedConv f = fold_conv_bn(h, head_prefix(i, t) + "0.", head_prefix(i, t) + "1.", true);
+            const FoldedConv f = fold_conv_bn(ts, head_prefix(i, t) + "0.", head_prefix(i, t) + "1.", true);
             if (i == 0) {      // the merged layer's rows of this tower (the tower's own layer-1 slot is not read)
                 const size_t ow = pk.alloc(f.w.size()), ob = pk.alloc(f.co);
                 conv_rows(f, ow, ob);
@@ -373,14 +436,14 @@ int finalize_generic(VtHandle h, cudaStream_t st) {
     const size_t w5 = pk.slot(g.head_w5, (size_t)5 * c5), b5 = pk.slot(g.head_b5, 5);
     for (int t = 0; t < 3; ++t) {
         const std::string p = std::string("box_head.conv5_") + kTowers[t] + ".";
-        const float *w = tensor(h, p + "weight"), *b = tensor(h, p + "bias");
+        const float *w = tensor(ts, p + "weight"), *b = tensor(ts, p + "bias");
         for (int o = 0; o < outs[t]; ++o) {
             pk.buf[b5 + row0[t] + o] = b[o];
             for (int k = 0; k < c5; ++k) pk.buf[w5 + (size_t)(row0[t] + o) * c5 + k] = w[(size_t)o * c5 + k];
         }
     }
     const size_t hann = pk.slot(g.hann, 256), lut = pk.slot(h->mw.lut, 768);         // the crop kernel reads the table through ModelW
-    fill_hann_and_lut(h, &pk.buf[hann], &pk.buf[lut]);
+    fill_hann_and_lut(ts, &pk.buf[hann], &pk.buf[lut]);
     for (const ConvImg& c : imgs) {
         const size_t o = pk.slot(*c.img, gen_img_bytes(c.co, 9 * c.ci) / 4);       // (allocating moves pk.buf: index, hold no pointer)
         gen_pack_weight_image(&pk.buf[c.w], c.co, 9 * c.ci, pk.bytes(o));
@@ -568,14 +631,17 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     DeviceGuard dg(h->cfg.device);
     VT_CUDA(h, dg.err);
     if (const int rc = check_missing(h)) return rc;
-    if (h->generic) return finalize_generic(h, st);
+    TensorMap ts = h->tensors;          // rebalanced on a copy: finalising again starts from the tensors as they were set
+    const int pnorm = rebalance(h->cfg, ts);
+    if (h->generic) return finalize_generic(h, ts, pnorm, st);
     Packer pk;
     ModelW& m = h->mw;
+    m.norm_tap_scale = ldexpf(1.f, pnorm);
 
     // ---- stem: BN folded, [co][ci][3][3] -> [ci][ky][kx][co]
     size_t stem_w[4], stem_b[4];
     for (int l = 0; l < 4; ++l) {
-        const FoldedConv f = fold_conv_bn(h, stem_prefix(l) + "c.", stem_prefix(l) + "bn.", false);
+        const FoldedConv f = fold_conv_bn(ts, stem_prefix(l) + "c.", stem_prefix(l) + "bn.", false);
         stem_w[l] = pk.slot(m.stem[l].w, f.w.size());
         stem_b[l] = pk.put(m.stem[l].b, f.b.data(), f.co);
         for (int co = 0; co < f.co; ++co)
@@ -601,7 +667,7 @@ int vt_finalize_weights(VtHandle h, void* stream) {
             for (int c = 0; c < cols_in; ++c) pk.buf[o + (size_t)c * rows_out + r] = src[(size_t)r * cols_in + c];
     };
     for (int b = 0; b < kDepth; ++b) {
-        const BlockTensors t = block_tensors(h, b);
+        const BlockTensors t = block_tensors(ts, b);
         BlockW& B = m.blk[b];
         pk.put(B.ln1_g, t.ln1_g, kC); pk.put(B.ln1_b, t.ln1_b, kC);
         transp(pk.slot(B.wqkv, kC * 3 * kC), t.wqkv, 3 * kC, kC);
@@ -617,10 +683,10 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     // ---- the same blocks for the tensor cores (vt_block_tc.cu)
     for (int b = 0; b < kDepth; ++b) {
         const size_t wa = pk.slot(m.tc[b].wa, kTcWaBytes / 4), wb = pk.slot(m.tc[b].wb, kTcWbBytes / 4), par = pk.slot(m.tc[b].par, kTcParFloats);
-        block_tc_pack(block_tensors(h, b), pk.bytes(wa), pk.bytes(wb), &pk.buf[par]);
+        block_tc_pack(block_tensors(ts, b), pk.bytes(wa), pk.bytes(wb), &pk.buf[par]);
     }
-    pk.put(m.norm_g, tensor(h, "norm.weight"), kC); pk.put(m.norm_b, tensor(h, "norm.bias"), kC);
-    pk.put(m.pos_z, tensor(h, "pos_embed_z"), kNz * kC); pk.put(m.pos_x, tensor(h, "pos_embed_x"), kNx * kC);
+    pk.put(m.norm_g, tensor(ts, "norm.weight"), kC); pk.put(m.norm_b, tensor(ts, "norm.bias"), kC);
+    pk.put(m.pos_z, tensor(ts, "pos_embed_z"), kNz * kC); pk.put(m.pos_x, tensor(ts, "pos_embed_x"), kNx * kC);
 
     // ---- head: conv(+bias) -> BN folded; layer i weights laid out [ci][k][tower][co_t]
     const float** head_w[4] = {&m.head.w1, &m.head.w2, &m.head.w3, &m.head.w4};
@@ -628,7 +694,7 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     size_t hw[4];
     for (int i = 0; i < 4; ++i) {
         FoldedConv f[3];
-        for (int t = 0; t < 3; ++t) f[t] = fold_conv_bn(h, head_prefix(i, t) + "0.", head_prefix(i, t) + "1.", true);
+        for (int t = 0; t < 3; ++t) f[t] = fold_conv_bn(ts, head_prefix(i, t) + "0.", head_prefix(i, t) + "1.", true);
         const int ci_n = f[0].ci, co_n = f[0].co;
         hw[i] = pk.slot(*head_w[i], (size_t)ci_n * 9 * 3 * co_n);
         const size_t hb = pk.slot(*head_b[i], 3 * co_n);
@@ -647,7 +713,7 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     const size_t w5 = pk.slot(m.head.w5, 3 * 4 * 2), b5 = pk.slot(m.head.b5, 3 * 2);
     for (int t = 0; t < 3; ++t) {
         const std::string p = std::string("box_head.conv5_") + kTowers[t] + ".";
-        const float *w = tensor(h, p + "weight"), *b = tensor(h, p + "bias");
+        const float *w = tensor(ts, p + "weight"), *b = tensor(ts, p + "bias");
         for (int o = 0; o < (t == 0 ? 1 : 2); ++o) {
             pk.buf[b5 + t * 2 + o] = b[o];
             for (int c = 0; c < 4; ++c) pk.buf[w5 + (t * 4 + c) * 2 + o] = w[o * 4 + c];
@@ -655,7 +721,7 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     }
     // ---- Hann window (hann.py:6-16) and normalisation table (data_utils.py:8-14) -----------------
     const size_t hann = pk.slot(m.hann, 256), lut = pk.slot(m.lut, 768);
-    fill_hann_and_lut(h, &pk.buf[hann], &pk.buf[lut]);
+    fill_hann_and_lut(ts, &pk.buf[hann], &pk.buf[lut]);
     if (const int rc = upload_weights(h, pk, st)) return rc;
     h->finalized = true;
     return VT_OK;

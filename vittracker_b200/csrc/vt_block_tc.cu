@@ -52,8 +52,10 @@ constexpr int kNS = 6;
 // low-order terms do not reach the arg-max: S feeds a softmax (a perturbation of S scales P by 1 + dS, and the row normalisation removes
 // its common part), |dS| ~ 2^-12 |q||k| / sqrt(48) ~ 1e-5 here.  Dropping either term of q k^T: 0 flips, score-map error 1e-6 (the noise
 // floor of the three-term scheme is 8e-7); every other contraction flips the arg-max when it loses a term (errors 2e-5 .. 1.5e-4).
-// That budget is measured on the specified workload (random-init weights: |S| < 1).  A trained checkpoint has sharper attention - larger
-// |q||k| and the same RELATIVE operand error - so the kernel is compiled in both forms and the handle chooses: VT_BLOCKS_TCGEN05 (single
+// That budget is measured on the specified workload (random-init weights: |S| < 1).  How a checkpoint splits scale between q and k (or
+// between a LayerNorm's gain and the next weights) does not reach the kernel: weight ingest rebalances it by powers of two (vt_api.cu:
+// rebalance), so each operand keeps the split's relative precision.  A trained checkpoint can still have sharper attention - a larger
+// product |q||k| and the same RELATIVE operand error - so the kernel is compiled in both forms and the handle chooses: VT_BLOCKS_TCGEN05 (single
 // pass, the default) or VT_BLOCKS_TCGEN05_3TERM (blocks_impl = "tcgen05_3term": three terms everywhere, ~9 % slower blocks).
 constexpr int kEpiWarps = 4 * kNS;
 constexpr int kEpiThreads = kEpiWarps * 32;

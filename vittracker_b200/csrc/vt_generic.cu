@@ -631,6 +631,11 @@ __global__ void __launch_bounds__(256) softmax_rows_kernel(float* __restrict__ s
     for (int c = lane; c < cols; c += 32) x[c] *= inv;
 }
 
+// out = in * s: the final LayerNorm's tap, scaled back to the model's LayerNorm (GenModelW::norm_tap_scale)
+__global__ void __launch_bounds__(256) scale_copy_kernel(const float* __restrict__ in, float* __restrict__ out, long long n, float s) {
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) out[i] = in[i] * s;
+}
+
 // raw conv5 outputs [n][256][5] (ctr, offset x, offset y, size w, size h) -> maps, arg-max, boxes, tracker state
 // Range guard: the tensor-core GEMMs take fp16 hi + lo operands, so an activation beyond fp16 range becomes inf and then inf / NaN
 // downstream.  Two chokepoints catch every such track: the final LayerNorm's output row (`ln_x`, first element: a non-finite input
@@ -846,7 +851,13 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
         if (taps && cudaMemcpyAsync(taps + (size_t)(b + 1) * tap_stride, tokens, tok_bytes, cudaMemcpyDeviceToDevice, st) != cudaSuccess) return -1;
     }
     GEN_TRY(ln(tokens, ws.ln, w.norm_g, w.norm_b));
-    if (taps && cudaMemcpyAsync(taps + (size_t)(w.depth + 1) * tap_stride, ws.ln, tok_bytes, cudaMemcpyDeviceToDevice, st) != cudaSuccess) return -1;
+    if (taps) {
+        const long long m = (long long)rows * C;
+        scale_copy_kernel<<<(int)((m + 255) / 256 < 148 * 32 ? (m + 255) / 256 : 148 * 32), 256, 0, st>>>(ws.ln, taps + (size_t)(w.depth + 1) * tap_stride,
+                                                                                                           m, w.norm_tap_scale);
+        if (cudaGetLastError() != cudaSuccess) return -1;
+        ++total;
+    }
 
     // ---- CENTER head on the 16 x 16 search feature map (tokens 64..319 of every track, NHWC) ----
     const int hc = w.hc, prow = n * 256;

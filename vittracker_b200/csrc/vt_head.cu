@@ -166,7 +166,8 @@ __device__ __forceinline__ void head_conv(const float* in, float* outp, const fl
     __syncthreads();
 }
 
-// Final LayerNorm of one token row (vit_dist.py:94); optionally stores the normalised row (tokens_norm tap).
+// Final LayerNorm of one token row (vit_dist.py:94); optionally stores the normalised row (tokens_norm tap, scaled back to the model's
+// LayerNorm by w.norm_tap_scale).
 // `bad` is raised when the row holds a non-finite value (an fp16-range overflow anywhere upstream on the tensor-core path ends as
 // inf / NaN in the residual stream: K / V' / q / P poison every query row of their track, the MLP its own row) or when the
 // normalised row itself would not fit the fp16 operand range.
@@ -205,7 +206,9 @@ __device__ __forceinline__ void head_norm_row(const HeadArgs& a, const ModelW& w
     if (a.tokens_norm) {
         float* t = a.tokens_norm + ((size_t)trk * kN + row) * kC;
 #pragma unroll
-        for (int k = 0; k < kC; k += 4) *reinterpret_cast<float4*>(t + k) = make_float4(y[k], y[k + 1], y[k + 2], y[k + 3]);
+        for (int k = 0; k < kC; k += 4)
+            *reinterpret_cast<float4*>(t + k) = make_float4(y[k] * w.norm_tap_scale, y[k + 1] * w.norm_tap_scale, y[k + 2] * w.norm_tap_scale,
+                                                            y[k + 3] * w.norm_tap_scale);
     }
 }
 

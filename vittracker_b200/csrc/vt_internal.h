@@ -140,6 +140,7 @@ struct ModelW {
     BlockW blk[kDepth];
     BlockTcW tc[kDepth];
     const float *norm_g, *norm_b;
+    float norm_tap_scale;          // 2^p: the final LayerNorm runs on weights rebalanced by 2^-p (vt_api.cu: rebalance); its tap is scaled back
     const float *pos_z, *pos_x;    // [64][48], [256][48]
     HeadW head;
     const uint8_t* stem_tc_w[3];   // stem conv2 / conv3 / conv4 for tcgen05 (vt_stem_tc.cu): fp16 hi | lo blobs in K-step order
@@ -343,6 +344,7 @@ struct GenModelW {
     const float* stem_w[4]; const float* stem_b[4];          // [cout][9 cin], [cout]
     GenBlockW blk[kGenMaxDepth];
     const float *norm_g, *norm_b, *pos_z, *pos_x;
+    float norm_tap_scale;                                    // as ModelW::norm_tap_scale
     const float* head_w1; const float* head_b1;              // three towers merged: [3 hc][9 C], [3 hc]  (ctr | offset | size)
     const float* head_w[3][3]; const float* head_b[3][3];    // [tower][layer 2..4]: [co][9 ci], [co]
     const float* head_w5; const float* head_b5;              // [5][hc / 8] rows ctr, offset x, offset y, size w, size h; [5]

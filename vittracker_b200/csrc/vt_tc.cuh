@@ -237,7 +237,10 @@ __device__ __forceinline__ void mbar_arrive_expect_tx_elect(uint64_t* bar, uint3
         : "memory");
 }
 // ---- fp32 -> fp16 hi/lo split ------------------------------------------------------------------------
-// v ~= hi + lo with hi = fp16(v), lo = fp16(v - hi): ~22 significant bits for |v| well inside fp16 range.
+// v ~= hi + lo with hi = fp16(v), lo = fp16(v - hi): ~22 significant bits while lo is a normal fp16 number and hi does not overflow,
+// i.e. for roughly 2^-3 <= |v| < 65504; below, the error is absolute (2^-25).  Weight ingest (vt_api.cu: rebalance) moves powers of
+// two between the factors of each LayerNorm / BatchNorm -> layer pair, q and k, and v and the output projection, so that the operands
+// stay near the magnitudes of a random-init model however a checkpoint splits its scale between them.
 // Two instructions per element: one packed conversion gives both hi halves, one mixed-precision FMA per element (sm_100
 // fma.rn.f32.f16: an fp16 product accumulated onto an fp32 addend, exact here) gives v - hi without unpacking, one packed conversion
 // gives both lo halves.
