@@ -49,6 +49,7 @@ typedef enum VtStatus {
                                    * tensor-core path (|v| >= 65504; operands are fp16 hi + lo): the result is
                                    * withheld (state kept, confidence -1, maps NaN) instead of silently wrong.
                                    * Rerun the track with VT_BLOCKS_SIMT_FP32 (all fp32).                    */
+#define VT_TRACK_BAD_SLOT 4       /* slot outside [0, max_tracks) or named by an earlier item of the same call */
 
 /* Which implementation of the ViT blocks vt_forward / vt_tracks_step use. */
 #define VT_BLOCKS_SIMT_FP32 0     /* fp32 CUDA-core kernel: bring-up / exact mode                 */
@@ -164,13 +165,36 @@ int vt_tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offse
                    const int32_t* frame_hw, int32_t first, int32_t n, double* out_boxes,
                    double* out_detail, int32_t update_state, void* stream);
 
+/* The same two calls for any set of tracks: item i works on track slots[i].  `slots` is a DEVICE int32 array of n entries in any
+ * order; every other array is per item, in item order, exactly as in vt_tracks_init / vt_tracks_step.  A multi-target caller adds a
+ * target by initialising a free slot, retires one by no longer listing it, and steps the live set in one call.
+ *   - The list is checked on the device, without a host synchronisation.  An entry outside [0, max_tracks), or equal to the slot
+ *     of an earlier item of the same call, is not processed: vt_tracks_init_slots sets out_status[i] = VT_TRACK_BAD_SLOT and writes
+ *     no state or template; vt_tracks_step_slots writes out_boxes[i] = (0, 0, 0, 0, -1), out_detail[i] with status
+ *     VT_TRACK_BAD_SLOT and arg-max -1, NaN maps, and reads or writes no state.  Among repeated slots the first item wins.
+ *   - VT_ERR_INVALID_ARG before any launch for a null handle, n < 0, n > max_tracks, or a null pointer (out_status and out_detail
+ *     may be null) when n > 0.  n == 0 is a no-op.  vt_tracks_step_slots before any init returns VT_ERR_STATE.
+ *   - No allocation and no host synchronisation: a call can be captured in a CUDA graph and replayed with new contents in `slots`.
+ *   - A slot that was never initialised holds the zero box vt_create gave it: stepping it returns VT_TRACK_TOO_SMALL.
+ *   - A track's outputs, maps and new state are the same bits whether it is stepped by range or by slot list, in any order and next
+ *     to any other items.
+ *   - After vt_tracks_step_slots, vt_tracks_last_maps(first, n) addresses item positions [first, first + n) of that call.
+ * Cost over the range calls: two small kernels that resolve the list per call, plus per chunk one row-copy kernel (the template
+ * scatter of an init; on configurations other than vit_48_h32, the template gather of a step). */
+int vt_tracks_init_slots(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
+                         const double* boxes_xywh, const int32_t* slots, int32_t n, int32_t* out_status, void* stream);
+int vt_tracks_step_slots(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
+                         const int32_t* slots, int32_t n, double* out_boxes, double* out_detail, int32_t update_state,
+                         void* stream);
+
 /* Read / overwrite the per-track boxes ([n][4] float64 device pointers). */
 int vt_tracks_get_state(VtHandle h, double* boxes_xywh, int32_t first, int32_t n, void* stream);
 int vt_tracks_set_state(VtHandle h, const double* boxes_xywh, int32_t first, int32_t n, void* stream);
 
 /* Maps of the most recent vt_tracks_step chunk-by-chunk copy: score [n][F*F], size [n][2][F*F],
  * offset [n][2][F*F] for tracks [first, first+n) of that step (debug / parity aid; any may be
- * NULL). Valid only if the step covered those tracks. */
+ * NULL). Valid only if the step covered those tracks.  After vt_tracks_step_slots: items
+ * [first, first+n) of that call. */
 int vt_tracks_last_maps(VtHandle h, int32_t first, int32_t n, float* score_map, float* size_map,
                         float* offset_map, void* stream);
 

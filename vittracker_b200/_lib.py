@@ -15,7 +15,7 @@ VT_OK = 0
 VT_BLOCKS_SIMT_FP32 = 0
 VT_BLOCKS_TCGEN05 = 1
 VT_BLOCKS_TCGEN05_3TERM = 2
-VT_TRACK_OK, VT_TRACK_TOO_SMALL, VT_TRACK_OUT_OF_DOMAIN, VT_TRACK_NUMERIC_RANGE = 0, 1, 2, 3
+VT_TRACK_OK, VT_TRACK_TOO_SMALL, VT_TRACK_OUT_OF_DOMAIN, VT_TRACK_NUMERIC_RANGE, VT_TRACK_BAD_SLOT = 0, 1, 2, 3, 4
 
 STATUS_NAMES = {0: "VT_OK", -1: "VT_ERR_INVALID_ARG", -2: "VT_ERR_CUDA", -3: "VT_ERR_WEIGHTS", -4: "VT_ERR_STATE",
                 -5: "VT_ERR_UNSUPPORTED", -6: "VT_ERR_NO_DEVICE"}
@@ -49,6 +49,8 @@ SIGNATURES = {
     "vt_cal_bbox": (C.c_int, [_P, _P, _P, _P, C.c_int32, _P, _P]),
     "vt_tracks_init": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P]),
     "vt_tracks_step": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, C.c_int32, _P]),
+    "vt_tracks_init_slots": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
+    "vt_tracks_step_slots": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, C.c_int32, _P]),
     "vt_tracks_get_state": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P]),
     "vt_tracks_set_state": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P]),
     "vt_tracks_last_maps": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P]),

@@ -168,9 +168,26 @@ class YuvSurfaces:
         return cls(format, f[:, :H], u, v)
 
 
+def check_slots(slots, max_tracks: int) -> list:
+    """A host sequence of track slots as a list of ints; ValueError for an entry outside [0, max_tracks) or named twice."""
+    out = [int(v) for v in slots]
+    seen = set()
+    for v in out:
+        if not 0 <= v < max_tracks:
+            raise ValueError(f"slot {v} outside [0, {max_tracks})")
+        if v in seen:
+            raise ValueError(f"slot {v} listed twice")
+        seen.add(v)
+    return out
+
+
 class BatchedTracker:
     """``initialize(pool, frame_index, boxes)`` / ``track(pool, frame_index)`` for n tracks at once:
-    the batched counterpart of ``Vit_dist.initialize`` / ``Vit_dist.track``."""
+    the batched counterpart of ``Vit_dist.initialize`` / ``Vit_dist.track``.
+
+    Without ``slots`` these calls work on tracks 0..n-1.  With ``slots`` (a host sequence of ints, checked here, or a CUDA integer
+    tensor, passed through: the device gives a bad entry status VT_TRACK_BAD_SLOT), item i works on track ``slots[i]`` and results come
+    back in slot-list order, so targets can be added to free slots, retired, and the live set stepped in one call."""
 
     def __init__(self, cfg, state_dict, max_tracks: int, device: Optional[int] = None, chunk_tracks: int = 0,
                  blocks_impl: str = "tcgen05", depth: Optional[int] = None):
@@ -185,34 +202,88 @@ class BatchedTracker:
         self.template_factor, self.search_factor = float(cfg.TEST.TEMPLATE_FACTOR), float(cfg.TEST.SEARCH_FACTOR)
         self._yuv_rgb: Optional[torch.Tensor] = None             # initialize_yuv / track_yuv: one RGB frame per track
         self._yuv_off: Optional[torch.Tensor] = None
+        # (H, W) of every slot's frames, for steps by slot list; row max_tracks takes the writes of bad entries
+        self._slot_hw = torch.zeros((max_tracks + 1, 2), dtype=torch.int32, device=self.device)
 
-    def initialize(self, pool: FramePool, frame_index: torch.Tensor, boxes) -> torch.Tensor:
+    def _slots(self, slots) -> torch.Tensor:
+        """The slot list as the contiguous int32 device tensor the engine takes."""
+        if torch.is_tensor(slots) and slots.is_cuda:
+            if slots.dtype not in (torch.int32, torch.int64) or slots.dim() != 1 or slots.device != self.device:
+                raise ValueError(f"slots: expected a 1-D integer tensor on {self.device}")
+            return slots.to(torch.int32).contiguous()
+        return torch.tensor(check_slots(slots.tolist() if torch.is_tensor(slots) else slots, self.max_tracks), dtype=torch.int32,
+                            device=self.device)
+
+    def _rows(self, slots: torch.Tensor) -> torch.Tensor:
+        """Per item the slot it works on, as the device resolves the list (first occurrence of an in-range slot), or max_tracks for a bad
+        entry: indexes per-slot tensors that have a spare last row, without a host synchronisation."""
+        mt, n = self.max_tracks, slots.shape[0]
+        s = slots.to(torch.int64)
+        item = torch.arange(n, dtype=torch.int64, device=self.device)
+        s = torch.where((s >= 0) & (s < mt), s, mt)
+        first = torch.full((mt + 1,), n, dtype=torch.int64, device=self.device).scatter_reduce_(0, s, item, "amin")
+        return torch.where(first[s] == item, s, mt)
+
+    def initialize(self, pool: FramePool, frame_index: torch.Tensor, boxes, slots=None) -> torch.Tensor:
         boxes = torch.as_tensor(boxes, dtype=torch.float64).reshape(-1, 4).to(self.device).contiguous()
         n = boxes.shape[0]
         if n > self.max_tracks:
             raise ValueError(f"{n} tracks > max_tracks {self.max_tracks}")
+        offs = pool.offsets(frame_index.to(self.device))
+        if slots is not None:
+            return self._init_slots(pool.data, offs, pool.hw(n), boxes, self._slots(slots))
         self.n = n
         self._hw = pool.hw(n)
-        status = self.engine.tracks_init(pool.data, pool.offsets(frame_index.to(self.device)), self._hw, boxes, first=0)
+        self._slot_hw[:n] = self._hw
+        status = self.engine.tracks_init(pool.data, offs, self._hw, boxes, first=0)
         return status
 
-    def set_state(self, boxes) -> None:
+    def _init_slots(self, frames, offsets, hw, boxes, slots: torch.Tensor) -> torch.Tensor:
+        if slots.shape[0] != boxes.shape[0]:
+            raise ValueError(f"{slots.shape[0]} slots for {boxes.shape[0]} boxes")
+        self._slot_hw[self._rows(slots)] = hw
+        return self.engine.tracks_init_slots(frames, offsets, hw, boxes, slots)
+
+    def set_state(self, boxes, slots=None) -> None:
+        """Overwrite the boxes of tracks 0..n-1, or of the listed slots (a bad entry of a CUDA slot tensor is skipped)."""
         boxes = torch.as_tensor(boxes, dtype=torch.float64).reshape(-1, 4).to(self.device).contiguous()
-        self.engine.tracks_set_state(boxes, first=0)
+        if slots is None:
+            self.engine.tracks_set_state(boxes, first=0)
+            return
+        slots = self._slots(slots)
+        state = torch.cat([self.engine.tracks_get_state(0, self.max_tracks), boxes.new_zeros((1, 4))])
+        state[self._rows(slots)] = boxes
+        self.engine.tracks_set_state(state[: self.max_tracks].contiguous(), first=0)
 
-    def get_state(self) -> torch.Tensor:
-        return self.engine.tracks_get_state(0, self.n)
+    def get_state(self, slots=None) -> torch.Tensor:
+        """Boxes [n, 4] of tracks 0..n-1, or of the listed slots in list order (NaN for a bad entry of a CUDA slot tensor)."""
+        if slots is None:
+            return self.engine.tracks_get_state(0, self.n)
+        slots = self._slots(slots)
+        state = torch.cat([self.engine.tracks_get_state(0, self.max_tracks), torch.full((1, 4), float("nan"), dtype=torch.float64,
+                                                                                          device=self.device)])
+        return state[self._rows(slots)]
 
-    def track(self, pool: FramePool, frame_index: torch.Tensor, update_state: bool = True, detail: bool = False):
-        """One step for all tracks; returns the device tensor [n,5] (x, y, w, h, confidence)."""
+    def track(self, pool: FramePool, frame_index: torch.Tensor, update_state: bool = True, detail: bool = False, slots=None):
+        """One step for all tracks (or for the listed slots, frame_index[i] for slots[i]); returns the device tensor [n,5] (x, y, w, h,
+        confidence)."""
         offs = pool.offsets(frame_index.to(self.device))
-        return self.track_offsets(pool.data, offs, update_state=update_state, detail=detail)
+        return self.track_offsets(pool.data, offs, update_state=update_state, detail=detail, slots=slots)
 
-    def track_offsets(self, frames: torch.Tensor, offsets: torch.Tensor, update_state: bool = True, detail: bool = False):
+    def track_offsets(self, frames: torch.Tensor, offsets: torch.Tensor, update_state: bool = True, detail: bool = False, slots=None):
+        if slots is not None:
+            slots = self._slots(slots)
+            return self._step_slots(frames, offsets, self._slot_hw[self._rows(slots)], slots, update_state, detail)
         out = self.out_boxes[: self.n]
         r = self.engine.tracks_step(frames, offsets, self._hw, first=0, n=self.n, out_boxes=out,
                                     update_state=update_state, detail=detail)
         return r
+
+    def _step_slots(self, frames, offsets, hw, slots: torch.Tensor, update_state: bool, detail: bool):
+        if offsets.shape[0] != slots.shape[0]:
+            raise ValueError(f"{offsets.shape[0]} frames for {slots.shape[0]} slots")
+        return self.engine.tracks_step_slots(frames, offsets, hw, slots, out_boxes=self.out_boxes[: slots.shape[0]],
+                                             update_state=update_state, detail=detail)
 
     def _yuv_frames(self, surfaces: YuvSurfaces) -> Tuple[torch.Tensor, torch.Tensor]:
         if surfaces.n > self.max_tracks:
@@ -221,30 +292,51 @@ class BatchedTracker:
             raise ValueError(f"surfaces on {surfaces.device}, tracker on {self.device}")
         if self._yuv_rgb is None or tuple(self._yuv_rgb.shape[1:3]) != (surfaces.H, surfaces.W):
             self._yuv_rgb = None
-            # zero-filled once: the crop kernels read the first pixels of a row with weight 0 for taps in the padding
-            self._yuv_rgb = torch.zeros((self.max_tracks, surfaces.H, surfaces.W, 3), dtype=torch.uint8, device=self.device)
-            self._yuv_off = torch.arange(self.max_tracks, dtype=torch.int64, device=self.device) * (surfaces.H * surfaces.W * 3)
+            # zero-filled once: the crop kernels read the first pixels of a row with weight 0 for taps in the padding.  The frame
+            # after the last track's takes the conversions of bad slot-list entries.
+            self._yuv_rgb = torch.zeros((self.max_tracks + 1, surfaces.H, surfaces.W, 3), dtype=torch.uint8, device=self.device)
+            self._yuv_off = torch.arange(self.max_tracks + 1, dtype=torch.int64, device=self.device) * (surfaces.H * surfaces.W * 3)
         return self._yuv_rgb, self._yuv_off[: surfaces.n]
 
-    def initialize_yuv(self, surfaces: YuvSurfaces, boxes) -> torch.Tensor:
+    def initialize_yuv(self, surfaces: YuvSurfaces, boxes, slots=None) -> torch.Tensor:
         """``initialize`` for tracks 0..n-1 from device-resident YUV surfaces (``YuvSurfaces``, track i on surface i): only the rectangle
         each template crop reads is converted (vt_yuv420_crop_to_rgb, bit for bit cv2.cvtColor), into an RGB frame per track that
         this tracker owns, then vt_tracks_init runs on it on the same stream.  Those frames cost max_tracks x H x W x 3 bytes of
-        device memory (2.76 MB per track at 720p, 6.2 MB at 1080p), allocated at the first call for a picture size."""
+        device memory (2.76 MB per track at 720p, 6.2 MB at 1080p), allocated at the first call for a picture size.  With ``slots``,
+        surface i belongs to track slots[i], whose RGB frame it is converted into."""
         boxes = torch.as_tensor(boxes, dtype=torch.float64).reshape(-1, 4).to(self.device).contiguous()
         if boxes.shape[0] != surfaces.n:
             raise ValueError(f"{boxes.shape[0]} boxes for {surfaces.n} surfaces")
         frames, offs = self._yuv_frames(surfaces)
+        if slots is not None:
+            slots = self._slots(slots)
+            offs = self._yuv_off[self._rows(slots)]
+            self.engine.yuv420_crop_to_rgb(surfaces.format, surfaces.planes, surfaces.pitches, surfaces.hw, frames, offs,
+                                           self.template_factor, boxes=boxes)
+            return self._init_slots(frames, offs, surfaces.hw, boxes, slots)
         self.engine.yuv420_crop_to_rgb(surfaces.format, surfaces.planes, surfaces.pitches, surfaces.hw, frames, offs,
                                        self.template_factor, boxes=boxes)
         self.n = surfaces.n
         self._hw = surfaces.hw
+        self._slot_hw[: self.n] = self._hw
         return self.engine.tracks_init(frames, offs, self._hw, boxes, first=0)
 
-    def track_yuv(self, surfaces: YuvSurfaces, update_state: bool = True, detail: bool = False):
+    def track_yuv(self, surfaces: YuvSurfaces, update_state: bool = True, detail: bool = False, slots=None):
         """``track`` from device-resident YUV surfaces (surface i for track i): the rectangle each search crop reads is computed on the
         device from the track's current state - the host never waits for it - and converted; then vt_tracks_step runs on the same
-        stream.  No allocation after the first call for a picture size, so a step can be captured in a CUDA graph."""
+        stream.  No allocation after the first call for a picture size, so a step can be captured in a CUDA graph.  With ``slots``,
+        surface i belongs to track slots[i]: its state is gathered on the device and the surface is converted into that track's frame."""
+        if slots is not None:
+            slots = self._slots(slots)
+            if slots.shape[0] != surfaces.n:
+                raise ValueError(f"{surfaces.n} surfaces for {slots.shape[0]} slots")
+            frames, _ = self._yuv_frames(surfaces)
+            rows = self._rows(slots)
+            boxes = self.engine.tracks_get_state(0, self.max_tracks)[rows.clamp(max=self.max_tracks - 1)]
+            offs = self._yuv_off[rows]
+            self.engine.yuv420_crop_to_rgb(surfaces.format, surfaces.planes, surfaces.pitches, surfaces.hw, frames, offs,
+                                           self.search_factor, boxes=boxes)
+            return self._step_slots(frames, offs, surfaces.hw, slots, update_state, detail)
         if surfaces.n != self.n:
             raise ValueError(f"{surfaces.n} surfaces for {self.n} tracks")
         frames, offs = self._yuv_frames(surfaces)

@@ -16,6 +16,7 @@
 
 using namespace vt;
 static_assert(vt::VT_TRACK_NUMERIC_RANGE_ == VT_TRACK_NUMERIC_RANGE, "status code shared with the kernels");
+static_assert(vt::VT_TRACK_BAD_SLOT_ == VT_TRACK_BAD_SLOT, "status code shared with the kernels");
 
 namespace {
 
@@ -53,7 +54,9 @@ struct VtContext {
     // per-track state
     double* d_state = nullptr;        // [max_tracks][4]
     float* d_tmpl = nullptr;          // [max_tracks][64][48] cached template tokens (+pos)
-    int32_t* d_status = nullptr;      // [max_tracks]
+    int32_t* d_status = nullptr;      // [max_tracks] crop status of the current call (by track for a range call, by item for a slot list)
+    uint32_t* d_claim = nullptr;      // [max_tracks] slot-list deduplication (vt_slots.cu), all 0xffffffff between calls
+    int32_t* d_eff = nullptr;         // [max_tracks] effective slot per item of the current slot-list call
     float* d_maps = nullptr;          // [max_tracks][1280] score | size | offset of the last step
     int last_first = 0, last_n = 0;
     // generic-configuration path (every configuration other than vit_48_h32; vt_generic.cu)
@@ -269,7 +272,7 @@ void free_all(VtHandle h) {
     for (auto e : h->evpool) cudaEventDestroy(e);
     cudaFree(h->d_weights); cudaFree(h->d_planes); cudaFree(h->d_scratch); cudaFree(h->d_taps); cudaFree(h->d_tokz);
     cudaFree(h->d_tokx); cudaFree(h->d_tok); cudaFree(h->d_state); cudaFree(h->d_tmpl);
-    cudaFree(h->d_status); cudaFree(h->d_maps); cudaFree(h->d_gwork);
+    cudaFree(h->d_status); cudaFree(h->d_claim); cudaFree(h->d_eff); cudaFree(h->d_maps); cudaFree(h->d_gwork);
 }
 
 int check_ready(VtHandle h, bool need_tracks) {
@@ -291,22 +294,25 @@ cudaEvent_t get_event(VtHandle h) {
     return e;
 }
 
-// Launch one pipeline stage; when profiling is on, bracket it with events on the launching stream.
+// Launch one pipeline stage; when profiling is on, bracket it with events on the launching stream.  kNoStage: the slot-list
+// bookkeeping of vt_slots.cu, counted as launches but not as a stage, so that a stage's items stay the number of tracks it processed.
+constexpr int kNoStage = -1;
 #define VT_LAUNCH(h, stage, items, st, where, expr)                               \
     do {                                                                          \
+        const bool prof__ = (h)->profiling && (stage) >= 0;                       \
         cudaEvent_t ea__ = nullptr, eb__ = nullptr;                               \
-        if ((h)->profiling) { ea__ = get_event(h); eb__ = get_event(h); cudaEventRecord(ea__, st); } \
+        if (prof__) { ea__ = get_event(h); eb__ = get_event(h); cudaEventRecord(ea__, st); } \
         const int k__ = (expr);                                                   \
         if (k__ < 0) return launch_fail(h, k__, where);                           \
         (h)->launches += k__;                                                     \
-        if ((h)->profiling) { cudaEventRecord(eb__, st); (h)->prof.push_back({stage, items, ea__, eb__}); } \
+        if (prof__) { cudaEventRecord(eb__, st); (h)->prof.push_back({stage, items, ea__, eb__}); } \
     } while (0)
 
-int run_blocks(VtHandle h, const float* tokz, int zs, const float* tokx, int xs, float* out, int n, float* taps,
+int run_blocks(VtHandle h, const float* tokz, int zs, const int32_t* zslots, const float* tokx, int xs, float* out, int n, float* taps,
                size_t tap_stride, cudaStream_t st) {
     if (h->cfg.blocks_impl == VT_BLOCKS_SIMT_FP32)
-        return launch_blocks_simt(tokz, zs, tokx, xs, out, n, h->mw, taps, tap_stride, st);
-    return launch_blocks_tc(tokz, zs, tokx, xs, out, n, h->mw, taps, tap_stride, h->num_sms, h->cfg.blocks_impl == VT_BLOCKS_TCGEN05_3TERM ? 3 : 1, st);
+        return launch_blocks_simt(tokz, zs, zslots, tokx, xs, out, n, h->mw, taps, tap_stride, st);
+    return launch_blocks_tc(tokz, zs, zslots, tokx, xs, out, n, h->mw, taps, tap_stride, h->num_sms, h->cfg.blocks_impl == VT_BLOCKS_TCGEN05_3TERM ? 3 : 1, st);
 }
 
 
@@ -329,16 +335,17 @@ LastMaps last_maps(VtHandle h, int first) {
     return {h->d_maps + (size_t)first * 256, h->d_maps + mt * 256 + (size_t)first * 512, h->d_maps + mt * 768 + (size_t)first * 512};
 }
 
-// HeadArgs of a tracking step over tracks [first + c0, first + c0 + m); frame_hw, out_boxes and out_detail are the step's arrays,
-// which start at track `first`
-HeadArgs track_head_args(VtHandle h, int first, int c0, int m, const int32_t* frame_hw, double* out_boxes, double* out_detail,
-                         int update_state) {
+// HeadArgs of a tracking step over items [c0, c0 + m); frame_hw, out_boxes and out_detail are the step's arrays.  Range step
+// (slots == NULL): item i is track first + i.  Slot list (first == 0): item i is track slots[i]; maps and status stay by item.
+HeadArgs track_head_args(VtHandle h, int first, const int32_t* slots, int c0, int m, const int32_t* frame_hw, double* out_boxes,
+                         double* out_detail, int update_state) {
     const int t0 = first + c0;
     const LastMaps maps = last_maps(h, t0);
     HeadArgs a{};
     a.n = m;
     a.score_map = maps.score; a.size_map = maps.size; a.offset_map = maps.offset;
-    a.state = h->d_state + (size_t)t0 * 4;
+    a.state = h->d_state + (size_t)(slots ? 0 : t0) * 4;
+    a.slots = slots ? slots + c0 : nullptr;
     a.frame_hw = frame_hw + 2 * c0;
     a.status = h->d_status + t0;
     a.out_boxes = out_boxes + (size_t)c0 * 5;
@@ -506,6 +513,91 @@ cudaError_t pack_upload(const PackRun* runs, int nruns, uint8_t* staging, uint8_
     return e;
 }
 
+
+// vt_tracks_init over items [0, n): item i initialises track first + i (slots == NULL), or track slots[i] (first == 0; slots resolved,
+// a negative entry initialises nothing).  A range init writes the template tokens, status and state in place; a slot list stages the
+// chunk's tokens and statuses by item and scatters them.
+int tracks_init(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes_xywh,
+                int first, const int32_t* slots, int n, int32_t* out_status, cudaStream_t st) {
+    const int C = h->cfg.embed_dim;
+    const size_t row = (size_t)kNz * C;
+    for (int c0 = 0; c0 < n; c0 += h->chunk) {
+        const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
+        int32_t* status = h->d_status + first + c0;
+        float* tok = slots ? (h->generic ? h->gws.tokz : h->d_tokz) : h->d_tmpl + (size_t)(first + c0) * row;
+        if (h->generic) {
+            VT_LAUNCH(h, VT_STAGE_CROP, m, st, "vt_tracks_init/crop",
+                      launch_crop_normalize(frames, frame_offsets + c0, frame_hw + 2 * c0, boxes_xywh + 4 * c0, nullptr, h->cfg.template_factor, kTz, m,
+                                            h->mw.lut, h->gws.crop, nullptr, nullptr, nullptr, status, st));
+            VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_init/stem", gen_launch_stem(h->gws.crop, kTz, m, h->gw, h->gws, tok, kNz, 0, st));
+        } else {
+            VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_init/crop+stem",
+                      launch_crop_stem(frames, frame_offsets + c0, frame_hw + 2 * c0, boxes_xywh + 4 * c0, nullptr, h->cfg.template_factor, kTz, m,
+                                       h->mw, h->d_scratch, tok, kNz, 0, status, h->d_planes, h->chunk, h->d_taps, st));
+        }
+        if (slots)
+            VT_LAUNCH(h, kNoStage, m, st, "vt_tracks_init_slots/scatter",
+                      launch_scatter_init(tok, h->d_tmpl, row, boxes_xywh + 4 * c0, h->d_state, status, out_status ? out_status + c0 : nullptr,
+                                          slots + c0, m, st));
+    }
+    if (!slots) {
+        VT_CUDA(h, cudaMemcpyAsync(h->d_state + (size_t)first * 4, boxes_xywh, (size_t)n * 4 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        if (out_status) VT_CUDA(h, cudaMemcpyAsync(out_status, h->d_status + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    }
+    h->tracks_ready = true;
+    return VT_OK;
+}
+
+// vt_tracks_step over items [0, n): item i steps track first + i (slots == NULL), or track slots[i] (first == 0; slots resolved).  The
+// state and template pointers start at track `first`; crop status and maps are kept at [first + i], i.e. by item for a slot list.
+int tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, int first, const int32_t* slots,
+                int n, double* out_boxes, double* out_detail, int update_state, cudaStream_t st) {
+    const double* state = h->d_state + (size_t)first * 4;
+    auto state_at = [&](int c0) { return slots ? state : state + (size_t)c0 * 4; };       // state row of the chunk's first item
+    auto slots_at = [&](int c0) { return slots ? slots + c0 : nullptr; };
+    if (h->generic) {
+        // every stage runs per chunk: crop -> stem into the chunk's token buffer, cached template tokens copied in front
+        const int C = h->cfg.embed_dim;
+        const float* tmpl = h->d_tmpl + (size_t)first * kNz * C;
+        for (int c0 = 0; c0 < n; c0 += h->chunk) {
+            const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
+            VT_LAUNCH(h, VT_STAGE_CROP, m, st, "vt_tracks_step/crop",
+                      launch_crop_normalize(frames, frame_offsets + c0, frame_hw + 2 * c0, state_at(c0), slots_at(c0), h->cfg.search_factor, kSx, m,
+                                            h->mw.lut, h->gws.crop, nullptr, nullptr, nullptr, h->d_status + first + c0, st));
+            if (slots)
+                VT_LAUNCH(h, kNoStage, m, st, "vt_tracks_step_slots/gather",
+                          launch_gather_rows(tmpl, (size_t)kNz * C, h->gws.tok, (size_t)kN * C, (size_t)kNz * C, slots + c0, m, st));
+            else
+                VT_CUDA(h, cudaMemcpy2DAsync(h->gws.tok, (size_t)kN * C * sizeof(float), tmpl + (size_t)c0 * kNz * C, (size_t)kNz * C * sizeof(float),
+                                             (size_t)kNz * C * sizeof(float), m, cudaMemcpyDeviceToDevice, st));
+            VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_step/stem", gen_launch_stem(h->gws.crop, kSx, m, h->gw, h->gws, h->gws.tok, kN, kNz, st));
+            const HeadArgs a = track_head_args(h, first, slots, c0, m, frame_hw, out_boxes, out_detail, update_state);
+            VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_tracks_step/blocks+head", gen_launch_blocks_head(h->gws.tok, m, h->gw, h->gws, a, nullptr, 0, st));
+        }
+        h->last_first = first; h->last_n = n;
+        return VT_OK;
+    }
+    // crop + stem run per chunk (their intermediates are large); blocks + head run once over all n tracks
+    for (int c0 = 0; c0 < n; c0 += h->chunk) {
+        const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
+        VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_step/crop+stem",
+                  launch_crop_stem(frames, frame_offsets + c0, frame_hw + 2 * c0, state_at(c0), slots_at(c0), h->cfg.search_factor, kSx, m,
+                                   h->mw, h->d_scratch, h->d_tokx + (size_t)c0 * kNx * kC, kNx, 0, h->d_status + first + c0,
+                                   h->d_planes, h->chunk, h->d_taps, st));
+    }
+    {
+        const int m = n;
+        VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_tracks_step/blocks",
+                  run_blocks(h, h->d_tmpl + (size_t)first * kNz * kC, kNz, slots, h->d_tokx, kNx, h->d_tok, m, nullptr, 0, st));
+        HeadArgs a = track_head_args(h, first, slots, 0, m, frame_hw, out_boxes, out_detail, update_state);
+        a.tokens = h->d_tok;
+        a.use_tc = h->cfg.blocks_impl != VT_BLOCKS_SIMT_FP32;
+        VT_LAUNCH(h, VT_STAGE_HEAD, m, st, "vt_tracks_step/head", launch_head(a, h->mw, st));
+    }
+    h->last_first = first; h->last_n = n;
+    return VT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -579,9 +671,12 @@ int vt_create(const VtConfig* cfg, VtHandle* out) {
     A((void**)&h->d_state, mt * 4 * sizeof(double));
     A((void**)&h->d_tmpl, mt * kNz * Cd * sizeof(float));
     A((void**)&h->d_status, mt * sizeof(int32_t));
+    A((void**)&h->d_claim, mt * sizeof(uint32_t));
+    A((void**)&h->d_eff, mt * sizeof(int32_t));
     A((void**)&h->d_maps, mt * 1280 * sizeof(float));
     if (e == cudaSuccess) e = cudaMemset(h->d_state, 0, mt * 4 * sizeof(double));
     if (e == cudaSuccess) e = cudaMemset(h->d_status, 0, mt * sizeof(int32_t));
+    if (e == cudaSuccess) e = cudaMemset(h->d_claim, 0xff, mt * sizeof(uint32_t));
     if (e != cudaSuccess) {
         fail(nullptr, VT_ERR_CUDA, "vt_create: device allocation failed: %s", cudaGetErrorString(e));
         free_all(h); delete h;
@@ -739,7 +834,7 @@ int vt_crop_normalize(VtHandle h, const uint8_t* frames, const int64_t* frame_of
     if (!(factor > 0)) return fail(h, VT_ERR_INVALID_ARG, "vt_crop_normalize: factor must be positive");
     DeviceGuard dg(h->cfg.device);
     VT_CUDA(h, dg.err);
-    const int k = launch_crop_normalize(frames, frame_offsets, frame_hw, boxes_xywh, factor, out_size, n, h->mw.lut, out_nchw,
+    const int k = launch_crop_normalize(frames, frame_offsets, frame_hw, boxes_xywh, nullptr, factor, out_size, n, h->mw.lut, out_nchw,
                                         out_u8_hwc, out_mask, out_resize_factor, out_status, (cudaStream_t)stream);
     if (k < 0) return fail(h, VT_ERR_CUDA, "crop kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     h->launches += k;
@@ -773,7 +868,7 @@ int vt_forward(VtHandle h, const float* z, const float* x, int32_t n, float* pre
         const int m = (n - first < h->chunk) ? n - first : h->chunk;
         VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_forward/stem(z)", launch_stem(z + (size_t)first * 3 * kTz * kTz, kTz, m, h->mw, h->d_scratch, h->d_tokz, kNz, 0, h->d_planes, h->chunk, st));
         VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_forward/stem(x)", launch_stem(x + (size_t)first * 3 * kSx * kSx, kSx, m, h->mw, h->d_scratch, h->d_tokx, kNx, 0, h->d_planes, h->chunk, st));
-        VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_forward/blocks", run_blocks(h, h->d_tokz, kNz, h->d_tokx, kNx, h->d_tok, m,
+        VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_forward/blocks", run_blocks(h, h->d_tokz, kNz, nullptr, h->d_tokx, kNx, h->d_tok, m,
                                                       taps ? taps + (size_t)first * kN * kC : nullptr, tap_stride, st));
         HeadArgs a = forward_head_args(first, m, pred_boxes, score_map, size_map, offset_map);
         a.tokens = h->d_tok;
@@ -803,28 +898,23 @@ int vt_tracks_init(VtHandle h, const uint8_t* frames, const int64_t* frame_offse
     if (n == 0) { h->tracks_ready = true; return VT_OK; }
     if (!frames || !frame_offsets || !frame_hw || !boxes_xywh) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init: null pointer");
     if (first < 0 || n < 0 || first + n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init: tracks [%d, %d) exceed max_tracks %d", first, first + n, h->cfg.max_tracks);
+    DeviceGuard dg(h->cfg.device);
+    VT_CUDA(h, dg.err);
+    return tracks_init(h, frames, frame_offsets, frame_hw, boxes_xywh, first, nullptr, n, out_status, (cudaStream_t)stream);
+}
+
+int vt_tracks_init_slots(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
+                         const double* boxes_xywh, const int32_t* slots, int32_t n, int32_t* out_status, void* stream) {
+    int rc = check_ready(h, false);
+    if (rc) return rc;
+    if (n < 0 || n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init_slots: n = %d outside [0, max_tracks %d]", n, h->cfg.max_tracks);
+    if (n == 0) { h->tracks_ready = true; return VT_OK; }
+    if (!frames || !frame_offsets || !frame_hw || !boxes_xywh || !slots) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init_slots: null pointer");
     cudaStream_t st = (cudaStream_t)stream;
     DeviceGuard dg(h->cfg.device);
     VT_CUDA(h, dg.err);
-    for (int c0 = 0; c0 < n && h->generic; c0 += h->chunk) {
-        const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
-        VT_LAUNCH(h, VT_STAGE_CROP, m, st, "vt_tracks_init/crop",
-                  launch_crop_normalize(frames, frame_offsets + c0, frame_hw + 2 * c0, boxes_xywh + 4 * c0, h->cfg.template_factor, kTz, m, h->mw.lut,
-                                        h->gws.crop, nullptr, nullptr, nullptr, h->d_status + first + c0, st));
-        VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_init/stem",
-                  gen_launch_stem(h->gws.crop, kTz, m, h->gw, h->gws, h->d_tmpl + (size_t)(first + c0) * kNz * h->cfg.embed_dim, kNz, 0, st));
-    }
-    for (int c0 = 0; c0 < n && !h->generic; c0 += h->chunk) {
-        const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
-        VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_init/crop+stem",
-                  launch_crop_stem(frames, frame_offsets + c0, frame_hw + 2 * c0, boxes_xywh + 4 * c0, h->cfg.template_factor, kTz, m,
-                                   h->mw, h->d_scratch, h->d_tmpl + (size_t)(first + c0) * kNz * kC, kNz, 0, h->d_status + first + c0,
-                                   h->d_planes, h->chunk, h->d_taps, st));
-    }
-    VT_CUDA(h, cudaMemcpyAsync(h->d_state + (size_t)first * 4, boxes_xywh, (size_t)n * 4 * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    if (out_status) VT_CUDA(h, cudaMemcpyAsync(out_status, h->d_status + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
-    h->tracks_ready = true;
-    return VT_OK;
+    VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_init_slots/resolve", launch_resolve_slots(slots, n, h->cfg.max_tracks, h->d_claim, h->d_eff, st));
+    return tracks_init(h, frames, frame_offsets, frame_hw, boxes_xywh, 0, h->d_eff, n, out_status, st);
 }
 
 int vt_tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
@@ -834,47 +924,23 @@ int vt_tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offse
     if (n == 0) return VT_OK;
     if (!frames || !frame_offsets || !frame_hw || !out_boxes) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step: null pointer");
     if (first < 0 || n < 0 || first + n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step: tracks [%d, %d) exceed max_tracks %d", first, first + n, h->cfg.max_tracks);
+    DeviceGuard dg(h->cfg.device);
+    VT_CUDA(h, dg.err);
+    return tracks_step(h, frames, frame_offsets, frame_hw, first, nullptr, n, out_boxes, out_detail, update_state, (cudaStream_t)stream);
+}
+
+int vt_tracks_step_slots(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
+                         const int32_t* slots, int32_t n, double* out_boxes, double* out_detail, int32_t update_state, void* stream) {
+    int rc = check_ready(h, true);
+    if (rc) return rc;
+    if (n < 0 || n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step_slots: n = %d outside [0, max_tracks %d]", n, h->cfg.max_tracks);
+    if (n == 0) return VT_OK;
+    if (!frames || !frame_offsets || !frame_hw || !out_boxes || !slots) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step_slots: null pointer");
     cudaStream_t st = (cudaStream_t)stream;
     DeviceGuard dg(h->cfg.device);
     VT_CUDA(h, dg.err);
-    if (h->generic) {
-        // every stage runs per chunk: crop -> stem into the chunk's token buffer, cached template tokens copied in front
-        const int C = h->cfg.embed_dim;
-        for (int c0 = 0; c0 < n; c0 += h->chunk) {
-            const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
-            const int t0 = first + c0;
-            VT_LAUNCH(h, VT_STAGE_CROP, m, st, "vt_tracks_step/crop",
-                      launch_crop_normalize(frames, frame_offsets + c0, frame_hw + 2 * c0, h->d_state + (size_t)t0 * 4, h->cfg.search_factor, kSx, m,
-                                            h->mw.lut, h->gws.crop, nullptr, nullptr, nullptr, h->d_status + t0, st));
-            VT_CUDA(h, cudaMemcpy2DAsync(h->gws.tok, (size_t)kN * C * sizeof(float), h->d_tmpl + (size_t)t0 * kNz * C, (size_t)kNz * C * sizeof(float),
-                                         (size_t)kNz * C * sizeof(float), m, cudaMemcpyDeviceToDevice, st));
-            VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_step/stem", gen_launch_stem(h->gws.crop, kSx, m, h->gw, h->gws, h->gws.tok, kN, kNz, st));
-            const HeadArgs a = track_head_args(h, first, c0, m, frame_hw, out_boxes, out_detail, update_state);
-            VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_tracks_step/blocks+head", gen_launch_blocks_head(h->gws.tok, m, h->gw, h->gws, a, nullptr, 0, st));
-        }
-        h->last_first = first; h->last_n = n;
-        return VT_OK;
-    }
-    // crop + stem run per chunk (their intermediates are large); blocks + head run once over all n tracks
-    for (int c0 = 0; c0 < n; c0 += h->chunk) {
-        const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
-        const int t0 = first + c0;
-        VT_LAUNCH(h, VT_STAGE_STEM, m, st, "vt_tracks_step/crop+stem",
-                  launch_crop_stem(frames, frame_offsets + c0, frame_hw + 2 * c0, h->d_state + (size_t)t0 * 4, h->cfg.search_factor, kSx, m,
-                                   h->mw, h->d_scratch, h->d_tokx + (size_t)c0 * kNx * kC, kNx, 0, h->d_status + t0,
-                                   h->d_planes, h->chunk, h->d_taps, st));
-    }
-    {
-        const int m = n;
-        VT_LAUNCH(h, VT_STAGE_BLOCKS, m, st, "vt_tracks_step/blocks",
-                  run_blocks(h, h->d_tmpl + (size_t)first * kNz * kC, kNz, h->d_tokx, kNx, h->d_tok, m, nullptr, 0, st));
-        HeadArgs a = track_head_args(h, first, 0, m, frame_hw, out_boxes, out_detail, update_state);
-        a.tokens = h->d_tok;
-        a.use_tc = h->cfg.blocks_impl != VT_BLOCKS_SIMT_FP32;
-        VT_LAUNCH(h, VT_STAGE_HEAD, m, st, "vt_tracks_step/head", launch_head(a, h->mw, st));
-    }
-    h->last_first = first; h->last_n = n;
-    return VT_OK;
+    VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_step_slots/resolve", launch_resolve_slots(slots, n, h->cfg.max_tracks, h->d_claim, h->d_eff, st));
+    return tracks_step(h, frames, frame_offsets, frame_hw, 0, h->d_eff, n, out_boxes, out_detail, update_state, st);
 }
 
 int vt_tracks_get_state(VtHandle h, double* boxes_xywh, int32_t first, int32_t n, void* stream) {

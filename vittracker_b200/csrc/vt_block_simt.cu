@@ -63,7 +63,7 @@ __device__ __forceinline__ void matvec48(const float (&in)[K], const float* W, i
 }
 
 __global__ void __launch_bounds__(kBlkThreads, 1)
-blocks_simt_kernel(const float* __restrict__ tok_z, int z_stride_rows, const float* __restrict__ tok_x,
+blocks_simt_kernel(const float* __restrict__ tok_z, int z_stride_rows, const int32_t* __restrict__ z_slots, const float* __restrict__ tok_x,
                    int x_stride_rows, float* __restrict__ out, ModelW w, float* __restrict__ taps,
                    size_t tap_stride) {
     extern __shared__ __align__(16) float smem[];
@@ -75,7 +75,7 @@ blocks_simt_kernel(const float* __restrict__ tok_z, int z_stride_rows, const flo
     // residual row of token i: template tokens first (vit_dist.py:84)
     float x[kC];
     {
-        const float* src = (i < kNz) ? tok_z + ((size_t)trk * z_stride_rows + i) * kC
+        const float* src = (i < kNz) ? tok_z + ((size_t)max(item_slot(z_slots, trk), 0) * z_stride_rows + i) * kC
                                      : tok_x + ((size_t)trk * x_stride_rows + (i - kNz)) * kC;
 #pragma unroll
         for (int k = 0; k < kC; k += 4) {
@@ -229,12 +229,12 @@ blocks_simt_kernel(const float* __restrict__ tok_z, int z_stride_rows, const flo
     for (int k = 0; k < kC; k += 4) *reinterpret_cast<float4*>(dst + k) = make_float4(x[k], x[k + 1], x[k + 2], x[k + 3]);
 }
 
-int launch_blocks_simt(const float* tok_z, int z_stride_rows, const float* tok_x, int x_stride_rows,
+int launch_blocks_simt(const float* tok_z, int z_stride_rows, const int32_t* z_slots, const float* tok_x, int x_stride_rows,
                        float* out, int n, const ModelW& w, float* taps, size_t tap_stride, cudaStream_t st) {
     if (n <= 0) return 0;
     static DeviceOnce once;
     if (!ensure_dyn_smem(once, blocks_simt_kernel, kBlkSmemBytes)) return -1;
-    blocks_simt_kernel<<<n, kBlkThreads, kBlkSmemBytes, st>>>(tok_z, z_stride_rows, tok_x, x_stride_rows, out, w, taps, tap_stride);
+    blocks_simt_kernel<<<n, kBlkThreads, kBlkSmemBytes, st>>>(tok_z, z_stride_rows, z_slots, tok_x, x_stride_rows, out, w, taps, tap_stride);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
 }
 

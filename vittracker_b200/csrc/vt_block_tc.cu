@@ -234,9 +234,12 @@ __device__ __forceinline__ void gelu_erf2(uint64_t v, float& h0, float& h1) {
 
 }  // namespace
 
-template <int kScoresTerms>
+// kSlots: template rows by slot list (z_slots); the range variant compiles without the lookup, so a range step runs the same code as
+// before slot lists existed.
+template <int kScoresTerms, bool kSlots>
 __global__ void __launch_bounds__(kTcThreads, 1)
-blocks_tc_kernel(const float* __restrict__ tok_z, int z_stride_rows, const float* __restrict__ tok_x, int x_stride_rows,
+blocks_tc_kernel(const float* __restrict__ tok_z, int z_stride_rows, const int32_t* __restrict__ z_slots, const float* __restrict__ tok_x,
+                 int x_stride_rows,
                  float* __restrict__ out, int n, ModelW w, float* __restrict__ taps, size_t tap_stride) {
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -422,11 +425,12 @@ blocks_tc_kernel(const float* __restrict__ tok_z, int z_stride_rows, const float
         for (int trk = blockIdx.x; trk < n; trk += gridDim.x) {
             // residual slice x[t][kCW]: tile t, row 128 t + row, columns [kCW s, kCW s + kCW)
             float x[3][kCW];
+            const size_t zrow = (size_t)(kSlots ? max(z_slots[trk], 0) : trk) * z_stride_rows;
 #pragma unroll
             for (int t = 0; t < 3; ++t) {
                 const int r = 128 * t + row;
                 const float* src = nullptr;
-                if (r < kNz) src = tok_z + ((size_t)trk * z_stride_rows + r) * kC + kCW * s;
+                if (r < kNz) src = tok_z + (zrow + r) * kC + kCW * s;
                 else if (r < kN) src = tok_x + ((size_t)trk * x_stride_rows + (r - kNz)) * kC + kCW * s;
 #pragma unroll
                 for (int i = 0; i < kCW; i += 4) {
@@ -662,14 +666,15 @@ extern "C" int vt_tc_trace_read(long long* host, int* n) {
 }
 #endif
 
-int launch_blocks_tc(const float* tok_z, int z_stride_rows, const float* tok_x, int x_stride_rows, float* out, int n,
+int launch_blocks_tc(const float* tok_z, int z_stride_rows, const int32_t* z_slots, const float* tok_x, int x_stride_rows, float* out, int n,
                      const ModelW& w, float* taps, size_t tap_stride, int num_sms, int scores_terms, cudaStream_t st) {
     if (n <= 0) return 0;
-    static DeviceOnce once1, once3;
-    if (!ensure_dyn_smem(once1, blocks_tc_kernel<1>, kTcSmemBytes) || !ensure_dyn_smem(once3, blocks_tc_kernel<3>, kTcSmemBytes)) return -1;
+    static DeviceOnce once[4];
+    auto kern = scores_terms == 1 ? (z_slots ? blocks_tc_kernel<1, true> : blocks_tc_kernel<1, false>)
+                                  : (z_slots ? blocks_tc_kernel<3, true> : blocks_tc_kernel<3, false>);
+    if (!ensure_dyn_smem(once[(scores_terms == 1 ? 0 : 2) + (z_slots ? 1 : 0)], kern, kTcSmemBytes)) return -1;
     const int grid = n < num_sms ? n : num_sms;
-    if (scores_terms == 1) blocks_tc_kernel<1><<<grid, kTcThreads, kTcSmemBytes, st>>>(tok_z, z_stride_rows, tok_x, x_stride_rows, out, n, w, taps, tap_stride);
-    else blocks_tc_kernel<3><<<grid, kTcThreads, kTcSmemBytes, st>>>(tok_z, z_stride_rows, tok_x, x_stride_rows, out, n, w, taps, tap_stride);
+    kern<<<grid, kTcThreads, kTcSmemBytes, st>>>(tok_z, z_stride_rows, z_slots, tok_x, x_stride_rows, out, n, w, taps, tap_stride);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
 }
 

@@ -18,7 +18,7 @@ constexpr int kCropRows = 8;      // output rows per CTA
 template <int S>
 __global__ void __launch_bounds__(kCropThreads)
 crop_normalize_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict__ frame_offsets,
-                      const int32_t* __restrict__ frame_hw, const double* __restrict__ boxes, double factor,
+                      const int32_t* __restrict__ frame_hw, const double* __restrict__ boxes, const int32_t* __restrict__ slots, double factor,
                       const float* __restrict__ lut, float* __restrict__ out_nchw,
                       uint8_t* __restrict__ out_u8, uint8_t* __restrict__ out_mask,
                       double* __restrict__ out_rf, int32_t* __restrict__ out_status) {
@@ -27,8 +27,9 @@ crop_normalize_kernel(const uint8_t* __restrict__ frames, const int64_t* __restr
 
     const int item = blockIdx.y;
     const int H = frame_hw[2 * item], W = frame_hw[2 * item + 1];
-    const double* bx = boxes + 4 * item;
-    const CropGeom g = crop_geometry(bx[0], bx[1], bx[2], bx[3], factor, S, H, W);
+    const int slot = item_slot(slots, item);
+    const double* bx = boxes + 4 * (size_t)(slot < 0 ? 0 : slot);
+    const CropGeom g = slot < 0 ? CropGeom{0, 0, 0, VT_TRACK_BAD_SLOT_, 0.0} : crop_geometry(bx[0], bx[1], bx[2], bx[3], factor, S, H, W);
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         if (out_rf) out_rf[item] = g.resize_factor;
         if (out_status) out_status[item] = g.status;
@@ -104,7 +105,7 @@ crop_normalize_kernel(const uint8_t* __restrict__ frames, const int64_t* __restr
 }
 
 int launch_crop_normalize(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
-                          const double* boxes, double factor, int S, int n, const float* lut,
+                          const double* boxes, const int32_t* slots, double factor, int S, int n, const float* lut,
                           float* out_nchw, uint8_t* out_u8, uint8_t* out_mask, double* out_rf,
                           int32_t* out_status, cudaStream_t st) {
     if (n <= 0) return 0;
@@ -119,12 +120,14 @@ int launch_crop_normalize(const uint8_t* frames, const int64_t* frame_offsets, c
         uint8_t* mk = out_mask ? out_mask + (size_t)first * plane : nullptr;
         double* rf = out_rf ? out_rf + first : nullptr;
         int32_t* stt = out_status ? out_status + first : nullptr;
+        const double* bx = slots ? boxes : boxes + 4 * first;
+        const int32_t* sl = slots ? slots + first : nullptr;
         if (S == 256)
             crop_normalize_kernel<256><<<grid, kCropThreads, 0, st>>>(frames, frame_offsets + first, frame_hw + 2 * first,
-                                                                     boxes + 4 * first, factor, lut, o, u, mk, rf, stt);
+                                                                     bx, sl, factor, lut, o, u, mk, rf, stt);
         else if (S == 128)
             crop_normalize_kernel<128><<<grid, kCropThreads, 0, st>>>(frames, frame_offsets + first, frame_hw + 2 * first,
-                                                                     boxes + 4 * first, factor, lut, o, u, mk, rf, stt);
+                                                                     bx, sl, factor, lut, o, u, mk, rf, stt);
         else
             return -1;
         ++launched;

@@ -52,14 +52,20 @@ __device__ __forceinline__ void decode_box(const HeadArgs& a, int trk, const flo
         pb[3] = numeric_status ? qnan : m_size[256 + raw_idx];
     }
     if (a.state) {
-        double* st = a.state + (size_t)trk * 4;
+        double* ob = a.out_boxes + (size_t)trk * 5;
+        double* od = a.out_detail ? a.out_detail + (size_t)trk * 8 : nullptr;
+        const int slot = item_slot(a.slots, trk);
+        if (slot < 0) {               // bad slot-list entry: no state to read or write
+            ob[0] = ob[1] = ob[2] = ob[3] = 0.0; ob[4] = -1.0;
+            if (od) { od[0] = od[1] = od[2] = od[3] = od[4] = 0.0; od[5] = -1.0; od[6] = (double)VT_TRACK_BAD_SLOT_; od[7] = 0.0; }
+            return;
+        }
+        double* st = a.state + (size_t)slot * 4;
         const double sx = st[0], sy = st[1], sw = st[2], sh = st[3];
         const int H = a.frame_hw[2 * trk], W = a.frame_hw[2 * trk + 1];
         const CropGeom g = crop_geometry(sx, sy, sw, sh, a.search_factor, kSx, H, W);
         int status = a.status ? a.status[trk] : g.status;
         if (status == 0) status = numeric_status;
-        double* ob = a.out_boxes + (size_t)trk * 5;
-        double* od = a.out_detail ? a.out_detail + (size_t)trk * 8 : nullptr;
         if (status != 0) {            // the reference raises here; keep the state and flag the track
             ob[0] = sx; ob[1] = sy; ob[2] = sw; ob[3] = sh; ob[4] = -1.0;
             if (od) { od[0] = od[1] = od[2] = od[3] = 0.0; od[4] = g.resize_factor; od[5] = -1.0; od[6] = (double)status; od[7] = 0.0; }

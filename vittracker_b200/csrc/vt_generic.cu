@@ -658,7 +658,7 @@ __global__ void __launch_bounds__(256) gen_decode_kernel(const float* __restrict
     if (a.score_map) a.score_map[(size_t)trk * 256 + tid] = sc;
     if (a.size_map) { a.size_map[(size_t)trk * 512 + tid] = sw; a.size_map[(size_t)trk * 512 + 256 + tid] = sh; }
     if (a.offset_map) { a.offset_map[(size_t)trk * 512 + tid] = ox; a.offset_map[(size_t)trk * 512 + 256 + tid] = oy; }
-    const int any_bad = __syncthreads_or(bad);
+    const int any_bad = __syncthreads_or(bad | (a.state && item_slot(a.slots, trk) < 0));
     if (any_bad) {                                   // never a silent wrong answer (see head_finish in vt_head.cu)
         const float qnan = __int_as_float(0x7fc00000);
         if (a.score_map) a.score_map[(size_t)trk * 256 + tid] = qnan;

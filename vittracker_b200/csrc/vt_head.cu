@@ -244,7 +244,7 @@ __device__ __forceinline__ void head_finish(const HeadArgs& a, const ModelW& w, 
         if (a.size_map) { a.size_map[(size_t)trk * 512 + tid] = sw; a.size_map[(size_t)trk * 512 + 256 + tid] = sh; }
         if (a.offset_map) { a.offset_map[(size_t)trk * 512 + tid] = o[1][0]; a.offset_map[(size_t)trk * 512 + 256 + tid] = o[1][1]; }
     }
-    const int any_bad = __syncthreads_or(bad);
+    const int any_bad = __syncthreads_or(bad | (a.state && item_slot(a.slots, trk) < 0));
     if (any_bad) {
         // never a silent wrong answer: the maps of a track whose activations left the representable range are NaN (ReLU and the
         // sigmoid would otherwise squash inf / NaN into plausible numbers), and the tracker output carries VT_TRACK_NUMERIC_RANGE

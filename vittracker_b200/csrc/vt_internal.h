@@ -19,6 +19,7 @@ constexpr int kSx = 256;        // search crop side
 constexpr float kLnEps = 1e-5f;
 constexpr float kF16Max = 65504.f;           // largest finite fp16: operands of the tensor-core path are fp16 hi + lo
 constexpr int VT_TRACK_NUMERIC_RANGE_ = 3;    // == VT_TRACK_NUMERIC_RANGE of include/vittrack_b200.h
+constexpr int VT_TRACK_BAD_SLOT_ = 4;         // == VT_TRACK_BAD_SLOT
 
 #ifdef __CUDACC__
 // Hardswish exactly as PyTorch evaluates it, x * relu6(x + 3) / 6 (vit_dist.py:41, torch.nn.Hardswish): the product is rounded to fp32 and
@@ -250,8 +251,13 @@ int launch_yuv420_rect(int format, const YuvDesc& d, int num_sms, cudaStream_t s
 int launch_yuv420_crop_to_rgb(int format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw, const double* boxes,
                               double factor, uint8_t* dst, const int64_t* dst_offsets, int n, int num_sms, cudaStream_t st);
 
+// Slot lists (the vt_tracks_*_slots entry points): a kernel that reads per-track state takes `slots` (nullable).  Item i reads the
+// state of track slots[i], or of track i of the pre-offset state pointer when slots == NULL (the range calls); a negative slot is a
+// bad entry (VT_TRACK_BAD_SLOT): its state is not read or written.
+__host__ __device__ inline int item_slot(const int32_t* slots, int item) { return slots ? slots[item] : item; }
+
 int launch_crop_normalize(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
-                          const double* boxes, double factor, int S, int n, const float* lut,
+                          const double* boxes, const int32_t* slots, double factor, int S, int n, const float* lut,
                           float* out_nchw, uint8_t* out_u8, uint8_t* out_mask, double* out_rf,
                           int32_t* out_status, cudaStream_t st);
 
@@ -272,25 +278,26 @@ __host__ __device__ constexpr size_t tc_planes_bytes_per_track() {
 int launch_stem34_tc(const uint8_t* planes3, int n, const ModelW& w, uint8_t* planes4, float* tokens, int tok_stride_rows, int tok_off,
                      cudaStream_t st);
 // Fused front of the search-branch stem (vt_stem_fused.cu): tap tables + crop gather -> conv1 -> conv2 on tcgen05 -> planes3
-int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes, double factor,
-                             int n, const ModelW& w, int32_t* out_status, void* tap_tables, uint8_t* planes3, cudaStream_t st);
+int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
+                             const int32_t* slots, double factor, int n, const ModelW& w, int32_t* out_status, void* tap_tables, uint8_t* planes3, cudaStream_t st);
 void stem1_tc_pack(const float* wf, const float* bf, uint8_t* blob, float* par);
 size_t stem_tc_weight_bytes(int layer);
 void stem_tc_pack_weights(int cin, int cch, int cout, int npad, const float* wf, uint8_t* hi8, uint8_t* lo8);
 
 // Crop + stem straight from raw uint8 frames (the first conv layer gathers its tile from the frame).
 int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
-                     double factor, int S, int n, const ModelW& w, float* scratch, float* tokens, int tok_stride_rows,
+                     const int32_t* slots, double factor, int S, int n, const ModelW& w, float* scratch, float* tokens, int tok_stride_rows,
                      int tok_off, int32_t* out_status, uint8_t* planes, int plane_tracks, void* tap_tables, cudaStream_t st);
 size_t crop_taps_bytes(int n);      // size of the tap-table buffer launch_crop_stem needs for n tracks
 
-// ViT blocks (fp32 SIMT): tokens_z [n][64][48] (stride z_stride rows per track), tokens_x likewise; in place
+// ViT blocks (fp32 SIMT): tokens_z [n][64][48] (stride z_stride rows per track; item i reads row block item_slot(z_slots, i), a negative
+// slot reads block 0), tokens_x likewise (by item); in place
 // result written to out [n][320][48]; taps (or null) receives [depth][n][320][48].
-int launch_blocks_simt(const float* tok_z, int z_stride_rows, const float* tok_x, int x_stride_rows,
+int launch_blocks_simt(const float* tok_z, int z_stride_rows, const int32_t* z_slots, const float* tok_x, int x_stride_rows,
                        float* out, int n, const ModelW& w, float* taps, size_t tap_stride, cudaStream_t st);
 
 // ViT blocks on the tcgen05 tensor cores (fp16 hi/lo split operands, fp32 accumulation in TMEM).
-int launch_blocks_tc(const float* tok_z, int z_stride_rows, const float* tok_x, int x_stride_rows,
+int launch_blocks_tc(const float* tok_z, int z_stride_rows, const int32_t* z_slots, const float* tok_x, int x_stride_rows,
                      float* out, int n, const ModelW& w, float* taps, size_t tap_stride, int num_sms, int scores_terms, cudaStream_t st);
 
 struct HeadArgs {
@@ -300,7 +307,8 @@ struct HeadArgs {
     float *pred_boxes, *score_map, *size_map, *offset_map;   // [n][4], [n][256], [n][2][256], [n][2][256]
     float* tokens_norm;       // [n][320][48] tap (nullable)
     // tracker outputs (nullable as a group: enabled when state != nullptr)
-    double* state;            // [n][4] previous boxes, updated in place when update_state
+    double* state;            // [n][4] previous boxes, updated in place when update_state; item i's is row item_slot(slots, i)
+    const int32_t* slots;     // [n] or null (see item_slot); a negative slot: maps NaN, status VT_TRACK_BAD_SLOT, state untouched
     const int32_t* frame_hw;  // [n][2]
     const int32_t* status;    // [n] VT_TRACK_* from the crop stage (nullable)
     double* out_boxes;        // [n][5]
@@ -365,5 +373,17 @@ int gen_launch_stem(const float* img, int S, int n, const GenModelW& w, const Ge
 // Blocks (in place on tokens [n][320][C]) + final LayerNorm (-> ws.ln) + head + decode.  taps: [depth + 2][n][320][C] or null.
 int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWork& ws, const HeadArgs& a, float* taps,
                            size_t tap_stride, cudaStream_t st);
+
+// ---- slot lists (vt_slots.cu) ---------------------------------------------------------------------
+// slots [n] as the caller gave them -> eff [n]: the slot, or -1 for an entry outside [0, max_tracks) or repeating an earlier item's.
+// claim: [max_tracks] uint32, all 0xffffffff between calls (the second kernel restores what the first changed).
+int launch_resolve_slots(const int32_t* slots, int n, int max_tracks, uint32_t* claim, int32_t* eff, cudaStream_t st);
+// Gather: dst + i * dst_stride <- src + eff[i] * src_stride, `row` floats (zeros for eff[i] < 0).
+int launch_gather_rows(const float* src, size_t src_stride, float* dst, size_t dst_stride, size_t row, const int32_t* eff, int n,
+                       cudaStream_t st);
+// Template scatter of vt_tracks_init_slots: for eff[i] >= 0, tmpl + eff[i] * row <- tok + i * row, state[eff[i]] <- boxes[i]; out_status[i]
+// (nullable) <- status[i], or VT_TRACK_BAD_SLOT for eff[i] < 0.
+int launch_scatter_init(const float* tok, float* tmpl, size_t row, const double* boxes, double* state, const int32_t* status,
+                        int32_t* out_status, const int32_t* eff, int n, cudaStream_t st);
 
 }  // namespace vt

@@ -487,12 +487,12 @@ size_t crop_taps_bytes(int n) { return (size_t)n * 2 * kTapPitch * sizeof(int4) 
 
 template <int S>
 static int run_crop_conv1(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
-                          double factor, int n, const ModelW& w, float* out, int32_t* out_status, int4* taps, cudaStream_t st) {
+                          const int32_t* slots, double factor, int n, const ModelW& w, float* out, int32_t* out_status, int4* taps, cudaStream_t st) {
     auto kern = crop_conv1_kernel<S>;
     static DeviceOnce once;
     if (!ensure_dyn_smem(once, kern, kCc1SmemBytes)) return -1;
     constexpr int tiles = (S / 64) * (S / 64);
-    crop_taps_kernel<S><<<n, 288, 0, st>>>(frame_hw, boxes, factor, taps, out_status, nullptr, 0);
+    crop_taps_kernel<S><<<n, 288, 0, st>>>(frame_hw, boxes, slots, factor, taps, out_status, nullptr, 0);
     int launched = 1;
     for (int first = 0; first < n; first += 32768) {
         const int m = min(32768, n - first);
@@ -505,7 +505,7 @@ static int run_crop_conv1(const uint8_t* frames, const int64_t* frame_offsets, c
 
 // Crop + stem straight from raw frames (fused first layer); same outputs as launch_crop_normalize + launch_stem.
 int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
-                     double factor, int S, int n, const ModelW& w, float* scratch, float* tokens, int tok_stride_rows,
+                     const int32_t* slots, double factor, int S, int n, const ModelW& w, float* scratch, float* tokens, int tok_stride_rows,
                      int tok_off, int32_t* out_status, uint8_t* planes, int plane_tracks, void* tap_tables, cudaStream_t st) {
     if (n <= 0) return 0;
     int4* taps = reinterpret_cast<int4*>(tap_tables);
@@ -519,13 +519,13 @@ int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const 
         // buffer keeps conv2's operand image first (launch_stem writes it), so conv3's image starts after it.
         uint8_t* planes3 = planes + (size_t)plane_tracks * tc_planes_bytes(kConv2Cch, kConv2Wout);
         uint8_t* planes4 = planes3 + (size_t)plane_tracks * tc_planes_bytes(kConv3Cch, kConv3Wout);
-        if ((r = launch_crop_stem12_fused(frames, frame_offsets, frame_hw, boxes, factor, n, w, out_status, tap_tables, planes3, st)) < 0) return r;
+        if ((r = launch_crop_stem12_fused(frames, frame_offsets, frame_hw, boxes, slots, factor, n, w, out_status, tap_tables, planes3, st)) < 0) return r;
         total += r;
         if ((r = launch_stem34_tc(planes3, n, w, planes4, tokens, tok_stride_rows, tok_off, st)) < 0) return r;
         return total + r;
     }
-    if (S == 256) r = run_crop_conv1<256>(frames, frame_offsets, frame_hw, boxes, factor, n, w, a1, out_status, taps, st);
-    else if (S == 128) r = run_crop_conv1<128>(frames, frame_offsets, frame_hw, boxes, factor, n, w, a1, out_status, taps, st);
+    if (S == 256) r = run_crop_conv1<256>(frames, frame_offsets, frame_hw, boxes, slots, factor, n, w, a1, out_status, taps, st);
+    else if (S == 128) r = run_crop_conv1<128>(frames, frame_offsets, frame_hw, boxes, slots, factor, n, w, a1, out_status, taps, st);
     else return -1;
     if (r < 0) return r;
     total += r;

@@ -460,8 +460,8 @@ stem12_fused_kernel(const uint8_t* __restrict__ frames, const int64_t* __restric
 
 // Search crop of n tracks straight from the raw frames -> conv3's operand image (planes3): tap tables + the fused kernel.
 // tap_tables: crop_taps_bytes(n) bytes; the fused kernel's work counter sits behind the n tables.
-int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes, double factor,
-                             int n, const ModelW& w, int32_t* out_status, void* tap_tables, uint8_t* planes3, cudaStream_t st) {
+int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
+                             const int32_t* slots, double factor, int n, const ModelW& w, int32_t* out_status, void* tap_tables, uint8_t* planes3, cudaStream_t st) {
     if (n <= 0) return 0;
     using F = Fused;
     auto kern = stem12_fused_kernel;
@@ -487,7 +487,7 @@ int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets
     const int grid = n_units < grid_caps[dev] ? n_units : grid_caps[dev];
     int4* taps = reinterpret_cast<int4*>(tap_tables);
     int* work_counter = reinterpret_cast<int*>(taps + (size_t)n * 2 * kTapPitch);
-    crop_taps_kernel<kSx><<<n, 288, 0, st>>>(frame_hw, boxes, factor, taps, out_status, work_counter, grid);
+    crop_taps_kernel<kSx><<<n, 288, 0, st>>>(frame_hw, boxes, slots, factor, taps, out_status, work_counter, grid);
     if (cudaGetLastError() != cudaSuccess) return -1;
     kern<<<grid, kFThreads, F::kSmemBytes, st>>>(frames, frame_offsets, taps, w.stem1_tc_w, w.stem1_tc_par, w.stem_tc_w[0], w.stem_tc_b[0],
                                                  planes3, n_units, n_big, unit_bands, work_counter);

@@ -13,11 +13,13 @@ namespace vt {
 // tap that is inside the image, so the six bytes read always are).  Rows: .x/.y = byte offsets of the two tap rows
 // (0 when the row is padding), .z = weights lo | hi << 16.  .w = 1 when the position is outside the resized crop
 // (= the convolution's zero padding, which is 0.0f and not the normalised pixel 0).
+// The box of item i is track item_slot(slots, i) of `boxes`; a bad slot gives status VT_TRACK_BAD_SLOT and empty tables.
 // `work_counter` (may be null) is the consumer kernel's dynamic work counter: block 0 resets it to `work_counter0` on the way.
 constexpr int kTapPitch = 264;
 template <int S>
 __global__ void __launch_bounds__(288)
-crop_taps_kernel(const int32_t* __restrict__ frame_hw, const double* __restrict__ boxes, double factor, int4* __restrict__ taps,
+crop_taps_kernel(const int32_t* __restrict__ frame_hw, const double* __restrict__ boxes, const int32_t* __restrict__ slots, double factor,
+                 int4* __restrict__ taps,
                  int32_t* __restrict__ out_status, int* __restrict__ work_counter, int work_counter0) {
     __shared__ CropGeom sg;
     __shared__ double s_scale;
@@ -25,9 +27,15 @@ crop_taps_kernel(const int32_t* __restrict__ frame_hw, const double* __restrict_
     const int H = frame_hw[2 * item], W = frame_hw[2 * item + 1];
     if (item == 0 && tid == 287 && work_counter) *work_counter = work_counter0;
     if (tid == 0) {
-        const double* bx = boxes + 4 * item;
-        sg = crop_geometry(bx[0], bx[1], bx[2], bx[3], factor, S, H, W);
-        s_scale = resize_scale(S, sg.crop_sz);
+        const int slot = item_slot(slots, item);
+        if (slot < 0) {
+            sg = CropGeom{0, 0, 0, VT_TRACK_BAD_SLOT_, 0.0};
+            s_scale = 0.0;
+        } else {
+            const double* bx = boxes + 4 * (size_t)slot;
+            sg = crop_geometry(bx[0], bx[1], bx[2], bx[3], factor, S, H, W);
+            s_scale = resize_scale(S, sg.crop_sz);
+        }
         if (out_status) out_status[item] = sg.status;
     }
     __syncthreads();

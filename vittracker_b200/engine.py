@@ -262,6 +262,37 @@ class Engine:
                                                 _ptr(out_boxes), _ptr(out_detail), 1 if update_state else 0, self._stream()))
         return (out_boxes, out_detail) if detail else out_boxes
 
+    def _slot_tensor(self, slots: torch.Tensor, n: int) -> torch.Tensor:
+        if slots.dtype != torch.int32 or slots.device != self.device or not slots.is_contiguous() or tuple(slots.shape) != (n,):
+            raise ValueError(f"slots: expected a contiguous int32 tensor of shape ({n},) on {self.device}")
+        return slots
+
+    def tracks_init_slots(self, frames, frame_offsets, frame_hw, boxes, slots: torch.Tensor) -> torch.Tensor:
+        """vt_tracks_init_slots: item i initialises track ``slots[i]`` (int32 device tensor [n]).  Returns the status per item
+        (VT_TRACK_BAD_SLOT for an entry outside [0, max_tracks) or repeating an earlier one)."""
+        n = boxes.shape[0]
+        assert boxes.dtype == torch.float64 and boxes.is_contiguous() and boxes.device == self.device
+        self._slot_tensor(slots, n)
+        status = torch.empty((n,), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_tracks_init_slots(self.handle, _ptr(frames), _ptr(frame_offsets), _ptr(frame_hw), _ptr(boxes),
+                                                      _ptr(slots), int(n), _ptr(status), self._stream()))
+        return status
+
+    def tracks_step_slots(self, frames, frame_offsets, frame_hw, slots: torch.Tensor, out_boxes: Optional[torch.Tensor] = None,
+                          out_detail: Optional[torch.Tensor] = None, update_state: bool = True, detail: bool = False):
+        """vt_tracks_step_slots: item i steps track ``slots[i]`` (int32 device tensor [n]); outputs are in item order."""
+        n = int(slots.shape[0])
+        self._slot_tensor(slots, n)
+        if out_boxes is None:
+            out_boxes = torch.empty((n, 5), dtype=torch.float64, device=self.device)
+        if detail and out_detail is None:
+            out_detail = torch.empty((n, 8), dtype=torch.float64, device=self.device)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_tracks_step_slots(self.handle, _ptr(frames), _ptr(frame_offsets), _ptr(frame_hw), _ptr(slots), n,
+                                                      _ptr(out_boxes), _ptr(out_detail), 1 if update_state else 0, self._stream()))
+        return (out_boxes, out_detail) if detail else out_boxes
+
     def tracks_get_state(self, first: int = 0, n: Optional[int] = None) -> torch.Tensor:
         n = self.max_tracks - first if n is None else n
         out = torch.empty((n, 4), dtype=torch.float64, device=self.device)

@@ -4,8 +4,8 @@ The reference evaluates a dataset with ``multiprocessing.Pool`` - one process, o
 worker, ``worker_id % num_gpu`` picks the GPU (lib/test/evaluation/running.py:105-113,159-187) - and
 ``Tracker._track_sequence`` (lib/test/evaluation/tracker.py:90-152) walks the frames.  Here ``slots`` sequences share one
 ``BatchedTracker``: every step uploads the next frame of each running sequence, advances all of them with one
-``vt_tracks_step``, and a slot whose sequence ended is re-initialised with the next pending one (ragged lengths, mixed
-frame sizes).  Outputs keep the reference's shape - per sequence ``{'target_bbox': [[x, y, w, h], ...], 'time': [...]}``
+``vt_tracks_step_slots`` over the running slots, and a slot whose sequence ended is re-initialised with the next pending one
+(ragged lengths, mixed frame sizes).  Outputs keep the reference's shape - per sequence ``{'target_bbox': [[x, y, w, h], ...], 'time': [...]}``
 with the init box as entry 0 - and ``save_tracker_output`` writes the same ``<seq>.txt`` / ``<seq>_time.txt`` files
 (running.py:14-102), so the analysis tooling reads them unchanged."""
 from __future__ import annotations
@@ -17,6 +17,8 @@ from concurrent.futures import Future, ThreadPoolExecutor
 from typing import Callable, Dict, List, Optional, Sequence as Seq, Union
 
 import numpy as np
+
+from .batched import check_slots
 
 Frame = Union[np.ndarray, str, bytes, list, Callable[[], np.ndarray]]
 
@@ -135,7 +137,7 @@ def crop_rect(box, factor: float, H: int, W: int) -> Optional[tuple]:
 
 
 class BatchedBackend:
-    """The device side of the driver: per-slot initialise, one step for a prefix of slots.  Split from the scheduler so
+    """The device side of the driver: per-slot initialise, one step for the running slots.  Split from the scheduler so
     that the scheduling logic is testable without a GPU.
 
     Uploads are ROW-STAGED like the batch-1 tracker's (tracker.py `_upload`): a step sends, per slot, only the frame rows its search
@@ -167,7 +169,9 @@ class BatchedBackend:
         self._pool = ThreadPoolExecutor(max_workers=stage_workers, thread_name_prefix="vt-stage") if stage_workers > 0 else None
         self._workers = max(1, stage_workers)
         self.bytes_uploaded = 0
-        # idle slots keep tracking a small black frame so that a step can always cover a contiguous slot range
+        self._slot_ids = torch.zeros((slots,), dtype=torch.int32).pin_memory()
+        self._slot_ids_np = self._slot_ids.numpy()
+        # step(): idle slots keep tracking a small black frame so that a step can cover a contiguous slot range
         self._dummy = np.zeros((64, 64, 3), dtype=np.uint8)
         self._dummy_box = [24.0, 24.0, 16.0, 16.0]
 
@@ -232,8 +236,8 @@ class BatchedBackend:
 
     def initialize_many(self, items) -> List[Optional[Exception]]:
         """items = [(slot, image, box), ...] -> per item None or the exception the reference's initialize() would have raised.  One staging
-        pass + upload for all of them (only the rows the template crop reads, like a step) and one vt_tracks_init per run of consecutive
-        slots, instead of a staging pass, a launch and a blocking status read per sequence."""
+        pass + upload for all of them (only the rows the template crop reads, like a step) and one vt_tracks_init_slots, instead of a
+        staging pass, a launch and a blocking status read per sequence."""
         torch = self.torch
         errors: List[Optional[Exception]] = [None] * len(items)
         ok = []
@@ -245,29 +249,23 @@ class BatchedBackend:
                 errors[k] = e
         if not ok:
             return errors
-        ok.sort(key=lambda k: items[k][0])
         frames = [items[k][1] for k in ok]
         rois = None
         if self.row_staging:
             rois = [crop_rows(items[k][2], self.template_factor, items[k][1].shape[0]) for k in ok]
         offs = self._stage(frames, rois)
         m = len(ok)
-        meta = np.zeros((m, 7), dtype=np.float64)               # H, W, offset (exact in fp64: < 2^53), box
+        meta = np.zeros((m, 8), dtype=np.float64)               # H, W, offset (exact in fp64: < 2^53), box, slot
         for j, k in enumerate(ok):
             f = frames[j]
             meta[j, 0], meta[j, 1], meta[j, 2] = f.shape[0], f.shape[1], offs[j]
             meta[j, 3:7] = [float(v) for v in items[k][2]]
+            meta[j, 7] = items[k][0]
         hw = torch.from_numpy(meta[:, 0:2].astype(np.int32)).to(self.dev)
         off = torch.from_numpy(meta[:, 2].astype(np.int64)).to(self.dev)
         bx = torch.from_numpy(np.ascontiguousarray(meta[:, 3:7])).to(self.dev)
-        status = torch.empty((m,), dtype=torch.int32, device=self.dev)
-        j = 0
-        while j < m:                                             # runs of consecutive slots
-            e = j + 1
-            while e < m and items[ok[e]][0] == items[ok[e - 1]][0] + 1:
-                e += 1
-            status[j:e] = self.bt.engine.tracks_init(self._devbuf, off[j:e], hw[j:e], bx[j:e], first=items[ok[j]][0])
-            j = e
+        slots = self.bt._slots(meta[:, 7].astype(np.int64))
+        status = self.bt._init_slots(self._devbuf, off, hw, bx, slots)
         codes = status.cpu().numpy()
         for j, k in enumerate(ok):
             code = int(codes[j])
@@ -289,13 +287,22 @@ class BatchedBackend:
         self.initialize(slot, self._dummy, self._dummy_box)
 
     def step(self, images: List[Optional[np.ndarray]]) -> np.ndarray:
-        """images[i] = next frame of slot i (None = idle); returns [len(images), 5] boxes + confidence."""
+        """images[i] = next frame of slot i (None = idle, tracking the parked dummy frame); returns [len(images), 5] boxes + confidence."""
+        return self._step(list(range(len(images))), [self._dummy if im is None else im for im in images], None)
+
+    def step_active(self, slots: List[int], images: List[np.ndarray]) -> np.ndarray:
+        """images[j] = next frame of slot slots[j]; stages and steps only those slots.  Returns [len(slots), 5] boxes + confidence, in the
+        order of `slots`."""
+        return self._step(check_slots(slots, self.slots), images, slots)
+
+    def _step(self, ids: List[int], frames: List[np.ndarray], slots: Optional[List[int]]) -> np.ndarray:
         torch = self.torch
-        n = len(images)
-        frames = [self._dummy if im is None else im for im in images]
+        n = len(frames)
+        if n == 0:
+            return np.zeros((0, 5))
         rois = None
         if self.row_staging:
-            rois = [crop_rows(self._state[i], self.search_factor, f.shape[0]) if self._state[i] is not None else None for i, f in enumerate(frames)]
+            rois = [crop_rows(self._state[t], self.search_factor, f.shape[0]) if self._state[t] is not None else None for t, f in zip(ids, frames)]
         offs = self._stage(frames, rois)
         hw_np, off_np = self._hw_np, self._off_np
         for i, f in enumerate(frames):
@@ -303,15 +310,19 @@ class BatchedBackend:
         off_np[:n] = offs
         hw = self._hw[:n].to(self.dev, non_blocking=True)
         off = self._off[:n].to(self.dev, non_blocking=True)
-        out = self.bt.engine.tracks_step(self._devbuf, off, hw, first=0, n=n, update_state=True)
+        if slots is None:
+            out = self.bt.engine.tracks_step(self._devbuf, off, hw, first=0, n=n, update_state=True)
+        else:
+            self._slot_ids_np[:n] = slots
+            out = self.bt._step_slots(self._devbuf, off, hw, self._slot_ids[:n].to(self.dev, non_blocking=True), True, False)
         self._out_pin[:n].copy_(out, non_blocking=True)
         torch.cuda.current_stream(self.dev).synchronize()
         res = self._out_pin[:n].numpy().copy()
         boxes = res[:, :4].tolist()
         good = (res[:, 4] >= 0).tolist()
-        for i in range(n):
+        for i, t in enumerate(ids):
             if good[i]:                                                # a flagged track keeps its state on the device too
-                self._state[i] = boxes[i]
+                self._state[t] = boxes[i]
         return res
 
 
@@ -439,7 +450,9 @@ class MultiSequenceRunner:
             if not active:
                 break
             high = max(active) + 1
-            for i in range(high):
+            # a backend with step_active steps just the running slots; otherwise a step covers slots [0, high), idle ones parked
+            step_active = getattr(self.backend, "step_active", None)
+            for i in range(high if step_active is None else 0):
                 if self.slots[i].seq is None and not self._parked[i]:
                     self.backend.park(i)
                     self._parked[i] = True
@@ -447,7 +460,12 @@ class MultiSequenceRunner:
             images = self._step_images(high)
             active = [i for i in active if self.slots[i].seq is not None]      # minus the sequences whose frame could not be read
             self._prefetch_next(active)                                        # decode step t + 1 while the device runs step t
-            boxes = self.backend.step(images)
+            if step_active is None:
+                boxes = self.backend.step(images)
+            else:
+                boxes = np.zeros((high, 5))
+                if active:
+                    boxes[active] = step_active(active, [images[i] for i in active])
             # `time`: the reference records the wall time of one sequence's track() call (tracker.py:139-146); a batched step
             # advances every running sequence at once, so each is charged its share of the step - sum(time) over all sequences
             # is the wall time spent tracking, and the printed FPS is this sequence's share of the batched throughput
