@@ -48,7 +48,8 @@ typedef enum VtStatus {
 #define VT_TRACK_NUMERIC_RANGE 3  /* an activation was non-finite, or left the fp16 operand range of the
                                    * tensor-core path (|v| >= 65504; operands are fp16 hi + lo): the result is
                                    * withheld (state kept, confidence -1, maps NaN) instead of silently wrong.
-                                   * Rerun the track with VT_BLOCKS_SIMT_FP32 (all fp32).                    */
+                                   * vt_set_range_fallback recomputes such tracks on the fp32 kernels within the
+                                   * same step call.                                                           */
 #define VT_TRACK_BAD_SLOT 4       /* slot outside [0, max_tracks) or named by an earlier item of the same call */
 
 /* Which implementation of the ViT blocks vt_forward / vt_tracks_step use. */
@@ -186,6 +187,28 @@ int vt_tracks_init_slots(VtHandle h, const uint8_t* frames, const int64_t* frame
 int vt_tracks_step_slots(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
                          const int32_t* slots, int32_t n, double* out_boxes, double* out_detail, int32_t update_state,
                          void* stream);
+
+/* Range fallback (off by default).  With enable != 0, every item of vt_tracks_step / vt_tracks_step_slots that the tensor-core
+ * kernels end with VT_TRACK_NUMERIC_RANGE is recomputed on the fp32 kernels of VT_BLOCKS_SIMT_FP32 before the call returns.
+ *   counter_dev  optional DEVICE int64: each step adds the number of items it recomputed (no host synchronisation to read it).
+ *                A CUDA graph captured while it is set keeps adding to that address on every replay: it must outlive such graphs.
+ * Contract:
+ *   1. A recomputed item's out_boxes, out_detail, maps (vt_tracks_last_maps) and new state are, bit for bit, what a
+ *      VT_BLOCKS_SIMT_FP32 handle with the same weights, template frame and box, and state gives for that track, for range and
+ *      slot-list steps, update_state 0 and 1, in any chunk.
+ *   2. An item that is not recomputed is bit-identical to the same handle with the fallback off.
+ *   3. An item the fp32 kernels flag too (a non-finite activation) keeps VT_TRACK_NUMERIC_RANGE, with the fp32 pass's outputs.
+ *   4. Items with VT_TRACK_TOO_SMALL, VT_TRACK_OUT_OF_DOMAIN or VT_TRACK_BAD_SLOT are never recomputed.
+ *   5. The step still allocates nothing and does not synchronise: it can be captured in a CUDA graph, and a replay recomputes
+ *      whichever items that replay flags.
+ * Detection: an item is recomputed when its confidence is -1 (a real one is a clamped sigmoid in [1e-4, 0.9999]), its crop status
+ * is 0 and its slot is valid.  The host never learns how many there are, so the fp32 kernels are launched as for every item of
+ * the step and work only on the items below the device count: nine extra launches per step at one chunk (one compaction, five for
+ * the fp32 crop + stem, blocks, head, one scatter), five more per further chunk.
+ * This call allocates the compacted per-item arrays and output rows (about 5.3 KB per track of max_tracks) the first time it
+ * enables the fallback.  VT_ERR_UNSUPPORTED for configurations other than vit_48_h32 (their fp32 route has no device-side item
+ * count); a VT_BLOCKS_SIMT_FP32 handle returns VT_OK and changes nothing (it has no fp16 operands). */
+int vt_set_range_fallback(VtHandle h, int32_t enable, int64_t* counter_dev);
 
 /* Read / overwrite the per-track boxes ([n][4] float64 device pointers). */
 int vt_tracks_get_state(VtHandle h, double* boxes_xywh, int32_t first, int32_t n, void* stream);

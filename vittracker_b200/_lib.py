@@ -51,6 +51,7 @@ SIGNATURES = {
     "vt_tracks_step": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, C.c_int32, _P]),
     "vt_tracks_init_slots": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "vt_tracks_step_slots": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, C.c_int32, _P]),
+    "vt_set_range_fallback": (C.c_int, [_P, C.c_int32, _P]),
     "vt_tracks_get_state": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P]),
     "vt_tracks_set_state": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P]),
     "vt_tracks_last_maps": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P]),

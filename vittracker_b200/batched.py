@@ -187,14 +187,22 @@ class BatchedTracker:
 
     Without ``slots`` these calls work on tracks 0..n-1.  With ``slots`` (a host sequence of ints, checked here, or a CUDA integer
     tensor, passed through: the device gives a bad entry status VT_TRACK_BAD_SLOT), item i works on track ``slots[i]`` and results come
-    back in slot-list order, so targets can be added to free slots, retired, and the live set stepped in one call."""
+    back in slot-list order, so targets can be added to free slots, retired, and the live set stepped in one call.
+
+    ``range_fallback=True`` recomputes, within the same step, every track the tensor-core kernels flag as out of fp16 range
+    (VT_TRACK_NUMERIC_RANGE) on the fp32 kernels: such a track gets the result a ``blocks_impl="simt"`` tracker would give instead of
+    confidence -1.  ``fallback_items`` counts the recomputed items."""
 
     def __init__(self, cfg, state_dict, max_tracks: int, device: Optional[int] = None, chunk_tracks: int = 0,
-                 blocks_impl: str = "tcgen05", depth: Optional[int] = None):
+                 blocks_impl: str = "tcgen05", depth: Optional[int] = None, range_fallback: bool = False):
         depth = int(getattr(cfg.MODEL.BACKBONE, "DEPTH", 3)) if depth is None else int(depth)
         self.engine = Engine(cfg, max_tracks=max_tracks, chunk_tracks=chunk_tracks, device=device, blocks_impl=blocks_impl, depth=depth)
         self.engine.load_state_dict(state_dict)
         self.device = self.engine.device
+        self._fallback_count = None
+        if range_fallback:
+            self._fallback_count = torch.zeros((1,), dtype=torch.int64, device=self.device)
+            self.engine.set_range_fallback(True, self._fallback_count)
         self.max_tracks = max_tracks
         self.n = 0
         self._hw = None
@@ -204,6 +212,11 @@ class BatchedTracker:
         self._yuv_off: Optional[torch.Tensor] = None
         # (H, W) of every slot's frames, for steps by slot list; row max_tracks takes the writes of bad entries
         self._slot_hw = torch.zeros((max_tracks + 1, 2), dtype=torch.int32, device=self.device)
+
+    @property
+    def fallback_items(self) -> int:
+        """Items recomputed on the fp32 kernels so far (0 without ``range_fallback``).  Reading it synchronises with the device."""
+        return 0 if self._fallback_count is None else int(self._fallback_count.item())
 
     def _slots(self, slots) -> torch.Tensor:
         """The slot list as the contiguous int32 device tensor the engine takes."""

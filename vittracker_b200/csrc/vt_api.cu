@@ -59,6 +59,11 @@ struct VtContext {
     int32_t* d_eff = nullptr;         // [max_tracks] effective slot per item of the current slot-list call
     float* d_maps = nullptr;          // [max_tracks][1280] score | size | offset of the last step
     int last_first = 0, last_n = 0;
+    // range fallback (vt_set_range_fallback): the flagged items of a tensor-core step, recomputed on the fp32 kernels
+    bool fallback = false;
+    int64_t* fallback_counter = nullptr;  // the caller's device counter (nullable)
+    void* d_fallback = nullptr;           // every array of `fb`, one allocation
+    RangeFallback fb{};
     // generic-configuration path (every configuration other than vit_48_h32; vt_generic.cu)
     bool generic = false;
     GenModelW gw{};
@@ -272,7 +277,7 @@ void free_all(VtHandle h) {
     for (auto e : h->evpool) cudaEventDestroy(e);
     cudaFree(h->d_weights); cudaFree(h->d_planes); cudaFree(h->d_scratch); cudaFree(h->d_taps); cudaFree(h->d_tokz);
     cudaFree(h->d_tokx); cudaFree(h->d_tok); cudaFree(h->d_state); cudaFree(h->d_tmpl);
-    cudaFree(h->d_status); cudaFree(h->d_claim); cudaFree(h->d_eff); cudaFree(h->d_maps); cudaFree(h->d_gwork);
+    cudaFree(h->d_status); cudaFree(h->d_claim); cudaFree(h->d_eff); cudaFree(h->d_maps); cudaFree(h->d_gwork); cudaFree(h->d_fallback);
 }
 
 int check_ready(VtHandle h, bool need_tracks) {
@@ -548,6 +553,14 @@ int tracks_init(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets,
     return VT_OK;
 }
 
+// Range fallback of a tensor-core step over items [0, n) (arguments as tracks_step's): the items the step flagged VT_TRACK_NUMERIC_RANGE
+// are compacted on the device and run through the chain a VT_BLOCKS_SIMT_FP32 handle's step runs (fp32 crop + stem per chunk, fp32
+// blocks, CUDA-core head) as a slot list, then scattered back to their item positions.  The host does not learn how many there are:
+// every launch is sized for n items, and the kernels work only on the items below the device count.  Stages are profiled with 0 items, so
+// that the per-stage item counts stay those of the tensor-core pass.
+int range_fallback(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, int first, const int32_t* slots,
+                   int n, double* out_boxes, double* out_detail, int update_state, cudaStream_t st);
+
 // vt_tracks_step over items [0, n): item i steps track first + i (slots == NULL), or track slots[i] (first == 0; slots resolved).  The
 // state and template pointers start at track `first`; crop status and maps are kept at [first + i], i.e. by item for a slot list.
 int tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, int first, const int32_t* slots,
@@ -595,6 +608,42 @@ int tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets,
         VT_LAUNCH(h, VT_STAGE_HEAD, m, st, "vt_tracks_step/head", launch_head(a, h->mw, st));
     }
     h->last_first = first; h->last_n = n;
+    return h->fallback ? range_fallback(h, frames, frame_offsets, frame_hw, first, slots, n, out_boxes, out_detail, update_state, st) : VT_OK;
+}
+
+int range_fallback(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, int first, const int32_t* slots,
+                   int n, double* out_boxes, double* out_detail, int update_state, cudaStream_t st) {
+    const RangeFallback& fb = h->fb;
+    VT_LAUNCH(h, VT_STAGE_HEAD, 0, st, "vt_tracks_step/fallback compact",
+              launch_fallback_compact(out_boxes, h->d_status + first, slots, first, frame_offsets, frame_hw, n, h->chunk, fb,
+                                      h->fallback_counter, st));
+    for (int c0 = 0; c0 < n; c0 += h->chunk) {
+        const int m = (n - c0 < h->chunk) ? n - c0 : h->chunk;
+        VT_LAUNCH(h, VT_STAGE_STEM, 0, st, "vt_tracks_step/fallback crop+stem",
+                  launch_crop_stem(frames, fb.frame_off + c0, fb.frame_hw + 2 * c0, h->d_state, fb.slot + c0, h->cfg.search_factor, kSx, m,
+                                   h->mw, h->d_scratch, h->d_tokx + (size_t)c0 * kNx * kC, kNx, 0, nullptr, nullptr, 0, h->d_taps, st,
+                                   fb.count + 1 + c0 / h->chunk));
+    }
+    VT_LAUNCH(h, VT_STAGE_BLOCKS, 0, st, "vt_tracks_step/fallback blocks",
+              launch_blocks_simt(h->d_tmpl, kNz, fb.slot, h->d_tokx, kNx, h->d_tok, n, h->mw, nullptr, 0, st, fb.count));
+    const size_t mt = h->cfg.max_tracks;
+    HeadArgs a{};
+    a.tokens = h->d_tok;
+    a.n = n;
+    a.score_map = fb.maps; a.size_map = fb.maps + mt * 256; a.offset_map = fb.maps + mt * 768;
+    a.state = h->d_state;
+    a.slots = fb.slot;
+    a.frame_hw = fb.frame_hw;
+    a.status = nullptr;               // crop status 0 (compaction rule): the head recomputes the same geometry from the state
+    a.out_boxes = fb.boxes;
+    a.out_detail = fb.detail;
+    a.update_state = update_state;
+    a.search_factor = h->cfg.search_factor;
+    a.use_tc = 0;
+    VT_LAUNCH(h, VT_STAGE_HEAD, 0, st, "vt_tracks_step/fallback head", launch_head(a, h->mw, st, fb.count));
+    const LastMaps maps = last_maps(h, first);
+    VT_LAUNCH(h, VT_STAGE_HEAD, 0, st, "vt_tracks_step/fallback scatter",
+              launch_fallback_scatter(fb, h->cfg.max_tracks, out_boxes, out_detail, maps.score, maps.size, maps.offset, n, st));
     return VT_OK;
 }
 
@@ -941,6 +990,29 @@ int vt_tracks_step_slots(VtHandle h, const uint8_t* frames, const int64_t* frame
     VT_CUDA(h, dg.err);
     VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_step_slots/resolve", launch_resolve_slots(slots, n, h->cfg.max_tracks, h->d_claim, h->d_eff, st));
     return tracks_step(h, frames, frame_offsets, frame_hw, 0, h->d_eff, n, out_boxes, out_detail, update_state, st);
+}
+
+int vt_set_range_fallback(VtHandle h, int32_t enable, int64_t* counter_dev) {
+    if (!h) return VT_ERR_INVALID_ARG;
+    if (h->generic) return fail(h, VT_ERR_UNSUPPORTED, "vt_set_range_fallback: only the vit_48_h32 configuration has the fp32 step chain it needs");
+    if (h->cfg.blocks_impl == VT_BLOCKS_SIMT_FP32) return VT_OK;        // no fp16 operands: nothing is ever flagged for range
+    if (enable && !h->d_fallback) {
+        DeviceGuard dg(h->cfg.device);
+        VT_CUDA(h, dg.err);
+        const size_t mt = h->cfg.max_tracks, chunks = (mt + h->chunk - 1) / h->chunk;
+        size_t off = 0;
+        auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+        const size_t o_count = carve((1 + chunks) * 4), o_item = carve(mt * 4), o_slot = carve(mt * 4), o_off = carve(mt * 8),
+                     o_hw = carve(mt * 8), o_boxes = carve(mt * 5 * 8), o_detail = carve(mt * 8 * 8), o_maps = carve(mt * 1280 * 4);
+        VT_CUDA(h, cudaMalloc(&h->d_fallback, off));
+        uint8_t* b = static_cast<uint8_t*>(h->d_fallback);
+        h->fb = RangeFallback{reinterpret_cast<int32_t*>(b + o_count), reinterpret_cast<int32_t*>(b + o_item), reinterpret_cast<int32_t*>(b + o_slot),
+                              reinterpret_cast<int64_t*>(b + o_off), reinterpret_cast<int32_t*>(b + o_hw), reinterpret_cast<double*>(b + o_boxes),
+                              reinterpret_cast<double*>(b + o_detail), reinterpret_cast<float*>(b + o_maps)};
+    }
+    h->fallback = enable != 0;
+    h->fallback_counter = enable ? counter_dev : nullptr;
+    return VT_OK;
 }
 
 int vt_tracks_get_state(VtHandle h, double* boxes_xywh, int32_t first, int32_t n, void* stream) {

@@ -62,14 +62,13 @@ __device__ __forceinline__ void matvec48(const float (&in)[K], const float* W, i
     }
 }
 
-__global__ void __launch_bounds__(kBlkThreads, 1)
-blocks_simt_kernel(const float* __restrict__ tok_z, int z_stride_rows, const int32_t* __restrict__ z_slots, const float* __restrict__ tok_x,
-                   int x_stride_rows, float* __restrict__ out, ModelW w, float* __restrict__ taps,
-                   size_t tap_stride) {
+// Track trk.
+__device__ __forceinline__ void blocks_simt_track(const float* __restrict__ tok_z, int z_stride_rows, const int32_t* __restrict__ z_slots,
+                                                  const float* __restrict__ tok_x, int x_stride_rows, float* __restrict__ out, const ModelW& w,
+                                                  float* __restrict__ taps, size_t tap_stride, int trk) {
     extern __shared__ __align__(16) float smem[];
     float* sA = smem;
     float* sKV = smem + kAFloats;
-    const int trk = blockIdx.x;
     const int i = threadIdx.x;
 
     // residual row of token i: template tokens first (vit_dist.py:84)
@@ -229,12 +228,35 @@ blocks_simt_kernel(const float* __restrict__ tok_z, int z_stride_rows, const int
     for (int k = 0; k < kC; k += 4) *reinterpret_cast<float4*>(dst + k) = make_float4(x[k], x[k + 1], x[k + 2], x[k + 3]);
 }
 
+// Track blockIdx.x; COUNTED (the range fallback of vt_api.cu, whose item count is known on the device only): tracks blockIdx.x,
+// blockIdx.x + gridDim.x, ... below *count.
+template <bool COUNTED>
+__global__ void __launch_bounds__(kBlkThreads, 1)
+blocks_simt_kernel(const float* __restrict__ tok_z, int z_stride_rows, const int32_t* __restrict__ z_slots, const float* __restrict__ tok_x,
+                   int x_stride_rows, float* __restrict__ out, ModelW w, float* __restrict__ taps,
+                   size_t tap_stride, const int32_t* __restrict__ count) {
+    if constexpr (COUNTED) {
+        for (int trk = blockIdx.x; trk < *count; trk += gridDim.x) {
+            blocks_simt_track(tok_z, z_stride_rows, z_slots, tok_x, x_stride_rows, out, w, taps, tap_stride, trk);
+            __syncthreads();                                 // the next track restages shared memory
+        }
+    } else {
+        blocks_simt_track(tok_z, z_stride_rows, z_slots, tok_x, x_stride_rows, out, w, taps, tap_stride, blockIdx.x);
+    }
+}
+
 int launch_blocks_simt(const float* tok_z, int z_stride_rows, const int32_t* z_slots, const float* tok_x, int x_stride_rows,
-                       float* out, int n, const ModelW& w, float* taps, size_t tap_stride, cudaStream_t st) {
+                       float* out, int n, const ModelW& w, float* taps, size_t tap_stride, cudaStream_t st, const int32_t* count) {
     if (n <= 0) return 0;
-    static DeviceOnce once;
-    if (!ensure_dyn_smem(once, blocks_simt_kernel, kBlkSmemBytes)) return -1;
-    blocks_simt_kernel<<<n, kBlkThreads, kBlkSmemBytes, st>>>(tok_z, z_stride_rows, z_slots, tok_x, x_stride_rows, out, w, taps, tap_stride);
+    static DeviceOnce once, once_counted;
+    if (count) {
+        if (!ensure_dyn_smem(once_counted, blocks_simt_kernel<true>, kBlkSmemBytes)) return -1;
+        blocks_simt_kernel<true><<<counted_rows(n, 1, 1), kBlkThreads, kBlkSmemBytes, st>>>(tok_z, z_stride_rows, z_slots, tok_x, x_stride_rows, out, w,
+                                                                                            taps, tap_stride, count);
+        return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    }
+    if (!ensure_dyn_smem(once, blocks_simt_kernel<false>, kBlkSmemBytes)) return -1;
+    blocks_simt_kernel<false><<<n, kBlkThreads, kBlkSmemBytes, st>>>(tok_z, z_stride_rows, z_slots, tok_x, x_stride_rows, out, w, taps, tap_stride, nullptr);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
 }
 

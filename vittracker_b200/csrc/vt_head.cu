@@ -263,7 +263,8 @@ __device__ __forceinline__ void head_finish(const HeadArgs& a, const ModelW& w, 
     HEAD_TRACE(7);
 }
 
-__global__ void __launch_bounds__(kHeadThreads, 1) head_kernel(HeadArgs a, ModelW w) {
+// Track trk on the CUDA cores.
+__device__ __forceinline__ void head_track(const HeadArgs& a, const ModelW& w, int trk) {
     extern __shared__ __align__(128) float smem[];
     float* feat = smem + kOffFeat;
     float* out1 = smem + kOffOut1;
@@ -271,7 +272,6 @@ __global__ void __launch_bounds__(kHeadThreads, 1) head_kernel(HeadArgs a, Model
     float* sb = smem + kOffBias;
     float* maps = smem + kOffMaps;
     float* red = smem + kOffRed;
-    const int trk = blockIdx.x;
     const int tid = threadIdx.x;
     int bad = 0;
 
@@ -313,6 +313,19 @@ __global__ void __launch_bounds__(kHeadThreads, 1) head_kernel(HeadArgs a, Model
     head_conv<8, 4, 3, true, 8>(out3, out4, w.head.w4, sb + 168, wbuf);            // 8 -> 4
 
     head_finish(a, w, trk, out4, sb, maps, red, 0xffffffffu, bad);
+}
+
+// Track blockIdx.x; COUNTED (the range fallback of vt_api.cu): tracks blockIdx.x, blockIdx.x + gridDim.x, ... below *count.
+template <bool COUNTED>
+__global__ void __launch_bounds__(kHeadThreads, 1) head_kernel(HeadArgs a, ModelW w, const int32_t* __restrict__ count) {
+    if constexpr (COUNTED) {
+        for (int trk = blockIdx.x; trk < *count; trk += gridDim.x) {
+            head_track(a, w, trk);
+            __syncthreads();                                 // the next track clears shared memory
+        }
+    } else {
+        head_track(a, w, blockIdx.x);
+    }
 }
 
 // Tensor-core head: conv1 (48 -> 96 merged) and conv2 (32 -> 16 per tower) on tcgen05, conv3-5 on CUDA cores.
@@ -664,10 +677,15 @@ __global__ void __launch_bounds__(kHeadThreads, 1) head_tc_kernel(HeadArgs a, Mo
     if (warp == 0) tc::tmem_dealloc(tbase, 512);
 }
 
-int launch_head(const HeadArgs& a, const ModelW& w, cudaStream_t st) {
+int launch_head(const HeadArgs& a, const ModelW& w, cudaStream_t st, const int32_t* count) {
     if (a.n <= 0) return 0;
-    static DeviceOnce once_simt, once_tc;
-    if (!ensure_dyn_smem(once_simt, head_kernel, kHeadSmemBytes) || !ensure_dyn_smem(once_tc, head_tc_kernel, kHeadTcSmemBytes)) return -1;
+    static DeviceOnce once_simt, once_tc, once_counted;
+    if (!ensure_dyn_smem(once_simt, head_kernel<false>, kHeadSmemBytes) || !ensure_dyn_smem(once_tc, head_tc_kernel, kHeadTcSmemBytes)) return -1;
+    if (count) {
+        if (!ensure_dyn_smem(once_counted, head_kernel<true>, kHeadSmemBytes)) return -1;
+        head_kernel<true><<<counted_rows(a.n, 1, 1), kHeadThreads, kHeadSmemBytes, st>>>(a, w, count);
+        return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    }
     if (a.use_tc) {
         static int sms[kMaxDevices] = {};
         int dev = 0;
@@ -675,7 +693,7 @@ int launch_head(const HeadArgs& a, const ModelW& w, cudaStream_t st) {
         if (sms[dev] == 0 && cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return -1;
         head_tc_kernel<<<a.n < sms[dev] ? a.n : sms[dev], kHeadThreads, kHeadTcSmemBytes, st>>>(a, w);      // persistent: one CTA (220 KB) per SM
     }
-    else head_kernel<<<a.n, kHeadThreads, kHeadSmemBytes, st>>>(a, w);
+    else head_kernel<false><<<a.n, kHeadThreads, kHeadSmemBytes, st>>>(a, w, nullptr);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
 }
 

@@ -229,6 +229,21 @@ struct DeviceGuard {
     DeviceGuard& operator=(const DeviceGuard&) = delete;
 };
 
+// Grid rows of a kernel that strides over a device-side item count (the range fallback of vt_api.cu), `tiles` CTAs per item: about
+// ctas_per_sm CTAs per SM in all (a grid that costs little when the count is 0), at least 1 and at most n.
+inline int counted_rows(int n, int tiles, int ctas_per_sm = 4) {
+    static int sms[kMaxDevices] = {};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) dev = -1;
+    int s = dev >= 0 ? sms[dev] : 0;
+    if (s == 0) {
+        if (cudaDeviceGetAttribute(&s, cudaDevAttrMultiProcessorCount, dev < 0 ? 0 : dev) != cudaSuccess || s <= 0) s = 148;
+        if (dev >= 0) sms[dev] = s;
+    }
+    const int rows = ctas_per_sm * s / tiles;
+    return rows < 1 ? 1 : rows > n ? n : rows;
+}
+
 // ---- kernel launchers (each returns the number of kernels it launched, or <0 on a CUDA error) -----
 // YUV 4:2:0 -> RGB (vt_yuv.cu).  One work item: an even w x h image whose luma rows are y_pitch apart and whose chroma rows
 // (one per two luma rows) are c_pitch apart; NV12 reads interleaved U V pairs at u, I420 reads U at u and V at v.
@@ -285,16 +300,18 @@ size_t stem_tc_weight_bytes(int layer);
 void stem_tc_pack_weights(int cin, int cch, int cout, int npad, const float* wf, uint8_t* hi8, uint8_t* lo8);
 
 // Crop + stem straight from raw uint8 frames (the first conv layer gathers its tile from the frame).
+// count (device, nullable): only items below *count are processed; given, the stem runs on the fp32 CUDA-core kernels whatever `planes`.
 int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
                      const int32_t* slots, double factor, int S, int n, const ModelW& w, float* scratch, float* tokens, int tok_stride_rows,
-                     int tok_off, int32_t* out_status, uint8_t* planes, int plane_tracks, void* tap_tables, cudaStream_t st);
+                     int tok_off, int32_t* out_status, uint8_t* planes, int plane_tracks, void* tap_tables, cudaStream_t st,
+                     const int32_t* count = nullptr);
 size_t crop_taps_bytes(int n);      // size of the tap-table buffer launch_crop_stem needs for n tracks
 
 // ViT blocks (fp32 SIMT): tokens_z [n][64][48] (stride z_stride rows per track; item i reads row block item_slot(z_slots, i), a negative
 // slot reads block 0), tokens_x likewise (by item); in place
-// result written to out [n][320][48]; taps (or null) receives [depth][n][320][48].
+// result written to out [n][320][48]; taps (or null) receives [depth][n][320][48].  count (device, nullable): only items below *count.
 int launch_blocks_simt(const float* tok_z, int z_stride_rows, const int32_t* z_slots, const float* tok_x, int x_stride_rows,
-                       float* out, int n, const ModelW& w, float* taps, size_t tap_stride, cudaStream_t st);
+                       float* out, int n, const ModelW& w, float* taps, size_t tap_stride, cudaStream_t st, const int32_t* count = nullptr);
 
 // ViT blocks on the tcgen05 tensor cores (fp16 hi/lo split operands, fp32 accumulation in TMEM).
 int launch_blocks_tc(const float* tok_z, int z_stride_rows, const int32_t* z_slots, const float* tok_x, int x_stride_rows,
@@ -317,7 +334,8 @@ struct HeadArgs {
     double search_factor;
     int use_tc;               // first (48 -> 96) convolution on the tcgen05 tensor cores
 };
-int launch_head(const HeadArgs& a, const ModelW& w, cudaStream_t st);
+// count (device, nullable; CUDA-core head only, use_tc == 0): only items below *count are processed.
+int launch_head(const HeadArgs& a, const ModelW& w, cudaStream_t st, const int32_t* count = nullptr);
 // Weights of the tensor-core head (vt_head.cu): blob sizes (0: conv1, 1: conv2, 2: conv3) and the host packer that fills them from
 // the folded HeadW layouts w1, w2, w3.
 size_t head_tc_weight_bytes(int layer);
@@ -385,5 +403,26 @@ int launch_gather_rows(const float* src, size_t src_stride, float* dst, size_t d
 // (nullable) <- status[i], or VT_TRACK_BAD_SLOT for eff[i] < 0.
 int launch_scatter_init(const float* tok, float* tmpl, size_t row, const double* boxes, double* state, const int32_t* status,
                         int32_t* out_status, const int32_t* eff, int n, cudaStream_t st);
+
+// ---- range fallback (vt_set_range_fallback; vt_slots.cu) ------------------------------------------------
+// The items of a tensor-core step that ended with VT_TRACK_NUMERIC_RANGE, compacted in item order, and the fp32 pass's rows for them.
+struct RangeFallback {
+    int32_t* count;        // [1 + chunks]: [0] flagged items of the step, [1 + k] of them in chunk k (items [k chunk, (k + 1) chunk))
+    int32_t* item;         // [max_tracks] item index of compacted entry j
+    int32_t* slot;         // [max_tracks] its track slot
+    int64_t* frame_off;    // [max_tracks] its frame offset
+    int32_t* frame_hw;     // [max_tracks][2]
+    double* boxes;         // [max_tracks][5] the fp32 pass's out_boxes rows
+    double* detail;        // [max_tracks][8] ... out_detail rows
+    float* maps;           // score [max_tracks][256] | size [max_tracks][512] | offset [max_tracks][512] ... maps
+};
+// Finds the flagged items of a step over n items: out_boxes[i][4] == -1, crop status[i] == 0 (status by item) and a valid slot (slot
+// first + i, or eff[i] >= 0 when eff is given).  Writes fb's per-item arrays and counts, and adds the count to *counter (nullable).
+int launch_fallback_compact(const double* out_boxes, const int32_t* status, const int32_t* eff, int first, const int64_t* frame_offsets,
+                            const int32_t* frame_hw, int n, int chunk, const RangeFallback& fb, int64_t* counter, cudaStream_t st);
+// Writes entry j < count[0] of the fp32 pass back to item fb.item[j]: out_boxes, out_detail (nullable) and the maps at score / size /
+// offset (the step's planar map rows from its first item, max_tracks rows per array in fb.maps).
+int launch_fallback_scatter(const RangeFallback& fb, int max_tracks, double* out_boxes, double* out_detail, float* score, float* size,
+                            float* offset, int n, cudaStream_t st);
 
 }  // namespace vt

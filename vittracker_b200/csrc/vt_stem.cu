@@ -261,11 +261,12 @@ __device__ __forceinline__ void conv_compute(const float* tile, const float* ws,
     }
 }
 
-template <int CIN, int COUT, int QG, int P, int TW, int TH, bool HSWISH, bool TOKENS, int TCOUT_CCH = 0>
-__global__ void __launch_bounds__(ConvCfg<CIN, COUT, QG, P, TW, TH>::kThreads)
-conv3x3s2_kernel(const float* __restrict__ in, int Hin, int Win, const float* __restrict__ wg,
-                 const float* __restrict__ bg, float* __restrict__ out, const float* __restrict__ pos,
-                 int tok_stride_rows, int tok_off) {
+// One image of a tile row of the grid: item `counted_item` (COUNTED), else blockIdx.y, read where the one-item kernel always read it
+// (that kernel then compiles to the instructions it had before the counted form existed).
+template <int CIN, int COUT, int QG, int P, int TW, int TH, bool HSWISH, bool TOKENS, int TCOUT_CCH, bool COUNTED>
+__device__ __forceinline__ void conv3x3s2_item(const float* __restrict__ in, int Hin, int Win, const float* __restrict__ wg,
+                                               const float* __restrict__ bg, float* __restrict__ out, const float* __restrict__ pos,
+                                               int tok_stride_rows, int tok_off, int counted_item) {
     using K = ConvCfg<CIN, COUT, QG, P, TW, TH>;
     extern __shared__ __align__(16) float smem[];
     float* tile = smem;
@@ -276,7 +277,7 @@ conv3x3s2_kernel(const float* __restrict__ in, int Hin, int Win, const float* __
     const int tiles_x = (Wout + TW - 1) / TW;
     const int tx0 = (blockIdx.x % tiles_x) * TW;
     const int ty0 = (blockIdx.x / tiles_x) * TH;
-    const int b = blockIdx.y;
+    const int b = COUNTED ? counted_item : blockIdx.y;
     const int tid = threadIdx.x;
 
     // weights / bias / input tile are staged with cp.async: every load is in flight at once (the tile
@@ -332,6 +333,23 @@ conv3x3s2_kernel(const float* __restrict__ in, int Hin, int Win, const float* __
     conv_compute<CIN, COUT, QG, P, TW, TH, HSWISH, TOKENS, TCOUT_CCH>(tile, ws, bs, tx0, ty0, Hout, Wout, b, out, pos, tok_stride_rows, tok_off);
 }
 
+// Item blockIdx.y; COUNTED (the range fallback of vt_api.cu, whose item count is known on the device only): items blockIdx.y,
+// blockIdx.y + gridDim.y, ... below *count, so that a grid sized for one wave costs little when there are none.
+template <int CIN, int COUT, int QG, int P, int TW, int TH, bool HSWISH, bool TOKENS, int TCOUT_CCH = 0, bool COUNTED = false>
+__global__ void __launch_bounds__(ConvCfg<CIN, COUT, QG, P, TW, TH>::kThreads)
+conv3x3s2_kernel(const float* __restrict__ in, int Hin, int Win, const float* __restrict__ wg,
+                 const float* __restrict__ bg, float* __restrict__ out, const float* __restrict__ pos,
+                 int tok_stride_rows, int tok_off, const int32_t* __restrict__ count) {
+    if constexpr (COUNTED) {
+        for (int b = blockIdx.y; b < *count; b += gridDim.y) {
+            conv3x3s2_item<CIN, COUT, QG, P, TW, TH, HSWISH, TOKENS, TCOUT_CCH, true>(in, Hin, Win, wg, bg, out, pos, tok_stride_rows, tok_off, b);
+            __syncthreads();                                  // the next item restages shared memory
+        }
+    } else {
+        conv3x3s2_item<CIN, COUT, QG, P, TW, TH, HSWISH, TOKENS, TCOUT_CCH, false>(in, Hin, Win, wg, bg, out, pos, tok_stride_rows, tok_off, 0);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------
 // Fused K1 + first stem layer: the 65 x 65 x 3 input tile of conv1 is gathered straight from the raw
 // uint8 frame (crop + zero pad + OpenCV-exact fixed-point bilinear + normalisation LUT, exactly the
@@ -344,11 +362,11 @@ constexpr int kCc1TileSide = 2 * 32 + 1;                                // 65 re
 constexpr int kCc1WFloats = 2 * Conv1Cfg::kWFloats;                    // conv1 weights duplicated {w, w} for the packed FMAs
 constexpr size_t kCc1SmemBytes = Conv1Cfg::kSmemBytes + Conv1Cfg::kWFloats * sizeof(float) + 64 + 2 * 80 * sizeof(int4);     // 4 CTAs / SM
 
-template <int S>
-__global__ void __launch_bounds__(kCc1Threads, 4)
-crop_conv1_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict__ frame_offsets,
-                  const int4* __restrict__ taps, const float* __restrict__ wg,
-                  const float* __restrict__ bg, float* __restrict__ out) {
+// Item `counted_item` (COUNTED), else blockIdx.y, read where the one-item kernel always read it (as conv3x3s2_item).
+template <int S, bool COUNTED>
+__device__ __forceinline__ void crop_conv1_item(const uint8_t* __restrict__ frames, const int64_t* __restrict__ frame_offsets,
+                                                const int4* __restrict__ taps, const float* __restrict__ wg,
+                                                const float* __restrict__ bg, float* __restrict__ out, int counted_item) {
     using K = Conv1Cfg;
     extern __shared__ __align__(16) float smem[];
     float* tile = smem;
@@ -361,7 +379,7 @@ crop_conv1_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict_
     constexpr int tiles_x = Hout / 32;
     const int tx0 = (blockIdx.x % tiles_x) * 32;
     const int ty0 = (blockIdx.x / tiles_x) * 32;
-    const int item = blockIdx.y;
+    const int item = COUNTED ? counted_item : blockIdx.y;
     const int tid = threadIdx.x;
 
     if (tid < 3 * 9 * 6) {                                                 // weights as {w, w} pairs (conv_compute PAIRED)
@@ -456,15 +474,37 @@ crop_conv1_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict_
     conv_compute<3, 6, 6, 4, 32, 32, true, false, 0, true>(tile, ws, bs, tx0, ty0, Hout, Hout, item, out, nullptr, 0, 0);
 }
 
+// Item blockIdx.y; COUNTED: a grid-stride loop over the items below *count, as conv3x3s2_kernel's.
+template <int S, bool COUNTED = false>
+__global__ void __launch_bounds__(kCc1Threads, 4)
+crop_conv1_kernel(const uint8_t* __restrict__ frames, const int64_t* __restrict__ frame_offsets,
+                  const int4* __restrict__ taps, const float* __restrict__ wg,
+                  const float* __restrict__ bg, float* __restrict__ out, const int32_t* __restrict__ count) {
+    if constexpr (COUNTED) {
+        for (int item = blockIdx.y; item < *count; item += gridDim.y) {
+            crop_conv1_item<S, true>(frames, frame_offsets, taps, wg, bg, out, item);
+            __syncthreads();                                  // the next item restages shared memory
+        }
+    } else {
+        crop_conv1_item<S, false>(frames, frame_offsets, taps, wg, bg, out, 0);
+    }
+}
+
 template <int CIN, int COUT, int QG, int P, int TW, int TH, bool HSWISH, bool TOKENS, int TCOUT_CCH = 0>
 static int run_conv(const float* in, int Hin, int n, const StemLayerW& w, float* out, const float* pos,
-                    int tok_stride_rows, int tok_off, cudaStream_t st) {
+                    int tok_stride_rows, int tok_off, cudaStream_t st, const int32_t* count = nullptr) {
     using K = ConvCfg<CIN, COUT, QG, P, TW, TH>;
     auto kern = conv3x3s2_kernel<CIN, COUT, QG, P, TW, TH, HSWISH, TOKENS, TCOUT_CCH>;
-    static DeviceOnce once;
+    static DeviceOnce once, once_counted;
     if (!ensure_dyn_smem(once, kern, K::kSmemBytes)) return -1;
     const int Hout = Hin / 2;
     const int tiles = ((Hout + TW - 1) / TW) * ((Hout + TH - 1) / TH);
+    if (count) {
+        auto kc = conv3x3s2_kernel<CIN, COUT, QG, P, TW, TH, HSWISH, TOKENS, TCOUT_CCH, true>;
+        if (!ensure_dyn_smem(once_counted, kc, K::kSmemBytes)) return -1;
+        kc<<<dim3(tiles, counted_rows(n, tiles)), K::kThreads, K::kSmemBytes, st>>>(in, Hin, Hin, w.w, w.b, out, pos, tok_stride_rows, tok_off, count);
+        return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    }
     int launched = 0;
     for (int first = 0; first < n; first += 32768) {
         const int m = min(32768, n - first);
@@ -472,7 +512,7 @@ static int run_conv(const float* in, int Hin, int n, const StemLayerW& w, float*
         const float* inp = in + (size_t)first * CIN * Hin * Hin;
         float* o = TCOUT_CCH > 0 ? reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(out) + (size_t)first * tc_planes_bytes(TCOUT_CCH, Hout / 2))
                    : TOKENS ? out + (size_t)first * tok_stride_rows * COUT : out + (size_t)first * COUT * Hout * Hout;
-        kern<<<grid, K::kThreads, K::kSmemBytes, st>>>(inp, Hin, Hin, w.w, w.b, o, pos, tok_stride_rows, tok_off);
+        kern<<<grid, K::kThreads, K::kSmemBytes, st>>>(inp, Hin, Hin, w.w, w.b, o, pos, tok_stride_rows, tok_off, nullptr);
         ++launched;
     }
     return cudaGetLastError() == cudaSuccess ? launched : -1;
@@ -487,17 +527,25 @@ size_t crop_taps_bytes(int n) { return (size_t)n * 2 * kTapPitch * sizeof(int4) 
 
 template <int S>
 static int run_crop_conv1(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
-                          const int32_t* slots, double factor, int n, const ModelW& w, float* out, int32_t* out_status, int4* taps, cudaStream_t st) {
+                          const int32_t* slots, double factor, int n, const ModelW& w, float* out, int32_t* out_status, int4* taps, cudaStream_t st,
+                          const int32_t* count) {
     auto kern = crop_conv1_kernel<S>;
-    static DeviceOnce once;
+    static DeviceOnce once, once_counted;
     if (!ensure_dyn_smem(once, kern, kCc1SmemBytes)) return -1;
     constexpr int tiles = (S / 64) * (S / 64);
-    crop_taps_kernel<S><<<n, 288, 0, st>>>(frame_hw, boxes, slots, factor, taps, out_status, nullptr, 0);
+    if (count) {
+        auto kc = crop_conv1_kernel<S, true>;
+        if (!ensure_dyn_smem(once_counted, kc, kCc1SmemBytes)) return -1;
+        crop_taps_kernel<S, true><<<n, 288, 0, st>>>(frame_hw, boxes, slots, factor, taps, out_status, nullptr, 0, count);
+        kc<<<dim3(tiles, counted_rows(n, tiles)), kCc1Threads, kCc1SmemBytes, st>>>(frames, frame_offsets, taps, w.stem[0].w, w.stem[0].b, out, count);
+        return cudaGetLastError() == cudaSuccess ? 2 : -1;
+    }
+    crop_taps_kernel<S><<<n, 288, 0, st>>>(frame_hw, boxes, slots, factor, taps, out_status, nullptr, 0, nullptr);
     int launched = 1;
     for (int first = 0; first < n; first += 32768) {
         const int m = min(32768, n - first);
         kern<<<dim3(tiles, m), kCc1Threads, kCc1SmemBytes, st>>>(frames, frame_offsets + first, taps + (size_t)first * 2 * kTapPitch,
-                                                                 w.stem[0].w, w.stem[0].b, out + (size_t)first * 6 * (S / 2) * (S / 2));
+                                                                 w.stem[0].w, w.stem[0].b, out + (size_t)first * 6 * (S / 2) * (S / 2), nullptr);
         ++launched;
     }
     return cudaGetLastError() == cudaSuccess ? launched : -1;
@@ -506,7 +554,8 @@ static int run_crop_conv1(const uint8_t* frames, const int64_t* frame_offsets, c
 // Crop + stem straight from raw frames (fused first layer); same outputs as launch_crop_normalize + launch_stem.
 int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw, const double* boxes,
                      const int32_t* slots, double factor, int S, int n, const ModelW& w, float* scratch, float* tokens, int tok_stride_rows,
-                     int tok_off, int32_t* out_status, uint8_t* planes, int plane_tracks, void* tap_tables, cudaStream_t st) {
+                     int tok_off, int32_t* out_status, uint8_t* planes, int plane_tracks, void* tap_tables, cudaStream_t st,
+                     const int32_t* count) {
     if (n <= 0) return 0;
     int4* taps = reinterpret_cast<int4*>(tap_tables);
     float* a1 = scratch;
@@ -514,7 +563,7 @@ int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const 
     float* a3 = a2 + (size_t)n * 12 * (S / 4) * (S / 4);
     const float* pos = (S == kSx) ? w.pos_x : w.pos_z;
     int total = 0, r;
-    if (planes && S == kSx && n <= plane_tracks) {
+    if (planes && !count && S == kSx && n <= plane_tracks) {
         // search branch: crop + conv1 + conv2 in one tcgen05 kernel (vt_stem_fused.cu), then layers 3-4 on tcgen05.  The planes
         // buffer keeps conv2's operand image first (launch_stem writes it), so conv3's image starts after it.
         uint8_t* planes3 = planes + (size_t)plane_tracks * tc_planes_bytes(kConv2Cch, kConv2Wout);
@@ -524,16 +573,16 @@ int launch_crop_stem(const uint8_t* frames, const int64_t* frame_offsets, const 
         if ((r = launch_stem34_tc(planes3, n, w, planes4, tokens, tok_stride_rows, tok_off, st)) < 0) return r;
         return total + r;
     }
-    if (S == 256) r = run_crop_conv1<256>(frames, frame_offsets, frame_hw, boxes, slots, factor, n, w, a1, out_status, taps, st);
-    else if (S == 128) r = run_crop_conv1<128>(frames, frame_offsets, frame_hw, boxes, slots, factor, n, w, a1, out_status, taps, st);
+    if (S == 256) r = run_crop_conv1<256>(frames, frame_offsets, frame_hw, boxes, slots, factor, n, w, a1, out_status, taps, st, count);
+    else if (S == 128) r = run_crop_conv1<128>(frames, frame_offsets, frame_hw, boxes, slots, factor, n, w, a1, out_status, taps, st, count);
     else return -1;
     if (r < 0) return r;
     total += r;
-    if ((r = run_conv<6, 12, 12, 2, 32, 16, true, false>(a1, S / 2, n, w.stem[1], a2, nullptr, 0, 0, st)) < 0) return r;
+    if ((r = run_conv<6, 12, 12, 2, 32, 16, true, false>(a1, S / 2, n, w.stem[1], a2, nullptr, 0, 0, st, count)) < 0) return r;
     total += r;
-    if ((r = run_conv<12, 24, 12, 2, 32, 8, true, false>(a2, S / 4, n, w.stem[2], a3, nullptr, 0, 0, st)) < 0) return r;
+    if ((r = run_conv<12, 24, 12, 2, 32, 8, true, false>(a2, S / 4, n, w.stem[2], a3, nullptr, 0, 0, st, count)) < 0) return r;
     total += r;
-    if ((r = run_conv<24, 48, 12, 4, 16, 16, false, true>(a3, S / 8, n, w.stem[3], tokens, pos, tok_stride_rows, tok_off, st)) < 0) return r;
+    if ((r = run_conv<24, 48, 12, 4, 16, 16, false, true>(a3, S / 8, n, w.stem[3], tokens, pos, tok_stride_rows, tok_off, st, count)) < 0) return r;
     total += r;
     return total;
 }

@@ -487,7 +487,7 @@ int launch_crop_stem12_fused(const uint8_t* frames, const int64_t* frame_offsets
     const int grid = n_units < grid_caps[dev] ? n_units : grid_caps[dev];
     int4* taps = reinterpret_cast<int4*>(tap_tables);
     int* work_counter = reinterpret_cast<int*>(taps + (size_t)n * 2 * kTapPitch);
-    crop_taps_kernel<kSx><<<n, 288, 0, st>>>(frame_hw, boxes, slots, factor, taps, out_status, work_counter, grid);
+    crop_taps_kernel<kSx><<<n, 288, 0, st>>>(frame_hw, boxes, slots, factor, taps, out_status, work_counter, grid, nullptr);
     if (cudaGetLastError() != cudaSuccess) return -1;
     kern<<<grid, kFThreads, F::kSmemBytes, st>>>(frames, frame_offsets, taps, w.stem1_tc_w, w.stem1_tc_par, w.stem_tc_w[0], w.stem_tc_b[0],
                                                  planes3, n_units, n_big, unit_bands, work_counter);

@@ -15,15 +15,18 @@ namespace vt {
 // (= the convolution's zero padding, which is 0.0f and not the normalised pixel 0).
 // The box of item i is track item_slot(slots, i) of `boxes`; a bad slot gives status VT_TRACK_BAD_SLOT and empty tables.
 // `work_counter` (may be null) is the consumer kernel's dynamic work counter: block 0 resets it to `work_counter0` on the way.
+// COUNTED: only items below *count are processed (the range fallback of vt_api.cu, whose item count is known on the device only);
+// the uncounted instantiation, which the fused tensor-core front launches, does not read `count`.
 constexpr int kTapPitch = 264;
-template <int S>
+template <int S, bool COUNTED = false>
 __global__ void __launch_bounds__(288)
 crop_taps_kernel(const int32_t* __restrict__ frame_hw, const double* __restrict__ boxes, const int32_t* __restrict__ slots, double factor,
                  int4* __restrict__ taps,
-                 int32_t* __restrict__ out_status, int* __restrict__ work_counter, int work_counter0) {
+                 int32_t* __restrict__ out_status, int* __restrict__ work_counter, int work_counter0, const int32_t* __restrict__ count) {
     __shared__ CropGeom sg;
     __shared__ double s_scale;
     const int item = blockIdx.x, tid = threadIdx.x;
+    if (COUNTED && item >= *count) return;
     const int H = frame_hw[2 * item], W = frame_hw[2 * item + 1];
     if (item == 0 && tid == 287 && work_counter) *work_counter = work_counter0;
     if (tid == 0) {

@@ -293,6 +293,18 @@ class Engine:
                                                       _ptr(out_boxes), _ptr(out_detail), 1 if update_state else 0, self._stream()))
         return (out_boxes, out_detail) if detail else out_boxes
 
+    def set_range_fallback(self, enable: bool, counter: Optional[torch.Tensor] = None) -> None:
+        """vt_set_range_fallback: with ``enable``, every item of a tracking step that the tensor-core kernels flag
+        VT_TRACK_NUMERIC_RANGE is recomputed on the fp32 kernels within the same call, bit for bit what a ``simt`` engine gives.
+        ``counter`` (optional int64 device tensor of one element) has the number of recomputed items added to it by every step."""
+        if counter is not None and (counter.dtype != torch.int64 or counter.device != self.device or counter.numel() != 1):
+            raise ValueError(f"counter: expected a one-element int64 tensor on {self.device}")
+        self._check(self.lib.vt_set_range_fallback(self.handle, 1 if enable else 0, _ptr(counter)))
+        # a CUDA graph captured while a counter was set keeps adding to its address on every replay, whatever the fallback's setting
+        # since: every counter handed over lives as long as this engine
+        if counter is not None:
+            self._fallback_counters = getattr(self, "_fallback_counters", []) + [counter]
+
     def tracks_get_state(self, first: int = 0, n: Optional[int] = None) -> torch.Tensor:
         n = self.max_tracks - first if n is None else n
         out = torch.empty((n, 4), dtype=torch.float64, device=self.device)

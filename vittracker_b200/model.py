@@ -32,7 +32,7 @@ class CenterHeadHandle:
 
 class OstrackDistB200:
     def __init__(self, cfg, depth: int = 3, mode: str = "eval", blocks_impl: str = "tcgen05", max_tracks: int = 1,
-                 chunk_tracks: int = 0):
+                 chunk_tracks: int = 0, range_fallback: bool = False):
         if mode != "eval":
             raise NotImplementedError("only mode='eval' (inference) is implemented; the distillation/training "
                                       "branches of OstrackDist (vit_dist.py:69-73,97-119) are out of scope")
@@ -46,6 +46,7 @@ class OstrackDistB200:
         self._blocks_impl = blocks_impl
         self._max_tracks = max_tracks
         self._chunk_tracks = chunk_tracks
+        self._range_fallback = range_fallback            # tracking steps recompute range-flagged tracks on the fp32 kernels
         self._engine: Optional[Engine] = None
         self._device: Optional[int] = None
         self._sd: Dict[str, torch.Tensor] = random_init_state_dict(cfg, depth)
@@ -88,6 +89,8 @@ class OstrackDistB200:
             self._engine = Engine(self.cfg, max_tracks=self._max_tracks, chunk_tracks=self._chunk_tracks,
                                   device=self._device, blocks_impl=self._blocks_impl, depth=self.depth)
             self._engine.load_state_dict(self._sd)
+            if self._range_fallback:
+                self._engine.set_range_fallback(True)
         return self._engine
 
     # -- inference -----------------------------------------------------------------------------

@@ -148,11 +148,12 @@ class BatchedBackend:
     _PAD = 256           # bytes between packed regions: the gather reads aligned words around a tap (< 16 bytes past a row's end)
 
     def __init__(self, cfg, state_dict, slots: int, device: Optional[int] = None, blocks_impl: str = "tcgen05", stage_workers: int = 8,
-                 row_staging: bool = True):
+                 row_staging: bool = True, range_fallback: bool = False):
         import torch
         from .batched import BatchedTracker
         self.torch = torch
-        self.bt = BatchedTracker(cfg, state_dict, max_tracks=slots, device=device, blocks_impl=blocks_impl)
+        # range_fallback: a step recomputes the tracks flagged as out of fp16 range on the fp32 kernels, so they are not dropped
+        self.bt = BatchedTracker(cfg, state_dict, max_tracks=slots, device=device, blocks_impl=blocks_impl, range_fallback=range_fallback)
         self.dev = self.bt.device
         self.slots = slots
         self.search_factor = float(cfg.TEST.SEARCH_FACTOR)
@@ -487,10 +488,12 @@ class MultiSequenceRunner:
 
 
 def run_sequences(sequences: Seq[Sequence], cfg, state_dict, slots: int = 64, results_dir: Optional[str] = None,
-                  device: Optional[int] = None, blocks_impl: str = "tcgen05", row_staging: bool = True, **kw) -> Dict[str, dict]:
-    """Track every sequence; ``slots`` run concurrently on one GPU."""
+                  device: Optional[int] = None, blocks_impl: str = "tcgen05", row_staging: bool = True, range_fallback: bool = False,
+                  **kw) -> Dict[str, dict]:
+    """Track every sequence; ``slots`` run concurrently on one GPU.  ``range_fallback``: see BatchedTracker."""
     slots = max(1, min(slots, len(sequences)))
-    backend = BatchedBackend(cfg, state_dict, slots, device=device, blocks_impl=blocks_impl, row_staging=row_staging)
+    backend = BatchedBackend(cfg, state_dict, slots, device=device, blocks_impl=blocks_impl, row_staging=row_staging,
+                             range_fallback=range_fallback)
     runner = MultiSequenceRunner(backend, slots, results_dir=results_dir, **kw)
     try:
         return runner.run(sequences)

@@ -63,7 +63,10 @@ class Vit_dist(BaseTracker):
         super().__init__(params)
         self.cfg = params.cfg
         depth = int(getattr(params, "depth", getattr(params.cfg.MODEL.BACKBONE, "DEPTH", 3)))
-        network = build_ostrack_dist(params.cfg, depth=depth, blocks_impl=getattr(params, "blocks_impl", "tcgen05"))
+        # params.range_fallback: a track the tensor-core kernels flag as out of fp16 range is recomputed on the fp32 kernels in the same
+        # step (the result a blocks_impl = 'simt' tracker gives) instead of raising FloatingPointError
+        network = build_ostrack_dist(params.cfg, depth=depth, blocks_impl=getattr(params, "blocks_impl", "tcgen05"),
+                                     range_fallback=bool(getattr(params, "range_fallback", False)))
         ckpt = getattr(params, "checkpoint", None)
         state_dict = getattr(params, "state_dict", None)         # in-memory alternative to a checkpoint file
         if state_dict is None:
@@ -231,7 +234,8 @@ class Vit_dist(BaseTracker):
             raise Exception('Too small bounding box.')
         if int(out[11]) == 3:
             raise FloatingPointError("an activation left the fp16 operand range of the tensor-core path (or was non-finite): result "
-                                     "withheld; construct the tracker with params.blocks_impl = 'simt' for these weights")
+                                     "withheld; set params.range_fallback = True to recompute such "
+                                     "frames on the fp32 kernels, or params.blocks_impl = 'simt' for these weights")
         if int(out[11]) != 0:
             raise ValueError("search crop lies outside the image (undefined behaviour in the reference)")
         pred_box = out[5:9]                                      # (cx, cy, w, h) as `.tolist()` of the fp32 tensor
