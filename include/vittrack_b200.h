@@ -51,6 +51,7 @@ typedef enum VtStatus {
                                    * vt_set_range_fallback recomputes such tracks on the fp32 kernels within the
                                    * same step call.                                                           */
 #define VT_TRACK_BAD_SLOT 4       /* slot outside [0, max_tracks) or named by an earlier item of the same call */
+#define VT_TRACK_BAD_RECORD 5     /* vt_tracks_import*: the record failed a check (header, fingerprint, checksum, box); nothing written */
 
 /* Which implementation of the ViT blocks vt_forward / vt_tracks_step use. */
 #define VT_BLOCKS_SIMT_FP32 0     /* fp32 CUDA-core kernel: bring-up / exact mode                 */
@@ -213,6 +214,69 @@ int vt_set_range_fallback(VtHandle h, int32_t enable, int64_t* counter_dev);
 /* Read / overwrite the per-track boxes ([n][4] float64 device pointers). */
 int vt_tracks_get_state(VtHandle h, double* boxes_xywh, int32_t first, int32_t n, void* stream);
 int vt_tracks_set_state(VtHandle h, const double* boxes_xywh, int32_t first, int32_t n, void* stream);
+
+/* Track records: a whole track state (box + cached template tokens) as a fixed-size, self-checking byte image, so that a track can
+ * be saved, restored, forked, or moved to another slot, handle or GPU and continue bit for bit.  A record is
+ * R = VT_TRACK_RECORD_HEADER_BYTES + 256 C bytes (12 352 at C = 48, 196 672 at C = 768), all fields little-endian:
+ *   offset  bytes  field
+ *        0      4  uint32 VT_TRACK_RECORD_MAGIC
+ *        4      4  uint32 VT_TRACK_RECORD_VERSION
+ *        8      8  uint64 weights fingerprint of the exporting handle (vt_weights_fingerprint)
+ *       16      4  int32  embed_dim C
+ *       20      4  int32  template token rows (64)
+ *       24      8  uint64 checksum of the payload (below)
+ *       32     32  float64 box x, y, w, h (the track state)
+ *       64  256 C  float32 template tokens [64][C]: stem output + pos_embed_z, as vt_tracks_init computed them
+ * Payload checksum: the payload is bytes [32, R) read as little-endian uint64 words w_0 .. w_{K-1} (K = 4 + 32 C; w_0 .. w_3 the
+ * box), and
+ *     checksum = sum over k of splitmix64(w_k + k * 0x9E3779B97F4A7C15)  (mod 2^64),
+ *     splitmix64(z): z += 0x9E3779B97F4A7C15; z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9; z = (z ^ (z >> 27)) * 0x94D049BB133111EB;
+ *                    return z ^ (z >> 31)           (all arithmetic mod 2^64)
+ * which depends on every word and its position, and not on the order in which the terms are added.
+ * Weights fingerprint, computed on the host by vt_finalize_weights: FNV-1a 64 (offset basis 0xcbf29ce484222325, prime
+ * 0x100000001b3) over 8-byte little-endian words of a byte stream (h ^= word; h *= prime), the last word zero-padded:
+ *   1. the 24 ASCII bytes "vittrack_b200 weights v1" (no terminator);
+ *   2. int32 embed_dim, num_heads, depth, mlp_ratio, head_channels, stride, template_size, search_size, then float64
+ *      template_factor, search_factor (max_tracks, chunk_tracks, device and blocks_impl are not hashed);
+ *   3. int32 template route: how the handle computes template tokens.  0: vit_48_h32 (fp32 crop + stem on the CUDA cores for every
+ *      blocks_impl); other configurations: 1 VT_BLOCKS_SIMT_FP32 (fp32 GEMMs), 2 tensor-core GEMMs, 3 tensor-core split-image GEMMs
+ *      (embed_dim % 128 == 0);
+ *   4. every tensor the handle holds ("*.num_batches_tracked" is never held; tracker.output_window is
+ *      when it was set) in byte-wise ascending name order: the name's bytes and a NUL, int32 ndim, int64 shape[ndim], then the fp32
+ *      data exactly as vt_set_tensor received it (before BatchNorm folding or scale rebalancing).
+ * Two handles with equal fingerprints compute the same template-token bits from the same frame and box, so a record moves freely
+ * between them (e.g. between the VT_BLOCKS_* of vit_48_h32, which share route 0).  Hashing is one multiply per 8 bytes: about
+ * 82 ms for the widest configuration's 381 MB on one Intel Xeon core, of the 1.8 s vt_finalize_weights takes there in all. */
+#define VT_TRACK_RECORD_MAGIC 0x52545456u     /* "VTTR" as little-endian bytes */
+#define VT_TRACK_RECORD_VERSION 1
+#define VT_TRACK_RECORD_HEADER_BYTES 64       /* bytes before the template tokens: the fields above and the box */
+
+/* The handle's weights fingerprint (host out_host); VT_ERR_STATE before vt_finalize_weights. */
+int vt_weights_fingerprint(VtHandle h, uint64_t* out_host);
+/* R, the size of one record of this handle, in bytes (host out_host). */
+int vt_track_record_bytes(VtHandle h, int64_t* out_host);
+/* Export tracks [first, first + n), or slots[i] for item i, into `records`; import records into tracks [first, first + n) or slots.
+ *   - `records` is a DEVICE array of n records R bytes apart, 16-byte aligned.  `slots` and out_status are device int32 [n]; out_status
+ *     may be null.  Export's out_status[i] is VT_TRACK_OK or VT_TRACK_BAD_SLOT; import's VT_TRACK_OK, VT_TRACK_BAD_SLOT or
+ *     VT_TRACK_BAD_RECORD.
+ *   - Export is VT_ERR_STATE before vt_finalize_weights.  A slot that was never initialised exports the zero box of vt_create.
+ *   - Import checks every record on the device, without a host synchronisation: magic, version, C, rows, a fingerprint equal to this
+ *     handle's, the checksum and a finite box.  A record that fails any check gets VT_TRACK_BAD_RECORD and writes nothing.
+ *   - Slot lists are checked as in vt_tracks_init_slots: an entry outside [0, max_tracks) or repeating an earlier item's slot gets
+ *     VT_TRACK_BAD_SLOT (which takes precedence over VT_TRACK_BAD_RECORD); the first item wins.  An export item with a bad slot writes
+ *     an all-zero record (magic 0: it can never be imported).
+ *   - Import writes the state and the template tokens in place (CUDA graphs captured earlier stay valid) and makes the handle ready
+ *     to step, as vt_tracks_init does.
+ *   - An accepted record continues exactly as the exported track would have: its out_boxes, out_detail, maps and new state are the
+ *     same bits, for range and slot-list steps, in any chunk, with the range fallback on or off.
+ *   - VT_ERR_INVALID_ARG before any launch for a null handle, n < 0, n > max_tracks, first < 0 or first + n > max_tracks, a null
+ *     pointer when n > 0, or a `records` that is not 16-byte aligned.  n == 0 is a no-op.
+ *   - No allocation and no host synchronisation: the calls can be captured in a CUDA graph and replayed with new contents in `slots`
+ *     and `records`.  One kernel launch per range call, two per slot-list call (the slot claim, then the copy). */
+int vt_tracks_export(VtHandle h, int32_t first, int32_t n, uint8_t* records, void* stream);
+int vt_tracks_export_slots(VtHandle h, const int32_t* slots, int32_t n, uint8_t* records, int32_t* out_status, void* stream);
+int vt_tracks_import(VtHandle h, const uint8_t* records, int32_t first, int32_t n, int32_t* out_status, void* stream);
+int vt_tracks_import_slots(VtHandle h, const uint8_t* records, const int32_t* slots, int32_t n, int32_t* out_status, void* stream);
 
 /* Maps of the most recent vt_tracks_step chunk-by-chunk copy: score [n][F*F], size [n][2][F*F],
  * offset [n][2][F*F] for tracks [first, first+n) of that step (debug / parity aid; any may be

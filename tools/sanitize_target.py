@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Small workload for compute-sanitizer (tools/sanitize.sh): every hand-written kernel once, at sizes a 10 - 100x slowdown can afford.
-Fast path (vit_48_h32): tracks_init + two closed-loop steps of 5 tracks on tcgen05 (crop_taps, crop_conv1, conv_s2_tc x3, blocks_tc,
+Fast path (vit_48_h32): tracks_init + two closed-loop steps of 5 tracks, then track records out and back in, on tcgen05 (crop_taps, crop_conv1, conv_s2_tc x3, blocks_tc,
 head_tc), the same on the fp32 CUDA-core kernels, vt_forward, vt_crop_normalize, vt_cal_bbox.  Generic path (C 96 / 3 heads / depth 2 /
 head 64): tracks + forward (im2col, gemm_tc_kernel NT / NN, sgemm, layernorm, softmax, decode)."""
 import os, sys
@@ -20,6 +20,9 @@ if which in ("all", "fast"):
         assert int(bt.initialize(pool, torch.zeros(5, dtype=torch.int64), boxes).abs().sum()) == 0
         for t in range(2):
             out = bt.track(pool, torch.full((5,), (t + 1) % 2, dtype=torch.int64), update_state=True)
+        recs = bt.export_tracks(slots=[4, 0, 2])                   # track records: export and import kernels, by range and by slot
+        assert int(bt.import_tracks(recs, slots=[1, 3, 0]).abs().sum()) == 0
+        assert int(bt.import_tracks(bt.export_tracks()).abs().sum()) == 0
         z = torch.randn(3, 3, 128, 128)
         x = torch.randn(3, 3, 256, 256)
         fw = bt.engine.forward(z, x, taps=True)

@@ -25,6 +25,9 @@ def __getattr__(name):
     if name in ("Sequence", "MultiSequenceRunner", "BatchedBackend", "run_sequences", "save_tracker_output", "read_image"):
         from . import sequences
         return getattr(sequences, name)
+    if name in ("TrackRecords",):
+        from . import records
+        return getattr(records, name)
     if name in ("CropPreprocessor", "NestedTensor"):
         from . import preprocess
         return getattr(preprocess, name)

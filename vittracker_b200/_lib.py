@@ -16,6 +16,7 @@ VT_BLOCKS_SIMT_FP32 = 0
 VT_BLOCKS_TCGEN05 = 1
 VT_BLOCKS_TCGEN05_3TERM = 2
 VT_TRACK_OK, VT_TRACK_TOO_SMALL, VT_TRACK_OUT_OF_DOMAIN, VT_TRACK_NUMERIC_RANGE, VT_TRACK_BAD_SLOT = 0, 1, 2, 3, 4
+VT_TRACK_BAD_RECORD = 5
 
 STATUS_NAMES = {0: "VT_OK", -1: "VT_ERR_INVALID_ARG", -2: "VT_ERR_CUDA", -3: "VT_ERR_WEIGHTS", -4: "VT_ERR_STATE",
                 -5: "VT_ERR_UNSUPPORTED", -6: "VT_ERR_NO_DEVICE"}
@@ -52,6 +53,12 @@ SIGNATURES = {
     "vt_tracks_init_slots": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "vt_tracks_step_slots": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, C.c_int32, _P]),
     "vt_set_range_fallback": (C.c_int, [_P, C.c_int32, _P]),
+    "vt_weights_fingerprint": (C.c_int, [_P, C.POINTER(C.c_uint64)]),
+    "vt_track_record_bytes": (C.c_int, [_P, C.POINTER(C.c_int64)]),
+    "vt_tracks_export": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P]),
+    "vt_tracks_export_slots": (C.c_int, [_P, _P, C.c_int32, _P, _P, _P]),
+    "vt_tracks_import": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, _P]),
+    "vt_tracks_import_slots": (C.c_int, [_P, _P, _P, C.c_int32, _P, _P]),
     "vt_tracks_get_state": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P]),
     "vt_tracks_set_state": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P]),
     "vt_tracks_last_maps": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P]),

@@ -13,6 +13,7 @@ import numpy as np
 import torch
 
 from .engine import YUV_FORMATS, Engine, yuv420_frame_hw, yuv_format
+from .records import TrackRecords
 
 
 class FramePool:
@@ -297,6 +298,47 @@ class BatchedTracker:
             raise ValueError(f"{offsets.shape[0]} frames for {slots.shape[0]} slots")
         return self.engine.tracks_step_slots(frames, offsets, hw, slots, out_boxes=self.out_boxes[: slots.shape[0]],
                                              update_state=update_state, detail=detail)
+
+    def export_tracks(self, slots=None) -> TrackRecords:
+        """Track records of tracks 0..n-1, or of the listed slots in list order, with each track's frame size: save them, or import them
+        into this or another tracker (``records.to("cuda:1")`` moves them to another GPU).  A bad entry of a CUDA slot tensor gets an
+        all-zero record, which every import rejects."""
+        if slots is None:
+            return TrackRecords(self.engine.tracks_export(0, self.n), self._slot_hw[: self.n].clone())
+        slots = self._slots(slots)
+        records, _ = self.engine.tracks_export_slots(slots)
+        return TrackRecords(records, self._slot_hw[self._rows(slots)])
+
+    def import_tracks(self, records: TrackRecords, slots=None) -> torch.Tensor:
+        """Continue exported tracks here, bit for bit: without ``slots`` as tracks 0..n-1 (as ``initialize`` sets them up), else into the
+        listed slots.  The device checks every record; returns the status per item: VT_TRACK_OK, VT_TRACK_BAD_RECORD (5: other weights,
+        another embed dim, or an altered record; the track is left as it was, records.describe_rejection says why) or, by slot,
+        VT_TRACK_BAD_SLOT.  Frame sizes are taken for the accepted items only, without a host synchronisation."""
+        if not isinstance(records, TrackRecords):
+            raise ValueError("records: expected a TrackRecords (BatchedTracker.export_tracks / TrackRecords.load)")
+        rec, hw = records.records, records.frame_hw
+        R, n = self.engine.track_record_bytes, len(records)
+        if rec.dtype != torch.uint8 or rec.dim() != 2 or rec.shape[1] != R:
+            raise ValueError(f"records of {tuple(rec.shape)} {rec.dtype}: this tracker's records are uint8 [n, {R}]")
+        if not (rec.is_contiguous() and hw.is_contiguous()) or rec.data_ptr() % 16:
+            raise ValueError("records: expected contiguous, 16-byte aligned tensors")
+        if rec.device != self.device or hw.device != self.device:
+            raise ValueError(f"records on {rec.device}, tracker on {self.device}: move them with records.to(...)")
+        if n > self.max_tracks:
+            raise ValueError(f"{n} records > max_tracks {self.max_tracks}")
+        if slots is None:
+            status = self.engine.tracks_import(rec, first=0)
+            self._slot_hw[:n] = torch.where((status == 0)[:, None], hw, self._slot_hw[:n])
+            self.n = n
+            self._hw = self._slot_hw[:n].clone()
+            return status
+        slots = self._slots(slots)
+        if slots.shape[0] != n:
+            raise ValueError(f"{slots.shape[0]} slots for {n} records")
+        rows = self._rows(slots)
+        status = self.engine.tracks_import_slots(rec, slots)
+        self._slot_hw[rows] = torch.where((status == 0)[:, None], hw, self._slot_hw[rows])
+        return status
 
     def _yuv_frames(self, surfaces: YuvSurfaces) -> Tuple[torch.Tensor, torch.Tensor]:
         if surfaces.n > self.max_tracks:

@@ -20,7 +20,7 @@ LIB_DIR = os.path.abspath(os.environ["VT_LIB_DIR"]) if os.environ.get("VT_LIB_DI
 LIB_PATH = os.path.join(LIB_DIR, "libvittrack_b200.so")
 STAMP = os.path.join(LIB_DIR, "build.stamp")
 
-SOURCES = ["vt_api.cu", "vt_crop.cu", "vt_stem.cu", "vt_stem_tc.cu", "vt_stem_fused.cu", "vt_block_simt.cu", "vt_block_tc.cu", "vt_head.cu", "vt_generic.cu", "vt_yuv.cu", "vt_slots.cu"]
+SOURCES = ["vt_api.cu", "vt_crop.cu", "vt_stem.cu", "vt_stem_tc.cu", "vt_stem_fused.cu", "vt_block_simt.cu", "vt_block_tc.cu", "vt_head.cu", "vt_generic.cu", "vt_yuv.cu", "vt_slots.cu", "vt_records.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fno-fast-math", "-Xcompiler", "-fopenmp", "--fmad=true", "-I", INCLUDE]
 

@@ -17,6 +17,7 @@
 using namespace vt;
 static_assert(vt::VT_TRACK_NUMERIC_RANGE_ == VT_TRACK_NUMERIC_RANGE, "status code shared with the kernels");
 static_assert(vt::VT_TRACK_BAD_SLOT_ == VT_TRACK_BAD_SLOT, "status code shared with the kernels");
+static_assert(vt::kNz * 4 == 256 && VT_TRACK_RECORD_HEADER_BYTES % 16 == 0, "record layout: 64 + 256 C bytes, 16-byte vectors");
 
 namespace {
 
@@ -36,6 +37,7 @@ struct VtContext {
     TensorMap tensors;
     bool finalized = false;
     bool tracks_ready = false;
+    uint64_t fingerprint = 0;         // of the weights finalised last (vt_weights_fingerprint)
     int64_t launches = 0;
 
     float* d_weights = nullptr;       // packed model
@@ -234,6 +236,52 @@ int rebalance(const VtConfig& c, TensorMap& ts) {
         for (int i = 0; i < 4; ++i)
             affine_to(head_prefix(i, t) + "1.", {i < 3 ? head_prefix(i + 1, t) + "0.weight" : std::string("box_head.conv5_") + kTowers[t] + ".weight"});
     return pnorm;
+}
+
+// FNV-1a 64 over 8-byte little-endian words of a byte stream, the last word zero-padded (the weights fingerprint of the header).
+// Word-wise rather than byte-wise: one multiply per 8 bytes.
+struct WordFnv {
+    uint64_t h = 0xcbf29ce484222325ull;
+    uint8_t tail[8];
+    size_t nt = 0;
+    void word(uint64_t w) { h = (h ^ w) * 0x100000001b3ull; }
+    void bytes(const void* p, size_t n) {
+        const uint8_t* b = static_cast<const uint8_t*>(p);
+        while (nt && n) { tail[nt++] = *b++; --n; if (nt == 8) { uint64_t w; memcpy(&w, tail, 8); word(w); nt = 0; } }
+        for (; n >= 8; b += 8, n -= 8) { uint64_t w; memcpy(&w, b, 8); word(w); }
+        while (n) { tail[nt++] = *b++; --n; }
+    }
+    template <typename T> void put(T v) { bytes(&v, sizeof v); }
+    uint64_t finish() {
+        if (nt) { memset(tail + nt, 0, 8 - nt); uint64_t w; memcpy(&w, tail, 8); word(w); nt = 0; }
+        return h;
+    }
+};
+
+// The template route of the fingerprint: which kernels compute a handle's template tokens.  vit_48_h32 crops and runs the template stem
+// on the fp32 CUDA-core kernels for every blocks_impl (launch_crop_stem takes the tensor-core branch for the search crop only); the
+// generic stem follows GenModelW's GEMM route.
+int32_t template_route(VtHandle h) {
+    if (!h->generic) return 0;
+    return h->gw.fp32_only ? 1 : h->gw.use_img ? 3 : 2;
+}
+
+uint64_t weights_fingerprint(VtHandle h) {
+    static const char kVersion[] = "vittrack_b200 weights v1";
+    WordFnv f;
+    f.bytes(kVersion, sizeof kVersion - 1);
+    const VtConfig& c = h->cfg;
+    for (int32_t v : {c.embed_dim, c.num_heads, c.depth, c.mlp_ratio, c.head_channels, c.stride, c.template_size, c.search_size}) f.put(v);
+    f.put(c.template_factor);
+    f.put(c.search_factor);
+    f.put(template_route(h));
+    for (const auto& e : h->tensors) {                 // std::map: ascending byte-wise name order
+        f.bytes(e.first.c_str(), e.first.size() + 1);
+        f.put((int32_t)e.second.shape.size());
+        for (int64_t d : e.second.shape) f.put(d);
+        f.bytes(e.second.data.data(), e.second.data.size() * sizeof(float));
+    }
+    return f.finish();
 }
 
 // The packed weights: one fp32 buffer of 16-byte aligned slots.  slot() allocates one for the ModelW / GenModelW member that will
@@ -647,6 +695,36 @@ int range_fallback(VtHandle h, const uint8_t* frames, const int64_t* frame_offse
     return VT_OK;
 }
 
+int64_t record_bytes(VtHandle h) { return VT_TRACK_RECORD_HEADER_BYTES + (int64_t)256 * h->cfg.embed_dim; }
+
+// Host checks shared by the four record calls, before any launch.
+int check_records_call(VtHandle h, const char* where, int first, int n, const void* records, const int32_t* slots, bool range) {
+    if (const int rc = check_ready(h, false)) return rc;
+    if (n < 0 || n > h->cfg.max_tracks || first < 0 || first + n > h->cfg.max_tracks)
+        return fail(h, VT_ERR_INVALID_ARG, "%s: tracks [%d, %d) exceed max_tracks %d", where, first, first + n, h->cfg.max_tracks);
+    if (n == 0) return VT_OK;
+    if (!records || (!range && !slots)) return fail(h, VT_ERR_INVALID_ARG, "%s: null pointer", where);
+    if (reinterpret_cast<uintptr_t>(records) % 16) return fail(h, VT_ERR_INVALID_ARG, "%s: records must be 16-byte aligned", where);
+    return VT_OK;
+}
+
+// Export (records written) or import (records read) over items [0, n): track first + i, or slots[i].  An import makes the handle ready
+// to step, as an init does.
+int tracks_records(VtHandle h, bool do_export, uint8_t* records, int first, const int32_t* slots, int n, int32_t* out_status,
+                   cudaStream_t st) {
+    DeviceGuard dg(h->cfg.device);
+    VT_CUDA(h, dg.err);
+    const RecordArgs a{h->d_state, h->d_tmpl, h->cfg.embed_dim, first, h->cfg.max_tracks, slots, h->d_claim, out_status, h->fingerprint};
+    if (slots) VT_LAUNCH(h, kNoStage, n, st, "track records/claim", launch_claim_slots(slots, n, h->cfg.max_tracks, h->d_claim, st));
+    if (do_export) {
+        VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_export", launch_tracks_export(a, records, n, st));
+    } else {
+        VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_import", launch_tracks_import(a, records, n, st));
+        h->tracks_ready = true;
+    }
+    return VT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -775,6 +853,7 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     DeviceGuard dg(h->cfg.device);
     VT_CUDA(h, dg.err);
     if (const int rc = check_missing(h)) return rc;
+    h->fingerprint = weights_fingerprint(h);
     TensorMap ts = h->tensors;          // rebalanced on a copy: finalising again starts from the tensors as they were set
     const int pnorm = rebalance(h->cfg, ts);
     if (h->generic) return finalize_generic(h, ts, pnorm, st);
@@ -1013,6 +1092,44 @@ int vt_set_range_fallback(VtHandle h, int32_t enable, int64_t* counter_dev) {
     h->fallback = enable != 0;
     h->fallback_counter = enable ? counter_dev : nullptr;
     return VT_OK;
+}
+
+int vt_weights_fingerprint(VtHandle h, uint64_t* out_host) {
+    if (const int rc = check_ready(h, false)) return rc;
+    if (!out_host) return fail(h, VT_ERR_INVALID_ARG, "vt_weights_fingerprint: null pointer");
+    *out_host = h->fingerprint;
+    return VT_OK;
+}
+
+int vt_track_record_bytes(VtHandle h, int64_t* out_host) {
+    if (!h) return VT_ERR_INVALID_ARG;
+    if (!out_host) return fail(h, VT_ERR_INVALID_ARG, "vt_track_record_bytes: null pointer");
+    *out_host = record_bytes(h);
+    return VT_OK;
+}
+
+int vt_tracks_export(VtHandle h, int32_t first, int32_t n, uint8_t* records, void* stream) {
+    if (const int rc = check_records_call(h, "vt_tracks_export", first, n, records, nullptr, true)) return rc;
+    if (n == 0) return VT_OK;
+    return tracks_records(h, true, records, first, nullptr, n, nullptr, (cudaStream_t)stream);
+}
+
+int vt_tracks_export_slots(VtHandle h, const int32_t* slots, int32_t n, uint8_t* records, int32_t* out_status, void* stream) {
+    if (const int rc = check_records_call(h, "vt_tracks_export_slots", 0, n, records, slots, false)) return rc;
+    if (n == 0) return VT_OK;
+    return tracks_records(h, true, records, 0, slots, n, out_status, (cudaStream_t)stream);
+}
+
+int vt_tracks_import(VtHandle h, const uint8_t* records, int32_t first, int32_t n, int32_t* out_status, void* stream) {
+    if (const int rc = check_records_call(h, "vt_tracks_import", first, n, records, nullptr, true)) return rc;
+    if (n == 0) return VT_OK;
+    return tracks_records(h, false, const_cast<uint8_t*>(records), first, nullptr, n, out_status, (cudaStream_t)stream);
+}
+
+int vt_tracks_import_slots(VtHandle h, const uint8_t* records, const int32_t* slots, int32_t n, int32_t* out_status, void* stream) {
+    if (const int rc = check_records_call(h, "vt_tracks_import_slots", 0, n, records, slots, false)) return rc;
+    if (n == 0) return VT_OK;
+    return tracks_records(h, false, const_cast<uint8_t*>(records), 0, slots, n, out_status, (cudaStream_t)stream);
 }
 
 int vt_tracks_get_state(VtHandle h, double* boxes_xywh, int32_t first, int32_t n, void* stream) {

@@ -396,6 +396,20 @@ int gen_launch_blocks_head(float* tokens, int n, const GenModelW& w, const GenWo
 // slots [n] as the caller gave them -> eff [n]: the slot, or -1 for an entry outside [0, max_tracks) or repeating an earlier item's.
 // claim: [max_tracks] uint32, all 0xffffffff between calls (the second kernel restores what the first changed).
 int launch_resolve_slots(const int32_t* slots, int n, int max_tracks, uint32_t* claim, int32_t* eff, cudaStream_t st);
+// Its first kernel alone: every valid entry claims its slot.  A kernel that runs next on the stream resolves item i with resolve_slot.
+int launch_claim_slots(const int32_t* slots, int n, int max_tracks, uint32_t* claim, cudaStream_t st);
+#ifdef __CUDACC__
+// Item i's effective slot after the claim, or -1; the winner releases its claim.  A losing item reads the winner's index or the released
+// value, neither of which is its own, so the release needs no ordering against it.
+__device__ __forceinline__ int resolve_slot(const int32_t* slots, int i, int max_tracks, uint32_t* claim) {
+    const int s = slots[i];
+    if (s >= 0 && s < max_tracks && claim[s] == (uint32_t)i) {
+        claim[s] = 0xffffffffu;
+        return s;
+    }
+    return -1;
+}
+#endif
 // Gather: dst + i * dst_stride <- src + eff[i] * src_stride, `row` floats (zeros for eff[i] < 0).
 int launch_gather_rows(const float* src, size_t src_stride, float* dst, size_t dst_stride, size_t row, const int32_t* eff, int n,
                        cudaStream_t st);
@@ -403,6 +417,21 @@ int launch_gather_rows(const float* src, size_t src_stride, float* dst, size_t d
 // (nullable) <- status[i], or VT_TRACK_BAD_SLOT for eff[i] < 0.
 int launch_scatter_init(const float* tok, float* tmpl, size_t row, const double* boxes, double* state, const int32_t* status,
                         int32_t* out_status, const int32_t* eff, int n, cudaStream_t st);
+
+// ---- track records (vt_tracks_export* / vt_tracks_import*; vt_records.cu) ------------------------------------------------
+// Item i of n works on track first + i (slots == NULL), or on slots[i] resolved against `claim` after launch_claim_slots (first == 0).
+// state [max_tracks][4] and tmpl [max_tracks][64][C] are the handle's; records [n][64 + 256 C] (16-byte aligned); out_status nullable.
+struct RecordArgs {
+    double* state;
+    float* tmpl;
+    int C, first, max_tracks;
+    const int32_t* slots;
+    uint32_t* claim;
+    int32_t* out_status;
+    uint64_t fingerprint;     // the handle's: written by export, required by import
+};
+int launch_tracks_export(const RecordArgs& a, uint8_t* records, int n, cudaStream_t st);
+int launch_tracks_import(const RecordArgs& a, const uint8_t* records, int n, cudaStream_t st);
 
 // ---- range fallback (vt_set_range_fallback; vt_slots.cu) ------------------------------------------------
 // The items of a tensor-core step that ended with VT_TRACK_NUMERIC_RANGE, compacted in item order, and the fp32 pass's rows for them.

@@ -15,19 +15,18 @@ __global__ void claim_slots_kernel(const int32_t* __restrict__ slots, int n, int
     if (s >= 0 && s < max_tracks) atomicMin(claim + s, (uint32_t)i);
 }
 
-// The winner of each slot reads its own index back and then releases the claim.  A losing item reads the winner's index or the
-// released value, neither of which is its own, so the release needs no ordering against it.
+// The winner of each slot reads its own index back and then releases the claim (resolve_slot).
 __global__ void resolve_slots_kernel(const int32_t* __restrict__ slots, int n, int max_tracks, uint32_t* __restrict__ claim,
                                      int32_t* __restrict__ eff) {
     const int i = blockIdx.x * kSlotThreads + threadIdx.x;
     if (i >= n) return;
-    const int s = slots[i];
-    int e = -1;
-    if (s >= 0 && s < max_tracks && claim[s] == (uint32_t)i) {
-        e = s;
-        claim[s] = 0xffffffffu;
-    }
-    eff[i] = e;
+    eff[i] = resolve_slot(slots, i, max_tracks, claim);
+}
+
+int launch_claim_slots(const int32_t* slots, int n, int max_tracks, uint32_t* claim, cudaStream_t st) {
+    if (n <= 0) return 0;
+    claim_slots_kernel<<<(n + kSlotThreads - 1) / kSlotThreads, kSlotThreads, 0, st>>>(slots, n, max_tracks, claim);
+    return cudaGetLastError() == cudaSuccess ? 1 : -1;
 }
 
 int launch_resolve_slots(const int32_t* slots, int n, int max_tracks, uint32_t* claim, int32_t* eff, cudaStream_t st) {

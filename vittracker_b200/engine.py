@@ -305,6 +305,68 @@ class Engine:
         if counter is not None:
             self._fallback_counters = getattr(self, "_fallback_counters", []) + [counter]
 
+    # ------------------------------------------------------------------------------------------
+    @property
+    def weights_fingerprint(self) -> int:
+        """vt_weights_fingerprint: the hash of the configuration, template route and tensors this engine's weights were finalised from
+        (records.weights_fingerprint restates it).  Equal fingerprints: a track record moves between the two engines bit for bit."""
+        out = C.c_uint64()
+        self._check(self.lib.vt_weights_fingerprint(self.handle, C.byref(out)))
+        return int(out.value)
+
+    @property
+    def track_record_bytes(self) -> int:
+        """R, the size of one track record of this engine (64 + 256 C bytes)."""
+        out = C.c_int64()
+        self._check(self.lib.vt_track_record_bytes(self.handle, C.byref(out)))
+        return int(out.value)
+
+    def _records(self, records: torch.Tensor, n: int) -> torch.Tensor:
+        R = self.track_record_bytes
+        if (records.dtype != torch.uint8 or records.device != self.device or not records.is_contiguous() or tuple(records.shape) != (n, R)
+                or records.data_ptr() % 16):
+            raise ValueError(f"records: expected a contiguous, 16-byte aligned uint8 tensor of shape ({n}, {R}) on {self.device}")
+        return records
+
+    def tracks_export(self, first: int = 0, n: Optional[int] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """vt_tracks_export: the records of tracks [first, first + n) as uint8 [n, R] (into ``out`` when given)."""
+        n = self.max_tracks - first if n is None else int(n)
+        out = torch.empty((n, self.track_record_bytes), dtype=torch.uint8, device=self.device) if out is None else self._records(out, n)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_tracks_export(self.handle, int(first), n, _ptr(out), self._stream()))
+        return out
+
+    def tracks_export_slots(self, slots: torch.Tensor, out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """vt_tracks_export_slots: record i of track ``slots[i]``; returns (records [n, R], status [n]: VT_TRACK_OK or
+        VT_TRACK_BAD_SLOT, whose record is all zeros)."""
+        n = int(slots.shape[0])
+        self._slot_tensor(slots, n)
+        out = torch.empty((n, self.track_record_bytes), dtype=torch.uint8, device=self.device) if out is None else self._records(out, n)
+        status = torch.empty((n,), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_tracks_export_slots(self.handle, _ptr(slots), n, _ptr(out), _ptr(status), self._stream()))
+        return out, status
+
+    def tracks_import(self, records: torch.Tensor, first: int = 0) -> torch.Tensor:
+        """vt_tracks_import: record i into track first + i, checked on the device.  Returns the status per item: VT_TRACK_OK, or
+        VT_TRACK_BAD_RECORD (header, fingerprint, checksum or box rejected; the track is left as it was)."""
+        n = int(records.shape[0])
+        self._records(records, n)
+        status = torch.empty((n,), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_tracks_import(self.handle, _ptr(records), int(first), n, _ptr(status), self._stream()))
+        return status
+
+    def tracks_import_slots(self, records: torch.Tensor, slots: torch.Tensor) -> torch.Tensor:
+        """vt_tracks_import_slots: record i into track ``slots[i]``; status per item as tracks_import's, or VT_TRACK_BAD_SLOT."""
+        n = int(slots.shape[0])
+        self._slot_tensor(slots, n)
+        self._records(records, n)
+        status = torch.empty((n,), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.vt_tracks_import_slots(self.handle, _ptr(records), _ptr(slots), n, _ptr(status), self._stream()))
+        return status
+
     def tracks_get_state(self, first: int = 0, n: Optional[int] = None) -> torch.Tensor:
         n = self.max_tracks - first if n is None else n
         out = torch.empty((n, 4), dtype=torch.float64, device=self.device)

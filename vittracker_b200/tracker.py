@@ -17,6 +17,7 @@ import torch
 from .batched import YuvSurfaces
 from .engine import yuv420_frame_hw, yuv_format
 from .model import build_ostrack_dist
+from .records import describe_rejection
 from .sequences import crop_rect
 from .weights import load_checkpoint
 
@@ -242,6 +243,31 @@ class Vit_dist(BaseTracker):
         self.state = clip_box(self.map_box_back(pred_box, resize_factor), H, W, margin=10)
         self.last_detail = {"argmax": int(out[10]), "resize_factor": out[9], "window_max": out[12], "device_box": out[0:4]}
         return {"target_bbox": self.state, "confidence": confidence}
+
+    def snapshot(self) -> dict:
+        """The tracker's state after the last frame, picklable: the track record (box and template tokens, bytes), the host ``state``
+        list as ``track`` returned it, ``frame_id`` and ``z_patch_arr``.  ``restore`` continues from it bit for bit: rewind this tracker,
+        fork a hypothesis into another one, or resume after a restart."""
+        if self.state is None:
+            raise RuntimeError("snapshot() needs an initialised tracker")
+        record = self.engine.tracks_export(0, 1)[0].cpu().numpy().tobytes()
+        return {"record": record, "state": list(self.state), "frame_id": self.frame_id, "z_patch_arr": self.z_patch_arr.copy()}
+
+    def restore(self, snapshot: dict) -> None:
+        """Continue from ``snapshot``: its record is imported into this tracker's track in place (a captured CUDA graph stays valid).
+        ValueError when the record is rejected, e.g. taken under other weights (fingerprint) or altered (checksum)."""
+        R = self.engine.track_record_bytes
+        rec = np.frombuffer(snapshot["record"], dtype=np.uint8)
+        if rec.size != R:
+            raise ValueError(f"snapshot record of {rec.size} bytes: this tracker's records have {R}")
+        status = int(self.engine.tracks_import(torch.from_numpy(rec.copy()).to(self._dev).view(1, R), first=0).item())
+        if status != 0:
+            why = describe_rejection(rec, self.engine.weights_fingerprint, self.engine.C)
+            raise ValueError(f"snapshot rejected by this tracker (status {status}): {why}")
+        self.state = list(snapshot["state"])
+        self.frame_id = int(snapshot["frame_id"])
+        self._z_patch_arr = np.array(snapshot["z_patch_arr"], copy=True)
+        self._z_patch_dev = None
 
     def _step_device(self) -> None:
         """State upload + one tracking step + result download for the single track.  Every buffer involved is allocated once (frame
