@@ -80,6 +80,25 @@ def test_unsupported_config_rejected():
     assert lib.vt_create(None, C.byref(h)) == -1
 
 
+def test_tensor_ptr_refuses_what_the_abi_would_misread():
+    from vittracker_b200.engine import tensor_ptr
+    cpu = torch.device("cpu")
+    boxes = torch.zeros((3, 4), dtype=torch.float64)
+    assert tensor_ptr(boxes, "boxes", torch.float64, cpu, (3, 4)).value == boxes.data_ptr()
+    assert tensor_ptr(None, "out_detail", torch.float64, cpu, (3, 8), optional=True).value is None
+    bad = {"None": None, "dtype": boxes.float(), "device": boxes.to("meta"), "non-contiguous": torch.zeros((4, 3), dtype=torch.float64).t(),
+           "short": boxes[:2], "numpy": boxes.numpy()}
+    for what, t in bad.items():
+        with pytest.raises(ValueError, match="boxes"):
+            tensor_ptr(t, "boxes", torch.float64, cpu, (3, 4))
+    R = 12352
+    base = torch.zeros(2 * R + 16, dtype=torch.uint8)
+    assert tensor_ptr(base[16:16 + 2 * R].view(2, R), "records", torch.uint8, cpu, (2, R), align=16).value == base.data_ptr() + 16
+    with pytest.raises(ValueError, match="16-byte aligned"):
+        tensor_ptr(base[1:1 + 2 * R].view(2, R), "records", torch.uint8, cpu, (2, R), align=16)
+    assert tensor_ptr(base, "frames", torch.uint8, cpu).value == base.data_ptr()            # no shape: any buffer
+
+
 def test_shard_range_partitions():
     from vittracker_b200.batched import shard_range
     for total in (0, 1, 7, 8, 1024, 8191, 8192):

@@ -335,6 +335,45 @@ int check_ready(VtHandle h, bool need_tracks) {
     return VT_OK;
 }
 
+// Tracks [first, first + n) lie in [lo, lo + count): no intermediate overflows, whatever int32 values a caller passes.
+bool tracks_in(int first, int n, int lo, int count) { return n >= 0 && first >= lo && first - lo <= count - n; }
+
+int check_tracks(VtHandle h, const char* where, int first, int n) {
+    if (tracks_in(first, n, 0, h->cfg.max_tracks)) return VT_OK;
+    return fail(h, VT_ERR_INVALID_ARG, "%s: tracks [%d, %lld) exceed max_tracks %d", where, first, (long long)first + n, h->cfg.max_tracks);
+}
+
+int check_yuv_format(VtHandle h, const char* where, int format) {
+    if (format == VT_FRAME_NV12 || format == VT_FRAME_I420) return VT_OK;
+    return fail(h, VT_ERR_INVALID_ARG, "%s: unknown format %d", where, format);
+}
+
+// The checks every entry point that enqueues work starts with, in this order: a null handle; readiness (`need`); n < 0, or with
+// `range` tracks [first, first + n) outside max_tracks (a slot list passes first = 0); an empty batch, a successful no-op whose
+// pointers may be null (kEmpty); a null `required` pointer.  VT_ENTER returns on anything but VT_OK.
+enum Need { kHandle, kWeights, kTracks };
+constexpr int kEmpty = 1;
+int enter(VtHandle h, const char* where, Need need, int first, int n, bool range, std::initializer_list<const void*> required) {
+    if (!h) return VT_ERR_INVALID_ARG;
+    if (need != kHandle)
+        if (const int rc = check_ready(h, need == kTracks)) return rc;
+    if (range) {
+        if (const int rc = check_tracks(h, where, first, n)) return rc;
+    } else if (n < 0) {
+        return fail(h, VT_ERR_INVALID_ARG, "%s: negative n", where);
+    }
+    if (n == 0) return kEmpty;
+    for (const void* p : required)
+        if (!p) return fail(h, VT_ERR_INVALID_ARG, "%s: null pointer", where);
+    return VT_OK;
+}
+
+// Returns the prologue's status, or VT_OK for an empty batch; past it the handle's device is current until the entry point returns.
+#define VT_ENTER(h, prologue)                                           \
+    if (const int rc__ = (prologue)) return rc__ == kEmpty ? VT_OK : rc__; \
+    DeviceGuard dg__((h)->cfg.device);                                  \
+    VT_CUDA(h, dg__.err)
+
 int launch_fail(VtHandle h, int k, const char* where) {
     if (k == -2) return fail(h, VT_ERR_UNSUPPORTED, "%s: blocks_impl %d is not available in this build", where, h->cfg.blocks_impl);
     return fail(h, VT_ERR_CUDA, "%s: kernel launch failed: %s", where, cudaGetErrorString(cudaGetLastError()));
@@ -697,29 +736,43 @@ int range_fallback(VtHandle h, const uint8_t* frames, const int64_t* frame_offse
 
 int64_t record_bytes(VtHandle h) { return VT_TRACK_RECORD_HEADER_BYTES + (int64_t)256 * h->cfg.embed_dim; }
 
-// Host checks shared by the four record calls, before any launch.
-int check_records_call(VtHandle h, const char* where, int first, int n, const void* records, const int32_t* slots, bool range) {
-    if (const int rc = check_ready(h, false)) return rc;
-    if (n < 0 || n > h->cfg.max_tracks || first < 0 || first + n > h->cfg.max_tracks)
-        return fail(h, VT_ERR_INVALID_ARG, "%s: tracks [%d, %d) exceed max_tracks %d", where, first, first + n, h->cfg.max_tracks);
-    if (n == 0) return VT_OK;
-    if (!records || (!range && !slots)) return fail(h, VT_ERR_INVALID_ARG, "%s: null pointer", where);
-    if (reinterpret_cast<uintptr_t>(records) % 16) return fail(h, VT_ERR_INVALID_ARG, "%s: records must be 16-byte aligned", where);
-    return VT_OK;
+// The entry points below come in pairs: a range call over tracks [first, first + n) (slots == NULL) and its _slots twin (list, first
+// == 0), in which item i works on track slots[i].  Each pair is one checked function.  Only a list requires `slots`: a range call
+// repeats another required pointer in its place.
+
+// vt_tracks_init / vt_tracks_init_slots; an empty init still makes the handle ready to step.
+int init_call(VtHandle h, const char* where, bool list, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
+              const double* boxes_xywh, int first, const int32_t* slots, int n, int32_t* out_status, void* stream) {
+    const int rc = enter(h, where, kWeights, first, n, true, {frames, frame_offsets, frame_hw, boxes_xywh, list ? (const void*)slots : frames});
+    if (rc == kEmpty) h->tracks_ready = true;
+    VT_ENTER(h, rc);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (list) VT_LAUNCH(h, kNoStage, n, st, where, launch_resolve_slots(slots, n, h->cfg.max_tracks, h->d_claim, h->d_eff, st));
+    return tracks_init(h, frames, frame_offsets, frame_hw, boxes_xywh, first, list ? h->d_eff : nullptr, n, out_status, st);
 }
 
-// Export (records written) or import (records read) over items [0, n): track first + i, or slots[i].  An import makes the handle ready
+// vt_tracks_step / vt_tracks_step_slots
+int step_call(VtHandle h, const char* where, bool list, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
+              int first, const int32_t* slots, int n, double* out_boxes, double* out_detail, int update_state, void* stream) {
+    VT_ENTER(h, enter(h, where, kTracks, first, n, true, {frames, frame_offsets, frame_hw, out_boxes, list ? (const void*)slots : frames}));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (list) VT_LAUNCH(h, kNoStage, n, st, where, launch_resolve_slots(slots, n, h->cfg.max_tracks, h->d_claim, h->d_eff, st));
+    return tracks_step(h, frames, frame_offsets, frame_hw, first, list ? h->d_eff : nullptr, n, out_boxes, out_detail, update_state, st);
+}
+
+// vt_tracks_export (records written) and vt_tracks_import (records read), with their _slots twins.  An import makes the handle ready
 // to step, as an init does.
-int tracks_records(VtHandle h, bool do_export, uint8_t* records, int first, const int32_t* slots, int n, int32_t* out_status,
-                   cudaStream_t st) {
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
+int records_call(VtHandle h, const char* where, bool do_export, bool list, uint8_t* records, int first, const int32_t* slots, int n,
+                 int32_t* out_status, void* stream) {
+    VT_ENTER(h, enter(h, where, kWeights, first, n, true, {records, list ? (const void*)slots : records}));
+    if (reinterpret_cast<uintptr_t>(records) % 16) return fail(h, VT_ERR_INVALID_ARG, "%s: records must be 16-byte aligned", where);
+    cudaStream_t st = (cudaStream_t)stream;
     const RecordArgs a{h->d_state, h->d_tmpl, h->cfg.embed_dim, first, h->cfg.max_tracks, slots, h->d_claim, out_status, h->fingerprint};
-    if (slots) VT_LAUNCH(h, kNoStage, n, st, "track records/claim", launch_claim_slots(slots, n, h->cfg.max_tracks, h->d_claim, st));
+    if (list) VT_LAUNCH(h, kNoStage, n, st, where, launch_claim_slots(slots, n, h->cfg.max_tracks, h->d_claim, st));
     if (do_export) {
-        VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_export", launch_tracks_export(a, records, n, st));
+        VT_LAUNCH(h, kNoStage, n, st, where, launch_tracks_export(a, records, n, st));
     } else {
-        VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_import", launch_tracks_import(a, records, n, st));
+        VT_LAUNCH(h, kNoStage, n, st, where, launch_tracks_import(a, records, n, st));
         h->tracks_ready = true;
     }
     return VT_OK;
@@ -802,6 +855,7 @@ int vt_create(const VtConfig* cfg, VtHandle* out) {
     A((void**)&h->d_eff, mt * sizeof(int32_t));
     A((void**)&h->d_maps, mt * 1280 * sizeof(float));
     if (e == cudaSuccess) e = cudaMemset(h->d_state, 0, mt * 4 * sizeof(double));
+    if (e == cudaSuccess) e = cudaMemset(h->d_tmpl, 0, mt * kNz * Cd * sizeof(float));     // never-initialised slots export zeros, not stale memory
     if (e == cudaSuccess) e = cudaMemset(h->d_status, 0, mt * sizeof(int32_t));
     if (e == cudaSuccess) e = cudaMemset(h->d_claim, 0xff, mt * sizeof(uint32_t));
     if (e != cudaSuccess) {
@@ -954,30 +1008,20 @@ int vt_crop_normalize(VtHandle h, const uint8_t* frames, const int64_t* frame_of
                       const double* boxes_xywh, double factor, int32_t out_size, int32_t n, float* out_nchw,
                       uint8_t* out_u8_hwc, uint8_t* out_mask, double* out_resize_factor, int32_t* out_status,
                       void* stream) {
-    int rc = check_ready(h, false);
-    if (rc) return rc;
-    if (n == 0) return VT_OK;                      // an empty batch is a no-op (its pointers may be null)
-    if (!frames || !frame_offsets || !frame_hw || !boxes_xywh || !out_nchw || n < 0) return fail(h, VT_ERR_INVALID_ARG, "vt_crop_normalize: null pointer or negative n");
+    VT_ENTER(h, enter(h, "vt_crop_normalize", kWeights, 0, n, false, {frames, frame_offsets, frame_hw, boxes_xywh, out_nchw}));
     if (out_size != 128 && out_size != 256) return fail(h, VT_ERR_UNSUPPORTED, "vt_crop_normalize: out_size must be 128 or 256");
     if (!(factor > 0)) return fail(h, VT_ERR_INVALID_ARG, "vt_crop_normalize: factor must be positive");
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
-    const int k = launch_crop_normalize(frames, frame_offsets, frame_hw, boxes_xywh, nullptr, factor, out_size, n, h->mw.lut, out_nchw,
-                                        out_u8_hwc, out_mask, out_resize_factor, out_status, (cudaStream_t)stream);
-    if (k < 0) return fail(h, VT_ERR_CUDA, "crop kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    h->launches += k;
+    cudaStream_t st = (cudaStream_t)stream;
+    VT_LAUNCH(h, kNoStage, n, st, "vt_crop_normalize",
+              launch_crop_normalize(frames, frame_offsets, frame_hw, boxes_xywh, nullptr, factor, out_size, n, h->mw.lut, out_nchw,
+                                    out_u8_hwc, out_mask, out_resize_factor, out_status, st));
     return VT_OK;
 }
 
 int vt_forward(VtHandle h, const float* z, const float* x, int32_t n, float* pred_boxes, float* score_map,
                float* size_map, float* offset_map, float* taps, void* stream) {
-    int rc = check_ready(h, false);
-    if (rc) return rc;
-    if (n == 0) return VT_OK;
-    if (!z || !x || n < 0) return fail(h, VT_ERR_INVALID_ARG, "vt_forward: null input or negative n");
+    VT_ENTER(h, enter(h, "vt_forward", kWeights, 0, n, false, {z, x}));
     cudaStream_t st = (cudaStream_t)stream;
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
     if (h->generic) {
         const int C = h->cfg.embed_dim;
         const size_t gtap = (size_t)n * kN * C;
@@ -1009,66 +1053,30 @@ int vt_forward(VtHandle h, const float* z, const float* x, int32_t n, float* pre
 
 int vt_cal_bbox(VtHandle h, const float* score, const float* size_map, const float* offset_map, int32_t n,
                 float* boxes, void* stream) {
-    if (!h) return VT_ERR_INVALID_ARG;
-    if (!score || !size_map || !offset_map || !boxes || n < 0) return fail(h, VT_ERR_INVALID_ARG, "vt_cal_bbox: null pointer or negative n");
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
-    const int k = launch_cal_bbox(score, size_map, offset_map, n, boxes, (cudaStream_t)stream);
-    if (k < 0) return fail(h, VT_ERR_CUDA, "cal_bbox launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    h->launches += k;
+    VT_ENTER(h, enter(h, "vt_cal_bbox", kHandle, 0, n, false, {score, size_map, offset_map, boxes}));
+    cudaStream_t st = (cudaStream_t)stream;
+    VT_LAUNCH(h, kNoStage, n, st, "vt_cal_bbox", launch_cal_bbox(score, size_map, offset_map, n, boxes, st));
     return VT_OK;
 }
 
 int vt_tracks_init(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
                    const double* boxes_xywh, int32_t first, int32_t n, int32_t* out_status, void* stream) {
-    int rc = check_ready(h, false);
-    if (rc) return rc;
-    if (n == 0) { h->tracks_ready = true; return VT_OK; }
-    if (!frames || !frame_offsets || !frame_hw || !boxes_xywh) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init: null pointer");
-    if (first < 0 || n < 0 || first + n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init: tracks [%d, %d) exceed max_tracks %d", first, first + n, h->cfg.max_tracks);
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
-    return tracks_init(h, frames, frame_offsets, frame_hw, boxes_xywh, first, nullptr, n, out_status, (cudaStream_t)stream);
+    return init_call(h, "vt_tracks_init", false, frames, frame_offsets, frame_hw, boxes_xywh, first, nullptr, n, out_status, stream);
 }
 
 int vt_tracks_init_slots(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
                          const double* boxes_xywh, const int32_t* slots, int32_t n, int32_t* out_status, void* stream) {
-    int rc = check_ready(h, false);
-    if (rc) return rc;
-    if (n < 0 || n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init_slots: n = %d outside [0, max_tracks %d]", n, h->cfg.max_tracks);
-    if (n == 0) { h->tracks_ready = true; return VT_OK; }
-    if (!frames || !frame_offsets || !frame_hw || !boxes_xywh || !slots) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_init_slots: null pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
-    VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_init_slots/resolve", launch_resolve_slots(slots, n, h->cfg.max_tracks, h->d_claim, h->d_eff, st));
-    return tracks_init(h, frames, frame_offsets, frame_hw, boxes_xywh, 0, h->d_eff, n, out_status, st);
+    return init_call(h, "vt_tracks_init_slots", true, frames, frame_offsets, frame_hw, boxes_xywh, 0, slots, n, out_status, stream);
 }
 
 int vt_tracks_step(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
                    int32_t first, int32_t n, double* out_boxes, double* out_detail, int32_t update_state, void* stream) {
-    int rc = check_ready(h, true);
-    if (rc) return rc;
-    if (n == 0) return VT_OK;
-    if (!frames || !frame_offsets || !frame_hw || !out_boxes) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step: null pointer");
-    if (first < 0 || n < 0 || first + n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step: tracks [%d, %d) exceed max_tracks %d", first, first + n, h->cfg.max_tracks);
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
-    return tracks_step(h, frames, frame_offsets, frame_hw, first, nullptr, n, out_boxes, out_detail, update_state, (cudaStream_t)stream);
+    return step_call(h, "vt_tracks_step", false, frames, frame_offsets, frame_hw, first, nullptr, n, out_boxes, out_detail, update_state, stream);
 }
 
 int vt_tracks_step_slots(VtHandle h, const uint8_t* frames, const int64_t* frame_offsets, const int32_t* frame_hw,
                          const int32_t* slots, int32_t n, double* out_boxes, double* out_detail, int32_t update_state, void* stream) {
-    int rc = check_ready(h, true);
-    if (rc) return rc;
-    if (n < 0 || n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step_slots: n = %d outside [0, max_tracks %d]", n, h->cfg.max_tracks);
-    if (n == 0) return VT_OK;
-    if (!frames || !frame_offsets || !frame_hw || !out_boxes || !slots) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_step_slots: null pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
-    VT_LAUNCH(h, kNoStage, n, st, "vt_tracks_step_slots/resolve", launch_resolve_slots(slots, n, h->cfg.max_tracks, h->d_claim, h->d_eff, st));
-    return tracks_step(h, frames, frame_offsets, frame_hw, 0, h->d_eff, n, out_boxes, out_detail, update_state, st);
+    return step_call(h, "vt_tracks_step_slots", true, frames, frame_offsets, frame_hw, 0, slots, n, out_boxes, out_detail, update_state, stream);
 }
 
 int vt_set_range_fallback(VtHandle h, int32_t enable, int64_t* counter_dev) {
@@ -1109,46 +1117,37 @@ int vt_track_record_bytes(VtHandle h, int64_t* out_host) {
 }
 
 int vt_tracks_export(VtHandle h, int32_t first, int32_t n, uint8_t* records, void* stream) {
-    if (const int rc = check_records_call(h, "vt_tracks_export", first, n, records, nullptr, true)) return rc;
-    if (n == 0) return VT_OK;
-    return tracks_records(h, true, records, first, nullptr, n, nullptr, (cudaStream_t)stream);
+    return records_call(h, "vt_tracks_export", true, false, records, first, nullptr, n, nullptr, stream);
 }
 
 int vt_tracks_export_slots(VtHandle h, const int32_t* slots, int32_t n, uint8_t* records, int32_t* out_status, void* stream) {
-    if (const int rc = check_records_call(h, "vt_tracks_export_slots", 0, n, records, slots, false)) return rc;
-    if (n == 0) return VT_OK;
-    return tracks_records(h, true, records, 0, slots, n, out_status, (cudaStream_t)stream);
+    return records_call(h, "vt_tracks_export_slots", true, true, records, 0, slots, n, out_status, stream);
 }
 
 int vt_tracks_import(VtHandle h, const uint8_t* records, int32_t first, int32_t n, int32_t* out_status, void* stream) {
-    if (const int rc = check_records_call(h, "vt_tracks_import", first, n, records, nullptr, true)) return rc;
-    if (n == 0) return VT_OK;
-    return tracks_records(h, false, const_cast<uint8_t*>(records), first, nullptr, n, out_status, (cudaStream_t)stream);
+    return records_call(h, "vt_tracks_import", false, false, const_cast<uint8_t*>(records), first, nullptr, n, out_status, stream);
 }
 
 int vt_tracks_import_slots(VtHandle h, const uint8_t* records, const int32_t* slots, int32_t n, int32_t* out_status, void* stream) {
-    if (const int rc = check_records_call(h, "vt_tracks_import_slots", 0, n, records, slots, false)) return rc;
-    if (n == 0) return VT_OK;
-    return tracks_records(h, false, const_cast<uint8_t*>(records), 0, slots, n, out_status, (cudaStream_t)stream);
+    return records_call(h, "vt_tracks_import_slots", false, true, const_cast<uint8_t*>(records), 0, slots, n, out_status, stream);
 }
 
 int vt_tracks_get_state(VtHandle h, double* boxes_xywh, int32_t first, int32_t n, void* stream) {
-    if (!h) return VT_ERR_INVALID_ARG;
-    if (!boxes_xywh || first < 0 || n < 0 || first + n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_get_state: bad range");
+    VT_ENTER(h, enter(h, "vt_tracks_get_state", kHandle, first, n, true, {boxes_xywh}));
     VT_CUDA(h, cudaMemcpyAsync(boxes_xywh, h->d_state + (size_t)first * 4, (size_t)n * 4 * sizeof(double), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return VT_OK;
 }
 
 int vt_tracks_set_state(VtHandle h, const double* boxes_xywh, int32_t first, int32_t n, void* stream) {
-    if (!h) return VT_ERR_INVALID_ARG;
-    if (!boxes_xywh || first < 0 || n < 0 || first + n > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "vt_tracks_set_state: bad range");
+    VT_ENTER(h, enter(h, "vt_tracks_set_state", kHandle, first, n, true, {boxes_xywh}));
     VT_CUDA(h, cudaMemcpyAsync(h->d_state + (size_t)first * 4, boxes_xywh, (size_t)n * 4 * sizeof(double), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return VT_OK;
 }
 
 int vt_tracks_last_maps(VtHandle h, int32_t first, int32_t n, float* score_map, float* size_map, float* offset_map, void* stream) {
-    if (!h) return VT_ERR_INVALID_ARG;
-    if (first < h->last_first || n < 0 || first + n > h->last_first + h->last_n) return fail(h, VT_ERR_STATE, "vt_tracks_last_maps: tracks [%d, %d) were not part of the last step", first, first + n);
+    if (h && !tracks_in(first, n, h->last_first, h->last_n))
+        return fail(h, VT_ERR_STATE, "vt_tracks_last_maps: tracks [%d, %lld) were not part of the last step", first, (long long)first + n);
+    VT_ENTER(h, enter(h, "vt_tracks_last_maps", kHandle, first, n, false, {}));
     cudaStream_t st = (cudaStream_t)stream;
     const LastMaps maps = last_maps(h, first);
     if (score_map) VT_CUDA(h, cudaMemcpyAsync(score_map, maps.score, (size_t)n * 256 * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -1179,9 +1178,8 @@ int vt_upload_frame_rect(const uint8_t* image, int32_t H, int32_t W, int32_t y0,
 
 int vt_upload_yuv420_rect(VtHandle h, int32_t format, const uint8_t* image, int32_t H, int32_t W, int32_t y0, int32_t y1,
                           int32_t x0, int32_t x1, uint8_t* staging, uint8_t* staging_dev, uint8_t* frame_rgb_dev, void* stream) {
-    if (!h) return VT_ERR_INVALID_ARG;
-    if (format != VT_FRAME_NV12 && format != VT_FRAME_I420) return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: unknown format %d", format);
-    if (!image || !staging || !staging_dev || !frame_rgb_dev) return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: null pointer");
+    VT_ENTER(h, enter(h, "vt_upload_yuv420_rect", kHandle, 0, 1, false, {image, staging, staging_dev, frame_rgb_dev}));      // one frame
+    if (const int rc = check_yuv_format(h, "vt_upload_yuv420_rect", format)) return rc;
     if (H < 2 || W < 2 || (H & 1) || (W & 1)) return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: frame %d x %d: H and W must be even and positive", H, W);
     if (y0 < 0 || y1 > H || y0 >= y1 || x0 < 0 || x1 > W || x0 >= x1)
         return fail(h, VT_ERR_INVALID_ARG, "vt_upload_yuv420_rect: rectangle [%d, %d) x [%d, %d) is empty or leaves the %d x %d frame", y0, y1, x0, x1, H, W);
@@ -1199,8 +1197,6 @@ int vt_upload_yuv420_rect(VtHandle h, int32_t format, const uint8_t* image, int3
         runs[nruns++] = {chroma + (size_t)(y0 / 2) * cw + x0 / 2, cw, (size_t)cols / 2, rows / 2};
         runs[nruns++] = {chroma + (size_t)(H / 2) * cw + (size_t)(y0 / 2) * cw + x0 / 2, cw, (size_t)cols / 2, rows / 2};
     }
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
     cudaStream_t st = (cudaStream_t)stream;
     VT_CUDA(h, pack_upload(runs, nruns, staging, staging_dev, st));
     YuvDesc d{};
@@ -1212,44 +1208,30 @@ int vt_upload_yuv420_rect(VtHandle h, int32_t format, const uint8_t* image, int3
     d.dst = frame_rgb_dev + ((size_t)y0 * W + x0) * 3;
     d.dst_pitch = (int64_t)W * 3;
     d.w = cols; d.h = rows;
-    const int k = launch_yuv420_rect(format, d, h->num_sms, st);
-    if (k < 0) return fail(h, VT_ERR_CUDA, "vt_upload_yuv420_rect: kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    h->launches += k;
+    VT_LAUNCH(h, kNoStage, 1, st, "vt_upload_yuv420_rect", launch_yuv420_rect(format, d, h->num_sms, st));
     return VT_OK;
 }
 
 int vt_yuv420_to_rgb(VtHandle h, int32_t format, const uint8_t* src, const int64_t* src_offsets, const int32_t* frame_hw,
                      uint8_t* dst, const int64_t* dst_offsets, int32_t n, void* stream) {
-    if (!h) return VT_ERR_INVALID_ARG;
-    if (format != VT_FRAME_NV12 && format != VT_FRAME_I420) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_to_rgb: unknown format %d", format);
-    if (n < 0) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_to_rgb: negative n");
-    if (n == 0) return VT_OK;
-    if (!src || !src_offsets || !frame_hw || !dst || !dst_offsets) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_to_rgb: null pointer");
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
-    const int k = launch_yuv420_to_rgb(format, src, src_offsets, frame_hw, dst, dst_offsets, n, h->num_sms, (cudaStream_t)stream);
-    if (k < 0) return fail(h, VT_ERR_CUDA, "vt_yuv420_to_rgb: kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    h->launches += k;
+    VT_ENTER(h, enter(h, "vt_yuv420_to_rgb", kHandle, 0, n, false, {src, src_offsets, frame_hw, dst, dst_offsets}));
+    if (const int rc = check_yuv_format(h, "vt_yuv420_to_rgb", format)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    VT_LAUNCH(h, kNoStage, n, st, "vt_yuv420_to_rgb", launch_yuv420_to_rgb(format, src, src_offsets, frame_hw, dst, dst_offsets, n, h->num_sms, st));
     return VT_OK;
 }
 
 int vt_yuv420_crop_to_rgb(VtHandle h, int32_t format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw,
                           const double* boxes_xywh, double factor, int32_t first, int32_t n, uint8_t* dst, const int64_t* dst_offsets,
                           void* stream) {
-    if (!h) return VT_ERR_INVALID_ARG;
-    if (format != VT_FRAME_NV12 && format != VT_FRAME_I420) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: unknown format %d", format);
-    if (n < 0) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: negative n");
-    if (n == 0) return VT_OK;
-    if (!planes || !pitches || !frame_hw || !dst || !dst_offsets) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: null pointer");
-    if (!(factor > 0)) return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: factor must be positive");
-    if (!boxes_xywh && (first < 0 || first + n > h->cfg.max_tracks))
-        return fail(h, VT_ERR_INVALID_ARG, "vt_yuv420_crop_to_rgb: tracks [%d, %d) exceed max_tracks %d", first, first + n, h->cfg.max_tracks);
-    DeviceGuard dg(h->cfg.device);
-    VT_CUDA(h, dg.err);
+    const char* where = "vt_yuv420_crop_to_rgb";
+    VT_ENTER(h, enter(h, where, kHandle, 0, n, false, {planes, pitches, frame_hw, dst, dst_offsets}));
+    if (const int rc = check_yuv_format(h, where, format)) return rc;
+    if (!(factor > 0)) return fail(h, VT_ERR_INVALID_ARG, "%s: factor must be positive", where);
+    if (const int rc = boxes_xywh ? VT_OK : check_tracks(h, where, first, n)) return rc;       // the boxes are the tracks' state
     const double* boxes = boxes_xywh ? boxes_xywh : h->d_state + (size_t)first * 4;
-    const int k = launch_yuv420_crop_to_rgb(format, planes, pitches, frame_hw, boxes, factor, dst, dst_offsets, n, h->num_sms, (cudaStream_t)stream);
-    if (k < 0) return fail(h, VT_ERR_CUDA, "vt_yuv420_crop_to_rgb: kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    h->launches += k;
+    cudaStream_t st = (cudaStream_t)stream;
+    VT_LAUNCH(h, kNoStage, n, st, where, launch_yuv420_crop_to_rgb(format, planes, pitches, frame_hw, boxes, factor, dst, dst_offsets, n, h->num_sms, st));
     return VT_OK;
 }
 

@@ -18,6 +18,21 @@ def _ptr(t: Optional[torch.Tensor]):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+def tensor_ptr(t: Optional[torch.Tensor], name: str, dtype: torch.dtype, device: torch.device, shape: Optional[tuple] = None,
+               align: int = 1, optional: bool = False) -> C.c_void_p:
+    """The address a C-ABI call takes for ``t``, once ``t`` is what the call reads there: a contiguous ``dtype`` tensor on ``device``,
+    of exactly ``shape`` when one is given (a per-item array is [n, ...]), at an address that is a multiple of ``align`` bytes.
+    ``None`` passes NULL where the call takes it (``optional``).  Anything else raises ValueError, before the call."""
+    if t is None and optional:
+        return C.c_void_p(0)
+    if (not torch.is_tensor(t) or t.dtype != dtype or t.device != device or not t.is_contiguous()
+            or (shape is not None and t.shape != shape) or t.data_ptr() % align):
+        got = f"{t.dtype} {tuple(t.shape)} on {t.device}" if torch.is_tensor(t) else type(t).__name__
+        raise ValueError(f"{name}: expected a contiguous {dtype} tensor{'' if shape is None else f' of shape {tuple(shape)}'} on {device}"
+                         f"{f', {align}-byte aligned' if align > 1 else ''}; got {got}")
+    return C.c_void_p(t.data_ptr())
+
+
 YUV_FORMATS = {"nv12": 1, "i420": 2}          # VT_FRAME_NV12, VT_FRAME_I420
 
 
@@ -87,6 +102,17 @@ class Engine:
     def _check(self, rc):
         _lib.check(self.handle, rc)
 
+    def _call(self, name: str, *args) -> None:
+        """``name``(handle, *args, stream) on this engine's device and its current stream; VtError for a failed status."""
+        with torch.cuda.device(self.device):
+            self._check(getattr(self.lib, name)(self.handle, *args, self._stream()))
+
+    def _frames(self, frames, frame_offsets, frame_hw, n: int) -> tuple:
+        """The frame arguments of a crop: uint8 frames, int64 frame_offsets [n] (bytes), int32 frame_hw [n, 2]."""
+        dev = self.device
+        return (tensor_ptr(frames, "frames", torch.uint8, dev), tensor_ptr(frame_offsets, "frame_offsets", torch.int64, dev, (n,)),
+                tensor_ptr(frame_hw, "frame_hw", torch.int32, dev, (n, 2)))
+
     @property
     def launch_count(self) -> int:
         return int(self.lib.vt_launch_count(self.handle))
@@ -130,8 +156,7 @@ class Engine:
         self._check(self.lib.vt_set_tensor(self.handle, b"tracker.output_window", C.c_void_p(win.data_ptr()), shape, 4))
         if strict and unexpected:
             raise RuntimeError(f"unexpected keys: {unexpected}")
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_finalize_weights(self.handle, self._stream()))
+        self._call("vt_finalize_weights")
         self.weights_loaded = True
         return [], unexpected
 
@@ -141,51 +166,47 @@ class Engine:
                        want_mask: bool = False):
         """sample_target + Preprocessor for n (frame, box) pairs.  frames: uint8 device buffer;
         frame_offsets int64 [n]; frame_hw int32 [n,2]; boxes float64 [n,4].  Returns a dict."""
-        n = boxes.shape[0]
+        n = int(boxes.shape[0])
         dev = self.device
-        assert frames.dtype == torch.uint8 and frame_offsets.dtype == torch.int64 and frame_hw.dtype == torch.int32
-        assert boxes.dtype == torch.float64 and boxes.is_contiguous()
         out = torch.empty((n, 3, out_size, out_size), dtype=torch.float32, device=dev)
         u8 = torch.empty((n, out_size, out_size, 3), dtype=torch.uint8, device=dev) if want_u8 else None
         mask = torch.empty((n, out_size, out_size), dtype=torch.uint8, device=dev) if want_mask else None
         rf = torch.empty((n,), dtype=torch.float64, device=dev)
         status = torch.empty((n,), dtype=torch.int32, device=dev)
-        with torch.cuda.device(dev):
-            self._check(self.lib.vt_crop_normalize(self.handle, _ptr(frames), _ptr(frame_offsets), _ptr(frame_hw), _ptr(boxes),
-                                                   float(factor), int(out_size), int(n), _ptr(out), _ptr(u8), _ptr(mask),
-                                                   _ptr(rf), _ptr(status), self._stream()))
+        self._call("vt_crop_normalize", *self._frames(frames, frame_offsets, frame_hw, n),
+                   tensor_ptr(boxes, "boxes", torch.float64, dev, (n, 4)), float(factor), int(out_size), n, _ptr(out), _ptr(u8), _ptr(mask),
+                   _ptr(rf), _ptr(status))
         return {"tensors": out, "u8": u8, "mask": mask, "resize_factor": rf, "status": status}
 
     def forward(self, z: torch.Tensor, x: torch.Tensor, taps: bool = False):
         """OstrackDist.forward(z, x): returns the reference's output dict (+ 'taps' when asked)."""
-        n = z.shape[0]
+        n = int(z.shape[0])
         dev = self.device
-        assert z.shape[1:] == (3, self.template_size, self.template_size) and x.shape == (n, 3, self.search_size, self.search_size)
         z = z.to(dev, torch.float32).contiguous()
         x = x.to(dev, torch.float32).contiguous()
-        F = self.search_size // 16
+        T, S = self.template_size, self.search_size
+        F = S // 16
         pred = torch.empty((n, 1, 4), dtype=torch.float32, device=dev)
         score = torch.empty((n, 1, F, F), dtype=torch.float32, device=dev)
         size = torch.empty((n, 2, F, F), dtype=torch.float32, device=dev)
         off = torch.empty((n, 2, F, F), dtype=torch.float32, device=dev)
         tp = torch.zeros((self.depth + 2, n, TEMPLATE_TOKENS + SEARCH_TOKENS, self.C), dtype=torch.float32, device=dev) if taps else None
-        with torch.cuda.device(dev):
-            self._check(self.lib.vt_forward(self.handle, _ptr(z), _ptr(x), int(n), _ptr(pred), _ptr(score), _ptr(size),
-                                            _ptr(off), _ptr(tp), self._stream()))
+        self._call("vt_forward", tensor_ptr(z, "z", torch.float32, dev, (n, 3, T, T)), tensor_ptr(x, "x", torch.float32, dev, (n, 3, S, S)), n,
+                   _ptr(pred), _ptr(score), _ptr(size), _ptr(off), _ptr(tp))
         out = {"pred_boxes": pred, "score_map": score, "size_map": size, "offset_map": off}
         if taps:
             out["taps"] = tp
         return out
 
     def cal_bbox(self, score: torch.Tensor, size_map: torch.Tensor, offset_map: torch.Tensor) -> torch.Tensor:
-        n = score.shape[0]
+        n = int(score.shape[0])
         dev = self.device
-        score = score.to(dev, torch.float32).contiguous()
-        size_map = size_map.to(dev, torch.float32).contiguous()
-        offset_map = offset_map.to(dev, torch.float32).contiguous()
+        F = self.search_size // 16
+        score, size_map, offset_map = (t.to(dev, torch.float32).contiguous() for t in (score, size_map, offset_map))
         boxes = torch.empty((n, 4), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            self._check(self.lib.vt_cal_bbox(self.handle, _ptr(score), _ptr(size_map), _ptr(offset_map), int(n), _ptr(boxes), self._stream()))
+        self._call("vt_cal_bbox", tensor_ptr(score, "score", torch.float32, dev, (n, 1, F, F)),
+                   tensor_ptr(size_map, "size_map", torch.float32, dev, (n, 2, F, F)),
+                   tensor_ptr(offset_map, "offset_map", torch.float32, dev, (n, 2, F, F)), n, _ptr(boxes))
         return boxes
 
     # ------------------------------------------------------------------------------------------
@@ -195,15 +216,11 @@ class Engine:
         ``src_offsets[i]`` of ``src`` becomes the H x W x 3 frame at byte ``dst_offsets[i]`` of ``dst``.  uint8 buffers, int64
         offsets [n], int32 frame_hw [n, 2] (even), all on this engine's device.  Returns ``dst``."""
         fmt = yuv_format(format)
-        for t, dt in ((src, torch.uint8), (dst, torch.uint8), (src_offsets, torch.int64), (dst_offsets, torch.int64), (frame_hw, torch.int32)):
-            if t.dtype != dt or t.device != self.device or not t.is_contiguous():
-                raise ValueError(f"yuv420_to_rgb: expected a contiguous {dt} tensor on {self.device}")
         n = int(src_offsets.shape[0])
-        if dst_offsets.shape != (n,) or frame_hw.shape != (n, 2):
-            raise ValueError("yuv420_to_rgb: src_offsets [n], dst_offsets [n] and frame_hw [n, 2] required")
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_yuv420_to_rgb(self.handle, fmt, _ptr(src), _ptr(src_offsets), _ptr(frame_hw), _ptr(dst),
-                                                  _ptr(dst_offsets), n, self._stream()))
+        dev = self.device
+        self._call("vt_yuv420_to_rgb", fmt, tensor_ptr(src, "src", torch.uint8, dev),
+                   tensor_ptr(src_offsets, "src_offsets", torch.int64, dev, (n,)), tensor_ptr(frame_hw, "frame_hw", torch.int32, dev, (n, 2)),
+                   tensor_ptr(dst, "dst", torch.uint8, dev), tensor_ptr(dst_offsets, "dst_offsets", torch.int64, dev, (n,)), n)
         return dst
 
     def upload_yuv420_rect(self, format: str, image: np.ndarray, y0: int, y1: int, x0: int, x1: int, staging: torch.Tensor,
@@ -216,9 +233,10 @@ class Engine:
         need = H * W * 3 // 2
         if staging.numel() < need or staging_dev.numel() < need or frame_rgb.numel() < H * W * 3:
             raise ValueError("upload_yuv420_rect: staging buffers need (H*3/2) x W bytes and frame_rgb H x W x 3")
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_upload_yuv420_rect(self.handle, fmt, image.ctypes.data, H, W, int(y0), int(y1), int(x0), int(x1),
-                                                       _ptr(staging), _ptr(staging_dev), _ptr(frame_rgb), self._stream()))
+        host, dev = torch.device("cpu"), self.device
+        self._call("vt_upload_yuv420_rect", fmt, image.ctypes.data, H, W, int(y0), int(y1), int(x0), int(x1),
+                   tensor_ptr(staging, "staging", torch.uint8, host), tensor_ptr(staging_dev, "staging_dev", torch.uint8, dev),
+                   tensor_ptr(frame_rgb, "frame_rgb", torch.uint8, dev))
 
     def yuv420_crop_to_rgb(self, format: str, planes: torch.Tensor, pitches: torch.Tensor, frame_hw: torch.Tensor, dst: torch.Tensor,
                            dst_offsets: torch.Tensor, factor: float, boxes: Optional[torch.Tensor] = None, first: int = 0) -> torch.Tensor:
@@ -228,78 +246,65 @@ class Engine:
         allocation and no synchronisation (capturable in a CUDA graph).  Returns ``dst``."""
         fmt = yuv_format(format)
         n = int(planes.shape[0])
-        want = [(planes, torch.int64, (n, 3)), (pitches, torch.int32, (n, 2)), (frame_hw, torch.int32, (n, 2)), (dst_offsets, torch.int64, (n,))]
-        if boxes is not None:
-            want.append((boxes, torch.float64, (n, 4)))
-        for t, dt, shape in want + [(dst, torch.uint8, tuple(dst.shape))]:
-            if t.dtype != dt or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape:
-                raise ValueError(f"yuv420_crop_to_rgb: expected a contiguous {dt} tensor of shape {shape} on {self.device}")
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_yuv420_crop_to_rgb(self.handle, fmt, _ptr(planes), _ptr(pitches), _ptr(frame_hw), _ptr(boxes),
-                                                       float(factor), int(first), n, _ptr(dst), _ptr(dst_offsets), self._stream()))
+        dev = self.device
+        self._call("vt_yuv420_crop_to_rgb", fmt, tensor_ptr(planes, "planes", torch.int64, dev, (n, 3)),
+                   tensor_ptr(pitches, "pitches", torch.int32, dev, (n, 2)), tensor_ptr(frame_hw, "frame_hw", torch.int32, dev, (n, 2)),
+                   tensor_ptr(boxes, "boxes", torch.float64, dev, (n, 4), optional=True), float(factor), int(first), n,
+                   tensor_ptr(dst, "dst", torch.uint8, dev), tensor_ptr(dst_offsets, "dst_offsets", torch.int64, dev, (n,)))
         return dst
 
     # ------------------------------------------------------------------------------------------
     def tracks_init(self, frames, frame_offsets, frame_hw, boxes, first: int = 0) -> torch.Tensor:
-        n = boxes.shape[0]
-        assert boxes.dtype == torch.float64 and boxes.is_contiguous() and boxes.device == self.device
+        n = int(boxes.shape[0])
         status = torch.empty((n,), dtype=torch.int32, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_init(self.handle, _ptr(frames), _ptr(frame_offsets), _ptr(frame_hw), _ptr(boxes),
-                                                int(first), int(n), _ptr(status), self._stream()))
+        self._call("vt_tracks_init", *self._frames(frames, frame_offsets, frame_hw, n),
+                   tensor_ptr(boxes, "boxes", torch.float64, self.device, (n, 4)), int(first), n, _ptr(status))
         return status
 
     def tracks_step(self, frames, frame_offsets, frame_hw, first: int = 0, n: Optional[int] = None,
                     out_boxes: Optional[torch.Tensor] = None, out_detail: Optional[torch.Tensor] = None,
                     update_state: bool = True, detail: bool = False):
-        n = frame_offsets.shape[0] if n is None else n
+        n = int(frame_offsets.shape[0] if n is None else n)
+        dev = self.device
         if out_boxes is None:
-            out_boxes = torch.empty((n, 5), dtype=torch.float64, device=self.device)
+            out_boxes = torch.empty((n, 5), dtype=torch.float64, device=dev)
         if detail and out_detail is None:
-            out_detail = torch.empty((n, 8), dtype=torch.float64, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_step(self.handle, _ptr(frames), _ptr(frame_offsets), _ptr(frame_hw), int(first), int(n),
-                                                _ptr(out_boxes), _ptr(out_detail), 1 if update_state else 0, self._stream()))
+            out_detail = torch.empty((n, 8), dtype=torch.float64, device=dev)
+        self._call("vt_tracks_step", *self._frames(frames, frame_offsets, frame_hw, n), int(first), n,
+                   tensor_ptr(out_boxes, "out_boxes", torch.float64, dev, (n, 5)),
+                   tensor_ptr(out_detail, "out_detail", torch.float64, dev, (n, 8), optional=True), 1 if update_state else 0)
         return (out_boxes, out_detail) if detail else out_boxes
-
-    def _slot_tensor(self, slots: torch.Tensor, n: int) -> torch.Tensor:
-        if slots.dtype != torch.int32 or slots.device != self.device or not slots.is_contiguous() or tuple(slots.shape) != (n,):
-            raise ValueError(f"slots: expected a contiguous int32 tensor of shape ({n},) on {self.device}")
-        return slots
 
     def tracks_init_slots(self, frames, frame_offsets, frame_hw, boxes, slots: torch.Tensor) -> torch.Tensor:
         """vt_tracks_init_slots: item i initialises track ``slots[i]`` (int32 device tensor [n]).  Returns the status per item
         (VT_TRACK_BAD_SLOT for an entry outside [0, max_tracks) or repeating an earlier one)."""
-        n = boxes.shape[0]
-        assert boxes.dtype == torch.float64 and boxes.is_contiguous() and boxes.device == self.device
-        self._slot_tensor(slots, n)
-        status = torch.empty((n,), dtype=torch.int32, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_init_slots(self.handle, _ptr(frames), _ptr(frame_offsets), _ptr(frame_hw), _ptr(boxes),
-                                                      _ptr(slots), int(n), _ptr(status), self._stream()))
+        n = int(boxes.shape[0])
+        dev = self.device
+        status = torch.empty((n,), dtype=torch.int32, device=dev)
+        self._call("vt_tracks_init_slots", *self._frames(frames, frame_offsets, frame_hw, n),
+                   tensor_ptr(boxes, "boxes", torch.float64, dev, (n, 4)), tensor_ptr(slots, "slots", torch.int32, dev, (n,)), n, _ptr(status))
         return status
 
     def tracks_step_slots(self, frames, frame_offsets, frame_hw, slots: torch.Tensor, out_boxes: Optional[torch.Tensor] = None,
                           out_detail: Optional[torch.Tensor] = None, update_state: bool = True, detail: bool = False):
         """vt_tracks_step_slots: item i steps track ``slots[i]`` (int32 device tensor [n]); outputs are in item order."""
         n = int(slots.shape[0])
-        self._slot_tensor(slots, n)
+        dev = self.device
         if out_boxes is None:
-            out_boxes = torch.empty((n, 5), dtype=torch.float64, device=self.device)
+            out_boxes = torch.empty((n, 5), dtype=torch.float64, device=dev)
         if detail and out_detail is None:
-            out_detail = torch.empty((n, 8), dtype=torch.float64, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_step_slots(self.handle, _ptr(frames), _ptr(frame_offsets), _ptr(frame_hw), _ptr(slots), n,
-                                                      _ptr(out_boxes), _ptr(out_detail), 1 if update_state else 0, self._stream()))
+            out_detail = torch.empty((n, 8), dtype=torch.float64, device=dev)
+        self._call("vt_tracks_step_slots", *self._frames(frames, frame_offsets, frame_hw, n),
+                   tensor_ptr(slots, "slots", torch.int32, dev, (n,)), n, tensor_ptr(out_boxes, "out_boxes", torch.float64, dev, (n, 5)),
+                   tensor_ptr(out_detail, "out_detail", torch.float64, dev, (n, 8), optional=True), 1 if update_state else 0)
         return (out_boxes, out_detail) if detail else out_boxes
 
     def set_range_fallback(self, enable: bool, counter: Optional[torch.Tensor] = None) -> None:
         """vt_set_range_fallback: with ``enable``, every item of a tracking step that the tensor-core kernels flag
         VT_TRACK_NUMERIC_RANGE is recomputed on the fp32 kernels within the same call, bit for bit what a ``simt`` engine gives.
         ``counter`` (optional int64 device tensor of one element) has the number of recomputed items added to it by every step."""
-        if counter is not None and (counter.dtype != torch.int64 or counter.device != self.device or counter.numel() != 1):
-            raise ValueError(f"counter: expected a one-element int64 tensor on {self.device}")
-        self._check(self.lib.vt_set_range_fallback(self.handle, 1 if enable else 0, _ptr(counter)))
+        ptr = tensor_ptr(counter, "counter", torch.int64, self.device, (1,), optional=True)
+        self._check(self.lib.vt_set_range_fallback(self.handle, 1 if enable else 0, ptr))
         # a CUDA graph captured while a counter was set keeps adding to its address on every replay, whatever the fallback's setting
         # since: every counter handed over lives as long as this engine
         if counter is not None:
@@ -321,69 +326,56 @@ class Engine:
         self._check(self.lib.vt_track_record_bytes(self.handle, C.byref(out)))
         return int(out.value)
 
-    def _records(self, records: torch.Tensor, n: int) -> torch.Tensor:
-        R = self.track_record_bytes
-        if (records.dtype != torch.uint8 or records.device != self.device or not records.is_contiguous() or tuple(records.shape) != (n, R)
-                or records.data_ptr() % 16):
-            raise ValueError(f"records: expected a contiguous, 16-byte aligned uint8 tensor of shape ({n}, {R}) on {self.device}")
-        return records
+    def _records(self, records: torch.Tensor, n: int) -> C.c_void_p:
+        return tensor_ptr(records, "records", torch.uint8, self.device, (n, self.track_record_bytes), align=16)
 
     def tracks_export(self, first: int = 0, n: Optional[int] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """vt_tracks_export: the records of tracks [first, first + n) as uint8 [n, R] (into ``out`` when given)."""
         n = self.max_tracks - first if n is None else int(n)
-        out = torch.empty((n, self.track_record_bytes), dtype=torch.uint8, device=self.device) if out is None else self._records(out, n)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_export(self.handle, int(first), n, _ptr(out), self._stream()))
+        out = torch.empty((n, self.track_record_bytes), dtype=torch.uint8, device=self.device) if out is None else out
+        self._call("vt_tracks_export", int(first), n, self._records(out, n))
         return out
 
     def tracks_export_slots(self, slots: torch.Tensor, out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """vt_tracks_export_slots: record i of track ``slots[i]``; returns (records [n, R], status [n]: VT_TRACK_OK or
         VT_TRACK_BAD_SLOT, whose record is all zeros)."""
         n = int(slots.shape[0])
-        self._slot_tensor(slots, n)
-        out = torch.empty((n, self.track_record_bytes), dtype=torch.uint8, device=self.device) if out is None else self._records(out, n)
+        out = torch.empty((n, self.track_record_bytes), dtype=torch.uint8, device=self.device) if out is None else out
         status = torch.empty((n,), dtype=torch.int32, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_export_slots(self.handle, _ptr(slots), n, _ptr(out), _ptr(status), self._stream()))
+        self._call("vt_tracks_export_slots", tensor_ptr(slots, "slots", torch.int32, self.device, (n,)), n, self._records(out, n),
+                   _ptr(status))
         return out, status
 
     def tracks_import(self, records: torch.Tensor, first: int = 0) -> torch.Tensor:
         """vt_tracks_import: record i into track first + i, checked on the device.  Returns the status per item: VT_TRACK_OK, or
         VT_TRACK_BAD_RECORD (header, fingerprint, checksum or box rejected; the track is left as it was)."""
         n = int(records.shape[0])
-        self._records(records, n)
         status = torch.empty((n,), dtype=torch.int32, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_import(self.handle, _ptr(records), int(first), n, _ptr(status), self._stream()))
+        self._call("vt_tracks_import", self._records(records, n), int(first), n, _ptr(status))
         return status
 
     def tracks_import_slots(self, records: torch.Tensor, slots: torch.Tensor) -> torch.Tensor:
         """vt_tracks_import_slots: record i into track ``slots[i]``; status per item as tracks_import's, or VT_TRACK_BAD_SLOT."""
         n = int(slots.shape[0])
-        self._slot_tensor(slots, n)
-        self._records(records, n)
         status = torch.empty((n,), dtype=torch.int32, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_import_slots(self.handle, _ptr(records), _ptr(slots), n, _ptr(status), self._stream()))
+        self._call("vt_tracks_import_slots", self._records(records, n), tensor_ptr(slots, "slots", torch.int32, self.device, (n,)), n,
+                   _ptr(status))
         return status
 
     def tracks_get_state(self, first: int = 0, n: Optional[int] = None) -> torch.Tensor:
-        n = self.max_tracks - first if n is None else n
+        n = self.max_tracks - first if n is None else int(n)
         out = torch.empty((n, 4), dtype=torch.float64, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_get_state(self.handle, _ptr(out), int(first), int(n), self._stream()))
+        self._call("vt_tracks_get_state", _ptr(out), int(first), n)
         return out
 
     def tracks_set_state(self, boxes: torch.Tensor, first: int = 0) -> None:
-        assert boxes.dtype == torch.float64 and boxes.is_contiguous() and boxes.device == self.device
-        with torch.cuda.device(self.device):
-            self._check(self.lib.vt_tracks_set_state(self.handle, _ptr(boxes), int(first), int(boxes.shape[0]), self._stream()))
+        n = int(boxes.shape[0])
+        self._call("vt_tracks_set_state", tensor_ptr(boxes, "boxes", torch.float64, self.device, (n, 4)), int(first), n)
 
     def tracks_last_maps(self, first: int, n: int):
         dev = self.device
         score = torch.empty((n, 1, 16, 16), dtype=torch.float32, device=dev)
         size = torch.empty((n, 2, 16, 16), dtype=torch.float32, device=dev)
         off = torch.empty((n, 2, 16, 16), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            self._check(self.lib.vt_tracks_last_maps(self.handle, int(first), int(n), _ptr(score), _ptr(size), _ptr(off), self._stream()))
+        self._call("vt_tracks_last_maps", int(first), int(n), _ptr(score), _ptr(size), _ptr(off))
         return {"score_map": score, "size_map": size, "offset_map": off}
