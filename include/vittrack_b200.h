@@ -364,6 +364,32 @@ int vt_yuv420_crop_to_rgb(VtHandle h, int32_t format, const uint64_t* planes, co
                           const double* boxes_xywh, double factor, int32_t first, int32_t n, uint8_t* dst,
                           const int64_t* dst_offsets, void* stream);
 
+/* Several tracks on one surface (many targets in one camera stream): each surface is converted once, into one RGB frame per
+ * surface, over the bounding rectangle of the crops of its items.  For m surfaces and n items:
+ *   planes, pitches, frame_hw   per surface ([m][3], [m][2], [m][2]), as for vt_yuv420_crop_to_rgb.
+ *   dst + dst_offsets[s]        surface s's H x W x 3 RGB frame ([m]); every item on surface s is then initialised or stepped on it.
+ *   item_surface [n] int32      the surface of item i.
+ *   boxes_xywh   [n][4]         float64 boxes, or NULL: the crop is taken around the track state, of track slots[i] when `slots` is
+ *                               given and of track first + i otherwise.
+ *   slots        [n] int32      track slots (as vt_tracks_init_slots / vt_tracks_step_slots take them), or NULL; `first` is ignored
+ *                               when they are given.
+ * Item i's rectangle is the one vt_yuv420_crop_to_rgb converts for its box and factor (the crop's rows and columns plus one spare
+ * column on either side, widened to even bounds).  An item is skipped when its surface index is outside [0, m), when `slots` is given
+ * and slots[i] is a bad slot as vt_tracks_init_slots defines it (outside [0, max_tracks) or repeating an earlier item's slot), or when
+ * vt_yuv420_crop_to_rgb would skip its rectangle (degenerate crop, odd or tiny frame, a pitch below the row width).  Surface s's
+ * frame gets the cvtColor bytes of the bounding rectangle of its valid items' rectangles, and no other byte of dst is written; a
+ * surface without a valid item is not written at all.  A track's crop reads only its own rectangle, which lies inside the bounding
+ * rectangle and holds there the bytes the per-item path writes, so vt_tracks_init / vt_tracks_step on these frames give, bit for
+ * bit, what they give on the per-item path's frames.  The bounding rectangle is not the exact union: at worst one whole frame per
+ * surface is converted.
+ * All arrays are device pointers.  No allocation and no host synchronisation (the handle owns a 16-byte rectangle and a counter per
+ * surface, left empty after each call): the call can be captured in a CUDA graph.  Bad host arguments (format, n < 0, m < 0 or
+ * m > max_tracks, factor <= 0, first + n > max_tracks when the state is read by range, null pointers when n > 0) return
+ * VT_ERR_INVALID_ARG before any launch; n == 0 is a no-op.  Launches: two, three with `slots`. */
+int vt_yuv420_crops_to_surface_rgb(VtHandle h, int32_t format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw,
+                                   int32_t m, const int32_t* item_surface, const double* boxes_xywh, const int32_t* slots, double factor,
+                                   int32_t first, int32_t n, uint8_t* dst, const int64_t* dst_offsets, void* stream);
+
 /* Development aid: which profiled stage launches (vt_profile_enable) have started / finished.  Non-blocking;
  * meant for a watchdog thread while the owning thread waits in a synchronisation (tools/hang_probe.py,
  * tests/test_gpu_soak.py).  out[i] = stage * 4 + (started ? 1 : 0) + (finished ? 2 : 0); returns the count. */

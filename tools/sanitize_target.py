@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Small workload for compute-sanitizer (tools/sanitize.sh): every hand-written kernel once, at sizes a 10 - 100x slowdown can afford.
-Fast path (vit_48_h32): tracks_init + two closed-loop steps of 5 tracks, then track records out and back in, on tcgen05 (crop_taps, crop_conv1, conv_s2_tc x3, blocks_tc,
+Fast path (vit_48_h32): tracks_init + two closed-loop steps of 5 tracks, then track records out and back in, then two targets per NV12 surface (surface union + surface conversion kernels), on tcgen05 (crop_taps, crop_conv1, conv_s2_tc x3, blocks_tc,
 head_tc), the same on the fp32 CUDA-core kernels, vt_forward, vt_crop_normalize, vt_cal_bbox.  Generic path (C 96 / 3 heads / depth 2 /
 head 64): tracks + forward (im2col, gemm_tc_kernel NT / NN, sgemm, layernorm, softmax, decode)."""
 import os, sys
@@ -8,7 +8,8 @@ import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import vt_oracle as O
-from vittracker_b200 import BatchedTracker, FramePool, load_cfg
+from oracle import yuv420 as Y
+from vittracker_b200 import BatchedTracker, FramePool, YuvSurfaces, load_cfg
 
 which = sys.argv[1] if len(sys.argv) > 1 else "all"
 frames = O.synth_frames(2, 360, 640, seed=7, smooth=True)
@@ -23,6 +24,9 @@ if which in ("all", "fast"):
         recs = bt.export_tracks(slots=[4, 0, 2])                   # track records: export and import kernels, by range and by slot
         assert int(bt.import_tracks(recs, slots=[1, 3, 0]).abs().sum()) == 0
         assert int(bt.import_tracks(bt.export_tracks()).abs().sum()) == 0
+        surf = YuvSurfaces.from_frames(torch.from_numpy(Y.synth_yuv420(2, 360, 640, seed=9)).to(bt.device), "nv12")
+        assert int(bt.initialize_yuv(surf, boxes, surface=[0, 1, 0, 1, 0]).abs().sum()) == 0
+        bt.track_yuv(surf, surface=torch.tensor([1, 0, 1, 0, 1], device=bt.device), slots=[4, 3, 2, 1, 0])
         z = torch.randn(3, 3, 128, 128)
         x = torch.randn(3, 3, 256, 256)
         fw = bt.engine.forward(z, x, taps=True)

@@ -71,6 +71,8 @@ SIGNATURES = {
     "vt_upload_yuv420_rect": (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                         _P, _P, _P, _P]),
     "vt_yuv420_crop_to_rgb": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, C.c_double, C.c_int32, C.c_int32, _P, _P, _P]),
+    "vt_yuv420_crops_to_surface_rgb": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_double, C.c_int32, C.c_int32,
+                                                 _P, _P, _P]),
 }
 
 _lib = None

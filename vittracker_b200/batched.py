@@ -211,6 +211,8 @@ class BatchedTracker:
         self.template_factor, self.search_factor = float(cfg.TEST.TEMPLATE_FACTOR), float(cfg.TEST.SEARCH_FACTOR)
         self._yuv_rgb: Optional[torch.Tensor] = None             # initialize_yuv / track_yuv: one RGB frame per track
         self._yuv_off: Optional[torch.Tensor] = None
+        self._surf_rgb: Optional[torch.Tensor] = None            # ... with surface=: one RGB frame per surface, plus one for bad entries
+        self._surf_off: Optional[torch.Tensor] = None
         # (H, W) of every slot's frames, for steps by slot list; row max_tracks takes the writes of bad entries
         self._slot_hw = torch.zeros((max_tracks + 1, 2), dtype=torch.int32, device=self.device)
 
@@ -353,13 +355,82 @@ class BatchedTracker:
             self._yuv_off = torch.arange(self.max_tracks + 1, dtype=torch.int64, device=self.device) * (surfaces.H * surfaces.W * 3)
         return self._yuv_rgb, self._yuv_off[: surfaces.n]
 
-    def initialize_yuv(self, surfaces: YuvSurfaces, boxes, slots=None) -> torch.Tensor:
+    def _surface_frames(self, surfaces: YuvSurfaces) -> Tuple[torch.Tensor, torch.Tensor]:
+        if surfaces.n > self.max_tracks:
+            raise ValueError(f"{surfaces.n} surfaces > max_tracks {self.max_tracks}")
+        if surfaces.device != self.device:
+            raise ValueError(f"surfaces on {surfaces.device}, tracker on {self.device}")
+        shape = (surfaces.n + 1, surfaces.H, surfaces.W, 3)
+        if self._surf_rgb is None or tuple(self._surf_rgb.shape) != shape:
+            self._surf_rgb = None
+            # zero-filled once, as the per-track frames; the last frame is the one bad entries of a CUDA surface tensor crop from
+            self._surf_rgb = torch.zeros(shape, dtype=torch.uint8, device=self.device)
+            self._surf_off = torch.arange(surfaces.n + 1, dtype=torch.int64, device=self.device) * (surfaces.H * surfaces.W * 3)
+        return self._surf_rgb, self._surf_off
+
+    def _surface_items(self, surfaces: YuvSurfaces, surface, n: int, slots: Optional[torch.Tensor]):
+        """Per item its surface (int32 device tensor [n]), frame offset and size, gathered on the device, and the slot list the step takes:
+        ``slots`` as given, or None for a range call; with a CUDA surface tensor, a list in which every entry whose surface lies outside
+        [0, m) is bad (-1), so that the device steps it as a bad slot-list entry."""
+        m = surfaces.n
+        frames, soff = self._surface_frames(surfaces)
+        if torch.is_tensor(surface) and surface.is_cuda:
+            if surface.dtype not in (torch.int32, torch.int64) or surface.dim() != 1 or surface.device != self.device:
+                raise ValueError(f"surface: expected a 1-D integer tensor on {self.device}")
+            if surface.shape[0] != n:
+                raise ValueError(f"{surface.shape[0]} surface entries for {n} items")
+            surf, checked = surface.to(torch.int32).contiguous(), False
+        else:
+            vals = [int(v) for v in (surface.tolist() if torch.is_tensor(surface) else surface)]
+            if len(vals) != n:
+                raise ValueError(f"{len(vals)} surface entries for {n} items")
+            for v in vals:
+                if not 0 <= v < m:
+                    raise ValueError(f"surface {v} outside [0, {m})")
+            surf, checked = torch.tensor(vals, dtype=torch.int32, device=self.device), True
+        s = surf.to(torch.int64)
+        ok = (s >= 0) & (s < m)
+        row = torch.where(ok, s, m)
+        offs, hw = soff[row], surfaces.hw[row.clamp(max=m - 1)]
+        if not checked:
+            base = slots if slots is not None else torch.arange(n, dtype=torch.int32, device=self.device)
+            slots = torch.where(ok, base, -1).to(torch.int32)
+        return frames, soff[:m], offs, hw, surf, slots
+
+    def _init_surfaces(self, surfaces: YuvSurfaces, boxes: torch.Tensor, slots, surface) -> torch.Tensor:
+        n = boxes.shape[0]
+        if n > self.max_tracks:
+            raise ValueError(f"{n} tracks > max_tracks {self.max_tracks}")
+        listed = None if slots is None else self._slots(slots)
+        if listed is not None and listed.shape[0] != n:
+            raise ValueError(f"{listed.shape[0]} slots for {n} boxes")
+        frames, soff, offs, hw, surf, eff = self._surface_items(surfaces, surface, n, listed)
+        self.engine.yuv420_crops_to_surface_rgb(surfaces.format, surfaces.planes, surfaces.pitches, surfaces.hw, frames, soff, surf,
+                                                self.template_factor, boxes=boxes, slots=eff)
+        if listed is None:
+            self.n = n
+            self._hw = hw
+            if eff is None:
+                self._slot_hw[:n] = hw
+                return self.engine.tracks_init(frames, offs, hw, boxes, first=0)
+        return self._init_slots(frames, offs, hw, boxes, eff)
+
+    def initialize_yuv(self, surfaces: YuvSurfaces, boxes, slots=None, surface=None) -> torch.Tensor:
         """``initialize`` for tracks 0..n-1 from device-resident YUV surfaces (``YuvSurfaces``, track i on surface i): only the rectangle
         each template crop reads is converted (vt_yuv420_crop_to_rgb, bit for bit cv2.cvtColor), into an RGB frame per track that
         this tracker owns, then vt_tracks_init runs on it on the same stream.  Those frames cost max_tracks x H x W x 3 bytes of
         device memory (2.76 MB per track at 720p, 6.2 MB at 1080p), allocated at the first call for a picture size.  With ``slots``,
-        surface i belongs to track slots[i], whose RGB frame it is converted into."""
+        surface i belongs to track slots[i], whose RGB frame it is converted into.
+
+        ``surface`` (several targets per surface): item i - box i, and track i or slots[i] - lies on ``surfaces`` entry ``surface[i]``,
+        a host sequence of ints (checked here: ValueError outside [0, surfaces.n)) or a CUDA integer tensor (passed through: an entry
+        outside [0, surfaces.n) makes the item a bad slot-list entry, VT_TRACK_BAD_SLOT, which touches no track state).  Each surface
+        is converted once, over the bounding rectangle of its items' crops (vt_yuv420_crops_to_surface_rgb), into one RGB frame per
+        surface: (surfaces.n + 1) x H x W x 3 bytes instead of (max_tracks + 1) x H x W x 3.  Results are bit for bit those of the
+        per-track path."""
         boxes = torch.as_tensor(boxes, dtype=torch.float64).reshape(-1, 4).to(self.device).contiguous()
+        if surface is not None:
+            return self._init_surfaces(surfaces, boxes, slots, surface)
         if boxes.shape[0] != surfaces.n:
             raise ValueError(f"{boxes.shape[0]} boxes for {surfaces.n} surfaces")
         frames, offs = self._yuv_frames(surfaces)
@@ -376,11 +447,26 @@ class BatchedTracker:
         self._slot_hw[: self.n] = self._hw
         return self.engine.tracks_init(frames, offs, self._hw, boxes, first=0)
 
-    def track_yuv(self, surfaces: YuvSurfaces, update_state: bool = True, detail: bool = False, slots=None):
+    def track_yuv(self, surfaces: YuvSurfaces, update_state: bool = True, detail: bool = False, slots=None, surface=None):
         """``track`` from device-resident YUV surfaces (surface i for track i): the rectangle each search crop reads is computed on the
         device from the track's current state - the host never waits for it - and converted; then vt_tracks_step runs on the same
         stream.  No allocation after the first call for a picture size, so a step can be captured in a CUDA graph.  With ``slots``,
-        surface i belongs to track slots[i]: its state is gathered on the device and the surface is converted into that track's frame."""
+        surface i belongs to track slots[i]: its state is gathered on the device and the surface is converted into that track's frame.
+
+        ``surface`` as for ``initialize_yuv``: item i (track i, or slots[i]) is on surface ``surface[i]``; each surface is converted once,
+        over the bounding rectangle of its items' search crops, computed on the device from the tracks' states.  With a CUDA surface
+        tensor (needed for CUDA-graph capture) the step runs as a slot list, so that an entry outside [0, surfaces.n) gets
+        VT_TRACK_BAD_SLOT and leaves its track as it was."""
+        if surface is not None:
+            listed = None if slots is None else self._slots(slots)
+            n = self.n if listed is None else listed.shape[0]
+            frames, soff, offs, hw, surf, eff = self._surface_items(surfaces, surface, n, listed)
+            self.engine.yuv420_crops_to_surface_rgb(surfaces.format, surfaces.planes, surfaces.pitches, surfaces.hw, frames, soff, surf,
+                                                    self.search_factor, boxes=None, slots=eff, first=0)
+            if eff is None:
+                self._hw = hw
+                return self.track_offsets(frames, offs, update_state=update_state, detail=detail)
+            return self._step_slots(frames, offs, hw, eff, update_state, detail)
         if slots is not None:
             slots = self._slots(slots)
             if slots.shape[0] != surfaces.n:

@@ -60,6 +60,8 @@ struct VtContext {
     uint32_t* d_claim = nullptr;      // [max_tracks] slot-list deduplication (vt_slots.cu), all 0xffffffff between calls
     int32_t* d_eff = nullptr;         // [max_tracks] effective slot per item of the current slot-list call
     float* d_maps = nullptr;          // [max_tracks][1280] score | size | offset of the last step
+    int32_t* d_surf_rect = nullptr;   // [max_tracks][4] bounding rectangle per surface (vt_yuv420_crops_to_surface_rgb), empty between calls
+    uint32_t* d_surf_done = nullptr;  // [max_tracks] conversion CTAs of the surface counted in, 0 between calls
     int last_first = 0, last_n = 0;
     // range fallback (vt_set_range_fallback): the flagged items of a tensor-core step, recomputed on the fp32 kernels
     bool fallback = false;
@@ -326,6 +328,7 @@ void free_all(VtHandle h) {
     cudaFree(h->d_weights); cudaFree(h->d_planes); cudaFree(h->d_scratch); cudaFree(h->d_taps); cudaFree(h->d_tokz);
     cudaFree(h->d_tokx); cudaFree(h->d_tok); cudaFree(h->d_state); cudaFree(h->d_tmpl);
     cudaFree(h->d_status); cudaFree(h->d_claim); cudaFree(h->d_eff); cudaFree(h->d_maps); cudaFree(h->d_gwork); cudaFree(h->d_fallback);
+    cudaFree(h->d_surf_rect); cudaFree(h->d_surf_done);
 }
 
 int check_ready(VtHandle h, bool need_tracks) {
@@ -854,10 +857,18 @@ int vt_create(const VtConfig* cfg, VtHandle* out) {
     A((void**)&h->d_claim, mt * sizeof(uint32_t));
     A((void**)&h->d_eff, mt * sizeof(int32_t));
     A((void**)&h->d_maps, mt * 1280 * sizeof(float));
+    A((void**)&h->d_surf_rect, mt * 4 * sizeof(int32_t));
+    A((void**)&h->d_surf_done, mt * sizeof(uint32_t));
     if (e == cudaSuccess) e = cudaMemset(h->d_state, 0, mt * 4 * sizeof(double));
     if (e == cudaSuccess) e = cudaMemset(h->d_tmpl, 0, mt * kNz * Cd * sizeof(float));     // never-initialised slots export zeros, not stale memory
     if (e == cudaSuccess) e = cudaMemset(h->d_status, 0, mt * sizeof(int32_t));
     if (e == cudaSuccess) e = cudaMemset(h->d_claim, 0xff, mt * sizeof(uint32_t));
+    if (e == cudaSuccess) {                                                                  // empty rectangles: {INT32_MAX, INT32_MAX, 0, 0}
+        std::vector<int32_t> empty(mt * 4, 0);
+        for (size_t s = 0; s < mt; ++s) empty[4 * s] = empty[4 * s + 1] = 0x7fffffff;
+        e = cudaMemcpy(h->d_surf_rect, empty.data(), mt * 4 * sizeof(int32_t), cudaMemcpyHostToDevice);
+    }
+    if (e == cudaSuccess) e = cudaMemset(h->d_surf_done, 0, mt * sizeof(uint32_t));
     if (e != cudaSuccess) {
         fail(nullptr, VT_ERR_CUDA, "vt_create: device allocation failed: %s", cudaGetErrorString(e));
         free_all(h); delete h;
@@ -1232,6 +1243,24 @@ int vt_yuv420_crop_to_rgb(VtHandle h, int32_t format, const uint64_t* planes, co
     const double* boxes = boxes_xywh ? boxes_xywh : h->d_state + (size_t)first * 4;
     cudaStream_t st = (cudaStream_t)stream;
     VT_LAUNCH(h, kNoStage, n, st, where, launch_yuv420_crop_to_rgb(format, planes, pitches, frame_hw, boxes, factor, dst, dst_offsets, n, h->num_sms, st));
+    return VT_OK;
+}
+
+int vt_yuv420_crops_to_surface_rgb(VtHandle h, int32_t format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw,
+                                   int32_t m, const int32_t* item_surface, const double* boxes_xywh, const int32_t* slots, double factor,
+                                   int32_t first, int32_t n, uint8_t* dst, const int64_t* dst_offsets, void* stream) {
+    const char* where = "vt_yuv420_crops_to_surface_rgb";
+    VT_ENTER(h, enter(h, where, kHandle, 0, n, false, {planes, pitches, frame_hw, item_surface, dst, dst_offsets}));
+    if (const int rc = check_yuv_format(h, where, format)) return rc;
+    if (!(factor > 0)) return fail(h, VT_ERR_INVALID_ARG, "%s: factor must be positive", where);
+    if (m < 0 || m > h->cfg.max_tracks) return fail(h, VT_ERR_INVALID_ARG, "%s: %d surfaces outside [0, max_tracks %d]", where, m, h->cfg.max_tracks);
+    if (const int rc = boxes_xywh || slots ? VT_OK : check_tracks(h, where, first, n)) return rc;      // the state, by range
+    if (slots) first = 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    const YuvSurfaceArgs a{planes, pitches, frame_hw, m, item_surface, boxes_xywh, h->d_state, slots, h->d_claim, first, h->cfg.max_tracks,
+                           factor, dst, dst_offsets, h->d_surf_rect, h->d_surf_done};
+    if (slots) VT_LAUNCH(h, kNoStage, n, st, where, launch_claim_slots(slots, n, h->cfg.max_tracks, h->d_claim, st));
+    VT_LAUNCH(h, kNoStage, n, st, where, launch_yuv420_crops_to_surface_rgb(format, a, n, h->num_sms, st));
     return VT_OK;
 }
 

@@ -265,6 +265,29 @@ int launch_yuv420_rect(int format, const YuvDesc& d, int num_sms, cudaStream_t s
 // and pitches below the row width are skipped.
 int launch_yuv420_crop_to_rgb(int format, const uint64_t* planes, const int32_t* pitches, const int32_t* frame_hw, const double* boxes,
                               double factor, uint8_t* dst, const int64_t* dst_offsets, int n, int num_sms, cudaStream_t st);
+// Shared surfaces: items [0, n) on m surfaces.  Item i's box is boxes[i], or the state of track slots[i] / first + i; it is skipped for a
+// surface index outside [0, m), a bad slot (outside [0, max_tracks) or repeating an earlier item's: the list is claimed first, with
+// launch_claim_slots) or a rectangle launch_yuv420_crop_to_rgb would skip.  Each surface's frame at dst + dst_off[s] gets the bounding
+// rectangle of its valid items' rectangles.  rect [m][4] int32 (y0, x0: minima; y1, x1: maxima) and done [m] are the handle's scratch,
+// empty between calls ({INT32_MAX, INT32_MAX, 0, 0} and 0).  Launches: one union pass, then one conversion per 32768 surfaces.
+struct YuvSurfaceArgs {
+    const uint64_t* planes;                               // [m][3] Y, U (NV12: UV), V
+    const int32_t* pitches;                               // [m][2] luma, chroma
+    const int32_t* hw;                                    // [m][2]
+    int m;
+    const int32_t* item_surface;                          // [n]
+    const double* boxes;                                  // [n][4] or null: the state
+    const double* state;                                  // [max_tracks][4]
+    const int32_t* slots;                                 // [n] or null: tracks first + i
+    uint32_t* claim;
+    int first, max_tracks;
+    double factor;
+    uint8_t* dst;
+    const int64_t* dst_off;                               // [m]
+    int32_t* rect;
+    uint32_t* done;
+};
+int launch_yuv420_crops_to_surface_rgb(int format, const YuvSurfaceArgs& a, int n, int num_sms, cudaStream_t st);
 
 // Slot lists (the vt_tracks_*_slots entry points): a kernel that reads per-track state takes `slots` (nullable).  Item i reads the
 // state of track slots[i], or of track i of the pre-offset state pointer when slots == NULL (the range calls); a negative slot is a

@@ -60,10 +60,37 @@ __device__ __forceinline__ bool make_desc(const YuvBatch& b, const YuvDesc& one,
     return true;
 }
 
-// The rectangle of a crop (vt_yuv420_crop_to_rgb): the box's crop geometry, computed by the code the crop kernels run, gives rows
-// [max(0, y1), min(H, y1 + crop_sz)) x columns [max(0, x1 - 1), min(W, x1 + crop_sz + 1)) (sequences.py crop_rect), widened to even
-// bounds (tracker.py even_rect); the descriptor addresses it inside the item's own planes and RGB frame.  False: nothing to write
-// (degenerate crop, odd or tiny frame, a pitch below its row's width).
+// The rectangle of a crop (vt_yuv420_crop_to_rgb, vt_yuv420_crops_to_surface_rgb): the box's crop geometry, computed by the code the
+// crop kernels run, gives rows [max(0, y1), min(H, y1 + crop_sz)) x columns [max(0, x1 - 1), min(W, x1 + crop_sz + 1)) (sequences.py
+// crop_rect), widened to even bounds (tracker.py even_rect): rows [r.y0, r.y1) x columns [r.x0, r.x1).  False: nothing to write
+// (degenerate crop, odd or tiny frame, a pitch below its row's width); the box is read only for a well-formed frame.
+struct EvenRect { int y0, x0, y1, x1; };
+
+template <int Layout>
+__device__ __forceinline__ bool crop_even_rect(const double* bx, double factor, int H, int W, int yp, int cp, EvenRect& r) {
+    if (H < 2 || W < 2 || (H & 1) || (W & 1) || yp < W || cp < (Layout == kYuvI420 ? W / 2 : W)) return false;
+    const CropGeom g = crop_geometry(bx[0], bx[1], bx[2], bx[3], factor, 1, H, W);
+    if (g.status != 0) return false;
+    const long long y0 = max(0, g.y1), y1 = min((long long)H, (long long)g.y1 + g.crop_sz);
+    const long long x0 = max(0, g.x1 - 1), x1 = min((long long)W, (long long)g.x1 + g.crop_sz + 1);
+    if (y1 <= y0 || x1 <= x0) return false;
+    r.y0 = (int)y0 & ~1; r.y1 = min(H, (int)(y1 + 1) & ~1); r.x0 = (int)x0 & ~1; r.x1 = min(W, (int)(x1 + 1) & ~1);
+    return true;
+}
+
+// The descriptor of the even rectangle r inside one picture's planes p (Y, U or UV, V) and its W-wide RGB frame at dst.
+template <int Layout>
+__device__ __forceinline__ void rect_desc(const uint64_t* p, int yp, int cp, int W, uint8_t* dst, const EvenRect& r, YuvDesc& d) {
+    d.y = reinterpret_cast<const uint8_t*>(p[0]) + (int64_t)r.y0 * yp + r.x0;
+    d.u = reinterpret_cast<const uint8_t*>(p[1]) + (int64_t)(r.y0 / 2) * cp + (Layout == kYuvI420 ? r.x0 / 2 : r.x0);
+    d.v = Layout == kYuvI420 ? reinterpret_cast<const uint8_t*>(p[2]) + (int64_t)(r.y0 / 2) * cp + r.x0 / 2 : d.u;
+    d.dst = dst + ((int64_t)r.y0 * W + r.x0) * 3;
+    d.y_pitch = yp;
+    d.c_pitch = cp;
+    d.dst_pitch = (int64_t)W * 3;
+    d.w = r.x1 - r.x0; d.h = r.y1 - r.y0;
+}
+
 struct YuvCropBatch {
     const uint64_t* planes;                               // [n][3] Y, U (NV12: UV), V
     const int32_t* pitches;                               // [n][2] luma, chroma
@@ -76,25 +103,10 @@ struct YuvCropBatch {
 
 template <int Layout>
 __device__ __forceinline__ bool make_crop_desc(const YuvCropBatch& b, int item, YuvDesc& d) {
-    const int H = b.hw[2 * item], W = b.hw[2 * item + 1];
-    const int yp = b.pitches[2 * item], cp = b.pitches[2 * item + 1];
-    if (H < 2 || W < 2 || (H & 1) || (W & 1) || yp < W || cp < (Layout == kYuvI420 ? W / 2 : W)) return false;
-    const double* bx = b.boxes + 4 * item;
-    const CropGeom g = crop_geometry(bx[0], bx[1], bx[2], bx[3], b.factor, 1, H, W);
-    if (g.status != 0) return false;
-    const long long y0 = max(0, g.y1), y1 = min((long long)H, (long long)g.y1 + g.crop_sz);
-    const long long x0 = max(0, g.x1 - 1), x1 = min((long long)W, (long long)g.x1 + g.crop_sz + 1);
-    if (y1 <= y0 || x1 <= x0) return false;
-    const int ya = (int)y0 & ~1, yb = min(H, (int)(y1 + 1) & ~1), xa = (int)x0 & ~1, xb = min(W, (int)(x1 + 1) & ~1);
-    const uint64_t* p = b.planes + 3 * item;
-    d.y = reinterpret_cast<const uint8_t*>(p[0]) + (int64_t)ya * yp + xa;
-    d.u = reinterpret_cast<const uint8_t*>(p[1]) + (int64_t)(ya / 2) * cp + (Layout == kYuvI420 ? xa / 2 : xa);
-    d.v = Layout == kYuvI420 ? reinterpret_cast<const uint8_t*>(p[2]) + (int64_t)(ya / 2) * cp + xa / 2 : d.u;
-    d.dst = b.dst + b.dst_off[item] + ((int64_t)ya * W + xa) * 3;
-    d.y_pitch = yp;
-    d.c_pitch = cp;
-    d.dst_pitch = (int64_t)W * 3;
-    d.w = xb - xa; d.h = yb - ya;
+    const int W = b.hw[2 * item + 1], yp = b.pitches[2 * item], cp = b.pitches[2 * item + 1];
+    EvenRect r;
+    if (!crop_even_rect<Layout>(b.boxes + 4 * item, b.factor, b.hw[2 * item], W, yp, cp, r)) return false;
+    rect_desc<Layout>(b.planes + 3 * item, yp, cp, W, b.dst + b.dst_off[item], r, d);
     return true;
 }
 
@@ -189,6 +201,57 @@ yuv420_crop_to_rgb_kernel(YuvCropBatch b) {
     convert_units<Layout>(d, s_row);
 }
 
+// Shared surfaces (vt_yuv420_crops_to_surface_rgb): pass 1 folds every valid item's rectangle into its surface's bounding rectangle,
+// pass 2 converts each surface's bounding rectangle once into the surface's own RGB frame.  An item's crop reads only its own
+// rectangle, which lies inside the bounding one, so every track reads the bytes the per-item path would have written for it.
+constexpr int kUnionThreads = 256;
+constexpr EvenRect kEmptyRect{0x7fffffff, 0x7fffffff, 0, 0};          // also the state of the scratch between calls
+
+// One thread per item.  Every item of a slot list resolves its entry (the winner releases its claim) before anything may skip it.
+template <int Layout>
+__global__ void __launch_bounds__(kUnionThreads)
+yuv420_surface_union_kernel(YuvSurfaceArgs a, int n) {
+    const int i = blockIdx.x * kUnionThreads + threadIdx.x;
+    if (i >= n) return;
+    const int slot = a.slots ? resolve_slot(a.slots, i, a.max_tracks, a.claim) : a.first + i;
+    const int s = a.item_surface[i];
+    if (slot < 0 || s < 0 || s >= a.m) return;
+    const double* bx = a.boxes ? a.boxes + 4 * i : a.state + 4 * (int64_t)slot;
+    EvenRect r;
+    if (!crop_even_rect<Layout>(bx, a.factor, a.hw[2 * s], a.hw[2 * s + 1], a.pitches[2 * s], a.pitches[2 * s + 1], r)) return;
+    int* u = a.rect + 4 * s;                                         // y0, x0: minima; y1, x1: maxima
+    atomicMin(u, r.y0);
+    atomicMin(u + 1, r.x0);
+    atomicMax(u + 2, r.y1);
+    atomicMax(u + 3, r.x1);
+}
+
+// gridDim.x CTAs per surface (blockIdx.y).  Each CTA reads the bounding rectangle, then counts itself in; the last one to do so empties
+// the scratch for the next call.  A surface without a valid item has an empty rectangle: nothing is written.
+template <int Layout>
+__global__ void __launch_bounds__(kYuvThreads)
+yuv420_surface_to_rgb_kernel(YuvSurfaceArgs a, int s0) {
+    __shared__ uint32_t s_row[2][kRowWords];
+    __shared__ EvenRect s_rect;
+    const int s = s0 + blockIdx.y;
+    if (threadIdx.x == 0) {
+        int* u = a.rect + 4 * s;
+        s_rect = EvenRect{u[0], u[1], u[2], u[3]};
+        __threadfence();                                              // the read above is complete before this CTA is counted
+        if (atomicAdd(a.done + s, 1u) == gridDim.x - 1) {
+            u[0] = kEmptyRect.y0; u[1] = kEmptyRect.x0; u[2] = kEmptyRect.y1; u[3] = kEmptyRect.x1;
+            a.done[s] = 0;
+        }
+    }
+    __syncthreads();
+    const EvenRect r = s_rect;
+    if (r.y1 <= r.y0) return;
+    const int W = a.hw[2 * s + 1];
+    YuvDesc d;
+    rect_desc<Layout>(a.planes + 3 * s, a.pitches[2 * s], a.pitches[2 * s + 1], W, a.dst + a.dst_off[s], r, d);
+    convert_units<Layout>(d, s_row);
+}
+
 namespace {
 
 int launch(int format, const YuvBatch& b, const YuvDesc& one, dim3 grid, cudaStream_t st) {
@@ -243,6 +306,28 @@ int launch_yuv420_crop_to_rgb(int format, const uint64_t* planes, const int32_t*
         ++launched;
     }
     return launched;
+}
+
+template <int Layout>
+int launch_surfaces(const YuvSurfaceArgs& a, int n, int num_sms, cudaStream_t st) {
+    yuv420_surface_union_kernel<Layout><<<(n + kUnionThreads - 1) / kUnionThreads, kUnionThreads, 0, st>>>(a, n);
+    if (cudaPeekAtLastError() != cudaSuccess) return -1;
+    // a bounding rectangle can be a whole frame: a fixed number of CTAs per surface, as for whole frames
+    const int per_surface = max(1, min(4096, num_sms * 32 * 2 / min(max(a.m, 1), 32768)));
+    int launched = 1;
+    for (int s0 = 0; s0 < a.m; s0 += 32768) {                              // gridDim.y is limited to 65535
+        yuv420_surface_to_rgb_kernel<Layout><<<dim3(per_surface, min(32768, a.m - s0)), kYuvThreads, 0, st>>>(a, s0);
+        if (cudaPeekAtLastError() != cudaSuccess) return -1;
+        ++launched;
+    }
+    return launched;
+}
+
+int launch_yuv420_crops_to_surface_rgb(int format, const YuvSurfaceArgs& a, int n, int num_sms, cudaStream_t st) {
+    if (n <= 0) return 0;
+    if (format == kYuvNV12) return launch_surfaces<kYuvNV12>(a, n, num_sms, st);
+    if (format == kYuvI420) return launch_surfaces<kYuvI420>(a, n, num_sms, st);
+    return -1;
 }
 
 }  // namespace vt

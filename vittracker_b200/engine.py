@@ -253,6 +253,26 @@ class Engine:
                    tensor_ptr(dst, "dst", torch.uint8, dev), tensor_ptr(dst_offsets, "dst_offsets", torch.int64, dev, (n,)))
         return dst
 
+    def yuv420_crops_to_surface_rgb(self, format: str, planes: torch.Tensor, pitches: torch.Tensor, frame_hw: torch.Tensor,
+                                    dst: torch.Tensor, dst_offsets: torch.Tensor, item_surface: torch.Tensor, factor: float,
+                                    boxes: Optional[torch.Tensor] = None, slots: Optional[torch.Tensor] = None,
+                                    first: int = 0) -> torch.Tensor:
+        """vt_yuv420_crops_to_surface_rgb: n items on m surfaces (``planes`` int64 [m, 3], ``pitches`` / ``frame_hw`` int32 [m, 2],
+        ``dst_offsets`` int64 [m]: one RGB frame per surface); item i lies on surface ``item_surface[i]`` (int32 [n]).  Each surface's
+        frame gets, bit for bit cv2.cvtColor, the bounding rectangle of the crops of its items, whose boxes are ``boxes`` (float64
+        [n, 4]) or the state of tracks ``slots[i]`` (int32 [n]) or [first, first + n).  Items with a surface outside [0, m), a bad slot or
+        a degenerate crop are skipped.  No allocation and no synchronisation (capturable in a CUDA graph).  Returns ``dst``."""
+        fmt = yuv_format(format)
+        m, n = int(planes.shape[0]), int(item_surface.shape[0])
+        dev = self.device
+        self._call("vt_yuv420_crops_to_surface_rgb", fmt, tensor_ptr(planes, "planes", torch.int64, dev, (m, 3)),
+                   tensor_ptr(pitches, "pitches", torch.int32, dev, (m, 2)), tensor_ptr(frame_hw, "frame_hw", torch.int32, dev, (m, 2)), m,
+                   tensor_ptr(item_surface, "item_surface", torch.int32, dev, (n,)),
+                   tensor_ptr(boxes, "boxes", torch.float64, dev, (n, 4), optional=True),
+                   tensor_ptr(slots, "slots", torch.int32, dev, (n,), optional=True), float(factor), int(first), n,
+                   tensor_ptr(dst, "dst", torch.uint8, dev), tensor_ptr(dst_offsets, "dst_offsets", torch.int64, dev, (m,)))
+        return dst
+
     # ------------------------------------------------------------------------------------------
     def tracks_init(self, frames, frame_offsets, frame_hw, boxes, first: int = 0) -> torch.Tensor:
         n = int(boxes.shape[0])
