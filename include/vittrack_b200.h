@@ -58,9 +58,17 @@ typedef enum VtStatus {
 #define VT_BLOCKS_TCGEN05 1       /* tcgen05 tensor-core kernels: fp16 hi/lo split operands (three products per contraction),
                                    * fp32 accumulation; the attention scores q k^T as a single fp16 pass - the one contraction whose
                                    * low-order terms the measured precision budget (profiles/r02_precision_budget*.json) shows
-                                   * never reach the arg-max on the specified (random-init) workload                          */
-#define VT_BLOCKS_TCGEN05_3TERM 2 /* the same kernels with three products for q k^T too: for checkpoints with sharp attention
-                                   * (large |q||k|), ~9 % slower blocks                                                       */
+                                   * never reach the arg-max on the specified (random-init) workload.  Its error grows with
+                                   * |q||k|: max |map - float64| (score / offset) over 1024 open-loop 720p tracks, NVIDIA B200 at
+                                   * 1000 W (tests/test_trained_weights.py), q and k scaled to a max |logit| of:
+                                   *                   random init        4                 16                64
+                                   *   single pass     8.8e-7 / 1.4e-5    3.6e-6 / 3.9e-5   4.0e-5 / 5.8e-4   4.2e-4 / 2.9e-3
+                                   *   three terms     6.0e-7 / 1.0e-5    6.4e-7 / 1.1e-5   9.0e-7 / 1.5e-5   1.0e-6 / 1.3e-5
+                                   * At 64 the single pass moves boxes past the 1e-2 parity bound, so vt_finalize_weights takes the
+                                   * three-term pass when a bound on |q.k|/sqrt(C) from the weights alone exceeds 512 (random-init
+                                   * weights: < 20)                                                                          */
+#define VT_BLOCKS_TCGEN05_3TERM 2 /* the same kernels with three products for q k^T too, whatever the weights: for checkpoints
+                                   * with sharp attention (large |q||k|), ~9 % slower blocks                                  */
 
 /* Model / tracker configuration: experiments/vit_dist/vit_48_h32_noKD.yaml:56-64,89-92,
  * lib/config/vit_dist/config.py:27-37, build_ostrack_dist(cfg, depth=3) vit_dist.py:159. */

@@ -37,6 +37,7 @@ struct VtContext {
     TensorMap tensors;
     bool finalized = false;
     bool tracks_ready = false;
+    int score_terms = 1;              // split terms of the tensor-core blocks' q k^T (vt_finalize_weights: score_terms)
     uint64_t fingerprint = 0;         // of the weights finalised last (vt_weights_fingerprint)
     int64_t launches = 0;
 
@@ -240,6 +241,61 @@ int rebalance(const VtConfig& c, TensorMap& ts) {
     return pnorm;
 }
 
+// Upper bound on the spectral norm of W [rows][cols]: ||W||_2^2 = lambda_max(W^T W) <= ||(W^T W)^32||_F^(1/32), at most 48^(1/64) ~ 6 %
+// above it for a 48-column W.  The powers are taken by squaring, renormalised at every step.
+double spectral_norm_bound(const float* W, int rows, int cols) {
+    std::vector<double> m((size_t)cols * cols, 0.0), t(m.size());
+    for (int r = 0; r < rows; ++r)
+        for (int i = 0; i < cols; ++i)
+            for (int j = 0; j < cols; ++j) m[(size_t)i * cols + j] += (double)W[(size_t)r * cols + i] * W[(size_t)r * cols + j];
+    auto frob = [&]() { double s = 0.0; for (double v : m) s += v * v; return sqrt(s); };
+    double log_scale = 0.0;                       // (W^T W)^(2^s) = m * exp(log_scale)
+    for (int s = 0; s < 5; ++s) {
+        const double f = frob();
+        if (!(f > 0.0) || !std::isfinite(f)) return f > 0.0 ? INFINITY : 0.0;
+        for (double& v : m) v /= f;
+        for (int i = 0; i < cols; ++i)
+            for (int j = 0; j < cols; ++j) {
+                double a = 0.0;
+                for (int k = 0; k < cols; ++k) a += m[(size_t)i * cols + k] * m[(size_t)k * cols + j];
+                t[(size_t)i * cols + j] = a;
+            }
+        m.swap(t);
+        log_scale = 2.0 * (log_scale + log(f));
+    }
+    return exp((log(frob()) + log_scale) / 64.0);
+}
+
+// Split terms of the tensor-core blocks' scores q k^T (vt_block_tc.cu: kScoresTerms).  The single pass rounds q and k to fp16, so its
+// error grows with |q||k|.  Each block bounds |q . k| / sqrt(C) from its weights alone: norm1's output has norm at most
+// R = sqrt(C) max|gamma| + ||beta||, so |q| <= ||W_q||_2 R + ||b_q|| and |k| likewise.  Random-init weights stay below 20
+// (tests/test_trained_weights.py); above kSharpScores the handle takes the three-term pass whatever blocks_impl asked for.
+constexpr double kSharpScores = 512.0;
+
+int score_terms(const VtConfig& c, const TensorMap& ts) {
+    if (c.blocks_impl == VT_BLOCKS_TCGEN05_3TERM) return 3;
+    const size_t C = c.embed_dim;
+    for (int b = 0; b < c.depth; ++b) {
+        const std::string p = "blocks." + std::to_string(b) + ".";
+        const std::vector<float>& g = ts.at(p + "norm1.weight").data;
+        const std::vector<float>& be = ts.at(p + "norm1.bias").data;
+        const std::vector<float>& w = ts.at(p + "attn.qkv.weight").data;
+        const std::vector<float>& bias = ts.at(p + "attn.qkv.bias").data;
+        double gmax = 0.0, bn = 0.0, bq = 0.0, bk = 0.0;
+        for (size_t i = 0; i < C; ++i) {
+            gmax = fmax(gmax, fabs((double)g[i]));
+            bn += (double)be[i] * be[i];
+            bq += (double)bias[i] * bias[i];
+            bk += (double)bias[C + i] * bias[C + i];
+        }
+        const double R = sqrt((double)C) * gmax + sqrt(bn);
+        const double q = spectral_norm_bound(w.data(), (int)C, (int)C) * R + sqrt(bq);
+        const double k = spectral_norm_bound(w.data() + C * C, (int)C, (int)C) * R + sqrt(bk);
+        if (!(q * k / sqrt((double)C) <= kSharpScores)) return 3;
+    }
+    return 1;
+}
+
 // FNV-1a 64 over 8-byte little-endian words of a byte stream, the last word zero-padded (the weights fingerprint of the header).
 // Word-wise rather than byte-wise: one multiply per 8 bytes.
 struct WordFnv {
@@ -407,7 +463,7 @@ int run_blocks(VtHandle h, const float* tokz, int zs, const int32_t* zslots, con
                size_t tap_stride, cudaStream_t st) {
     if (h->cfg.blocks_impl == VT_BLOCKS_SIMT_FP32)
         return launch_blocks_simt(tokz, zs, zslots, tokx, xs, out, n, h->mw, taps, tap_stride, st);
-    return launch_blocks_tc(tokz, zs, zslots, tokx, xs, out, n, h->mw, taps, tap_stride, h->num_sms, h->cfg.blocks_impl == VT_BLOCKS_TCGEN05_3TERM ? 3 : 1, st);
+    return launch_blocks_tc(tokz, zs, zslots, tokx, xs, out, n, h->mw, taps, tap_stride, h->num_sms, h->score_terms, st);
 }
 
 
@@ -922,6 +978,7 @@ int vt_finalize_weights(VtHandle h, void* stream) {
     TensorMap ts = h->tensors;          // rebalanced on a copy: finalising again starts from the tensors as they were set
     const int pnorm = rebalance(h->cfg, ts);
     if (h->generic) return finalize_generic(h, ts, pnorm, st);
+    h->score_terms = score_terms(h->cfg, ts);
     Packer pk;
     ModelW& m = h->mw;
     m.norm_tap_scale = ldexpf(1.f, pnorm);

@@ -56,7 +56,8 @@ constexpr int kNS = 6;
 // between a LayerNorm's gain and the next weights) does not reach the kernel: weight ingest rebalances it by powers of two (vt_api.cu:
 // rebalance), so each operand keeps the split's relative precision.  A trained checkpoint can still have sharper attention - a larger
 // product |q||k| and the same RELATIVE operand error - so the kernel is compiled in both forms and the handle chooses: VT_BLOCKS_TCGEN05 (single
-// pass, the default) or VT_BLOCKS_TCGEN05_3TERM (blocks_impl = "tcgen05_3term": three terms everywhere, ~9 % slower blocks).
+// pass, the default, unless a bound on |q||k| from the weights says they are sharp: vt_api.cu, score_terms) or VT_BLOCKS_TCGEN05_3TERM
+// (blocks_impl = "tcgen05_3term": three terms everywhere, ~9 % slower blocks).
 constexpr int kEpiWarps = 4 * kNS;
 constexpr int kEpiThreads = kEpiWarps * 32;
 constexpr int kTcThreads = kEpiThreads + 32;   // + the control warp
