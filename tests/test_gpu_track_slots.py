@@ -269,9 +269,6 @@ def test_sequence_driver_steps_only_running_sequences():
     log = []
 
     class Profiled(BatchedBackend):
-        def park(self, slot):
-            raise AssertionError("a backend with step_active is never asked to park a slot")
-
         def step_active(self, slots, images):
             self.bt.engine.profile_read()
             r = super().step_active(slots, images)

@@ -9,30 +9,45 @@ from vittracker_b200.sequences import MultiSequenceRunner, Sequence, results_pat
 
 
 class FakeBackend:
-    """Box of a slot after k steps = init box + k in x; remembers which slot served which frame."""
+    """Box of a slot after k steps = init box + k in x; remembers which slot served which frame, the slots of every initialisation
+    and every step, and checks that each step lists exactly the slots whose sequence is running (see _runner)."""
 
     def __init__(self, slots):
         self.state = [None] * slots
         self.log = []
+        self.batches = []
+        self.calls = []
+        self.runner = None
 
-    def initialize(self, slot, image, box):
-        if box[2] <= 0:
-            raise Exception("Too small bounding box.")
-        self.state[slot] = [float(v) for v in box]
+    def initialize_many(self, items):
+        self.batches.append([slot for (slot, _, _) in items])
+        errors = []
+        for slot, image, box in items:
+            if box[2] <= 0:
+                errors.append(Exception("Too small bounding box."))
+                continue
+            self.state[slot] = [float(v) for v in box]
+            errors.append(None)
+        return errors
 
-    def park(self, slot):
-        self.state[slot] = [0.0, 0.0, 1.0, 1.0]
-
-    def step(self, images):
-        out = np.zeros((len(images), 5))
-        for i, im in enumerate(images):
-            if im is not None:
-                assert self.state[i] is not None
-                self.state[i][0] += 1.0
-                self.log.append((i, int(im[0, 0, 0])))
-            out[i, :4] = self.state[i]
-            out[i, 4] = 0.5
+    def step_active(self, slots, images):
+        running = [i for i, s in enumerate(self.runner.slots) if s.seq is not None]
+        assert list(slots) == running and len(images) == len(slots)
+        self.calls.append(list(slots))
+        out = np.zeros((len(slots), 5))
+        for j, (i, im) in enumerate(zip(slots, images)):
+            assert self.state[i] is not None
+            self.state[i][0] += 1.0
+            self.log.append((i, int(im[0, 0, 0])))
+            out[j, :4] = self.state[i]
+            out[j, 4] = 0.5
         return out
+
+
+def _runner(be, slots, **kw):
+    """A runner over the fake backend `be`, which checks every step against this runner's running slots."""
+    be.runner = MultiSequenceRunner(be, slots, **kw)
+    return be.runner
 
 
 def _frames(n, tag):
@@ -44,8 +59,10 @@ def test_scheduler_ragged_sequences_and_result_files(tmp_path):
     seqs = [Sequence(f"s{i}", _frames(n, i), [10.0 * i + 0.7, 5.9, 20.5, 30.2], dataset="got10k" if i == 2 else "") for i, n in enumerate(lengths)]
     seqs.append(Sequence("bad", _frames(3, 9), [1.0, 1.0, 0.0, 5.0]))          # init fails: reported and skipped
     be = FakeBackend(3)
-    res = MultiSequenceRunner(be, 3, results_dir=str(tmp_path)).run(seqs)
+    res = _runner(be, 3, results_dir=str(tmp_path)).run(seqs)
     assert set(res) == {f"s{i}" for i in range(len(lengths))}
+    assert sum(len(c) for c in be.calls) == sum(n - 1 for n in lengths)         # every tracked frame stepped once, nothing else
+    assert any(len(c) < 3 for c in be.calls)                                    # the run drains: the last steps list fewer slots
     for i, n in enumerate(lengths):
         out = res[f"s{i}"]
         if n == 1:
@@ -63,41 +80,26 @@ def test_scheduler_ragged_sequences_and_result_files(tmp_path):
     assert np.loadtxt(results_path(str(tmp_path), seqs[0]) + "_time.txt").shape == (5,)
     # resumable: sequences whose results exist are skipped (running.py:116-131)
     be2 = FakeBackend(3)
-    res2 = MultiSequenceRunner(be2, 3, results_dir=str(tmp_path)).run(seqs[:5])
+    res2 = _runner(be2, 3, results_dir=str(tmp_path)).run(seqs[:5])
     assert set(res2) == {"s1"} and not be2.log            # s1 has a single frame: no box file is ever written for it
 
 
 def test_free_slots_are_initialised_together_when_the_backend_can(tmp_path):
-    """A backend with initialize_many gets every free slot in ONE call per refill round; a sequence whose initialisation fails is reported,
-    skipped and its slot offered to the next pending sequence (running.py:135-142); results equal the one-by-one path."""
-    class Batching(FakeBackend):
-        def __init__(self, slots):
-            super().__init__(slots)
-            self.batches = []
-
-        def initialize_many(self, items):
-            self.batches.append([slot for (slot, _, _) in items])
-            errors = []
-            for slot, image, box in items:
-                try:
-                    self.initialize(slot, image, box)
-                    errors.append(None)
-                except Exception as e:
-                    errors.append(e)
-            return errors
-
+    """The backend gets every free slot in ONE initialize_many call per refill round; a sequence whose initialisation fails is reported,
+    skipped and its slot offered to the next pending sequence (running.py:135-142); every other sequence is tracked to its end."""
     lengths = [4, 2, 6, 3, 5, 1, 4]
-    def make():
-        seqs = [Sequence(f"s{i}", _frames(n, i), [10.0 * i + 1, 5.0, 20.0, 30.0]) for i, n in enumerate(lengths)]
-        seqs.insert(2, Sequence("bad", _frames(3, 9), [1.0, 1.0, 0.0, 5.0]))            # fails inside the first batch
-        return seqs
-    be = Batching(3)
-    res = MultiSequenceRunner(be, 3).run(make())
-    ref = MultiSequenceRunner(FakeBackend(3), 3).run(make())
-    assert set(res) == set(ref) == {f"s{i}" for i in range(len(lengths))}
-    for name in ref:
-        assert res[name].get("target_bbox") == ref[name].get("target_bbox")
-        assert len(res[name]["time"]) == len(ref[name]["time"])
+    seqs = [Sequence(f"s{i}", _frames(n, i), [10.0 * i + 1, 5.0, 20.0, 30.0]) for i, n in enumerate(lengths)]
+    seqs.insert(2, Sequence("bad", _frames(3, 9), [1.0, 1.0, 0.0, 5.0]))                # fails inside the first batch
+    be = FakeBackend(3)
+    res = _runner(be, 3).run(seqs)
+    assert set(res) == {f"s{i}" for i in range(len(lengths))}
+    for i, n in enumerate(lengths):
+        out = res[f"s{i}"]
+        assert len(out["time"]) == n
+        if n == 1:
+            assert "target_bbox" not in out
+            continue
+        assert out["target_bbox"] == [[10.0 * i + 1 + k, 5.0, 20.0, 30.0] for k in range(n)]
     assert be.batches[0] == [0, 1, 2]                       # all three slots at once ...
     assert be.batches[1] == [2]                             # ... and the failed one again, with the next pending sequence
     assert all(len(b) >= 1 for b in be.batches)
@@ -121,16 +123,15 @@ def test_threaded_frame_ingest_from_image_files(tmp_path):
         seqs.append(Sequence(f"s{i}", paths, [10.0 * i, 5.0, 20.0, 30.0]))
 
     class Recorder(FakeBackend):
-        def step(self, images):
-            for i, im in enumerate(images):
-                if im is not None:
-                    assert im.shape == (6, 8, 3) and int(im[0, 0, 2]) == 200          # RGB order restored
-                    self.log.append(("frame", i, int(im[0, 0, 0]), int(im[0, 0, 1])))
-            return super().step(images)
+        def step_active(self, slots, images):
+            for i, im in zip(slots, images):
+                assert im.shape == (6, 8, 3) and int(im[0, 0, 2]) == 200              # RGB order restored
+                self.log.append(("frame", i, int(im[0, 0, 0]), int(im[0, 0, 1])))
+            return super().step_active(slots, images)
 
     def run(workers, sequences):
         be = Recorder(2)
-        r = MultiSequenceRunner(be, 2, read_workers=workers)
+        r = _runner(be, 2, read_workers=workers)
         try:
             return r.run(sequences), be
         finally:

@@ -14,7 +14,7 @@ import math
 import os
 import time
 from concurrent.futures import Future, ThreadPoolExecutor
-from typing import Callable, Dict, List, Optional, Sequence as Seq, Union
+from typing import Callable, Dict, List, Optional, Sequence as Seq, Tuple, Union
 
 import numpy as np
 
@@ -137,8 +137,8 @@ def crop_rect(box, factor: float, H: int, W: int) -> Optional[tuple]:
 
 
 class BatchedBackend:
-    """The device side of the driver: per-slot initialise, one step for the running slots.  Split from the scheduler so
-    that the scheduling logic is testable without a GPU.
+    """The device side of the driver: one initialisation for any set of free slots, one step for the running slots.  Split from the
+    scheduler so that the scheduling logic is testable without a GPU.
 
     Uploads are ROW-STAGED like the batch-1 tracker's (tracker.py `_upload`): a step sends, per slot, only the frame rows its search
     crop can read (the state is known on the host: it is what the previous step returned), packed back to back in one pinned buffer
@@ -172,9 +172,6 @@ class BatchedBackend:
         self.bytes_uploaded = 0
         self._slot_ids = torch.zeros((slots,), dtype=torch.int32).pin_memory()
         self._slot_ids_np = self._slot_ids.numpy()
-        # step(): idle slots keep tracking a small black frame so that a step can cover a contiguous slot range
-        self._dummy = np.zeros((64, 64, 3), dtype=np.uint8)
-        self._dummy_box = [24.0, 24.0, 16.0, 16.0]
 
     def _stage(self, frames: List[np.ndarray], rois: Optional[List[Optional[tuple]]] = None):
         """Pack the frames (or, with `rois`, the rows [ya, yb) of each) into one pinned buffer, upload with one copy; returns per-frame
@@ -278,44 +275,26 @@ class BatchedBackend:
                 self._state[items[k][0]] = [float(v) for v in items[k][2]]
         return errors
 
-    def initialize(self, slot: int, image: np.ndarray, box) -> None:
-        err = self.initialize_many([(slot, image, box)])[0]
-        if err is not None:
-            raise err
-
-    def park(self, slot: int) -> None:
-        """Give an idle slot a valid template / state on the dummy frame."""
-        self.initialize(slot, self._dummy, self._dummy_box)
-
-    def step(self, images: List[Optional[np.ndarray]]) -> np.ndarray:
-        """images[i] = next frame of slot i (None = idle, tracking the parked dummy frame); returns [len(images), 5] boxes + confidence."""
-        return self._step(list(range(len(images))), [self._dummy if im is None else im for im in images], None)
-
     def step_active(self, slots: List[int], images: List[np.ndarray]) -> np.ndarray:
         """images[j] = next frame of slot slots[j]; stages and steps only those slots.  Returns [len(slots), 5] boxes + confidence, in the
         order of `slots`."""
-        return self._step(check_slots(slots, self.slots), images, slots)
-
-    def _step(self, ids: List[int], frames: List[np.ndarray], slots: Optional[List[int]]) -> np.ndarray:
         torch = self.torch
-        n = len(frames)
+        ids = check_slots(slots, self.slots)
+        n = len(images)
         if n == 0:
             return np.zeros((0, 5))
         rois = None
         if self.row_staging:
-            rois = [crop_rows(self._state[t], self.search_factor, f.shape[0]) if self._state[t] is not None else None for t, f in zip(ids, frames)]
-        offs = self._stage(frames, rois)
+            rois = [crop_rows(self._state[t], self.search_factor, f.shape[0]) if self._state[t] is not None else None for t, f in zip(ids, images)]
+        offs = self._stage(images, rois)
         hw_np, off_np = self._hw_np, self._off_np
-        for i, f in enumerate(frames):
+        for i, f in enumerate(images):
             hw_np[i, 0], hw_np[i, 1] = f.shape[0], f.shape[1]
         off_np[:n] = offs
         hw = self._hw[:n].to(self.dev, non_blocking=True)
         off = self._off[:n].to(self.dev, non_blocking=True)
-        if slots is None:
-            out = self.bt.engine.tracks_step(self._devbuf, off, hw, first=0, n=n, update_state=True)
-        else:
-            self._slot_ids_np[:n] = slots
-            out = self.bt._step_slots(self._devbuf, off, hw, self._slot_ids[:n].to(self.dev, non_blocking=True), True, False)
+        self._slot_ids_np[:n] = ids
+        out = self.bt._step_slots(self._devbuf, off, hw, self._slot_ids[:n].to(self.dev, non_blocking=True), True, False)
         self._out_pin[:n].copy_(out, non_blocking=True)
         torch.cuda.current_stream(self.dev).synchronize()
         res = self._out_pin[:n].numpy().copy()
@@ -332,14 +311,15 @@ class MultiSequenceRunner:
 
     def __init__(self, backend, slots: int, results_dir: Optional[str] = None, skip_existing: bool = True, verbose: bool = False,
                  read_workers: int = 8):
-        """read_workers: threads that decode frames (SURVEY 8f rank 2, frame ingest: cv.imread + BGR2RGB release the GIL).  The frames of a
+        """backend: ``initialize_many([(slot, image, box), ...]) -> [None or exception, ...]`` and ``step_active(slots, images) ->
+        [len(slots), 5]`` boxes + confidence, as BatchedBackend offers them.
+        read_workers: threads that decode frames (SURVEY 8f rank 2, frame ingest: cv.imread + BGR2RGB release the GIL).  The frames of a
         step are decoded in parallel, and the frames of step t + 1 while the device runs step t; 0 = decode on the calling thread."""
         self.backend = backend
         self.slots = [_Slot() for _ in range(slots)]
         self.results_dir = results_dir
         self.skip_existing = skip_existing
         self.verbose = verbose
-        self._parked = [False] * slots
         self._readers = ThreadPoolExecutor(max_workers=read_workers, thread_name_prefix="vt-read") if read_workers > 0 else None
 
     def close(self) -> None:
@@ -352,28 +332,29 @@ class MultiSequenceRunner:
             slot.prefetch.cancel()
         slot.seq, slot.output, slot.prefetch, slot.prefetch_idx = None, None, None, -1
 
-    def _step_images(self, high: int) -> List[Optional[np.ndarray]]:
-        """The next frame of every running slot below `high` (None for idle slots).  A sequence whose frame cannot be read is reported
-        and dropped, like a sequence that raises inside the reference's run_sequence (running.py:135-142)."""
-        futs: List[Optional[Future]] = [None] * high
-        for i, s in enumerate(self.slots[:high]):
-            if s.seq is None:
-                continue
+    def _step_images(self, active: List[int]) -> Tuple[List[int], List[np.ndarray]]:
+        """(slots, images): the running slots of `active` and the next frame of each.  A sequence whose frame cannot be read is reported,
+        dropped and left out, like a sequence that raises inside the reference's run_sequence (running.py:135-142)."""
+        futs: List[Optional[Future]] = []
+        for i in active:
+            s = self.slots[i]
             if s.prefetch is not None and s.prefetch_idx == s.next_frame:
-                futs[i] = s.prefetch
+                futs.append(s.prefetch)
             elif self._readers is not None:
-                futs[i] = self._readers.submit(read_image, s.seq.frames[s.next_frame])
+                futs.append(self._readers.submit(read_image, s.seq.frames[s.next_frame]))
+            else:
+                futs.append(None)
             s.prefetch, s.prefetch_idx = None, -1
-        images: List[Optional[np.ndarray]] = [None] * high
-        for i, s in enumerate(self.slots[:high]):
-            if s.seq is None:
-                continue
+        slots, images = [], []
+        for i, fut in zip(active, futs):
+            s = self.slots[i]
             try:
-                images[i] = futs[i].result() if futs[i] is not None else read_image(s.seq.frames[s.next_frame])
+                images.append(fut.result() if fut is not None else read_image(s.seq.frames[s.next_frame]))
+                slots.append(i)
             except Exception as e:
                 print(e)
                 self._drop(s)
-        return images
+        return slots, images
 
     def _prefetch_next(self, active: List[int]) -> None:
         if self._readers is None:
@@ -408,7 +389,7 @@ class MultiSequenceRunner:
         results: Dict[str, dict] = {}
         while True:
             # (re)fill free slots; a sequence whose initialisation fails is reported and skipped (running.py:135-142).  The slots that
-            # are free at this point are initialised together when the backend can do that (one staging pass, one upload).
+            # are free at this point are initialised together (one staging pass, one upload).
             while pending:
                 free = [i for i, slot in enumerate(self.slots) if slot.seq is None]
                 if not free:
@@ -425,17 +406,7 @@ class MultiSequenceRunner:
                         print(e)
                 if not batch:
                     continue
-                many = getattr(self.backend, "initialize_many", None)
-                if many is not None:
-                    errors = many([(i, im, seq.init_bbox) for (i, seq, im) in batch])
-                else:
-                    errors = []
-                    for (i, seq, im) in batch:
-                        try:
-                            self.backend.initialize(i, im, seq.init_bbox)
-                            errors.append(None)
-                        except Exception as e:
-                            errors.append(e)
+                errors = self.backend.initialize_many([(i, im, seq.init_bbox) for (i, seq, im) in batch])
                 dt = (time.time() - t0) / len(batch)
                 for (i, seq, im), err in zip(batch, errors):
                     if err is not None:
@@ -444,42 +415,28 @@ class MultiSequenceRunner:
                     slot = self.slots[i]
                     slot.seq, slot.next_frame = seq, 1
                     slot.output = {"target_bbox": [list(seq.init_bbox)], "time": [dt]}
-                    self._parked[i] = False
                     if len(seq.frames) == 1:
                         self._finish(slot, results)
             active = [i for i, s in enumerate(self.slots) if s.seq is not None]
             if not active:
                 break
-            high = max(active) + 1
-            # a backend with step_active steps just the running slots; otherwise a step covers slots [0, high), idle ones parked
-            step_active = getattr(self.backend, "step_active", None)
-            for i in range(high if step_active is None else 0):
-                if self.slots[i].seq is None and not self._parked[i]:
-                    self.backend.park(i)
-                    self._parked[i] = True
             t0 = time.time()
-            images = self._step_images(high)
-            active = [i for i in active if self.slots[i].seq is not None]      # minus the sequences whose frame could not be read
+            active, images = self._step_images(active)                         # minus the sequences whose frame could not be read
             self._prefetch_next(active)                                        # decode step t + 1 while the device runs step t
-            if step_active is None:
-                boxes = self.backend.step(images)
-            else:
-                boxes = np.zeros((high, 5))
-                if active:
-                    boxes[active] = step_active(active, [images[i] for i in active])
+            boxes = self.backend.step_active(active, images) if active else np.zeros((0, 5))
             # `time`: the reference records the wall time of one sequence's track() call (tracker.py:139-146); a batched step
             # advances every running sequence at once, so each is charged its share of the step - sum(time) over all sequences
             # is the wall time spent tracking, and the printed FPS is this sequence's share of the batched throughput
             dt = (time.time() - t0) / max(1, len(active))
-            for i in active:
+            for j, i in enumerate(active):
                 slot = self.slots[i]
-                if boxes[i, 4] < 0:
+                if boxes[j, 4] < 0:
                     # per-track failure flagged by vt_tracks_step (confidence -1, state kept: crop too small / outside the image /
                     # numeric range): the reference's track() would have raised and run_sequence dropped the sequence (running.py:135-142)
                     print(f"{slot.seq.name}: tracking failed at frame {slot.next_frame} (track status != 0), sequence dropped")
                     self._drop(slot)
                     continue
-                slot.output["target_bbox"].append([float(v) for v in boxes[i, :4]])
+                slot.output["target_bbox"].append([float(v) for v in boxes[j, :4]])
                 slot.output["time"].append(dt)
                 slot.next_frame += 1
                 if slot.next_frame >= len(slot.seq.frames):
